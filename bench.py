@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N>1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference --gpus N --steps K --warmup W
+    python bench.py --steps K --warmup W --dump-outputs DIR  (also writes the last timed step's results to DIR/*.npy)
 
 Workload (config.workload = "cfg1"): 4024x3036 u8 source (seeded synthetic stand-in for the missing
 Src7.bmp: blurred noise + Dst7 at three jittered README poses), the real 762x521 Dst7 template,
@@ -32,6 +33,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True        # the bench writes nothing into the tree (which may be read-only)
 
 METRIC = "images/sec (4024x3036 src, 762x521 tpl, +-180deg)"
 UNIT = "images/s"
@@ -112,7 +114,6 @@ def _cpu_worker(args):
 def cpu_throughput(wl, workers: int, images_per_worker: int, workload: str = "cfg1"):
     """images/sec of the CPU oracle with `workers` processes (one single-threaded matcher each)."""
     import multiprocessing as mp
-    subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "libncc_rowdot.so", "liboracle_cpu_match.so"], capture_output=True)
     ctx = mp.get_context("spawn")
     with ctx.Pool(workers) as pool:
         t0 = time.perf_counter()
@@ -237,6 +238,18 @@ def int8_peak_measured():
         return None
 
 
+def dump_outputs(out_dir: str, res, counts, B: int, cap: int):
+    """What one batch match hands its caller, as float64 .npy files: counts.npy [B] targets per frame, results.npy
+    [B, cap, 12] (score, angle, cx, cy, lt, rt, rb, lb per target; slots past a frame's count are zero)."""
+    import numpy as np
+    n = np.frombuffer(counts, dtype=np.int32, count=B).copy()
+    rows = np.frombuffer(res, dtype=np.float64, count=B * cap * 12).reshape(B, cap, 12).copy()
+    rows[np.arange(cap)[None, :] >= n[:, None]] = 0.0
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "counts.npy"), n.astype(np.float64))
+    np.save(os.path.join(out_dir, "results.npy"), rows)
+
+
 def percentile(v, q):
     v = sorted(v)
     if not v:
@@ -298,7 +311,11 @@ def main():
                     help="run only warm-up + timed device-resident steps and exit (clean launch list for ncu; prints no bench line)")
     ap.add_argument("--cpu-images", type=int, default=0, help="images per worker for the CPU baseline (0 = auto)")
     ap.add_argument("--h2d-chunk", type=int, default=0, help="frames per H2D chunk of the e2e path (0 = library default)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed device-resident step to DIR/*.npy (throughput mode)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.mode != "throughput" or args.device_steps_only):
+        ap.error("--dump-outputs needs the default throughput run (--impl b200 --mode throughput)")
     if args.workload is None:
         args.workload = "cfg5" if args.mode == "latency" else "cfg1"
     wl = WORKLOADS[args.workload]
@@ -332,7 +349,7 @@ def main():
     import numpy as np
     import torch
     import ctypes as C
-    from fastest_image_pattern_matching_b200 import TemplateMatcher, build
+    from fastest_image_pattern_matching_b200 import TemplateMatcher
     from fastest_image_pattern_matching_b200 import _lib as L
 
     if world > 1:
@@ -342,10 +359,6 @@ def main():
         dist = None
     torch.cuda.set_device(local_rank)
     numa = bind_to_gpu_numa(local_rank) if world > 1 else "single process, not bound"
-    if rank == 0:
-        build()
-    if dist:
-        dist.barrier()
     B, K, W = args.batch, args.steps, max(args.warmup, 3)
     int8_peak = int8_peak_measured() if rank == 0 and not args.device_steps_only else None
 
@@ -398,15 +411,15 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def timed(step_fn, inner):
-        """K steps x `inner` repeats inside ONE timed region (CUDA events on the library's stream, max over ranks)"""
+    def timed(step_fn):
+        """K steps inside ONE timed region (CUDA events on the library's stream, max over ranks)"""
         for i in range(W):
             step_fn(i)
         barrier()
         l0 = m.launchCount()
         m.timerRecord(0)
         t0 = time.perf_counter()
-        for i in range(K * inner):
+        for i in range(K):
             step_fn(i)
         m.timerRecord(1)
         ms = m.timerElapsedMs()
@@ -437,23 +450,13 @@ def main():
     found = [counts[b] for b in range(B)]
     ok_found = all(f == wl["expect"] for f in found)
 
-    # K steps alone are ~30 ms of device time: repeat them inside the timed region until it is >= 0.5 s, so that the clock
-    # sampler sees >= 25 samples under load; ms_per_step = region / (K * inner)
-    barrier()
-    m.timerRecord(0); step_device(0); step_device(1); m.timerRecord(1)
-    probe_ms = m.timerElapsedMs() / 2
-    inner = max(1, int(600.0 / max(probe_ms * K, 1e-3) + 0.999))
-    if dist:
-        t = torch.tensor([float(inner)], device="cuda")
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        inner = int(t.item())
-
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    dev_ms, dev_wall_ms, launches = timed(step_device, inner)
-    e2e_inner = max(1, inner // 4)
-    e2e_ms, e2e_wall_ms, _ = timed(step_host, e2e_inner)
+    dev_ms, dev_wall_ms, launches = timed(step_device)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res, counts, B, cap)
+    e2e_ms, e2e_wall_ms, _ = timed(step_host)
     clocks = sampler.stop() if rank == 0 else None
 
     # raw pinned-host -> device copy rate of one step's frames (context for e2e: the PCIe bound)
@@ -487,9 +490,9 @@ def main():
             dist.destroy_process_group()
         return 0
 
-    total_images = world * B * K * inner
+    total_images = world * B * K
     value = total_images / (dev_ms / 1000.0)
-    e2e_value = world * B * K * e2e_inner / (e2e_ms / 1000.0)
+    e2e_value = world * B * K / (e2e_ms / 1000.0)
 
     peaks = {}
     try:
@@ -578,12 +581,12 @@ def main():
     pcie_bound = world * h2d_gbps * 1e9 / (H * Wd)
     line = {
         "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": world, "steps": K, "warmup": W,
-        "ms_per_step": dev_ms / (K * inner), "higher_is_better": True, "scaling": "weak",
+        "ms_per_step": dev_ms / K, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "u8", "data": "synthetic",
         "config": workload_config(args.workload, wl, B),
         "run": {"global_batch": world * B, "sharding": "frames over ranks, no data-path collective",
                 "concurrent_half_batches": bool(split_default and B >= split_default and wl["tol"] > 0),
-                "inner_repeats": inner, "timed_region_ms": dev_ms, "e2e_inner_repeats": e2e_inner, "e2e_timed_region_ms": e2e_ms,
+                "timed_region_ms": dev_ms, "e2e_timed_region_ms": e2e_ms,
                 "distinct_frames_per_set": n_distinct},
         "p50_ms_per_match": percentile(l_pin, 0.5),
         "latency": {"what": "wall clock around one blocking fpm_match call, %d samples" % ns,
@@ -591,7 +594,7 @@ def main():
                     "host_pageable_p50_ms": percentile(l_pag, 0.5), "host_pageable_p90_ms": percentile(l_pag, 0.9),
                     "device_resident_p50_ms": percentile(l_dev, 0.5), "h2d_bytes": H * Wd},
         "e2e": {"value": e2e_value, "unit": UNIT, "h2d_bytes_per_step": B * H * Wd, "d2h_bytes_per_step": B * cap * 96 + B * 4,
-                "ms_per_step": e2e_ms / (K * e2e_inner), "h2d_copy_only_GBps": h2d_gbps, "host_numa": numa,
+                "ms_per_step": e2e_ms / K, "h2d_copy_only_GBps": h2d_gbps, "host_numa": numa,
                 "pcie_bound_images_per_s": pcie_bound, "bound": "h2d", "frac_of_bound": e2e_value / pcie_bound,
                 "note": "bound by the host->device copy of the frames (measured copy-only rate of the same pinned buffers); "
                         "at N>1 the ranks share the VM's host memory / PCIe root, see h2d_copy_only_GBps per N"},
@@ -603,7 +606,7 @@ def main():
         "int8_peak_measured": int8_peak,
         "cpu_baseline": cpu_baseline,
         "targets_found_per_frame_ok": ok_found,
-        "wall_ms_per_step": dev_wall_ms / (K * inner),
+        "wall_ms_per_step": dev_wall_ms / K,
     }
     emit(line)
     m.close()
@@ -619,7 +622,7 @@ def run_latency(args, wl, rank, world, local_rank):
     import ctypes as C
     import numpy as np
     import torch
-    from fastest_image_pattern_matching_b200 import TemplateMatcher, build
+    from fastest_image_pattern_matching_b200 import TemplateMatcher
     from fastest_image_pattern_matching_b200 import dist as D
     from fastest_image_pattern_matching_b200 import _lib as L
 
@@ -629,10 +632,6 @@ def run_latency(args, wl, rank, world, local_rank):
     else:
         dist = None
     torch.cuda.set_device(local_rank)
-    if rank == 0:
-        build()
-    if dist:
-        dist.barrier()
     ns, W = max(args.samples, 20), max(args.warmup, 3)
     tpl, frames_np = make_frames(1, 4242, args.workload)          # the SAME frame on every rank
     frame = np.ascontiguousarray(frames_np[0])

@@ -97,6 +97,27 @@ def ocr_case():
                                    rb=list(r.ptRB), lb=list(r.ptLB)) for r in res] for ch, res in per.items()})
 
 
+def imconv_golden():
+    """tests/golden/imconv_ref.json: the values the reference's IM_Conv_SIMD stands for on the pin's seeded inputs -- the
+    exact integer dot product of each row pair, and for each cell the float sum of its row dot products in row order
+    (src/TemplateMatcher.cpp:505-508: `*r_matResult = *r_matResult + IM_Conv_SIMD(...)`).  Computed here from that
+    definition, independently of the oracle; the pin checks the reference's own build (oracle/_ref) against them
+    wherever that build is present."""
+    from tests.helpers import imconv_pin_digest, imconv_pin_inputs
+    rows, cells = imconv_pin_inputs()
+    row_dot = [int((k.astype(np.int64) * c).sum()) for k, c in rows]
+    cell = []
+    for tpl, src in cells:
+        acc = np.float32(0)
+        for t, s in zip(tpl, src):
+            acc = np.float32(acc + np.float32(int((t.astype(np.int64) * s).sum())))
+        cell.append(float(acc))
+    out = dict(inputs="tests.helpers.imconv_pin_inputs()", inputs_sha256=imconv_pin_digest(rows, cells),
+               row_dot=row_dot, cell=cell)
+    with open(os.path.join(HERE, "imconv_ref.json"), "w") as f:
+        json.dump(out, f, indent=1)
+
+
 def main():
     os.makedirs(os.path.join(HERE, "images"), exist_ok=True)
     for f in FIXTURES:
@@ -118,7 +139,11 @@ def main():
     print("ocr_m12 ->", repr(cases["ocr_m12"]["text"]))
     with open(os.path.join(HERE, "cases.json"), "w") as f:
         json.dump(cases, f, indent=1)
+    imconv_golden()
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:] == ["imconv"]:
+        imconv_golden()
+    else:
+        main()

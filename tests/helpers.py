@@ -1,6 +1,30 @@
+import hashlib
+
 import numpy as np
 
 import fpm_workloads as synth
+
+# inputs of the IM_Conv_SIMD pin (tests/golden/imconv_ref.json): row lengths around the 16-byte SIMD blocks, and cells of
+# bright rows whose float accumulation rounds
+IMCONV_ROW_LENGTHS = [1, 7, 15, 16, 17, 54, 762, 1024, 4000]
+IMCONV_CELLS = [(762, 521), (1024, 300), (54, 54)]
+
+
+def imconv_pin_inputs():
+    """([(kernel row, source row)], [(template, source) cell]) drawn from one seeded stream, rows first."""
+    rng = np.random.default_rng(1)
+    rows = [(rng.integers(0, 256, n, dtype=np.uint8), rng.integers(0, 256, n, dtype=np.uint8)) for n in IMCONV_ROW_LENGTHS]
+    cells = [(rng.integers(200, 256, (th, tw), dtype=np.uint8), rng.integers(200, 256, (th, tw), dtype=np.uint8))
+             for (tw, th) in IMCONV_CELLS]
+    return rows, cells
+
+
+def imconv_pin_digest(rows, cells):
+    h = hashlib.sha256()
+    for a, b in rows + cells:
+        h.update(a.tobytes())
+        h.update(b.tobytes())
+    return h.hexdigest()
 
 
 def get_image(name):

@@ -1,6 +1,7 @@
 """CPU tests: the oracle against its pins (known answers, golden vectors, the reference's own
 IM_Conv_SIMD build, cv2 for every OpenCV model the CUDA kernels restate)."""
 import ctypes
+import json
 import os
 
 import cv2
@@ -9,7 +10,7 @@ import pytest
 
 from oracle import oracle as O
 from oracle import models as M
-from tests.helpers import assert_results_match, configure, get_image
+from tests.helpers import assert_results_match, configure, get_image, imconv_pin_digest, imconv_pin_inputs
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
 
@@ -49,40 +50,35 @@ def test_numpy_and_sse2_numerators_agree(oracle_lib):
         assert np.array_equal(a, b)
 
 
-def test_restated_simd_matches_reference_build():
-    """oracle/_ref/libimconv_ref.so is the reference's own IM_Conv_SIMD compiled from its source."""
-    ref_path = os.path.join(ROOT, "oracle", "_ref", "libimconv_ref.so")
-    if not os.path.exists(ref_path):
-        # policy: where the reference is mounted the pin must run -- build it, and fail (not skip) if that does not work;
-        # only a box without /root/reference (the GPU box) may skip, and then only if the prebuilt .so did not travel
-        if os.path.isdir("/root/reference"):
-            import subprocess
-            subprocess.run(["bash", os.path.join(ROOT, "oracle", "build_ref.sh")], check=False, capture_output=True)
-            assert os.path.exists(ref_path), "oracle/_ref could not be built from /root/reference (oracle/build_ref.sh)"
-        else:
-            pytest.skip("oracle/_ref not present and /root/reference not mounted")
-    ref = ctypes.CDLL(ref_path)
-    ref.ref_IM_Conv_SIMD.restype = ctypes.c_int
-    ref.ref_cell.restype = ctypes.c_float
+def test_restated_simd_matches_reference_build(oracle_lib):
+    """The oracle's restatements of the reference's IM_Conv_SIMD (SSE2 C and numpy) return the stored values of
+    tests/golden/imconv_ref.json; so does oracle/_ref/libimconv_ref.so, the reference's own IM_Conv_SIMD compiled from
+    its source (oracle/build_ref.sh), wherever that build is present."""
+    with open(os.path.join(ROOT, "tests", "golden", "imconv_ref.json")) as f:
+        golden = json.load(f)
+    rows, cells = imconv_pin_inputs()
+    assert imconv_pin_digest(rows, cells) == golden["inputs_sha256"], "the seeded stream no longer draws the stored inputs"
     lib = O._load_rowdot()
-    if not lib:
-        pytest.skip("oracle C helper not built")
+    assert lib, "oracle/libncc_rowdot.so not built"
     lib.oracle_row_dot.restype = ctypes.c_int
-    rng = np.random.default_rng(1)
-    for n in [1, 7, 15, 16, 17, 54, 762, 1024, 4000]:
-        k = rng.integers(0, 256, n, dtype=np.uint8)
-        c = rng.integers(0, 256, n, dtype=np.uint8)
-        want = int((k.astype(np.int64) * c).sum())
-        assert ref.ref_IM_Conv_SIMD(k.ctypes.data, c.ctypes.data, n) == want
-        assert lib.oracle_row_dot(k.ctypes.data, c.ctypes.data, n) == want
+    for (k, c), want in zip(rows, golden["row_dot"]):
+        assert int((k.astype(np.int64) * c).sum()) == want
+        assert lib.oracle_row_dot(k.ctypes.data, c.ctypes.data, k.size) == want
     # bright rows: float accumulation rounds -- restatement must round identically
-    for (tw, th) in [(762, 521), (1024, 300), (54, 54)]:
-        tpl = rng.integers(200, 256, (th, tw), dtype=np.uint8)
-        src = rng.integers(200, 256, (th, tw), dtype=np.uint8)
-        want = ref.ref_cell(tpl.ctypes.data, tw, th, src.ctypes.data, tw)
+    for (tpl, src), want in zip(cells, golden["cell"]):
         got = O.match_template_simd(src, tpl)[0, 0]
         assert np.float32(want) == got
         assert O.match_template_simd_numpy(src, tpl)[0, 0] == got
+    ref_path = os.path.join(ROOT, "oracle", "_ref", "libimconv_ref.so")
+    if os.path.exists(ref_path):
+        ref = ctypes.CDLL(ref_path)
+        ref.ref_IM_Conv_SIMD.restype = ctypes.c_int
+        ref.ref_cell.restype = ctypes.c_float
+        for (k, c), want in zip(rows, golden["row_dot"]):
+            assert ref.ref_IM_Conv_SIMD(k.ctypes.data, c.ctypes.data, k.size) == want
+        for (tpl, src), want in zip(cells, golden["cell"]):
+            th, tw = tpl.shape
+            assert np.float32(ref.ref_cell(tpl.ctypes.data, tw, th, src.ctypes.data, tw)) == np.float32(want)
 
 
 # ---- OpenCV models the CUDA kernels restate, pinned against cv2 itself ----
