@@ -50,6 +50,12 @@ SIGNATURES = {
     "fpm_ingested_pixels": (_i, [_vp, _vp]),
     "fpm_match_ingested": (_i, [_vp, _vp, _i, _pi]),
     "fpm_learn_ingested": (_i, [_vp]),
+    "fpm_ingest_jpeg_batch": (_i, [_vp, _vp, _vp, _i, _pi, _pi]),
+    "fpm_ingested_count": (_i, [_vp]),
+    "fpm_ingested_frame_pixels": (_i, [_vp, _i, _vp]),
+    "fpm_match_ingested_batch": (_i, [_vp, _vp, _i, _vp]),
+    "fpm_dbg_jpeg_luma_parallel_batch": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i]),
+    "fpm_dbg_jpeg_unstuff": (_i, [_vp, _sz, _i, _vp, _sz, _vp, _i, _vp, _pi, _pi]),
     "fpm_match_batch_device": (_i, [_vp, _vp, _i, _i, _i, _i, _sz, _vp, _i, _vp]),
     "fpm_last_time_ms": (_d, [_vp]),
     "fpm_set_user_rect": (None, [_vp, _i, _i, _i, _i]),

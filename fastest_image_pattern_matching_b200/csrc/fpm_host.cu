@@ -174,8 +174,9 @@ struct fpm_handle {
     int mfc_compat = 0;            // 1: MFC result convention (angle sign/wrap, TargetNum truncation, double corners)
     int async_descent = -1;        // FPM_PARAM_ASYNC_DESCENT: -1 auto (batches < 8 frames), 0 never, 1 always
     int jpeg_device_huffman = 1;   // FPM_PARAM_JPEG_DEVICE_HUFFMAN
-    int jpeg_passes = 0;           // synchronisation passes of the last device-decoded JPEG scan (0: decoded on the host)
-    DevBuf d_jpeg;                 // unstuffed scan, tables, decoder states, DC values
+    int jpeg_passes = 0;           // synchronisation passes of the last JPEG ingest (0: decoded on the host)
+    DevBuf d_jpeg_scan;            // JPEG ingest: the uploaded files, their unstuffed scans, restart positions
+    DevBuf d_jpeg;                 // JPEG ingest: file descriptors, decoder states, DC values of a decode wave
     int cur_batch = 1;             // frames of the match in flight
     bool err_check_pending = false;
     int use_tc = 1;                // 0 = dp4a only, 1 = tcgen05 for large levels, 2 = tcgen05 wherever possible
@@ -187,7 +188,8 @@ struct fpm_handle {
     int tpl0_w = 0, tpl0_h = 0;
     std::vector<TplLevelHost> tpl;
     DevBuf d_tpl, d_tsh, d_raw, d_inv, d_numer, d_totS, d_totQ, d_ingest_raw, d_ingest;
-    int ingest_w = 0, ingest_h = 0, ingest_pitch = 0;      // last ingested frame (device resident)
+    int ingest_w = 0, ingest_h = 0, ingest_pitch = 0;      // last ingested frames (device resident, [count][h][pitch])
+    int ingest_count = 0;
     // user rect (pure storage)
     int ur[4] = {0, 0, 0, 0};
     int has_ur = 0;
@@ -216,8 +218,8 @@ struct fpm_handle {
     std::vector<cudaEvent_t> ev_pool;
     struct ProfRec { int kid; cudaEvent_t a, b; double work; };
     std::vector<ProfRec> prof_pending;
-    double prof_ms[16] = {0}, prof_work[16] = {0};
-    long long prof_launches[16] = {0};
+    double prof_ms[24] = {0}, prof_work[24] = {0};
+    long long prof_launches[24] = {0};
     cudaEvent_t prof_cur = nullptr;
     // trace
     std::vector<double> tr_cands;                 // n*4
@@ -247,11 +249,15 @@ namespace {
 
 // CNT_LAYER + l: candidates entering pyramid layer l (descent without host round trips)
 enum { CNT_FLAT = 0, CNT_NEXT = 1, CNT_REFINED = 2, CNT_TOTAL = 3, CNT_ERR = 4, CNT_LAYER = 8, CNT_N = 8 + FPM_MAX_LEVELS };
-enum { K_PYRDOWN = 0, K_WARP_TOP, K_TOP_SCORE, K_TOP_PEAKS, K_COLLECT, K_PREP, K_WARP_ROI, K_CORR, K_FINALIZE, K_FINAL, K_CORR_MMA, K_CORR_FUSED, K_CORR_WARP, K_COUNT };
+enum { K_PYRDOWN = 0, K_WARP_TOP, K_TOP_SCORE, K_TOP_PEAKS, K_COLLECT, K_PREP, K_WARP_ROI, K_CORR, K_FINALIZE, K_FINAL, K_CORR_MMA, K_CORR_FUSED, K_CORR_WARP,
+       K_JPEG_UPLOAD, K_JPEG_UNSTUFF, K_JPEG_PASSES, K_JPEG_SCAN, K_JPEG_WRITE, K_JPEG_IDCT, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"fpm_pyrdown_kernel", "fpm_warp_kernel(top)", "fpm_top_score_kernel", "fpm_top_peaks_kernel",
                                            "fpm_collect_sort_kernel", "fpm_refine_prep_kernel", "fpm_warp_kernel(roi)",
                                            "fpm_corr_rows_kernel", "fpm_refine_finalize_kernel", "fpm_final_kernel",
-                                           "fpm_corr_mma_kernel", "fpm_corr_fused_kernel", "fpm_corr_warp_kernel"};
+                                           "fpm_corr_mma_kernel", "fpm_corr_fused_kernel", "fpm_corr_warp_kernel",
+                                           "jpeg_upload(H2D copy)", "fpm_jpeg_unstuff_count/write_kernel", "fpm_jpeg_cold/sync_kernel(passes)",
+                                           "fpm_jpeg_block_tile/dc_tile/offsets_kernel(scans)", "fpm_jpeg_write_kernel", "fpm_ingest_jpeg_idct_kernel"};
+static_assert(K_COUNT <= 24, "profile arrays");
 
 cudaEvent_t prof_event(fpm_handle* h)
 {
@@ -1406,6 +1412,7 @@ void fpm_destroy(fpm_handle* h)
     for (DevBuf* b : bufs) b->release();
     h->h_counts.release(); h->h_results.release(); h->h_stage.release();
     h->d_jpeg.release();
+    h->d_jpeg_scan.release();
     for (int i = 0; i < 2; i++) { cudaEventDestroy(h->ev_copy[i]); cudaEventDestroy(h->ev_done[i]); }
     cudaEventDestroy(h->ev_t0); cudaEventDestroy(h->ev_t1);
     prof_collect(h);
@@ -1738,6 +1745,7 @@ uint32_t rd16(const uint8_t* p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8);
 int fpm_ingest_bmp(fpm_handle* h, const uint8_t* file, size_t nbytes, int* width, int* height)
 {
     if (!h) return FPM_ERR_INVALID;
+    h->ingest_count = 0;
     if (!file || nbytes < 54 || file[0] != 'B' || file[1] != 'M') { h->err = "not a BMP file"; return FPM_ERR_INVALID; }
     const uint32_t off = rd32(file + 10), dib = rd32(file + 14);
     if (dib < 40) { h->err = "unsupported BMP header (OS/2 core header)"; return FPM_ERR_INVALID; }
@@ -1784,17 +1792,17 @@ int fpm_ingest_bmp(fpm_handle* h, const uint8_t* file, size_t nbytes, int* width
                                                        h->d_ingest.as<uint8_t>(), pitch);
     CKL();
     CK(cudaStreamSynchronize(h->stream));                             // the caller's file buffer is free again
-    h->ingest_w = w; h->ingest_h = hh; h->ingest_pitch = pitch;
+    h->ingest_w = w; h->ingest_h = hh; h->ingest_pitch = pitch; h->ingest_count = 1;
     if (width) *width = w;
     if (height) *height = hh;
     return FPM_OK;
 }
 
 // ---- JPEG ingest ------------------------------------------------------------------------------------------------------
-enum { FPM_ERR_UNSUPPORTED_LOCAL = -1000 };                             // internal: "take the host decoder instead"
 // entropy-coded segment without the 0xFF00 stuffing and without the RSTn markers (their positions go to rst_bits: first bit of
 // every restart interval + a final sentinel); stops at the first other marker (EOI).  out needs n - begin + 16 bytes; the 16
-// bytes after the data are zero (the device reader looks a few bytes ahead).  Returns the number of data bytes.
+// bytes after the data are zero (the device reader looks a few bytes ahead).  Returns the number of data bytes.  The sequential
+// reference of the device unstuffing (jp_unstuff_*, fpm_jpeg_par.cuh): fpm_dbg_jpeg_unstuff runs both.
 size_t jpeg_unstuff(const uint8_t* d, size_t n, size_t begin, uint8_t* out, std::vector<unsigned>* rst_bits)
 {
     size_t i = begin, o = 0;
@@ -1871,167 +1879,363 @@ bool jpeg_device_ok(const fpm_jpeg::Frame& fr, size_t file_bytes)
     return slots <= JP_MAX_SLOTS && file_bytes < (400u << 20);
 }
 
-// Huffman decoding on the device: the unstuffed scan + the tables are the only H2D traffic.  Leaves the AC coefficients in
-// d_ingest_raw ([bh*bw][64] int16), the DC values in scan order in *dcval_out (each short of its 4096-value tile's offset
-// (*tile_off_out)[L / 4096]); fills *sc.
-int jpeg_decode_device(fpm_handle* h, const fpm_jpeg::Frame& fr, const uint8_t* file, size_t nbytes, JpScan* sc_out, const int** dcval_out,
-                       const int** tile_off_out)
+// ---- batches: the files of one fpm_ingest_jpeg_batch call (one file for fpm_ingest_jpeg) --------------------------------
+struct JpegBatchFile {
+    fpm_jpeg::Frame fr;
+    size_t off = 0, nbytes = 0;    // the file is data[off, off + nbytes)
+    bool device = false;           // Huffman decoding on the device (else on the host, fpm_jpeg.h)
+};
+
+std::string jpeg_file_prefix(int i, int n) { return n > 1 ? "JPEG file " + std::to_string(i) + " of the batch: " : std::string(); }
+
+// headers of every file (the host reads nothing past them); same_size: all frames must have file 0's size
+int jpeg_batch_parse(const uint8_t* data, const size_t* offsets, int n, bool same_size, std::vector<JpegBatchFile>* fs, std::string* err)
 {
-    const size_t cap = nbytes - fr.scan_begin + 16;
-    const size_t tab_bytes = 8 * sizeof(JpTable);
-    CK(h->h_stage.ensure(align_up(cap, 256) + tab_bytes));
-    uint8_t* hbits = h->h_stage.as<uint8_t>();
-    std::vector<unsigned> rst;
-    const size_t scan_bytes = jpeg_unstuff(file, nbytes, fr.scan_begin, hbits, fr.restart_interval ? &rst : nullptr);
-    JpTable* htabs = reinterpret_cast<JpTable*>(hbits + align_up(cap, 256));
-    JpScan sc;
-    jpeg_device_tables(fr, htabs, &sc, scan_bytes);
-    if (sc.nsub <= 0) { h->err = "JPEG without image data"; return FPM_ERR_INVALID; }
-    if (fr.restart_interval) {
-        sc.nint = (int)rst.size() - 1;
-        if (sc.nint != jpeg_expected_intervals(fr)) return FPM_ERR_UNSUPPORTED_LOCAL;     // damaged: the host decoder says what is wrong
+    if (n <= 0) { *err = "empty JPEG batch"; return FPM_ERR_INVALID; }
+    if (!data || !offsets) { *err = "null JPEG batch buffer or offsets"; return FPM_ERR_INVALID; }
+    for (int i = 0; i < n; i++)
+        if (offsets[i + 1] < offsets[i]) { *err = "JPEG batch offsets decrease at file " + std::to_string(i); return FPM_ERR_INVALID; }
+    fs->resize(n);
+    for (int i = 0; i < n; i++) {
+        JpegBatchFile& f = (*fs)[i];
+        f.off = offsets[i];
+        f.nbytes = offsets[i + 1] - offsets[i];
+        const std::string why = fpm_jpeg::parse(data + f.off, f.nbytes, &f.fr);
+        if (!why.empty()) { *err = jpeg_file_prefix(i, n) + why; return FPM_ERR_INVALID; }
+        if ((size_t)f.fr.height * f.fr.width > ((size_t)1 << 30)) {
+            *err = jpeg_file_prefix(i, n) + "JPEG too large (more than 2^30 pixels, OpenCV's own limit)";
+            return FPM_ERR_LIMIT;
+        }
+        const fpm_jpeg::Frame& f0 = (*fs)[0].fr;
+        if (same_size && (f.fr.width != f0.width || f.fr.height != f0.height)) {
+            *err = "JPEG file " + std::to_string(i) + " of the batch is " + std::to_string(f.fr.width) + "x" + std::to_string(f.fr.height) +
+                   ", file 0 is " + std::to_string(f0.width) + "x" + std::to_string(f0.height) + ": the frames of a batch must have one size";
+            return FPM_ERR_INVALID;
+        }
     }
-    const size_t nluma = (size_t)sc.mcux * sc.mcuy * sc.luma_slots;
-    // device layout: [bits + tables | 3 state arrays | first-block index | DC values | flag]
-    const size_t o_tabs = align_up(cap, 256), o_st = o_tabs + align_up(tab_bytes, 256), st_bytes = align_up((size_t)sc.nsub * sizeof(JpState), 256);
-    const int ntiles = (int)((nluma + JP_DC_TILE - 1) / JP_DC_TILE);
-    const size_t o_first = o_st + 3 * st_bytes, o_dc = o_first + align_up((size_t)sc.nsub * 4, 256), o_tile = o_dc + align_up(nluma * 4, 256);
-    const int nbtiles = (sc.nsub + 4095) / 4096;
-    const size_t o_btile = o_tile + align_up((size_t)ntiles * 4, 256), o_flag = o_btile + align_up((size_t)nbtiles * 4, 256);
-    const size_t o_rst = o_flag + 256;
-    CK(h->d_jpeg.ensure(o_rst + align_up(rst.size() * 4 + 4, 256)));
-    uint8_t* base = h->d_jpeg.as<uint8_t>();
-    if (fr.restart_interval) {
-        CK(cudaMemcpyAsync(base + o_rst, rst.data(), rst.size() * 4, cudaMemcpyHostToDevice, h->stream));
-        sc.rst = reinterpret_cast<const unsigned*>(base + o_rst);
+    return FPM_OK;
+}
+
+// where every file's unstuffing reads and writes (offsets relative to data[offsets[0]]); files decoded on the host get no tiles
+struct JpUnstuffPlan {
+    std::vector<JpUnstuff> u;
+    std::vector<int> tile_first;   // n + 1
+    size_t out_bytes = 0, rst_entries = 0;
+};
+
+void jpeg_unstuff_plan(const std::vector<JpegBatchFile>& fs, size_t base, JpUnstuffPlan* p)
+{
+    const int n = (int)fs.size();
+    p->u.assign(n, JpUnstuff{});
+    p->tile_first.assign(n + 1, 0);
+    int tiles = 0;
+    for (int i = 0; i < n; i++) {
+        JpUnstuff& u = p->u[i];
+        p->tile_first[i] = tiles;
+        if (!fs[i].device) continue;
+        u.begin = fs[i].off - base + fs[i].fr.scan_begin;
+        u.end = fs[i].off - base + fs[i].nbytes;
+        u.stop = u.end;
+        u.out = p->out_bytes;
+        p->out_bytes += align_up(u.end - u.begin, 4) + 16;
+        u.restart = fs[i].fr.restart_interval != 0;
+        u.rst = p->rst_entries;
+        u.rst_cap = u.restart ? jpeg_expected_intervals(fs[i].fr) + 2 : 0;     // more markers than that: the host decoder takes it
+        p->rst_entries += u.rst_cap;
+        tiles += (int)((u.end - u.begin + 1 + JP_UNSTUFF_TILE - 1) / JP_UNSTUFF_TILE);
     }
-    const size_t cbytes = nluma * 64 * sizeof(int16_t);
+    p->tile_first[n] = tiles;
+}
+
+// the unstuffing kernels run tile by tile, thread by thread on the CPU (d = data[offsets[0]])
+void jpeg_unstuff_emulate(const uint8_t* d, JpUnstuffPlan* p, uint8_t* out, unsigned* rst)
+{
+    const int n = (int)p->u.size(), ntiles = p->tile_first[n];
+    std::vector<unsigned long long> tile_sum(ntiles);
+    for (int t = 0; t < ntiles; t++) {                                  // fpm_jpeg_unstuff_count_kernel
+        const int fi = jp_file_of(p->tile_first.data(), n, t);
+        JpUnstuff& f = p->u[fi];
+        unsigned long long sum = 0;
+        for (int k = 0; k < JP_UNSTUFF_THREADS; k++) {
+            unsigned long long a, b, s = ~0ull;
+            unsigned e = 0, r = 0;
+            jp_unstuff_chunk(f, t - p->tile_first[fi], k, &a, &b);
+            if (a < b) jp_unstuff_count(d, f, a, b, &e, &r, &s);
+            f.stop = std::min(f.stop, s);
+            sum += ((unsigned long long)e << 32) | r;
+        }
+        tile_sum[t] = sum;
+    }
+    for (int fi = 0; fi < n; fi++) {                                    // fpm_jpeg_offsets_kernel
+        unsigned long long run = 0;
+        for (int t = p->tile_first[fi]; t < p->tile_first[fi + 1]; t++) { const unsigned long long v = tile_sum[t]; tile_sum[t] = run; run += v; }
+    }
+    for (int t = 0; t < ntiles; t++) {                                  // fpm_jpeg_unstuff_write_kernel
+        const int fi = jp_file_of(p->tile_first.data(), n, t);
+        JpUnstuff& f = p->u[fi];
+        unsigned long long x = tile_sum[t];
+        for (int k = 0; k < JP_UNSTUFF_THREADS; k++) {
+            unsigned long long a, b, s;
+            unsigned e = 0, r = 0;
+            jp_unstuff_chunk(f, t - p->tile_first[fi], k, &a, &b);
+            if (a < b) jp_unstuff_count(d, f, a, b, &e, &r, &s);
+            if (a < b && a <= f.stop) jp_unstuff_write(d, f, a, b, (unsigned)(x >> 32), (unsigned)x, out, rst);
+            x += ((unsigned long long)e << 32) | r;
+        }
+    }
+}
+
+// decoder descriptors of the files [f0, f1) of a batch (after the unstuffing); rst_base: the rst array the decoder reads
+struct JpWave {
+    std::vector<JpFile> files;
+    std::vector<int> cta_first, bseg, dseg;        // f1 - f0 + 1 entries each
+    size_t coef_elems = 0;
+    int nsub = 0, nluma = 0, max_nsub = 0;         // state / DC array lengths (padded per file)
+};
+
+void jpeg_wave_plan(const std::vector<JpegBatchFile>& fs, const JpUnstuffPlan& up, int f0, int f1, const unsigned* rst_base, int pitch, JpWave* w)
+{
+    const int m = f1 - f0;
+    w->files.assign(m, JpFile{});
+    w->cta_first.assign(m + 1, 0); w->bseg.assign(m + 1, 0); w->dseg.assign(m + 1, 0);
+    int ctas = 0;
+    for (int k = 0; k < m; k++) {
+        const JpegBatchFile& b = fs[f0 + k];
+        const JpUnstuff& u = up.u[f0 + k];
+        JpFile& f = w->files[k];
+        memset(&f, 0, sizeof(f));
+        jpeg_device_tables(b.fr, f.tabs, &f.sc, b.device ? u.nbits / 8 : 0);
+        if (!b.device) f.sc.nsub = 0;
+        else if (b.fr.restart_interval) { f.sc.nint = u.nint; f.sc.rst = rst_base + u.rst; }
+        memcpy(f.quant, b.fr.qt[b.fr.comp[0].tq], sizeof(f.quant));
+        f.bits = u.out;
+        f.coef = w->coef_elems;
+        w->coef_elems += (size_t)f.sc.bw * f.sc.mcuy * f.sc.luma_v * 64;
+        f.frame = (size_t)(f0 + k) * pitch * b.fr.height;
+        f.sub0 = w->nsub;
+        f.luma0 = w->nluma;
+        f.width = b.fr.width; f.height = b.fr.height;
+        f.device_huffman = b.device;
+        w->cta_first[k] = ctas; w->bseg[k] = f.sub0 / 4096; w->dseg[k] = f.luma0 / JP_DC_TILE;
+        ctas += (f.sc.nsub + JP_THREADS - 1) / JP_THREADS;
+        w->nsub += (int)align_up(f.sc.nsub, 4096);
+        if (b.device) w->nluma += (int)align_up((size_t)f.sc.mcux * f.sc.mcuy * f.sc.luma_slots, JP_DC_TILE);
+        w->max_nsub = std::max(w->max_nsub, f.sc.nsub);
+    }
+    w->cta_first[m] = ctas; w->bseg[m] = w->nsub / 4096; w->dseg[m] = w->nluma / JP_DC_TILE;
+}
+
+// device bytes one file needs in a decode wave: coefficients (2 B per luma pixel), decoder states, DC values
+size_t jpeg_wave_bytes(const JpegBatchFile& b, const JpUnstuff& u)
+{
+    const size_t luma = (size_t)b.fr.mcux * b.fr.comp[0].h * b.fr.mcuy * b.fr.comp[0].v;
+    size_t bytes = luma * 64 * sizeof(int16_t);
+    if (b.device) {
+        const size_t nsub = (u.nbits + JP_SUB_BITS - 1) / JP_SUB_BITS;
+        bytes += align_up(nsub, 4096) * (3 * sizeof(JpState) + 4) + align_up(luma, JP_DC_TILE) * 4 * 2;
+    }
+    return bytes;
+}
+
+// Huffman decoding of the device files of a wave + dequantisation / IDCT of all its files into their frame slots
+int jpeg_decode_wave(fpm_handle* h, const std::vector<JpegBatchFile>& fs, const uint8_t* data, const JpUnstuffPlan& up, int f0, int f1,
+                     const uint8_t* bits, const unsigned* rst, int pitch, int* passes_out)
+{
+    const int m = f1 - f0;
+    JpWave w;
+    jpeg_wave_plan(fs, up, f0, f1, rst, pitch, &w);
+    std::vector<fpm_jpeg::Luma> host(m);
+    for (int k = 0; k < m; k++)
+        if (!fs[f0 + k].device) {
+            const JpegBatchFile& b = fs[f0 + k];
+            const std::string why = fpm_jpeg::decode_scan_host(b.fr, data + b.off, b.nbytes, &host[k]);
+            if (!why.empty()) { h->err = jpeg_file_prefix(f0 + k, (int)fs.size()) + why; return FPM_ERR_INVALID; }
+        }
+    // d_jpeg: [descriptors | cta_first | bseg | dseg] [3 state arrays | first-block index | block tile offsets | DC values |
+    // DC tile offsets | flag]
+    const size_t o_cta = align_up((size_t)m * sizeof(JpFile), 256), o_bseg = o_cta + align_up((m + 1) * 4, 256);
+    const size_t o_dseg = o_bseg + align_up((m + 1) * 4, 256), desc_bytes = o_dseg + (m + 1) * 4;
+    const size_t S = (size_t)w.nsub, L = (size_t)w.nluma, st_bytes = align_up(S * sizeof(JpState), 256);
+    const size_t o_st = align_up(desc_bytes, 256), o_first = o_st + 3 * st_bytes, o_btile = o_first + align_up(S * 4, 256);
+    const size_t o_dc = o_btile + align_up(S / 4096 * 4 + 4, 256), o_dtile = o_dc + align_up(L * 4, 256);
+    const size_t o_flag = o_dtile + align_up(L / JP_DC_TILE * 4 + 4, 256);
+    CK(h->d_jpeg.ensure(o_flag + 256));
+    const size_t cbytes = w.coef_elems * sizeof(int16_t);
     CK(h->d_ingest_raw.ensure(cbytes));
-    CK(cudaMemcpyAsync(base, hbits, o_tabs + tab_bytes, cudaMemcpyHostToDevice, h->stream));
-    CK(cudaMemsetAsync(h->d_ingest_raw.p, 0, cbytes, h->stream));
-    const uint8_t* bits = base;
-    const JpTable* tabs = reinterpret_cast<const JpTable*>(base + o_tabs);
+    CK(h->h_stage.ensure(desc_bytes));
+    uint8_t* hs = h->h_stage.as<uint8_t>();
+    memcpy(hs, w.files.data(), (size_t)m * sizeof(JpFile));
+    memcpy(hs + o_cta, w.cta_first.data(), (m + 1) * 4);
+    memcpy(hs + o_bseg, w.bseg.data(), (m + 1) * 4);
+    memcpy(hs + o_dseg, w.dseg.data(), (m + 1) * 4);
+    uint8_t* base = h->d_jpeg.as<uint8_t>();
+    CK(cudaMemcpyAsync(base, hs, desc_bytes, cudaMemcpyHostToDevice, h->stream));
+    const JpFile* files = reinterpret_cast<const JpFile*>(base);
+    const int* cta_first = reinterpret_cast<const int*>(base + o_cta);
+    int16_t* coef = h->d_ingest_raw.as<int16_t>();
+    CK(cudaMemsetAsync(coef, 0, cbytes, h->stream));
+    for (int k = 0; k < m; k++)
+        if (!fs[f0 + k].device)
+            CK(cudaMemcpyAsync(coef + w.files[k].coef, host[k].coef.data(), host[k].coef.size() * sizeof(int16_t), cudaMemcpyHostToDevice, h->stream));
     JpState* st[2] = {reinterpret_cast<JpState*>(base + o_st), reinterpret_cast<JpState*>(base + o_st + st_bytes)};
     JpState* used = reinterpret_cast<JpState*>(base + o_st + 2 * st_bytes);
     unsigned* first = reinterpret_cast<unsigned*>(base + o_first);
-    int* dcval = reinterpret_cast<int*>(base + o_dc);
-    int* flag = reinterpret_cast<int*>(base + o_flag);
-    int* tile_off = reinterpret_cast<int*>(base + o_tile);
-    const int nb = (sc.nsub + JP_THREADS - 1) / JP_THREADS;
-    fpm_jpeg_cold_kernel<<<nb, JP_THREADS, 0, h->stream>>>(bits, tabs, sc, st[0], used);
-    CKL();
-    // synchronisation passes, two per flag read-back (a pass in which no entry state moved costs a few microseconds: its CTAs
-    // leave before they stage anything)
-    int cur = 0, passes = 0;
-    CK(h->h_counts.ensure(256));
-    int* hflag = h->h_counts.as<int>();
-    for (;;) {
-        if (passes > sc.nsub + 2) { h->err = "JPEG scan did not synchronise"; return FPM_ERR_INVALID; }
-        CK(cudaMemsetAsync(flag, 0, 8, h->stream));
-        for (int k = 0; k < 2; k++) {
-            fpm_jpeg_sync_kernel<<<nb, JP_THREADS, 0, h->stream>>>(bits, tabs, sc, st[cur], st[cur ^ 1], used, flag + k);
-            CKL();
-            cur ^= 1;
-        }
-        CK(cudaMemcpyAsync(hflag, flag, 8, cudaMemcpyDeviceToHost, h->stream));
-        CK(cudaStreamSynchronize(h->stream));
-        passes += hflag[0] ? 2 : 1;                                   // passes that did work (+ the one that found the fixed point)
-        if (!hflag[1]) break;
-    }
-    h->jpeg_passes = passes;
     int* btile_off = reinterpret_cast<int*>(base + o_btile);
-    fpm_jpeg_block_tile_kernel<<<nbtiles, 256, 0, h->stream>>>(st[cur], sc.nsub, first, btile_off);
-    CKL();
-    fpm_jpeg_dc_offsets_kernel<<<1, 1024, 0, h->stream>>>(nbtiles, btile_off);
-    CKL();
-    fpm_jpeg_write_kernel<<<nb, JP_THREADS, 0, h->stream>>>(bits, tabs, sc, st[cur], first, btile_off, h->d_ingest_raw.as<int16_t>(), dcval);
-    CKL();
-    fpm_jpeg_dc_tile_kernel<<<ntiles, 256, 0, h->stream>>>((int)nluma, dcval, tile_off);
-    CKL();
-    fpm_jpeg_dc_offsets_kernel<<<1, 1024, 0, h->stream>>>(ntiles, tile_off);
-    CKL();
-    *sc_out = sc;
-    *dcval_out = dcval;
-    *tile_off_out = tile_off;
+    int* dcval = reinterpret_cast<int*>(base + o_dc);
+    int* dtile_off = reinterpret_cast<int*>(base + o_dtile);
+    int* flag = reinterpret_cast<int*>(base + o_flag);
+    const int nb = w.cta_first[m];
+    int passes = 0;
+    if (nb > 0) {
+        KL(K_JPEG_PASSES, S, fpm_jpeg_cold_kernel<<<nb, JP_THREADS, 0, h->stream>>>(files, cta_first, m, bits, st[0], used));
+        // synchronisation passes, two per flag read-back (a pass in which no entry state moved costs a few microseconds: its
+        // CTAs leave before they stage anything)
+        int cur = 0;
+        CK(h->h_counts.ensure(256));
+        int* hflag = h->h_counts.as<int>();
+        for (;;) {
+            if (passes > w.max_nsub + 2) { h->err = "JPEG scan did not synchronise"; return FPM_ERR_INVALID; }
+            CK(cudaMemsetAsync(flag, 0, 8, h->stream));
+            for (int k = 0; k < 2; k++) {
+                KL(K_JPEG_PASSES, S, fpm_jpeg_sync_kernel<<<nb, JP_THREADS, 0, h->stream>>>(files, cta_first, m, bits, st[cur], st[cur ^ 1], used, flag + k));
+                cur ^= 1;
+            }
+            CK(cudaMemcpyAsync(hflag, flag, 8, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            passes += hflag[0] ? 2 : 1;                               // passes that did work (+ the one that found the fixed point)
+            if (!hflag[1]) break;
+        }
+        const int* bseg = reinterpret_cast<const int*>(base + o_bseg);
+        const int* dseg = reinterpret_cast<const int*>(base + o_dseg);
+        KL(K_JPEG_SCAN, S * 16, fpm_jpeg_block_tile_kernel<<<(int)(S / 4096), 256, 0, h->stream>>>(st[cur], (int)S, first, btile_off));
+        KL(K_JPEG_SCAN, S / 4096 * 4, fpm_jpeg_offsets_kernel<int><<<m, 1024, 0, h->stream>>>(bseg, btile_off));
+        KL(K_JPEG_WRITE, cbytes, fpm_jpeg_write_kernel<<<nb, JP_THREADS, 0, h->stream>>>(files, cta_first, m, bits, st[cur], first, btile_off, coef, dcval));
+        if (L > 0) {
+            KL(K_JPEG_SCAN, L * 8, fpm_jpeg_dc_tile_kernel<<<(int)(L / JP_DC_TILE), 256, 0, h->stream>>>((int)L, dcval, dtile_off));
+            KL(K_JPEG_SCAN, L / JP_DC_TILE * 4, fpm_jpeg_offsets_kernel<int><<<m, 1024, 0, h->stream>>>(dseg, dtile_off));
+        }
+    }
+    int max_blocks = 0;
+    for (const JpFile& f : w.files) max_blocks = std::max(max_blocks, f.sc.bw * f.sc.mcuy * f.sc.luma_v);
+    KL(K_JPEG_IDCT, cbytes, fpm_ingest_jpeg_idct_kernel<<<dim3((max_blocks + 127) / 128, m), 128, 0, h->stream>>>(
+                                files, coef, dcval, dtile_off, h->d_ingest.as<uint8_t>(), pitch));
+    CK(cudaStreamSynchronize(h->stream));                             // the stage buffer and the host coefficients are free again
+    *passes_out = passes;
     return FPM_OK;
 }
 
-// JPEG file image -> grayscale frame like cv::imread(path, IMREAD_GRAYSCALE): luma only, libjpeg's ISLOW IDCT.  Scans without
-// restart intervals are Huffman-decoded on the device (fpm_jpeg_par.cuh: the compressed scan is the only H2D traffic); the
-// others on the host (fpm_jpeg.h), their quantised luma coefficients go to the device.  Dequantisation + IDCT + range limit
-// run on the device in both cases.
-static int ingest_jpeg_impl(fpm_handle* h, const uint8_t* file, size_t nbytes, int* width, int* height);
+// n JPEG file images -> n device-resident frames [n][height][pitch].  The host reads the headers only: the span of all files
+// goes to the device in one copy, the unstuffing kernels read back one record per file (nbits, nint), and the files are
+// decoded in waves that fit FPM_PARAM_WORKSPACE_MB.  A file whose restart markers do not match its header (damaged) is
+// Huffman-decoded on the host, like every file with FPM_PARAM_JPEG_DEVICE_HUFFMAN = 0; dequantisation + IDCT + range limit
+// run on the device for all.
+static int ingest_jpeg_batch_impl(fpm_handle* h, const uint8_t* data, const size_t* offsets, int n, int* width, int* height)
+{
+    std::vector<JpegBatchFile> fs;
+    int rc = jpeg_batch_parse(data, offsets, n, true, &fs, &h->err);
+    if (rc) return rc;
+    for (JpegBatchFile& f : fs) f.device = h->jpeg_device_huffman && jpeg_device_ok(f.fr, f.nbytes);
+    CK(cudaSetDevice(h->device));
+    const size_t base = offsets[0], span = offsets[n] - base;
+    JpUnstuffPlan up;
+    jpeg_unstuff_plan(fs, base, &up);
+    const int ntiles = up.tile_first[n];
+    // d_jpeg_scan: [the files | unstuffed scans | rst | unstuffing records | tile_first | tile sums]
+    const size_t o_out = align_up(span, 256), o_rst = o_out + align_up(up.out_bytes, 256), o_u = o_rst + align_up(up.rst_entries * 4, 256);
+    const size_t o_tf = o_u + align_up((size_t)n * sizeof(JpUnstuff), 256), o_ts = o_tf + align_up((size_t)(n + 1) * 4, 256);
+    CK(h->d_jpeg_scan.ensure(o_ts + (size_t)ntiles * 8 + 256));
+    uint8_t* sb = h->d_jpeg_scan.as<uint8_t>();
+    if (ntiles > 0) {
+        prof_begin(h);
+        CK(cudaMemcpyAsync(sb, data + base, span, cudaMemcpyHostToDevice, h->stream));
+        prof_end(h, K_JPEG_UPLOAD, (double)span);
+        const size_t rec_bytes = o_ts - o_u;
+        CK(h->h_stage.ensure(rec_bytes));
+        uint8_t* hs = h->h_stage.as<uint8_t>();
+        memcpy(hs, up.u.data(), (size_t)n * sizeof(JpUnstuff));
+        memcpy(hs + (o_tf - o_u), up.tile_first.data(), (size_t)(n + 1) * 4);
+        CK(cudaMemcpyAsync(sb + o_u, hs, rec_bytes, cudaMemcpyHostToDevice, h->stream));
+        JpUnstuff* u_dev = reinterpret_cast<JpUnstuff*>(sb + o_u);
+        const int* tf_dev = reinterpret_cast<const int*>(sb + o_tf);
+        unsigned long long* ts_dev = reinterpret_cast<unsigned long long*>(sb + o_ts);
+        KL(K_JPEG_UNSTUFF, span, fpm_jpeg_unstuff_count_kernel<<<ntiles, JP_UNSTUFF_THREADS, 0, h->stream>>>(sb, u_dev, tf_dev, n, ts_dev));
+        KL(K_JPEG_SCAN, ntiles * 8, fpm_jpeg_offsets_kernel<unsigned long long><<<n, 1024, 0, h->stream>>>(tf_dev, ts_dev));
+        KL(K_JPEG_UNSTUFF, span, fpm_jpeg_unstuff_write_kernel<<<ntiles, JP_UNSTUFF_THREADS, 0, h->stream>>>(sb, u_dev, tf_dev, n, ts_dev, sb + o_out,
+                                                                                                     reinterpret_cast<unsigned*>(sb + o_rst)));
+        CK(cudaMemcpyAsync(hs, u_dev, (size_t)n * sizeof(JpUnstuff), cudaMemcpyDeviceToHost, h->stream));
+        CK(cudaStreamSynchronize(h->stream));
+        memcpy(up.u.data(), hs, (size_t)n * sizeof(JpUnstuff));
+    }
+    for (int i = 0; i < n; i++) {
+        if (!fs[i].device) continue;
+        if (up.u[i].nbits == 0) { h->err = jpeg_file_prefix(i, n) + "JPEG without image data"; return FPM_ERR_INVALID; }
+        if (fs[i].fr.restart_interval && up.u[i].nint != jpeg_expected_intervals(fs[i].fr))
+            fs[i].device = false;                                   // e.g. a restart marker is missing: the host decoder says what is wrong
+    }
+    const int W = fs[0].fr.width, H = fs[0].fr.height, pitch = (int)align_up(W, 128);
+    CK(h->d_ingest.ensure((size_t)n * pitch * H));
+    const size_t budget = (size_t)std::max(0.0, h->workspace_mb * 1024.0 * 1024.0);
+    int max_passes = 0;
+    for (int f0 = 0; f0 < n;) {
+        size_t need = 0;
+        int f1 = f0;
+        while (f1 < n && f1 - f0 < 65535) {                         // grid rows of the IDCT kernel
+            const size_t c = jpeg_wave_bytes(fs[f1], up.u[f1]);
+            if (f1 > f0 && need + c > budget) break;
+            need += c;
+            f1++;
+        }
+        int passes = 0;
+        rc = jpeg_decode_wave(h, fs, data, up, f0, f1, sb + o_out, reinterpret_cast<const unsigned*>(sb + o_rst), pitch, &passes);
+        if (rc) return rc;
+        max_passes = std::max(max_passes, passes);
+        f0 = f1;
+    }
+    h->jpeg_passes = max_passes;
+    h->ingest_w = W; h->ingest_h = H; h->ingest_pitch = pitch; h->ingest_count = n;
+    if (width) *width = W;
+    if (height) *height = H;
+    return FPM_OK;
+}
+
+// nothing may be thrown across the C ABI; an error leaves no frame and nothing in flight
+static int ingest_jpeg_batch(fpm_handle* h, const uint8_t* data, const size_t* offsets, int n, int* width, int* height)
+{
+    h->ingest_count = 0;
+    int rc;
+    try {
+        rc = ingest_jpeg_batch_impl(h, data, offsets, n, width, height);
+    } catch (const std::bad_alloc&) {
+        h->err = "out of host memory while decoding the JPEG";
+        rc = FPM_ERR_LIMIT;
+    }
+    if (rc != FPM_OK) {
+        cudaStreamSynchronize(h->stream);
+        h->ingest_count = 0;
+    }
+    return rc;
+}
+
+// JPEG file image -> grayscale frame like cv::imread(path, IMREAD_GRAYSCALE): luma only, libjpeg's ISLOW IDCT.  A batch of one.
 int fpm_ingest_jpeg(fpm_handle* h, const uint8_t* file, size_t nbytes, int* width, int* height)
 {
     if (!h) return FPM_ERR_INVALID;
-    if (!file) { h->err = "null JPEG buffer"; return FPM_ERR_INVALID; }
-    try {                                                             // nothing may be thrown across the C ABI
-        return ingest_jpeg_impl(h, file, nbytes, width, height);
-    } catch (const std::bad_alloc&) {
-        h->err = "out of host memory while decoding the JPEG";
-        return FPM_ERR_LIMIT;
-    }
+    if (!file) { h->ingest_count = 0; h->err = "null JPEG buffer"; return FPM_ERR_INVALID; }
+    const size_t offsets[2] = {0, nbytes};
+    return ingest_jpeg_batch(h, file, offsets, 1, width, height);
 }
 
-static int ingest_jpeg_impl(fpm_handle* h, const uint8_t* file, size_t nbytes, int* width, int* height)
+int fpm_ingest_jpeg_batch(fpm_handle* h, const uint8_t* data, const size_t* offsets, int n, int* width, int* height)
 {
-    fpm_jpeg::Frame fr;
-    {
-        const std::string why = fpm_jpeg::parse(file, nbytes, &fr);
-        if (!why.empty()) { h->err = why; return FPM_ERR_INVALID; }
-    }
-    if ((size_t)fr.height * fr.width > ((size_t)1 << 30)) { h->err = "JPEG too large (more than 2^30 pixels, OpenCV's own limit)"; return FPM_ERR_LIMIT; }
-    bool on_device = h->jpeg_device_huffman && jpeg_device_ok(fr, nbytes);
-    JpScan sc;
-    const int *dcval = nullptr, *tile_off = nullptr;
-    if (on_device) {
-        CK(cudaSetDevice(h->device));
-        int rc = jpeg_decode_device(h, fr, file, nbytes, &sc, &dcval, &tile_off);
-        if (rc == FPM_ERR_UNSUPPORTED_LOCAL) on_device = false;          // e.g. a restart marker is missing: host decoder
-        else if (rc) return rc;
-    }
-    if (on_device) {
-        const int pitch = (int)align_up(fr.width, 128);
-        CK(h->d_ingest.ensure((size_t)pitch * fr.height));
-        FpmJpegQuant qt;
-        memcpy(qt.q, fr.qt[fr.comp[0].tq], sizeof(qt.q));
-        const int bw = sc.bw, bh = sc.mcuy * sc.luma_v, nblk = bw * bh;
-        fpm_ingest_jpeg_idct_kernel<<<(nblk + 127) / 128, 128, 0, h->stream>>>(h->d_ingest_raw.as<int16_t>(), qt, bw, bh, fr.width, fr.height,
-                                                                               h->d_ingest.as<uint8_t>(), pitch, dcval, tile_off, sc);
-        CKL();
-        CK(cudaStreamSynchronize(h->stream));
-        h->ingest_w = fr.width; h->ingest_h = fr.height; h->ingest_pitch = pitch;
-        if (width) *width = fr.width;
-        if (height) *height = fr.height;
-        return FPM_OK;
-    }
-    h->jpeg_passes = 0;
-    fpm_jpeg::Luma im;
-    const std::string why = fpm_jpeg::decode_scan_host(fr, file, nbytes, &im);
-    if (!why.empty()) { h->err = why; return FPM_ERR_INVALID; }
-    CK(cudaSetDevice(h->device));
-    const size_t cbytes = im.coef.size() * sizeof(int16_t);
-    CK(h->d_ingest_raw.ensure(cbytes));
-    const int pitch = (int)align_up(im.width, 128);
-    CK(h->d_ingest.ensure((size_t)pitch * im.height));
-    CK(cudaMemcpyAsync(h->d_ingest_raw.p, im.coef.data(), cbytes, cudaMemcpyHostToDevice, h->stream));
-    FpmJpegQuant qt;
-    memcpy(qt.q, im.quant, sizeof(qt.q));
-    const int nblk = im.bw * im.bh;
-    fpm_ingest_jpeg_idct_kernel<<<(nblk + 127) / 128, 128, 0, h->stream>>>(h->d_ingest_raw.as<int16_t>(), qt, im.bw, im.bh, im.width,
-                                                                           im.height, h->d_ingest.as<uint8_t>(), pitch, nullptr, nullptr, JpScan{});
-    CKL();
-    CK(cudaStreamSynchronize(h->stream));                             // the coefficient vector dies with this call
-    h->ingest_w = im.width; h->ingest_h = im.height; h->ingest_pitch = pitch;
-    if (width) *width = im.width;
-    if (height) *height = im.height;
-    return FPM_OK;
+    if (!h) return FPM_ERR_INVALID;
+    return ingest_jpeg_batch(h, data, offsets, n, width, height);
 }
 
 // what cv::imread does first: pick the decoder by the file's signature (two of the reference's "*.jpg" Test Images are BMP data)
 int fpm_ingest_image(fpm_handle* h, const uint8_t* file, size_t nbytes, int* width, int* height)
 {
     if (!h) return FPM_ERR_INVALID;
+    h->ingest_count = 0;
     if (!file || nbytes < 2) { h->err = "empty image file"; return FPM_ERR_INVALID; }
     if (file[0] == 'B' && file[1] == 'M') return fpm_ingest_bmp(h, file, nbytes, width, height);
     if (file[0] == 0xFF && file[1] == 0xD8) return fpm_ingest_jpeg(h, file, nbytes, width, height);
@@ -2064,59 +2268,144 @@ try {
     return FPM_ERR_LIMIT;
 }
 
-// the PARALLEL decoder (fpm_jpeg_par.cuh) run thread by thread on the CPU, no device: same outputs as fpm_dbg_jpeg_luma;
-// *passes = synchronisation passes it took
-int fpm_dbg_jpeg_luma_parallel(const uint8_t* file, size_t nbytes, int16_t* coef, size_t coef_capacity, int* passes, char* err, int err_capacity)
+// the PARALLEL decoder of a batch (unstuffing + passes + scans, fpm_jpeg_par.cuh) run CTA by CTA, thread by thread on the CPU,
+// no device: file i's coefficients go to coef + coef_offsets[i] (n + 1 entries: file i owns [coef_offsets[i], coef_offsets[i+1])),
+// passes[i] = the synchronisation passes file i took (the pass in which it last moved + 1)
+int fpm_dbg_jpeg_luma_parallel_batch(const uint8_t* data, const size_t* offsets, int n, int16_t* coef, const size_t* coef_offsets,
+                                     int* passes, char* err, int err_capacity)
 try {
-    auto fail = [&](const std::string& why) {
+    auto fail = [&](const std::string& why, int rc = FPM_ERR_INVALID) {
         if (err && err_capacity > 0) { strncpy(err, why.c_str(), err_capacity - 1); err[err_capacity - 1] = 0; }
-        return FPM_ERR_INVALID;
+        return rc;
     };
-    fpm_jpeg::Frame fr;
-    const std::string why = fpm_jpeg::parse(file, nbytes, &fr);
-    if (!why.empty()) return fail(why);
-    if (!jpeg_device_ok(fr, nbytes)) return fail("scan not eligible for the parallel decoder");
-    std::vector<uint8_t> bits(nbytes - fr.scan_begin + 16);
-    std::vector<unsigned> rst;
-    const size_t scan_bytes = jpeg_unstuff(file, nbytes, fr.scan_begin, bits.data(), fr.restart_interval ? &rst : nullptr);
-    std::vector<JpTable> tabs(8);
-    JpScan sc;
-    jpeg_device_tables(fr, tabs.data(), &sc, scan_bytes);
-    if (fr.restart_interval) {
-        sc.nint = (int)rst.size() - 1;
-        sc.rst = rst.data();
-        if (sc.nint != jpeg_expected_intervals(fr)) return fail("restart markers do not match the frame header");
+    std::vector<JpegBatchFile> fs;
+    std::string why;
+    const int rc = jpeg_batch_parse(data, offsets, n, false, &fs, &why);
+    if (rc) return fail(why, rc);
+    if (!coef || !coef_offsets) return fail("null coefficient buffer");
+    for (int i = 0; i < n; i++) {
+        if (!jpeg_device_ok(fs[i].fr, fs[i].nbytes)) return fail(jpeg_file_prefix(i, n) + "scan not eligible for the parallel decoder");
+        fs[i].device = true;
     }
-    const size_t nluma = (size_t)sc.mcux * sc.mcuy * sc.luma_slots;
-    if (coef_capacity < nluma * 64) return FPM_ERR_LIMIT;
-    memset(coef, 0, nluma * 64 * sizeof(int16_t));
-    std::vector<JpState> st[2] = {std::vector<JpState>(sc.nsub), std::vector<JpState>(sc.nsub)}, used(sc.nsub);
-    const JpBytes src{bits.data()};
-    for (int i = 0; i < sc.nsub; i++) jp_pass_cold(i, src, tabs.data(), sc, st[0].data(), used.data());
+    JpUnstuffPlan up;
+    jpeg_unstuff_plan(fs, offsets[0], &up);
+    std::vector<uint8_t> bits(up.out_bytes);
+    std::vector<unsigned> rst(up.rst_entries);
+    jpeg_unstuff_emulate(data + offsets[0], &up, bits.data(), rst.data());
+    for (int i = 0; i < n; i++)
+        if (fs[i].fr.restart_interval && up.u[i].nint != jpeg_expected_intervals(fs[i].fr))
+            return fail(jpeg_file_prefix(i, n) + "restart markers do not match the frame header");
+    JpWave w;
+    jpeg_wave_plan(fs, up, 0, n, rst.data(), 0, &w);
+    for (int i = 0; i < n; i++) {
+        const JpScan& sc = w.files[i].sc;
+        const size_t need = (size_t)sc.mcux * sc.mcuy * sc.luma_slots * 64;
+        if (coef_offsets[i + 1] < coef_offsets[i] || coef_offsets[i + 1] - coef_offsets[i] < need) return FPM_ERR_LIMIT;
+        memset(coef + coef_offsets[i], 0, need * sizeof(int16_t));
+    }
+    std::vector<JpState> st[2] = {std::vector<JpState>(w.nsub), std::vector<JpState>(w.nsub)}, used(w.nsub);
+    const int nb = w.cta_first[n];
+    auto each_thread = [&](auto fn) {                                 // blockIdx.x -> file by the same search as the kernels
+        for (int b = 0; b < nb; b++) {
+            const int fi = jp_file_of(w.cta_first.data(), n, b), cta = b - w.cta_first[fi];
+            const JpFile& f = w.files[fi];
+            for (int t = 0; t < JP_THREADS; t++) fn(fi, f, JpBytes{bits.data() + f.bits}, cta * JP_THREADS + t);
+        }
+    };
+    each_thread([&](int, const JpFile& f, const JpBytes& src, int i) { jp_pass_cold(i, src, f.tabs, f.sc, st[0].data() + f.sub0, used.data() + f.sub0); });
     int cur = 0, np = 0;
+    std::vector<int> last(n, 0), changed(n);
     for (;;) {
-        if (++np > sc.nsub + 1) return fail("JPEG scan did not synchronise");
-        int changed = 0;
-        for (int i = 0; i < sc.nsub; i++) jp_pass_sync(i, src, tabs.data(), sc, st[cur].data(), st[cur ^ 1].data(), used.data(), &changed);
+        if (++np > w.max_nsub + 1) return fail("JPEG scan did not synchronise");
+        std::fill(changed.begin(), changed.end(), 0);
+        each_thread([&](int fi, const JpFile& f, const JpBytes& src, int i) {
+            jp_pass_sync(i, src, f.tabs, f.sc, st[cur].data() + f.sub0, st[cur ^ 1].data() + f.sub0, used.data() + f.sub0, &changed[fi]);
+        });
         cur ^= 1;
-        if (!changed) break;
+        bool any = false;
+        for (int i = 0; i < n; i++)
+            if (changed[i]) { last[i] = np; any = true; }
+        if (!any) break;
     }
-    std::vector<unsigned> first(sc.nsub);
-    unsigned run = 0;
-    for (int i = 0; i < sc.nsub; i++) { first[i] = run; run += st[cur][i].nblk; }
-    std::vector<int> dcval(nluma, 0);
-    for (int i = 0; i < sc.nsub; i++) jp_pass_write(i, src, tabs.data(), sc, st[cur].data(), first.data(), nullptr, coef, dcval.data());
-    int acc = 0;
-    const int bh = sc.mcuy * sc.luma_v;
-    const size_t seg = sc.restart_blocks ? (size_t)sc.restart_blocks / sc.nslots * sc.luma_slots : 0;
-    for (size_t L = 0; L < nluma; L++) {
-        if (seg && L % seg == 0) acc = 0;                               // the DC prediction restarts with every interval
-        acc += dcval[L];
-        dcval[L] = acc;
+    std::vector<unsigned> first(w.nsub);
+    std::vector<int> dcval(w.nluma, 0);
+    for (const JpFile& f : w.files) {
+        unsigned run = 0;
+        for (int i = 0; i < f.sc.nsub; i++) { first[f.sub0 + i] = run; run += st[cur][f.sub0 + i].nblk; }
     }
-    for (int r = 0; r < bh; r++)
-        for (int c = 0; c < sc.bw; c++) coef[((size_t)r * sc.bw + c) * 64] = (int16_t)dcval[jp_luma_scan_index(sc, r, c)];
-    if (passes) *passes = np;
+    each_thread([&](int fi, const JpFile& f, const JpBytes& src, int i) {
+        jp_pass_write(i, src, f.tabs, f.sc, st[cur].data() + f.sub0, first.data() + f.sub0, nullptr, coef + coef_offsets[fi], dcval.data() + f.luma0);
+    });
+    for (int fi = 0; fi < n; fi++) {
+        const JpScan& sc = w.files[fi].sc;
+        int* dc = dcval.data() + w.files[fi].luma0;
+        int16_t* c = coef + coef_offsets[fi];
+        const size_t nluma = (size_t)sc.mcux * sc.mcuy * sc.luma_slots;
+        const size_t seg = sc.restart_blocks ? (size_t)sc.restart_blocks / sc.nslots * sc.luma_slots : 0;
+        int acc = 0;
+        for (size_t L = 0; L < nluma; L++) {
+            if (seg && L % seg == 0) acc = 0;                           // the DC prediction restarts with every interval
+            acc += dc[L];
+            dc[L] = acc;
+        }
+        const int bh = sc.mcuy * sc.luma_v;
+        for (int r = 0; r < bh; r++)
+            for (int col = 0; col < sc.bw; col++) c[((size_t)r * sc.bw + col) * 64] = (int16_t)dc[jp_luma_scan_index(sc, r, col)];
+        if (passes) passes[fi] = last[fi] + 1;
+    }
+    return FPM_OK;
+} catch (const std::bad_alloc&) {
+    return FPM_ERR_LIMIT;
+}
+
+// the same for one file
+int fpm_dbg_jpeg_luma_parallel(const uint8_t* file, size_t nbytes, int16_t* coef, size_t coef_capacity, int* passes, char* err, int err_capacity)
+{
+    const size_t offsets[2] = {0, nbytes}, coef_offsets[2] = {0, coef_capacity};
+    return fpm_dbg_jpeg_luma_parallel_batch(file, offsets, 1, coef, coef_offsets, passes, err, err_capacity);
+}
+
+// unstuffing of one file without a device: emulated = 1 runs the phase functions of the unstuffing kernels, 0 the sequential
+// jpeg_unstuff.  out: the unstuffed bytes + 16 zero bytes (out_cap >= file size - scan start + 20); rst: the first bit of every
+// restart interval and rst[nint] = nbits (0, nbits without restart intervals), up to rst_cap entries
+int fpm_dbg_jpeg_unstuff(const uint8_t* file, size_t nbytes, int emulated, uint8_t* out, size_t out_cap, unsigned* rst, int rst_cap,
+                         unsigned* nbits, int* nint, int* tile)
+try {
+    if (tile) *tile = JP_UNSTUFF_TILE;
+    if (!file || !out) return FPM_ERR_INVALID;
+    fpm_jpeg::Frame fr;
+    if (!fpm_jpeg::parse(file, nbytes, &fr).empty()) return FPM_ERR_INVALID;
+    const size_t cap = align_up(nbytes - fr.scan_begin, 4) + 16;
+    if (out_cap < cap) return FPM_ERR_LIMIT;
+    std::vector<unsigned> rv;
+    unsigned nb;
+    int ni;
+    if (!emulated) {
+        std::vector<uint8_t> tmp(cap);
+        const size_t o = jpeg_unstuff(file, nbytes, fr.scan_begin, tmp.data(), fr.restart_interval ? &rv : nullptr);
+        memcpy(out, tmp.data(), o + 16);
+        nb = (unsigned)(o * 8);
+        ni = fr.restart_interval ? (int)rv.size() - 1 : 1;
+    } else {
+        std::vector<JpegBatchFile> fs(1);
+        fs[0].fr = fr;
+        fs[0].nbytes = nbytes;
+        fs[0].device = true;
+        JpUnstuffPlan up;
+        jpeg_unstuff_plan(fs, 0, &up);
+        if (fr.restart_interval) up.u[0].rst_cap = std::max(rst_cap, 0);
+        std::vector<uint8_t> tmp(up.out_bytes);
+        rv.assign(up.u[0].rst_cap, 0);
+        jpeg_unstuff_emulate(file, &up, tmp.data(), rv.data());
+        nb = up.u[0].nbits;
+        ni = up.u[0].nint;
+        memcpy(out, tmp.data(), nb / 8 + 16);
+        if (fr.restart_interval) rv.resize(std::min<size_t>(rv.size(), (size_t)ni + 1));
+    }
+    if (!fr.restart_interval) rv = {0u, nb};
+    for (int i = 0; i < rst_cap && i < (int)rv.size(); i++) rst[i] = rv[i];
+    if (nbits) *nbits = nb;
+    if (nint) *nint = ni;
     return FPM_OK;
 } catch (const std::bad_alloc&) {
     return FPM_ERR_LIMIT;
@@ -2125,6 +2414,7 @@ try {
 int fpm_ingest_rgb32(fpm_handle* h, const uint32_t* pixels, int width, int height, int stride_bytes)
 {
     if (!h) return FPM_ERR_INVALID;
+    h->ingest_count = 0;
     if (!pixels || width <= 0 || height <= 0 || height > 65535 || width > (1 << 20) || stride_bytes < 4 * width || (stride_bytes & 3)) {
         h->err = "bad RGB32 frame";
         return FPM_ERR_INVALID;
@@ -2140,31 +2430,64 @@ int fpm_ingest_rgb32(fpm_handle* h, const uint32_t* pixels, int width, int heigh
                                                          h->d_ingest.as<uint8_t>(), pitch);
     CKL();
     CK(cudaStreamSynchronize(h->stream));
-    h->ingest_w = width; h->ingest_h = height; h->ingest_pitch = pitch;
+    h->ingest_w = width; h->ingest_h = height; h->ingest_pitch = pitch; h->ingest_count = 1;
+    return FPM_OK;
+}
+
+namespace {
+// the single-frame accessors: exactly one ingested frame (a batch goes through the _batch / _frame_ functions)
+int ingest_single(fpm_handle* h)
+{
+    if (h->ingest_count == 1) return FPM_OK;
+    h->err = h->ingest_count == 0 ? std::string("no ingested frame")
+                                  : "the last ingest left " + std::to_string(h->ingest_count) +
+                                        " frames: use fpm_ingested_frame_pixels / fpm_match_ingested_batch";
+    return FPM_ERR_INVALID;
+}
+}  // namespace
+
+int fpm_ingested_count(const fpm_handle* h) { return h ? h->ingest_count : 0; }
+
+int fpm_ingested_frame_pixels(fpm_handle* h, int index, uint8_t* out)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (!out) { h->err = "null output buffer"; return FPM_ERR_INVALID; }
+    if (index < 0 || index >= h->ingest_count) {
+        h->err = "ingested frame " + std::to_string(index) + " out of range (" + std::to_string(h->ingest_count) + " frames)";
+        return FPM_ERR_INVALID;
+    }
+    CK(cudaSetDevice(h->device));
+    const uint8_t* src = h->d_ingest.as<uint8_t>() + (size_t)index * h->ingest_pitch * h->ingest_h;
+    CK(cudaMemcpy2D(out, (size_t)h->ingest_w, src, (size_t)h->ingest_pitch, (size_t)h->ingest_w, h->ingest_h, cudaMemcpyDeviceToHost));
     return FPM_OK;
 }
 
 int fpm_ingested_pixels(fpm_handle* h, uint8_t* out)
 {
     if (!h || !out) return FPM_ERR_INVALID;
-    if (h->ingest_w <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
-    CK(cudaSetDevice(h->device));
-    CK(cudaMemcpy2D(out, (size_t)h->ingest_w, h->d_ingest.p, (size_t)h->ingest_pitch, (size_t)h->ingest_w, h->ingest_h, cudaMemcpyDeviceToHost));
-    return FPM_OK;
+    if (int rc = ingest_single(h)) return rc;
+    return fpm_ingested_frame_pixels(h, 0, out);
 }
 
 int fpm_match_ingested(fpm_handle* h, fpm_result* out, int cap, int* n)
 {
     if (!h) return FPM_ERR_INVALID;
-    if (h->ingest_w <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
-    return fpm_match_batch_device(h, h->d_ingest.as<uint8_t>(), 1, h->ingest_w, h->ingest_h, h->ingest_pitch,
-                                  (size_t)h->ingest_pitch * h->ingest_h, out, cap, n);
+    if (int rc = ingest_single(h)) return rc;
+    return fpm_match_ingested_batch(h, out, cap, n);
+}
+
+int fpm_match_ingested_batch(fpm_handle* h, fpm_result* out, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (h->ingest_count <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
+    return fpm_match_batch_device(h, h->d_ingest.as<uint8_t>(), h->ingest_count, h->ingest_w, h->ingest_h, h->ingest_pitch,
+                                  (size_t)h->ingest_pitch * h->ingest_h, out, cap, counts);
 }
 
 int fpm_learn_ingested(fpm_handle* h)
 {
     if (!h) return FPM_ERR_INVALID;
-    if (h->ingest_w <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
+    if (int rc = ingest_single(h)) return rc;
     std::vector<uint8_t> px((size_t)h->ingest_w * h->ingest_h);
     int rc = fpm_ingested_pixels(h, px.data());
     if (rc) return rc;
@@ -2832,7 +3155,7 @@ void fpm_profile_reset(fpm_handle* h)
 {
     if (!h) return;
     prof_collect(h);
-    for (int i = 0; i < 16; i++) { h->prof_ms[i] = 0; h->prof_work[i] = 0; h->prof_launches[i] = 0; }
+    for (int i = 0; i < 24; i++) { h->prof_ms[i] = 0; h->prof_work[i] = 0; h->prof_launches[i] = 0; }
     if (h->twin) fpm_profile_reset(h->twin);
 }
 

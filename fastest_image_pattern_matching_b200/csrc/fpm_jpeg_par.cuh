@@ -2,8 +2,8 @@
 // traffic of a JPEG ingest: 1.5 MB for the reference's 12 MP Src6.jpg instead of 24 MB of coefficients or 12 MB of pixels).
 //
 // A Huffman stream has no index, but it is self-synchronising: a decoder that starts at a wrong bit falls into step with
-// the true symbol sequence after a few symbols.  The scan (0xFF00 stuffing removed on the host) is cut into sub-sequences
-// of SUB bits, one thread each:
+// the true symbol sequence after a few symbols.  The scan (0xFF00 stuffing and RST markers removed on the device by a
+// stream compaction, jp_unstuff_*) is cut into sub-sequences of SUB bits, one thread each:
 //   pass 0     every thread decodes its sub-sequence from its first bit as if a block started there and records its EXIT
 //              state: the bit where its last symbol ended (inside the next sub-sequence), the block slot inside the MCU
 //              and the coefficient index it was at, and how many blocks it completed;
@@ -14,8 +14,11 @@
 //   then       an exclusive scan of the block counts gives every thread the index of its first block; a last pass decodes
 //              once more and writes the coefficients of the luma blocks (DC as differences); a scan over the luma blocks in
 //              scan order turns the DC differences into values.
-// Every phase function is __host__ __device__: fpm_dbg_jpeg_luma_parallel runs the same code thread by thread on the CPU and
-// tests/test_ingest.py checks it against the sequential decoder (fpm_jpeg.h) in the GPU-less container.
+// Every phase function is __host__ __device__: fpm_dbg_jpeg_luma_parallel(_batch) runs the same code thread by thread on the
+// CPU and tests/test_ingest.py, tests/test_ingest_batch.py check it against the sequential decoder (fpm_jpeg.h) without a GPU.
+// A batch of files is decoded by the same launches: every file has a descriptor (JpFile), a CTA finds its file by a binary
+// search over the first-CTA prefix, and each file's sub-sequences / luma blocks start on a 4096 / JP_DC_TILE boundary of the
+// shared state / DC arrays so that the tile scans run over the concatenation unchanged.
 // Restart intervals are exact entry points: a decoder that reaches the (all-ones, < 8 bits) padding at the end of an interval,
 // or runs over its end while it is out of step, restarts at the first bit of the next interval; the DC differences are then
 // summed per interval.
@@ -279,10 +282,121 @@ FPM_HD unsigned jp_luma_scan_index(const JpScan& sc, int row, int col)
     return (unsigned)(my * sc.mcux + mx) * sc.luma_slots + (unsigned)(sy * sc.luma_h + sx);
 }
 
+// ---- batches -----------------------------------------------------------------------------------------------------------
+// last i in [0, n) with first[i] <= x (first non-decreasing, first[0] <= x): the file of a CTA or tile.  Files with no CTAs
+// share their first[] value with the next file and are never picked.
+FPM_HD int jp_file_of(const int* first, int n, int x)
+{
+    int lo = 0, hi = n;
+    while (hi - lo > 1) {
+        const int mid = (lo + hi) >> 1;
+        if (first[mid] <= x) lo = mid; else hi = mid;
+    }
+    return lo;
+}
+
+// Unstuffing as a stream compaction over the entropy-coded segments of all files.  Whether byte i is emitted depends on
+// d[i-1], d[i], d[i+1] only (jp_unstuff_class); the output position of an emitted byte is an exclusive scan of the emit flags,
+// the restart interval a RST marker opens a scan of the RST flags.  The scan ends at the first other marker (a min-reduction
+// over the file) or at the position after the file's last byte; the thread that owns that position writes nbits / nint, the
+// sentinel rst[nint] and the 16 zero bytes the decoder reads ahead.  The output equals the sequential jpeg_unstuff
+// (fpm_host.cu) for every input, damaged and truncated files included.
+#define JP_UNSTUFF_THREADS 256
+#define JP_UNSTUFF_BYTES 16                                          // per thread
+#define JP_UNSTUFF_TILE (JP_UNSTUFF_THREADS * JP_UNSTUFF_BYTES)      // per CTA; a tile never spans two files
+
+struct JpUnstuff {                 // one file of a batch (offsets into the uploaded batch buffer / the output arrays)
+    unsigned long long begin, end; // entropy-coded data: from the byte after SOS to the end of the file
+    unsigned long long out;        // output slot, 4-aligned, align4(end - begin) + 16 bytes
+    unsigned long long rst;        // first of the file's rst_cap entries of rst[]
+    unsigned long long stop;       // in: end; out: the position where the scan ends
+    int rst_cap;
+    int restart;                   // DRI present: RSTn separates intervals; otherwise it ends the scan like any other marker
+    unsigned nbits;                // out: unstuffed length in bits
+    int nint;                      // out: restart intervals (RST markers before the stop + 1)
+};
+enum { JP_EMIT = 1, JP_RST = 2, JP_STOP = 4 };
+
+FPM_HD int jp_unstuff_class(const uint8_t* d, const JpUnstuff& f, unsigned long long i)
+{
+    if (i >= f.end) return JP_STOP;                                      // the position after the last byte
+    const unsigned b = d[i];
+    if (b != 0xFF) return i > f.begin && d[i - 1] == 0xFF ? 0 : JP_EMIT; // an FF is never the second byte of a pair, so this
+                                                                         // byte is the second byte of FF xx exactly when d[i-1] is FF
+    if (i + 1 >= f.end) return 0;                                        // 0xFF as the last byte
+    const unsigned c = d[i + 1];
+    if (c == 0x00) return JP_EMIT;                                       // stuffed 0xFF
+    if (c == 0xFF) return 0;                                             // fill byte
+    if (f.restart && c >= 0xD0 && c <= 0xD7) return JP_RST;
+    return JP_STOP;
+}
+
+// positions [a, b) of one thread's chunk: emitted bytes, RST markers, first stop (~0 if none)
+FPM_HD void jp_unstuff_count(const uint8_t* d, const JpUnstuff& f, unsigned long long a, unsigned long long b, unsigned* emit,
+                             unsigned* rst, unsigned long long* stop)
+{
+    unsigned e = 0, r = 0;
+    unsigned long long s = ~0ull;
+    for (unsigned long long i = a; i < b; i++) {
+        const int c = jp_unstuff_class(d, f, i);
+        e += c & JP_EMIT;
+        r += (c >> 1) & 1;
+        if ((c & JP_STOP) && s == ~0ull) s = i;
+    }
+    *emit = e; *rst = r; *stop = s;
+}
+
+// the same chunk again, f.stop final: o / r = bytes emitted / RST markers met before position a
+FPM_HD void jp_unstuff_write(const uint8_t* d, JpUnstuff& f, unsigned long long a, unsigned long long b, unsigned o, unsigned r,
+                             uint8_t* out, unsigned* rst)
+{
+    const unsigned long long stop = f.stop;
+    uint8_t* dst = out + f.out;
+    unsigned* rs = rst + f.rst;
+    const unsigned cap = (unsigned)f.rst_cap;
+    for (unsigned long long i = a; i < b && i <= stop; i++) {
+        if (i == stop) {
+            for (unsigned k = o; k < ((o + 3) & ~3u) + 16; k++) dst[k] = 0;
+            if (cap > 0) rs[0] = 0;
+            if (r + 1 < cap) rs[r + 1] = o * 8;                      // sentinel rst[nint] = nbits
+            f.nbits = o * 8;
+            f.nint = (int)r + 1;
+            return;
+        }
+        const int c = jp_unstuff_class(d, f, i);
+        if (c & JP_EMIT) dst[o++] = d[i];
+        if (c & JP_RST) {
+            r++;
+            if (r < cap) rs[r] = o * 8;
+        }
+    }
+}
+
+// positions [a, b) of thread `t` of tile `tile` of the file (b <= end + 1: end itself is the position that may stop the scan)
+FPM_HD void jp_unstuff_chunk(const JpUnstuff& f, int tile, int t, unsigned long long* a, unsigned long long* b)
+{
+    *a = f.begin + (unsigned long long)tile * JP_UNSTUFF_TILE + (unsigned long long)t * JP_UNSTUFF_BYTES;
+    *b = *a + JP_UNSTUFF_BYTES < f.end + 1 ? *a + JP_UNSTUFF_BYTES : f.end + 1;
+}
+
+struct JpFile {                    // one file of a decode wave
+    JpTable tabs[8];
+    JpScan sc;                     // sc.rst points at the file's entries of the batch's rst array
+    uint16_t quant[64];            // luma quantisation table, natural order
+    unsigned long long bits;       // byte offset of the unstuffed scan (4-aligned)
+    unsigned long long coef;       // first coefficient of luma block 0 in the wave's coefficient array
+    unsigned long long frame;      // byte offset of the output frame
+    int sub0;                      // first sub-sequence in the state arrays (a multiple of 4096)
+    int luma0;                     // first luma block in the DC array (a multiple of JP_DC_TILE)
+    int width, height;
+    int device_huffman;            // 0: Huffman-decoded on the host, coef holds its coefficients with the DC values
+    int pad;
+};
+
 #ifdef __CUDACC__
 // A decoder thread is one long chain of dependent loads (window -> table -> next window): out of global memory that is
 // ~1.4 us per symbol with one warp per SM sub-partition.  The CTA therefore stages its 128 sub-sequences (16 KB + the few
-// bytes the last symbol may reach into the next one) and the eight tables (11 KB) in shared memory first.
+// bytes the last symbol may reach into the next one) and its file's eight tables (11 KB) in shared memory first.
 #define JP_THREADS 128
 #define JP_CHUNK_BYTES (JP_THREADS * JP_SUB_BITS / 8)
 
@@ -293,11 +407,12 @@ struct JpShared {
     uint32_t words[JP_CHUNK_WORDS + JP_CHUNK_WORDS / JP_SUB_WORDS + 8];
 };
 
+// chunk `cta` of the file's unstuffed scan
 __device__ __forceinline__ JpWords jp_stage(JpShared& sh, const uint8_t* __restrict__ bits, const JpTable* __restrict__ tabs,
-                                            const JpScan& sc)
+                                            const JpScan& sc, int cta)
 {
-    const size_t byte0 = (size_t)blockIdx.x * JP_CHUNK_BYTES;
-    const size_t total = (((size_t)sc.nbits + 7) / 8 + 16 + 3) & ~(size_t)3;     // data + the zero padding the host appended
+    const size_t byte0 = (size_t)cta * JP_CHUNK_BYTES;
+    const size_t total = (((size_t)sc.nbits + 7) / 8 + 16 + 3) & ~(size_t)3;     // data + the zero padding after it
     const uint32_t* gt = reinterpret_cast<const uint32_t*>(tabs);
     uint32_t* st = reinterpret_cast<uint32_t*>(sh.tabs);
     for (int i = threadIdx.x; i < (int)(sizeof(sh.tabs) / 4); i += JP_THREADS) st[i] = gt[i];
@@ -314,45 +429,58 @@ __device__ __forceinline__ JpWords jp_stage(JpShared& sh, const uint8_t* __restr
     return src;
 }
 
+// the decoder grids: cta_first[i] = first CTA of file i (n + 1 entries), blockIdx.x -> (file, CTA of the file)
 __global__ void __launch_bounds__(JP_THREADS)
-fpm_jpeg_cold_kernel(const uint8_t* bits, const JpTable* tabs, JpScan sc, JpState* exit_state, JpState* entry_used)
+fpm_jpeg_cold_kernel(const JpFile* __restrict__ files, const int* __restrict__ cta_first, int n, const uint8_t* bits,
+                     JpState* exit_state, JpState* entry_used)
 {
     __shared__ JpShared sh;
-    const JpWords b = jp_stage(sh, bits, tabs, sc);
-    jp_pass_cold(blockIdx.x * JP_THREADS + threadIdx.x, b, sh.tabs, sh.sc, exit_state, entry_used);
+    const int fi = jp_file_of(cta_first, n, blockIdx.x), cta = blockIdx.x - cta_first[fi];
+    const JpFile& f = files[fi];
+    const JpWords b = jp_stage(sh, bits + f.bits, f.tabs, f.sc, cta);
+    jp_pass_cold(cta * JP_THREADS + threadIdx.x, b, sh.tabs, sh.sc, exit_state + f.sub0, entry_used + f.sub0);
 }
 
+// one changed-flag for the whole wave: the pass loop ends when no file moved
 __global__ void __launch_bounds__(JP_THREADS)
-fpm_jpeg_sync_kernel(const uint8_t* bits, const JpTable* tabs, JpScan sc, const JpState* prev, JpState* next,
-                     JpState* entry_used, int* changed)
+fpm_jpeg_sync_kernel(const JpFile* __restrict__ files, const int* __restrict__ cta_first, int n, const uint8_t* bits,
+                     const JpState* prev, JpState* next, JpState* entry_used, int* changed)
 {
     __shared__ JpShared sh;
-    // a CTA whose entry states did not move has nothing to decode: skip the staging too
-    const int i = blockIdx.x * JP_THREADS + threadIdx.x;
+    const int fi = jp_file_of(cta_first, n, blockIdx.x), cta = blockIdx.x - cta_first[fi];
+    const JpFile& f = files[fi];
+    const int nsub = f.sc.nsub;
+    prev += f.sub0; next += f.sub0; entry_used += f.sub0;
+    // a CTA whose entry states did not move (its file has converged) has nothing to decode: skip the staging too
+    const int i = cta * JP_THREADS + threadIdx.x;
     bool work = false;
-    if (i > 0 && i < sc.nsub) {
+    if (i > 0 && i < nsub) {
         const JpState in = prev[i - 1], used = entry_used[i];
         work = in.p != used.p || in.slot_k != used.slot_k;
     }
     if (!__syncthreads_or(work)) {
-        if (i < sc.nsub) next[i] = prev[i];
+        if (i < nsub) next[i] = prev[i];
         return;
     }
-    const JpWords b = jp_stage(sh, bits, tabs, sc);
+    const JpWords b = jp_stage(sh, bits + f.bits, f.tabs, f.sc, cta);
     jp_pass_sync(i, b, sh.tabs, sh.sc, prev, next, entry_used, changed);
 }
 
 __global__ void __launch_bounds__(JP_THREADS)
-fpm_jpeg_write_kernel(const uint8_t* bits, const JpTable* tabs, JpScan sc, const JpState* state, const unsigned* blk_first,
-                      const int* blk_tile_off, int16_t* coef, int* dcval)
+fpm_jpeg_write_kernel(const JpFile* __restrict__ files, const int* __restrict__ cta_first, int n, const uint8_t* bits,
+                      const JpState* state, const unsigned* blk_first, const int* blk_tile_off, int16_t* coef, int* dcval)
 {
     __shared__ JpShared sh;
-    const JpWords b = jp_stage(sh, bits, tabs, sc);
-    jp_pass_write(blockIdx.x * JP_THREADS + threadIdx.x, b, sh.tabs, sh.sc, state, blk_first, blk_tile_off, coef, dcval);
+    const int fi = jp_file_of(cta_first, n, blockIdx.x), cta = blockIdx.x - cta_first[fi];
+    const JpFile& f = files[fi];
+    const JpWords b = jp_stage(sh, bits + f.bits, f.tabs, f.sc, cta);
+    jp_pass_write(cta * JP_THREADS + threadIdx.x, b, sh.tabs, sh.sc, state + f.sub0, blk_first + f.sub0, blk_tile_off + f.sub0 / 4096,
+                  coef + f.coef, dcval + f.luma0);
 }
 
 // Exclusive scan of the block counts: tiles of 4096 sub-sequences by one CTA each (blk_first[i] = blocks before i inside its
-// tile, tile_sum = the tile's total), fpm_jpeg_dc_offsets_kernel scans the totals, the write pass adds its tile's offset.
+// tile, tile_sum = the tile's total), fpm_jpeg_offsets_kernel scans the totals of every file, the write pass adds its tile's
+// offset.  A file's sub-sequences start on a tile boundary, so no tile mixes two files.
 __global__ void __launch_bounds__(256)
 fpm_jpeg_block_tile_kernel(const JpState* __restrict__ state, int n, unsigned* __restrict__ blk_first, int* __restrict__ tile_sum)
 {
@@ -379,7 +507,7 @@ fpm_jpeg_block_tile_kernel(const JpState* __restrict__ state, int n, unsigned* _
 }
 
 // DC differences -> DC values: an inclusive scan over the luma blocks in scan order.  Tiles of 4096 values are scanned in
-// place by one CTA each (fpm_jpeg_dc_tile_kernel), the tile totals by one CTA (fpm_jpeg_dc_offsets_kernel); the IDCT kernel
+// place by one CTA each (fpm_jpeg_dc_tile_kernel), the tile totals of every file by fpm_jpeg_offsets_kernel; the IDCT kernel
 // adds the offset of a value's tile when it reads it.
 #define JP_DC_TILE 4096
 __global__ void __launch_bounds__(256)
@@ -407,23 +535,82 @@ fpm_jpeg_dc_tile_kernel(int n, int* __restrict__ dcval, int* __restrict__ tile_s
     if (t == 255) tile_sum[blockIdx.x] = woff + inc;
 }
 
-// exclusive scan of the tile totals in place, one CTA (a 12 MP image has 47 tiles)
+// exclusive scan in place of the tile totals v[seg[b] .. seg[b+1]) of file b, one CTA per file (a 12 MP image has 47 DC
+// tiles, a 1.5 MB scan 370 unstuffing tiles)
+template <class T>
 __global__ void __launch_bounds__(1024)
-fpm_jpeg_dc_offsets_kernel(int ntiles, int* __restrict__ tile_sum)
+fpm_jpeg_offsets_kernel(const int* __restrict__ seg, T* __restrict__ v)
 {
-    __shared__ int s_sum[1024];
+    __shared__ T s_sum[1024];
+    T* tile_sum = v + seg[blockIdx.x];
+    const int ntiles = seg[blockIdx.x + 1] - seg[blockIdx.x];
     const int t = threadIdx.x, per = (ntiles + 1023) / 1024, a = min(ntiles, t * per), b = min(ntiles, a + per);
-    int sum = 0;
+    T sum = 0;
     for (int i = a; i < b; i++) sum += tile_sum[i];
     s_sum[t] = sum;
     __syncthreads();
     for (int o = 1; o < 1024; o <<= 1) {
-        const int v = t >= o ? s_sum[t - o] : 0;
+        const T u = t >= o ? s_sum[t - o] : (T)0;
         __syncthreads();
-        s_sum[t] += v;
+        s_sum[t] += u;
         __syncthreads();
     }
-    int run = s_sum[t] - sum;
-    for (int i = a; i < b; i++) { const int v = tile_sum[i]; tile_sum[i] = run; run += v; }
+    T run = s_sum[t] - sum;
+    for (int i = a; i < b; i++) { const T u = tile_sum[i]; tile_sum[i] = run; run += u; }
+}
+
+// ---- unstuffing kernels: tile_first[i] = first tile of file i (n + 1 entries), a tile = JP_UNSTUFF_TILE positions ----------
+
+// exclusive scan over the CTA of (emitted << 32 | rst), 256 threads
+__device__ __forceinline__ unsigned long long jp_unstuff_block_scan(unsigned long long v, unsigned long long* total)
+{
+    __shared__ unsigned long long s_warp[JP_UNSTUFF_THREADS / 32];
+    const int t = threadIdx.x;
+    unsigned long long inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned long long u = __shfl_up_sync(0xffffffffu, inc, o);
+        if ((t & 31) >= o) inc += u;
+    }
+    if ((t & 31) == 31) s_warp[t >> 5] = inc;
+    __syncthreads();
+    unsigned long long woff = 0, all = 0;
+    for (int w = 0; w < JP_UNSTUFF_THREADS / 32; w++) {
+        if (w < (t >> 5)) woff += s_warp[w];
+        all += s_warp[w];
+    }
+    *total = all;
+    return woff + inc - v;
+}
+
+__global__ void __launch_bounds__(JP_UNSTUFF_THREADS)
+fpm_jpeg_unstuff_count_kernel(const uint8_t* __restrict__ d, JpUnstuff* files, const int* __restrict__ tile_first, int n,
+                              unsigned long long* __restrict__ tile_sum)
+{
+    const int fi = jp_file_of(tile_first, n, blockIdx.x);
+    JpUnstuff& f = files[fi];
+    unsigned long long a, b, s = ~0ull;
+    jp_unstuff_chunk(f, blockIdx.x - tile_first[fi], threadIdx.x, &a, &b);
+    unsigned e = 0, r = 0;
+    if (a < b) jp_unstuff_count(d, f, a, b, &e, &r, &s);
+    if (s != ~0ull) atomicMin(&f.stop, s);
+    unsigned long long total;
+    jp_unstuff_block_scan(((unsigned long long)e << 32) | r, &total);
+    if (threadIdx.x == 0) tile_sum[blockIdx.x] = total;
+}
+
+__global__ void __launch_bounds__(JP_UNSTUFF_THREADS)
+fpm_jpeg_unstuff_write_kernel(const uint8_t* __restrict__ d, JpUnstuff* files, const int* __restrict__ tile_first, int n,
+                              const unsigned long long* __restrict__ tile_off, uint8_t* __restrict__ out, unsigned* __restrict__ rst)
+{
+    const int fi = jp_file_of(tile_first, n, blockIdx.x);
+    JpUnstuff& f = files[fi];
+    unsigned long long a, b, s;
+    jp_unstuff_chunk(f, blockIdx.x - tile_first[fi], threadIdx.x, &a, &b);
+    unsigned e = 0, r = 0;
+    if (a < b) jp_unstuff_count(d, f, a, b, &e, &r, &s);
+    unsigned long long total;
+    const unsigned long long x = jp_unstuff_block_scan(((unsigned long long)e << 32) | r, &total) + tile_off[blockIdx.x];
+    if (a < b && a <= f.stop) jp_unstuff_write(d, f, a, b, (unsigned)(x >> 32), (unsigned)x, out, rst);
 }
 #endif

@@ -1505,8 +1505,8 @@ __global__ void fpm_ingest_rgb32_kernel(const uint32_t* __restrict__ px, int spi
 // JPEG luma blocks -> u8 pixels: dequantisation + libjpeg's accurate integer IDCT (JDCT_ISLOW, jidctint.c: the decoder
 // behind cv::imread, 13-bit constants, 2 extra bits after the column pass, descale by 18 after the row pass) + the
 // post-IDCT range limit (10-bit wrap, +128, clamp).  One thread per 8x8 block; integer-exact, so the frame is bit-identical
-// to cv2.imdecode(IMREAD_GRAYSCALE) (tests/test_ingest.py).  The Huffman decoding happened on the host (fpm_jpeg.h).
-struct FpmJpegQuant { uint16_t q[64]; };
+// to cv2.imdecode(IMREAD_GRAYSCALE) (tests/test_ingest.py).  The Huffman decoding happened on the device (fpm_jpeg_par.cuh)
+// or on the host (fpm_jpeg.h).
 
 __device__ __forceinline__ void fpm_idct_islow_1d(const int (&in)[8], int (&out)[8], int shift)
 {
@@ -1533,15 +1533,21 @@ __device__ __forceinline__ void fpm_idct_islow_1d(const int (&in)[8], int (&out)
     out[3] = (tmp13 + tmp0 + r) >> shift; out[4] = (tmp13 - tmp0 + r) >> shift;
 }
 
-// dcval (optional): DC values of the luma blocks in scan order, each still short of its tile's offset dc_tile_off[L / 4096]
-// (device Huffman path: fpm_jpeg_par.cuh); else coef[b][0]
+// One file of the wave per grid row (blockIdx.y).  Files decoded on the device take their DC values from dcval (luma blocks in
+// scan order from f.luma0, each still short of its tile's offset dc_tile_off[L / 4096], fpm_jpeg_par.cuh); files decoded on
+// the host from coef[b][0].  Frame of file f at frames + f.frame.
 __global__ void __launch_bounds__(128)
-fpm_ingest_jpeg_idct_kernel(const int16_t* __restrict__ coef, FpmJpegQuant qt, int bw, int bh, int w, int h,
-                            uint8_t* __restrict__ dst, int dpitch, const int* __restrict__ dcval, const int* __restrict__ dc_tile_off,
-                            JpScan sc)
+fpm_ingest_jpeg_idct_kernel(const JpFile* __restrict__ files, const int16_t* __restrict__ coef, const int* __restrict__ dcval,
+                            const int* __restrict__ dc_tile_off, uint8_t* __restrict__ frames, int dpitch)
 {
+    const JpFile& f = files[blockIdx.y];
+    const JpScan& sc = f.sc;
+    const int bw = sc.bw, bh = sc.mcuy * sc.luma_v, w = f.width, h = f.height;
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= bw * bh) return;
+    const uint16_t* q = f.quant;
+    uint8_t* dst = frames + f.frame;
+    coef += f.coef;
     const int by = b / bw, bx = b - by * bw;
     const uint4* c4 = reinterpret_cast<const uint4*>(coef + (size_t)b * 64);
     int ws[8][8];
@@ -1551,18 +1557,20 @@ fpm_ingest_jpeg_idct_kernel(const int16_t* __restrict__ coef, FpmJpegQuant qt, i
         const uint32_t u[4] = {v.x, v.y, v.z, v.w};
 #pragma unroll
         for (int k = 0; k < 4; k++) {
-            ws[r][2 * k] = (int)(int16_t)(u[k] & 0xffffu) * (int)qt.q[8 * r + 2 * k];
-            ws[r][2 * k + 1] = (int)(int16_t)(u[k] >> 16) * (int)qt.q[8 * r + 2 * k + 1];
+            ws[r][2 * k] = (int)(int16_t)(u[k] & 0xffffu) * (int)q[8 * r + 2 * k];
+            ws[r][2 * k + 1] = (int)(int16_t)(u[k] >> 16) * (int)q[8 * r + 2 * k + 1];
         }
     }
-    if (dcval) {
+    if (f.device_huffman) {
+        dcval += f.luma0;
+        dc_tile_off += f.luma0 / JP_DC_TILE;
         const unsigned L = jp_luma_scan_index(sc, by, bx);
         int dc = dcval[L] + dc_tile_off[L / JP_DC_TILE];
         if (sc.restart_blocks) {                                        // the DC prediction restarts with every interval
             const unsigned seg = sc.restart_blocks / sc.nslots * sc.luma_slots, s0 = L / seg * seg;
             if (s0) dc -= dcval[s0 - 1] + dc_tile_off[(s0 - 1) / JP_DC_TILE];
         }
-        ws[0][0] = (int)(int16_t)dc * (int)qt.q[0];
+        ws[0][0] = (int)(int16_t)dc * (int)q[0];
     }
 #pragma unroll
     for (int c = 0; c < 8; c++) {                                       // pass 1: columns, results scaled up by 4

@@ -193,6 +193,49 @@ class TemplateMatcher:
         self._check(self._lib.fpm_learn_ingested(self._h))
         return True
 
+    def ingestJpegBatch(self, files, offsets=None) -> tuple:
+        """n JPEG file images of one frame size -> n device-resident grayscale frames; returns (width, height).
+        files: a list of bytes-like objects (packed here into one buffer), or a 1-D uint8 buffer holding the files back to back
+        with offsets (n + 1 entries): a numpy array, or the data_ptr() of a pinned torch CPU tensor (no copy, PCIe rate)."""
+        if offsets is None:
+            parts = [np.frombuffer(bytes(f), np.uint8) for f in files]
+            offs = np.zeros(len(parts) + 1, np.uint64)
+            offs[1:] = np.cumsum([p.size for p in parts])
+            buf = np.concatenate(parts) if parts else np.zeros(0, np.uint8)
+            ptr = buf.ctypes.data
+        else:
+            offs = np.ascontiguousarray(offsets, np.uint64)
+            if isinstance(files, int):
+                buf, ptr = None, files
+            else:
+                buf = np.ascontiguousarray(files, np.uint8)
+                if buf.ndim != 1:
+                    raise FpmError("the packed JPEG buffer must be 1-D uint8")
+                if offs.size and int(offs[-1]) > buf.size:
+                    raise FpmError("JPEG batch offsets run past the buffer")
+                ptr = buf.ctypes.data
+        n = max(int(offs.size) - 1, 0)
+        w, h = C.c_int(0), C.c_int(0)
+        self._check(self._lib.fpm_ingest_jpeg_batch(self._h, ptr, offs.ctypes.data, n, C.byref(w), C.byref(h)))
+        self._ingest_shape = (h.value, w.value)
+        return w.value, h.value
+
+    def ingestedCount(self) -> int: return int(self._lib.fpm_ingested_count(self._h))
+
+    def ingestedFramePixels(self, index: int) -> np.ndarray:
+        out = np.zeros(self._ingest_shape, np.uint8)
+        self._check(self._lib.fpm_ingested_frame_pixels(self._h, int(index), out.ctypes.data))
+        return out
+
+    def matchIngestedBatch(self) -> List[List[SingleTargetMatch]]:
+        """the frames of the last ingest matched as one batch: one result list per frame"""
+        B = self.ingestedCount()
+        cap = self.result_capacity
+        res = (L.fpm_result * (cap * max(B, 1)))()
+        n = (C.c_int * max(B, 1))()
+        self._check(self._lib.fpm_match_ingested_batch(self._h, res, cap, n))
+        return [_convert(res[b * cap:(b + 1) * cap], min(n[b], cap)) for b in range(B)]
+
     def matchBatch(self, frames: np.ndarray) -> List[List[SingleTargetMatch]]:
         """frames: [B, H, W] uint8 in host memory (pinned for full PCIe speed)."""
         f = np.asarray(frames)

@@ -68,7 +68,8 @@ enum fpm_param {
                                       counts read on the device): -1 = automatic (batches of fewer than 8 frames), 0 = never, 1 = always */
     FPM_PARAM_JPEG_DEVICE_HUFFMAN = 23, /* fpm_ingest_jpeg: 1 (default) = the scan is Huffman-decoded on the device (the compressed scan is the
                                            only H2D traffic), 0 = on the host (sequential; its coefficients are uploaded) */
-    FPM_PARAM_JPEG_PASSES = 24,    /* read-only: synchronisation passes of the last device-decoded JPEG scan (0 = it was decoded on the host) */
+    FPM_PARAM_JPEG_PASSES = 24,    /* read-only: synchronisation passes of the last JPEG ingest (0 = decoded on the host); a batch iterates
+                                      as one, so this is the count of its slowest file */
     FPM_PARAM_COUNT_
 };
 
@@ -142,6 +143,22 @@ int fpm_ingest_rgb32(fpm_handle* h, const uint32_t* pixels, int width, int heigh
 int fpm_ingested_pixels(fpm_handle* h, uint8_t* out);
 int fpm_match_ingested(fpm_handle* h, fpm_result* out, int cap, int* n);
 int fpm_learn_ingested(fpm_handle* h);
+/* Batched JPEG ingest: n JPEG file images packed back to back in ONE host buffer, file i = data[offsets[i], offsets[i+1]) (offsets
+ * has n+1 entries).  All files must decode to frames of one width x height.  Result: n device-resident frames [n][height][pitch]
+ * owned by the handle, frame i bit-identical to cv::imread(IMREAD_GRAYSCALE) of file i (what fpm_ingest_jpeg gives for that file
+ * alone).  The host reads only the marker segments in front of each scan; the bytes data[offsets[0], offsets[n]) go to the device
+ * in one cudaMemcpyAsync (pinned memory: PCIe rate), where the stuffing is removed and all files are Huffman-decoded by the same
+ * launches, in waves of consecutive files that fit FPM_PARAM_WORKSPACE_MB.  FPM_ERR_INVALID (the message names the file) for an
+ * empty batch, null pointers, decreasing offsets, a file fpm_ingest_jpeg rejects, or a frame size that differs from file 0's;
+ * FPM_ERR_LIMIT above 2^30 pixels per frame.
+ * Every ingest leaves fpm_ingested_count frames (1 for the single-file calls, 0 after an error).  fpm_ingested_pixels,
+ * fpm_match_ingested and fpm_learn_ingested need exactly one; fpm_ingested_frame_pixels copies frame `index` (width*height
+ * bytes), fpm_match_ingested_batch matches all of them (= fpm_match_batch_device on the frames: out holds count*cap records,
+ * counts holds count totals). */
+int fpm_ingest_jpeg_batch(fpm_handle* h, const uint8_t* data, const size_t* offsets, int n, int* width, int* height);
+int fpm_ingested_count(const fpm_handle* h);
+int fpm_ingested_frame_pixels(fpm_handle* h, int index, uint8_t* out);
+int fpm_match_ingested_batch(fpm_handle* h, fpm_result* out, int cap, int* counts);
 
 /* getLastExecutionTime (include/TemplateMatcher.h:40), milliseconds of the last match call. */
 double fpm_last_time_ms(const fpm_handle* h);
@@ -223,6 +240,16 @@ int fpm_dbg_jpeg_luma(const uint8_t* file, size_t nbytes, int* width, int* heigh
 /* the parallel (device) Huffman decoder of fpm_ingest_jpeg run thread by thread on the CPU: same coefficients as fpm_dbg_jpeg_luma */
 int fpm_dbg_jpeg_luma_parallel(const uint8_t* file, size_t nbytes, int16_t* coef, size_t coef_capacity, int* passes, char* err,
                                int err_capacity);
+/* CPU emulation of the whole batched device decoder (unstuffing + passes + scans), thread by thread, no device: quantised luma
+   coefficients of every file, file i's [bh*bw][64] blocks at coef + coef_offsets[i] (coef_offsets has n+1 entries: file i owns
+   [coef_offsets[i], coef_offsets[i+1])); passes[i] = the synchronisation passes of file i.  Files may differ in size. */
+int fpm_dbg_jpeg_luma_parallel_batch(const uint8_t* data, const size_t* offsets, int n, int16_t* coef, const size_t* coef_offsets,
+                                     int* passes, char* err, int err_capacity);
+/* unstuffing of one file's entropy-coded segment, no device: emulated = 1 runs the device phase functions thread by thread, 0 the
+   sequential host reference.  out (out_cap >= file size - scan start + 20): the bytes + 16 zero bytes; rst: first bit of every
+   restart interval, rst[nint] = nbits (0, nbits without restart intervals); *tile = the compaction tile size in bytes */
+int fpm_dbg_jpeg_unstuff(const uint8_t* file, size_t nbytes, int emulated, uint8_t* out, size_t out_cap, unsigned* rst, int rst_cap,
+                         unsigned* nbits, int* nint, int* tile);
 /* one launch of the two-level pyramid kernel: dst1 = pyrDown(src), dst2 = pyrDown(dst1) (dst2 may be NULL: one level).
    misalign: byte offset of the device copy of src past a 128-byte boundary, also added to its pitch (0 / 8 / 4 / odd select
    the 16- / 8- / 4-byte cp.async and the byte staging paths). */
