@@ -101,6 +101,8 @@ SIGNATURES = {
     "fpm_trace_num_evals": (_i, [_vp, _i]),
     "fpm_trace_evals": (_i, [_vp, _i, _vp]),
     "fpm_trace_level": (_i, [_vp, _i, _vp, _pi, _pi]),
+    "fpm_trace_eval_scores": (_i, [_vp, _i, _vp]),
+    "fpm_trace_eval_rois": (_i, [_vp, _i, _vp, _pi, _pi, _pi]),
 }
 
 _lib = None

@@ -224,6 +224,9 @@ struct fpm_handle {
     // trace
     std::vector<double> tr_cands;                 // n*4
     std::vector<std::vector<double>> tr_evals;    // per level, n*5
+    std::vector<std::vector<float>> tr_scores;    // per level, n*49: the 7x7 score patch of every row of tr_evals
+    struct TraceRois { int w = 0, h = 0, pitch = 0; std::vector<uint8_t> px; };
+    std::vector<TraceRois> tr_rois;               // per level, n ROI patches of h rows at full pitch (none on warp-fused levels)
 };
 
 namespace {
@@ -904,7 +907,11 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
     double layer_score[FPM_MAX_LEVELS + 1];
     layer_score[0] = h->score;
     for (int l = 1; l <= top; l++) layer_score[l] = layer_score[l - 1] * 0.9;
-    if (h->trace) h->tr_evals.assign(top + 1, std::vector<double>());
+    if (h->trace) {
+        h->tr_evals.assign(top + 1, std::vector<double>());
+        h->tr_scores.assign(top + 1, std::vector<float>());
+        h->tr_rois.assign(top + 1, fpm_handle::TraceRois());
+    }
     const size_t budget = (size_t)(h->workspace_mb * 1024.0 * 1024.0);
     // the descent without host round trips needs every layer to fit one workspace wave at the top-layer count
     bool async = !h->trace && n_cands <= 65535 && (h->async_descent == 1 || (h->async_descent < 0 && h->cur_batch < 8));
@@ -931,6 +938,12 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
         if (h->trace) {
             CK(h->d_trace.ensure((size_t)n * n_ang * sizeof(FpmEvalTrace)));
             CK(cudaMemsetAsync(h->d_trace.p, 0, (size_t)n * n_ang * sizeof(FpmEvalTrace), h->stream));
+            // all-ones bytes are NaN: a score cell the finalize kernel does not write cannot pass for a result
+            CK(h->d_trace_sc.ensure((size_t)n * n_ang * FPM_NCELL * sizeof(float)));
+            CK(cudaMemsetAsync(h->d_trace_sc.p, 0xff, (size_t)n * n_ang * FPM_NCELL * sizeof(float), h->stream));
+            fpm_handle::TraceRois& tr = h->tr_rois[layer];
+            tr.w = t.w + FPM_ROI_PAD; tr.h = t.h + FPM_ROI_PAD; tr.pitch = rpitch;
+            tr.px.assign(warp_fused ? 0 : (size_t)n * n_ang * roi_stride, 0);
         }
         // live candidates of this layer / where the survivors are counted
         const int* n_dev = !async ? nullptr : (layer == top - 1 ? counters + CNT_FLAT : counters + CNT_LAYER + layer);
@@ -1000,9 +1013,13 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                        L.h, layer_score[layer], h->use_simd, layer == stop ? 1 : 0, stop ? 2 : 1, (h->subpixel && layer == 0) ? 1 : 0,
                        h->d_cand[cur ^ 1].as<FpmCand>(),
                        next_cnt, ref_out, ref_cnt,
-                       h->trace ? h->d_trace.as<FpmEvalTrace>() + (size_t)c0 * n_ang : nullptr, nullptr,
+                       h->trace ? h->d_trace.as<FpmEvalTrace>() + (size_t)c0 * n_ang : nullptr,
+                       h->trace ? h->d_trace_sc.as<float>() + (size_t)c0 * n_ang * FPM_NCELL : nullptr,
                        fused ? h->d_numer.as<float>() : nullptr, h->d_totS.as<long long>(), h->d_totQ.as<long long>(), raw_tile_evals, n_dev));
             }
+            if (h->trace && !warp_fused)                    // this wave's ROI patches, before the next wave overwrites them
+                CK(cudaMemcpyAsync(h->tr_rois[layer].px.data() + (size_t)c0 * n_ang * roi_stride, h->d_roi.p, (size_t)ne * roi_stride,
+                                   cudaMemcpyDeviceToHost, h->stream));
         }
         cur ^= 1;
         if (async) continue;                                  // n stays the top-layer count: an upper bound of every layer's list
@@ -1021,6 +1038,9 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                     rows.push_back(cc2[i].id); rows.push_back(e.angle); rows.push_back(e.score);
                     rows.push_back(e.locx); rows.push_back(e.locy);
                 }
+            std::vector<float>& sc = h->tr_scores[layer];
+            sc.resize((size_t)n * n_ang * FPM_NCELL);
+            CK(cudaMemcpy(sc.data(), h->d_trace_sc.p, sc.size() * sizeof(float), cudaMemcpyDeviceToHost));
         }
         if (hc[CNT_ERR]) { h->err = "fpm_corr_warp_kernel: source box larger than its staging buffer"; return FPM_ERR_LIMIT; }
         n = (layer == stop) ? 0 : hc[CNT_NEXT];
@@ -3180,6 +3200,25 @@ int fpm_trace_evals(const fpm_handle* h, int level, double* rows)
     if (!h || !rows || level < 0 || level >= (int)h->tr_evals.size()) return FPM_ERR_INVALID;
     for (size_t i = 0; i < h->tr_evals[level].size(); i++) rows[i] = h->tr_evals[level][i];
     return FPM_OK;
+}
+
+int fpm_trace_eval_scores(const fpm_handle* h, int level, float* out)
+{
+    if (!h || !out || level < 0 || level >= (int)h->tr_scores.size()) return FPM_ERR_INVALID;
+    std::copy(h->tr_scores[level].begin(), h->tr_scores[level].end(), out);
+    return FPM_OK;
+}
+
+int fpm_trace_eval_rois(const fpm_handle* h, int level, uint8_t* out, int* w, int* hgt, int* pitch)
+{
+    if (!h || level < 0 || level >= (int)h->tr_rois.size()) return FPM_ERR_INVALID;
+    const fpm_handle::TraceRois& r = h->tr_rois[level];
+    if (w) *w = r.w;
+    if (hgt) *hgt = r.h;
+    if (pitch) *pitch = r.pitch;
+    if (out) std::copy(r.px.begin(), r.px.end(), out);
+    const size_t per = (size_t)r.h * r.pitch;
+    return per ? (int)(r.px.size() / per) : 0;
 }
 
 int fpm_trace_level(const fpm_handle* hc, int level, uint8_t* out, int* w, int* hgt)

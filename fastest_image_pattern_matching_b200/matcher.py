@@ -306,6 +306,29 @@ class TemplateMatcher:
             self._check(self._lib.fpm_trace_evals(self._h, level, rows.ctypes.data))
         return rows
 
+    def traceEvalScores(self, level: int) -> np.ndarray:
+        """[n, 7, 7] float32: the score patch of every refinement eval of `level`, rows as in traceEvals(level)"""
+        n = self._lib.fpm_trace_num_evals(self._h, level)
+        out = np.zeros((n, 7, 7), np.float32)
+        if n:
+            self._check(self._lib.fpm_trace_eval_scores(self._h, level, out.ctypes.data))
+        return out
+
+    def traceEvalRois(self, level: int) -> Optional[np.ndarray]:
+        """[n, h, pitch] uint8: the ROI patch of every refinement eval of `level` at the device pitch (the patch is
+        [:, :, :w] with w = template width + 6), rows as in traceEvals(level); None where the ROIs are warped inside the
+        correlation kernel and never stored"""
+        w, h, p = C.c_int(), C.c_int(), C.c_int()
+        n = self._lib.fpm_trace_eval_rois(self._h, level, None, C.byref(w), C.byref(h), C.byref(p))
+        if n < 0:
+            self._check(n)
+        if n == 0:
+            return None
+        out = np.zeros((n, h.value, p.value), np.uint8)
+        rc = self._lib.fpm_trace_eval_rois(self._h, level, out.ctypes.data, C.byref(w), C.byref(h), C.byref(p))
+        self._check(rc if rc < 0 else 0)
+        return out
+
     def traceLevel(self, level: int) -> Optional[np.ndarray]:
         w, h = C.c_int(), C.c_int()
         if self._lib.fpm_trace_level(self._h, level, None, C.byref(w), C.byref(h)) != 0:

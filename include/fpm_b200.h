@@ -282,6 +282,12 @@ int fpm_trace_candidates(const fpm_handle* h, double* rows /* n*4: x, y, score, 
 int fpm_trace_num_evals(const fpm_handle* h, int level);
 int fpm_trace_evals(const fpm_handle* h, int level, double* rows /* n*5: cand id, angle, score, locx, locy */);
 int fpm_trace_level(const fpm_handle* h, int level, uint8_t* out /* w*h of the source pyramid */, int* w, int* hgt);
+/* the 7x7 float32 score patch of every refinement eval of `level`, in the row order of fpm_trace_evals */
+int fpm_trace_eval_scores(const fpm_handle* h, int level, float* out /* n*49, row-major per eval */);
+/* the ROI patch of every refinement eval of `level` (getRotatedROI: template size + 6), in the row order of fpm_trace_evals,
+ * at the device pitch: out (may be null) receives n * hgt * pitch bytes, columns w .. pitch-1 as the device holds them.
+ * Returns n (>= 0); 0 on levels whose ROIs are warped inside the correlation kernel (FPM_PARAM_TENSOR_CORES = 6). */
+int fpm_trace_eval_rois(const fpm_handle* h, int level, uint8_t* out, int* w, int* hgt, int* pitch);
 
 #ifdef __cplusplus
 }

@@ -249,11 +249,9 @@ def ccorr_exact_dense(src, tpl):
     return acc.astype(f32)
 
 
-def ccoeff_denominator(src, td: TemplData, result, layer):
-    """CCOEFF_Denominator, src/TemplateMatcher.cpp:527-598 (vectorised, same op order)."""
-    if td.result_equal1[layer]:
-        result[:] = 1
-        return result
+def ccoeff_num_den(src, td: TemplData, result, layer):
+    """The centred numerator and the denominator of every cell of CCOEFF_Denominator (float64, same op order);
+    den == 0 where the window is flat."""
     tpl = td.pyramid[layer]
     th, tw = tpl.shape
     s, q = cv2.integral2(src, sdepth=cv2.CV_64F, sqdepth=cv2.CV_64F)
@@ -267,6 +265,30 @@ def ccoeff_denominator(src, td: TemplData, result, layer):
     diff2 = np.maximum(wnd_sum2 - wnd_mean2, 0.0)
     den = np.where(diff2 <= np.minimum(0.5, 10 * FLT_EPSILON * wnd_sum2), 0.0,
                    np.sqrt(diff2) * td.templ_norm[layer])
+    return num, den
+
+
+# outcomes of the CCOEFF_NORMED epilogue per cell (ccoeff_branches)
+BRANCH_FLAT, BRANCH_CLAMP, BRANCH_QUOTIENT, BRANCH_ZERO, BRANCH_EQUAL1 = range(5)
+
+
+def ccoeff_branches(src, td: TemplData, result, layer):
+    """Which branch of the epilogue every cell takes: den == 0 (score 0), den <= |num| < 1.125 den (score +-1),
+    |num| < den (num / den), |num| >= 1.125 den > 0 (score 0), or a flat template (score 1)."""
+    if td.result_equal1[layer]:
+        return np.full(result.shape, BRANCH_EQUAL1, np.int8)
+    num, den = ccoeff_num_den(src, td, result, layer)
+    absn = np.abs(num)
+    return np.where(den == 0, BRANCH_FLAT, np.where(absn < den, BRANCH_QUOTIENT,
+                    np.where(absn < den * 1.125, BRANCH_CLAMP, BRANCH_ZERO))).astype(np.int8)
+
+
+def ccoeff_denominator(src, td: TemplData, result, layer):
+    """CCOEFF_Denominator, src/TemplateMatcher.cpp:527-598 (vectorised, same op order)."""
+    if td.result_equal1[layer]:
+        result[:] = 1
+        return result
+    num, den = ccoeff_num_den(src, td, result, layer)
     absn = np.abs(num)
     with np.errstate(divide="ignore", invalid="ignore"):
         out = np.where(absn < den, num / den,

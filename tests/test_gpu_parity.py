@@ -572,39 +572,6 @@ def test_random_scenes_match_live_oracle(matcher, seed):
     assert_results_match(got, want, ordered=not ties)
 
 
-# ---------------- T6: per-layer refinement records against the oracle trace ----------------
-@pytest.mark.parametrize("case", ["src8", "cfg1_synth"])
-def test_refinement_records_match_oracle_trace(matcher, golden_cases, case):
-    c = golden_cases[case]
-    configure(matcher, c["params"])
-    tpl, src = get_image(c["tpl"]), get_image(c["src"])
-    matcher.learnPattern(tpl)
-    matcher.setTrace(True)
-    try:
-        matcher.match(src)
-        levels = len(matcher.templateLevels())
-        got = {}
-        for lvl in range(levels - 1):
-            rows = matcher.traceEvals(lvl)
-            seen = {}
-            for r in rows:                                   # rows: cand id, angle, score, locx, locy (3 per candidate, in order)
-                j = seen.get(int(r[0]), 0)
-                seen[int(r[0])] = j + 1
-                got[(lvl, int(r[0]), j)] = (r[1], np.float32(r[2]), int(r[3]), int(r[4]))
-    finally:
-        matcher.setTrace(False)
-    om = configure(O.OracleMatcher(), c["params"])
-    om.trace = {}
-    om.learn_pattern(tpl)
-    om.match(src)
-    want = {(e["layer"], e["cand"], e["j"]): (e["angle"], np.float32(e["val"]), e["loc"][0], e["loc"][1]) for e in om.trace["refine"]}
-    assert set(got) == set(want), "different (layer, candidate, angle) evaluation sets: the same candidates must survive each layer"
-    for k in want:
-        ga, gs, gx, gy = got[k]
-        wa, ws, wx, wy = want[k]
-        assert abs(ga - wa) <= 1e-9 and (gx, gy) == (wx, wy) and abs(float(gs) - float(ws)) <= 1e-6, (k, got[k], want[k])
-
-
 def test_unaligned_device_frames(matcher, golden_cases):
     """frames at an odd device address / odd pitch take the byte-granular load paths of pyrDown and warp."""
     import torch
