@@ -35,6 +35,10 @@ SIGNATURES = {
     "fpm_set_param": (_i, [_vp, _i, _d]),
     "fpm_get_param": (_d, [_vp, _i]),
     "fpm_learn": (_i, [_vp, _vp, _i, _i, _i]),
+    "fpm_learn_set": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    "fpm_set_size": (_i, [_vp]),
+    "fpm_match_set_batch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _vp, _i, _vp]),
+    "fpm_match_ingested_set_batch": (_i, [_vp, _vp, _i, _vp]),
     "fpm_is_learned": (_i, [_vp]),
     "fpm_clear": (None, [_vp]),
     "fpm_match": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _pi]),

@@ -29,12 +29,33 @@ struct FpmLevel {
 };
 
 // Per-level template statistics (s_TemplData, DataStructures.h:16-55)
+struct FpmTplStat {
+    double mean, norm, inv_area;
+    int result_equal1;
+};
+
+// One level of a template group: n_tpl templates of one size, template k at ptr + k * tpl_stride with statistics
+// stats[k].  The inline statistics are template 0's.  Virtual image v of a group = frame v / n_tpl x template v % n_tpl.
 struct FpmTplLevel {
     const uint8_t* ptr;     // [h][pitch] u8, rows zero padded to pitch (pitch % 16 == 0)
     int w, h, pitch;
     double mean, norm, inv_area;
     int result_equal1;
+    int n_tpl;              // templates in the group (1: a single template, stats unused)
+    size_t tpl_stride;
+    const FpmTplStat* stats;
 };
+
+// template k of a group level
+FPM_HD FpmTplLevel fpm_tpl_member(FpmTplLevel t, int k)
+{
+    if (t.n_tpl > 1) {
+        t.ptr += (size_t)k * t.tpl_stride;
+        const FpmTplStat s = t.stats[k];
+        t.mean = s.mean; t.norm = s.norm; t.inv_area = s.inv_area; t.result_equal1 = s.result_equal1;
+    }
+    return t;
+}
 
 // One warpAffine job (dst <- src), matrix already inverted the way cv::warpAffine does it.
 struct FpmWarpJob {
@@ -49,7 +70,7 @@ struct FpmCand {
     double angle;           // dMatchAngle
     double score;           // dMatchScore
     float ptx, pty;         // top layer: pt ; refinement: ptLT (cv::Point2f)
-    int img;                // image index in the batch
+    int img;                // image index in the batch (virtual image of a template group)
     int id;                 // rank in the score-sorted top-layer list of its image
 };
 

@@ -136,6 +136,8 @@ struct TplLevelHost {
     double mean = 0, norm = 0, inv_area = 1;
     int equal1 = 0;
     std::vector<uint8_t> pix;    // w*h
+    size_t tpl_stride = 0;       // template groups: bytes from one member's level to the next one's
+    size_t stat_off = 0;         // template groups: index of member 0's FpmTplStat of this level in d_tstat
 };
 
 struct TopPlan {                  // cached per (source size, parameters); always the WHOLE angle schedule
@@ -147,6 +149,21 @@ struct TopPlan {                  // cached per (source size, parameters); alway
     int n_ang = 0;                // angles.size()
     bool valid = false;
 };
+
+// Templates of a set with the same level-0 size and border colour: they share the top layer, the angle schedule, the
+// canvases, the ROI sizes and the NMS rectangle, and run through the pipeline together as virtual images
+// v = frame * n + member.  The group being matched lives in the handle's fields (tpl, border, tpl0_w/h, members, plan,
+// d_jobs_top, d_angles, d_ftx, d_fty); group 0 is there at rest, the others are swapped in for their pass.
+struct TplGroup {
+    std::vector<int> members;      // set indices, ascending
+    std::vector<TplLevelHost> tpl; // levels (statistics and pixels of members[0])
+    int border = 0, w0 = 0, h0 = 0;
+    TopPlan plan;
+    DevBuf d_jobs_top, d_angles, d_ftx, d_fty;
+    void release() { d_jobs_top.release(); d_angles.release(); d_ftx.release(); d_fty.release(); }
+};
+
+struct SetTpl { std::vector<uint8_t> px; int w = 0, h = 0; };
 
 }  // namespace
 
@@ -184,8 +201,11 @@ struct fpm_handle {
     bool learned = false;
     int learned_mra = -1;
     int border = 0;
-    std::vector<uint8_t> tpl0;    // level-0 copy for re-learning when MinReduceArea changes
-    int tpl0_w = 0, tpl0_h = 0;
+    std::vector<SetTpl> set;       // the learned templates (fpm_learn: one), kept for re-learning when MinReduceArea changes
+    std::vector<TplGroup> groups;  // their groups; groups[0]'s state is in the fields below (see TplGroup)
+    DevBuf d_tstat;                // FpmTplStat of every (group, level, member)
+    std::vector<int> members;      // current group: its set indices
+    int tpl0_w = 0, tpl0_h = 0;    // current group: level-0 size
     std::vector<TplLevelHost> tpl;
     DevBuf d_tpl, d_tsh, d_raw, d_inv, d_numer, d_totS, d_totQ, d_ingest_raw, d_ingest;
     int ingest_w = 0, ingest_h = 0, ingest_pitch = 0;      // last ingested frames (device resident, [count][h][pitch])
@@ -210,7 +230,7 @@ struct fpm_handle {
     std::vector<FpmLevel> levels; // source pyramid of the current batch
     const std::vector<FpmLevel>* shared_levels = nullptr;   // fpm_match_multi: the pyramid built once by the first handle
     TopPlan plan;
-    std::string err;
+    mutable std::string err;       // also set by the const accessors that refuse a template set
     double last_ms = 0;
     long long launches = 0, collectives = 0;
     // per-kernel profiling (CUDA events on the launch stream)
@@ -315,6 +335,9 @@ FpmTplLevel tpl_level_dev(const fpm_handle* h, int l)
     d.ptr = h->d_tpl.as<uint8_t>() + t.dev_off;
     d.w = t.w; d.h = t.h; d.pitch = t.pitch;
     d.mean = t.mean; d.norm = t.norm; d.inv_area = t.inv_area; d.result_equal1 = t.equal1;
+    d.n_tpl = std::max((int)h->members.size(), 1);
+    d.tpl_stride = t.tpl_stride;
+    d.stats = d.n_tpl > 1 ? h->d_tstat.as<FpmTplStat>() + t.stat_off : nullptr;
     return d;
 }
 
@@ -377,10 +400,11 @@ int launch_pyramid_chain(fpm_handle* h, const std::vector<FpmLevel>& lv, int top
     return FPM_OK;
 }
 
-// launch geometry of fpm_corr_rows_kernel for a template level
+// launch geometry of fpm_corr_rows_kernel for a template level (per_eval_tpl: every eval stages its own template rows,
+// the evals of a CTA may belong to different templates of a group)
 struct CorrCfg { int rb, evals_per_cta, threads; size_t smem; int blocks_y_rows; };
 
-CorrCfg corr_config(int tpl_h)
+CorrCfg corr_config(int tpl_h, bool per_eval_tpl = false)
 {
     CorrCfg c;
     const int rh = tpl_h + FPM_ROI_PAD;
@@ -396,7 +420,7 @@ CorrCfg corr_config(int tpl_h)
     }
     c.threads = (int)align_up((size_t)c.rb * c.evals_per_cta, 32);
     const size_t n_srow = (size_t)c.evals_per_cta * c.rb, n_trow = (size_t)c.rb + FPM_ROI_PAD;
-    size_t stage = (n_srow + n_trow) * CR_PW * 4;
+    size_t stage = (n_srow + (per_eval_tpl ? c.evals_per_cta : 1) * n_trow) * CR_PW * 4;
     size_t outb = (size_t)c.evals_per_cta * n_trow * FPM_NCELL * 4;
     c.smem = std::max(2 * stage, outb);      // two slab buffers (cp.async double buffering)
     return c;
@@ -461,9 +485,11 @@ int make_map_3d(fpm_handle* h, CUtensorMap* map, const void* base, uint64_t d0, 
 }
 
 // which correlation path a template level takes: 0 = dp4a (fpm_corr_rows_kernel), 1 = tensor cores
+// The tensor-core kernels share one B operand (the pre-shifted template) across the 128 evals of a tile: groups of
+// more than one template take dp4a (bit-identical results).
 bool mma_usable(const fpm_handle* h, int tw)
 {
-    if (h->use_tc == 0) return false;
+    if (h->use_tc == 0 || h->members.size() > 1) return false;
     if (!get_encode_tiled()) return false;
     return (h->use_tc == 2 || h->use_tc == 4) ? true : tw >= 64;     // modes 1, 3, 5, 6: large levels
 }
@@ -472,7 +498,7 @@ bool mma_usable(const fpm_handle* h, int tw)
 // 22..70-byte ROI row), the fused kernel does as soon as the level has enough evals to fill the SMs
 bool mma_narrow_fused(const fpm_handle* h, int tw)
 {
-    return (h->use_tc == 1 || h->use_tc == 6) && h->use_simd && get_encode_tiled() && tw >= 16 && tw < 64;
+    return (h->use_tc == 1 || h->use_tc == 6) && h->use_simd && h->members.size() <= 1 && get_encode_tiled() && tw >= 16 && tw < 64;
 }
 
 // The fused kernel keeps one CTA on 128 evals for all ROI rows: it wins when the evals fill the SMs and the rows are
@@ -576,7 +602,7 @@ bool fw_box_fits(int vec)
 
 bool corr_warp_usable(const fpm_handle* h, int tw, int n_ang, const FpmLevel& L)
 {
-    if (h->use_tc != 6) return false;                        // opt-in: bit-identical, less DRAM traffic, but slower than warp + MMA today
+    if (h->use_tc != 6 || h->members.size() > 1) return false;   // opt-in: bit-identical, less DRAM traffic, but slower than warp + MMA today
     if (n_ang != 3 || tw < 64 || !get_encode_tiled()) return false;
     return level_copy_vec(L) >= 4 && fw_box_fits(4);       // the box is staged with 4-byte copies
 }
@@ -605,81 +631,128 @@ int launch_corr_warp(fpm_handle* h, const FpmLevel& L, const FpmWarpJob* jobs, c
     return FPM_OK;
 }
 
-// ---- learnPattern, src/TemplateMatcher.cpp:45-95 ------------------------------------
+// ---- learnPattern, src/TemplateMatcher.cpp:45-95, for every template of the set ---------------------
+// Device layout: group by group and level by level, the members of a group level back to back (a set of one: today's
+// single-template layout).  Each group's template pyramids are built by one pyramid chain over its members.
 int do_learn(fpm_handle* h)
 {
-    const int w0 = h->tpl0_w, h0 = h->tpl0_h;
     CK(cudaSetDevice(h->device));
-    int top = get_top_layer(w0, h0, (int)sqrt((double)h->min_reduce_area));
-    if (top + 1 > FPM_MAX_LEVELS) { h->err = "too many pyramid levels"; return FPM_ERR_LIMIT; }
-    h->tpl.assign(top + 1, TplLevelHost());
-    size_t off = 0;
-    int w = w0, hh = h0;
-    for (int l = 0; l <= top; l++) {
-        TplLevelHost& t = h->tpl[l];
-        t.w = w; t.h = hh; t.pitch = (int)align_up(w, 16);
-        t.dev_off = off;
-        off += align_up((size_t)t.pitch * hh, 256);
-        w = (w + 1) / 2; hh = (hh + 1) / 2;
+    h->learned = false;
+    for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
+    h->groups.clear();
+    std::vector<TplGroup> gs;
+    for (int i = 0; i < (int)h->set.size(); i++) {
+        const SetTpl& st = h->set[i];
+        unsigned long long S = 0;
+        for (uint8_t v : st.px) S += v;
+        const int border = ((double)S / ((double)st.h * st.w)) < 128 ? 255 : 0;     // iBorderColor (:58-59)
+        size_t g = 0;
+        while (g < gs.size() && !(gs[g].w0 == st.w && gs[g].h0 == st.h && gs[g].border == border)) g++;
+        if (g == gs.size()) { gs.emplace_back(); gs[g].w0 = st.w; gs[g].h0 = st.h; gs[g].border = border; }
+        gs[g].members.push_back(i);
+    }
+    size_t off = 0, toff = 0, n_stat = 0;
+    for (TplGroup& G : gs) {
+        const int top = get_top_layer(G.w0, G.h0, (int)sqrt((double)h->min_reduce_area));
+        if (top + 1 > FPM_MAX_LEVELS) { h->err = "too many pyramid levels"; return FPM_ERR_LIMIT; }
+        const int T = (int)G.members.size();
+        G.tpl.assign(top + 1, TplLevelHost());
+        int w = G.w0, hh = G.h0;
+        for (int l = 0; l <= top; l++) {
+            TplLevelHost& t = G.tpl[l];
+            t.w = w; t.h = hh; t.pitch = (int)align_up(w, 16);
+            t.dev_off = off;
+            t.tpl_stride = align_up((size_t)t.pitch * hh, 256);
+            off += t.tpl_stride * T;
+            t.stat_off = n_stat;
+            n_stat += T;
+            if (T == 1) {                                          // 8 pre-shifted copies for the tensor-core path
+                t.bpitch = (int)align_up(t.w + 8, 16);
+                t.tsh_off = toff;
+                toff += align_up((size_t)8 * t.h * t.bpitch, 256);
+            }
+            w = (w + 1) / 2; hh = (hh + 1) / 2;
+        }
     }
     CK(h->d_tpl.ensure(off));
     CK(cudaMemsetAsync(h->d_tpl.p, 0, off, h->stream));
-    CK(cudaMemcpy2DAsync(h->d_tpl.as<uint8_t>() + h->tpl[0].dev_off, h->tpl[0].pitch, h->tpl0.data(), w0, w0, h0,
-                         cudaMemcpyHostToDevice, h->stream));
-    {
+    for (const TplGroup& G : gs) {
+        const TplLevelHost& t0 = G.tpl[0];
+        for (size_t k = 0; k < G.members.size(); k++)
+            CK(cudaMemcpy2DAsync(h->d_tpl.as<uint8_t>() + t0.dev_off + k * t0.tpl_stride, t0.pitch, h->set[G.members[k]].px.data(), G.w0,
+                                 G.w0, G.h0, cudaMemcpyHostToDevice, h->stream));
+        const int top = (int)G.tpl.size() - 1, T = (int)G.members.size();
         std::vector<FpmLevel> lv(top + 1);
-        for (int l = 0; l <= top; l++) lv[l] = FpmLevel{h->d_tpl.as<uint8_t>() + h->tpl[l].dev_off, h->tpl[l].w, h->tpl[l].h, h->tpl[l].pitch, 0};
-        int rc = launch_pyramid_chain(h, lv, top, 1);
+        for (int l = 0; l <= top; l++)
+            lv[l] = FpmLevel{h->d_tpl.as<uint8_t>() + G.tpl[l].dev_off, G.tpl[l].w, G.tpl[l].h, G.tpl[l].pitch, T > 1 ? G.tpl[l].tpl_stride : 0};
+        int rc = launch_pyramid_chain(h, lv, top, T);
         if (rc) return rc;
     }
-    {
-        size_t toff = 0;
-        for (int l = 0; l <= top; l++) {
-            TplLevelHost& t = h->tpl[l];
-            t.bpitch = (int)align_up(t.w + 8, 16);
-            t.tsh_off = toff;
-            toff += align_up((size_t)8 * t.h * t.bpitch, 256);
-        }
-        CK(h->d_tsh.ensure(toff));
-        for (int l = 0; l <= top; l++) {
-            TplLevelHost& t = h->tpl[l];
+    CK(h->d_tsh.ensure(toff));
+    for (const TplGroup& G : gs) {
+        if (G.members.size() != 1) continue;
+        for (const TplLevelHost& t : G.tpl) {
             dim3 g((t.bpitch + 127) / 128, t.h, 8);
             fpm_shift_template_kernel<<<g, 128, 0, h->stream>>>(h->d_tpl.as<uint8_t>() + t.dev_off, t.w, t.h, t.pitch,
                                                                 h->d_tsh.as<uint8_t>() + t.tsh_off, t.bpitch);
             CKL();
         }
     }
-    for (int l = 0; l <= top; l++) {
-        TplLevelHost& t = h->tpl[l];
-        t.pix.resize((size_t)t.w * t.h);
-        CK(cudaMemcpy2DAsync(t.pix.data(), t.w, h->d_tpl.as<uint8_t>() + t.dev_off, t.pitch, t.w, t.h,
-                             cudaMemcpyDeviceToHost, h->stream));
-    }
+    std::vector<uint8_t> all(off);
+    CK(cudaMemcpyAsync(all.data(), h->d_tpl.p, off, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
-    // iBorderColor = mean(templ) < 128 ? 255 : 0  (:58-59)
-    for (int l = 0; l <= top; l++) {
-        TplLevelHost& t = h->tpl[l];
-        unsigned long long S = 0, Q = 0;
-        for (uint8_t v : t.pix) { S += v; Q += (unsigned long long)v * v; }
-        double N = (double)t.h * t.w;
-        // cv::meanStdDev (u8): scale = 1/N; mean = S*scale; var = max(Q*scale - mean^2, 0); sdv = sqrt(var)
-        double scale = 1.0 / N;
-        double mean = (double)S * scale;
-        double var = std::max((double)Q * scale - mean * mean, 0.0);
-        double sdv = sqrt(var);
-        double invArea = 1.0 / ((double)t.h * t.w);
-        double templNorm = sdv * sdv;                       // :74
-        t.equal1 = templNorm < DBL_EPSILON ? 1 : 0;         // :77
-        templNorm = sqrt(templNorm);                        // :85
-        templNorm /= sqrt(invArea);                         // :86
-        t.mean = mean; t.norm = templNorm; t.inv_area = invArea;
-        if (l == 0) h->border = ((double)S / N) < 128 ? 255 : 0;
-    }
+    std::vector<FpmTplStat> stats(n_stat);
+    for (TplGroup& G : gs)
+        for (TplLevelHost& t : G.tpl)
+            for (size_t k = 0; k < G.members.size(); k++) {
+                const uint8_t* base = all.data() + t.dev_off + k * t.tpl_stride;
+                unsigned long long S = 0, Q = 0;
+                for (int y = 0; y < t.h; y++)
+                    for (int x = 0; x < t.w; x++) { const unsigned v = base[(size_t)y * t.pitch + x]; S += v; Q += (unsigned long long)v * v; }
+                double N = (double)t.h * t.w;
+                // cv::meanStdDev (u8): scale = 1/N; mean = S*scale; var = max(Q*scale - mean^2, 0); sdv = sqrt(var)
+                double scale = 1.0 / N;
+                double mean = (double)S * scale;
+                double var = std::max((double)Q * scale - mean * mean, 0.0);
+                double sdv = sqrt(var);
+                double invArea = 1.0 / ((double)t.h * t.w);
+                double templNorm = sdv * sdv;                       // :74
+                const int equal1 = templNorm < DBL_EPSILON ? 1 : 0; // :77
+                templNorm = sqrt(templNorm);                        // :85
+                templNorm /= sqrt(invArea);                         // :86
+                stats[t.stat_off + k] = FpmTplStat{mean, templNorm, invArea, equal1};
+                if (k == 0) {
+                    t.mean = mean; t.norm = templNorm; t.inv_area = invArea; t.equal1 = equal1;
+                    t.pix.resize((size_t)t.w * t.h);
+                    for (int y = 0; y < t.h; y++) memcpy(t.pix.data() + (size_t)y * t.w, base + (size_t)y * t.pitch, t.w);
+                }
+            }
+    CK(h->d_tstat.ensure(n_stat * sizeof(FpmTplStat)));
+    CK(cudaMemcpy(h->d_tstat.p, stats.data(), n_stat * sizeof(FpmTplStat), cudaMemcpyHostToDevice));
+    // group 0 goes into the handle's fields (its plan buffers stay the handle's), the others wait in groups[1..]
+    TplGroup& G0 = gs[0];
+    h->tpl.swap(G0.tpl); h->members.swap(G0.members);
+    h->border = G0.border; h->tpl0_w = G0.w0; h->tpl0_h = G0.h0;
+    h->groups.swap(gs);
     h->learned = true;
     h->learned_mra = h->min_reduce_area;
     h->plan.valid = false;
     return FPM_OK;
 }
+
+// runs group g's pass with its state in the handle's fields, then puts it back
+struct GroupScope {
+    fpm_handle* h; size_t g;
+    static void swap(fpm_handle* h, TplGroup& G)
+    {
+        std::swap(h->tpl, G.tpl); std::swap(h->members, G.members); std::swap(h->border, G.border);
+        std::swap(h->tpl0_w, G.w0); std::swap(h->tpl0_h, G.h0); std::swap(h->plan, G.plan);
+        std::swap(h->d_jobs_top, G.d_jobs_top); std::swap(h->d_angles, G.d_angles);
+        std::swap(h->d_ftx, G.d_ftx); std::swap(h->d_fty, G.d_fty);
+    }
+    GroupScope(fpm_handle* hh, size_t gg) : h(hh), g(gg) { if (g) swap(h, h->groups[g]); }
+    ~GroupScope() { if (g) swap(h, h->groups[g]); }
+};
 
 // ---- source pyramid -----------------------------------------------------------------
 int build_pyramid(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt, int stride, size_t frame_stride, int top)
@@ -784,71 +857,74 @@ float top_reject_below(const fpm_handle* h, int top)
     return t > 0.05 ? (float)(t - 0.01) : -INFINITY;
 }
 
-// ---- top-layer sweep: warp + score + peaks for jobs [j0, j0 + nj) of the plan's (image, angle) list -----
-// picks go to picks_out[nj][max_picks], counts to cnt_out[nj]
+// ---- top-layer sweep: warp + score + peaks for jobs [j0, j0 + nj) of the plan's (frame, angle) list -----
+// Each (frame, angle) canvas is warped once and scored against every template of the group.  picks go to
+// picks_out[slot][max_picks], counts to cnt_out[slot]: slot = job - j0 for one template, (frame * n_tpl + template) *
+// n_angles + angle for a group (whole sweeps only).  The sweep runs in chunks of canvases whose n_tpl score maps each fit
+// FPM_PARAM_WORKSPACE_MB and whose jobs fit gridDim.y / gridDim.z.
 int run_top(fpm_handle* h, int top, int j0, int nj, FpmPick* picks_out, int* cnt_out)
 {
     TopPlan& p = h->plan;
     const int max_picks = h->max_pos + FPM_MATCH_CANDIDATE_NUM;
     if (nj <= 0) return FPM_OK;
     const TplLevelHost& t = h->tpl[top];
+    const int n_tpl = std::max((int)h->members.size(), 1);
     const int rpitch = (int)align_up(p.maxW, 16);
     const size_t rot_stride = (size_t)rpitch * p.maxH;
     const int maxRW = std::max(p.maxW - t.w + 1, 1), maxRH = std::max(p.maxH - t.h + 1, 1);
     const int spitch = (int)align_up(maxRW, 4);
     const size_t score_stride = (size_t)spitch * maxRH;
-    CK(h->d_rot.ensure(rot_stride * nj));
-    CK(h->d_score.ensure(score_stride * nj * sizeof(float)));
     const FpmWarpJob* jobs = h->d_jobs_top.as<FpmWarpJob>() + j0;
     const int kMaxGridYZ = 65535;                              // gridDim.y / gridDim.z limit: larger sweeps run in chunks
+    const size_t budget = (size_t)(h->workspace_mb * 1024.0 * 1024.0);
+    const int chunk = (int)std::min<size_t>({(size_t)kMaxGridYZ, (size_t)nj,
+                                             std::max<size_t>(1, budget / ((size_t)n_tpl * score_stride * sizeof(float)))});
+    CK(h->d_rot.ensure(rot_stride * chunk));
+    CK(h->d_score.ensure(score_stride * chunk * n_tpl * sizeof(float)));
     const size_t smem_ts = top_score_smem(t.w, t.h);
     if (smem_ts > 200 * 1024) { h->err = "top-layer template too large for the score kernel"; return FPM_ERR_LIMIT; }
     if (smem_ts > 48 * 1024)
-        CK(ensure_dyn_smem((const void*)fpm_top_score_kernel, h->device, smem_ts));
-    for (int c0 = 0; c0 < nj; c0 += kMaxGridYZ) {
-        const int nc = std::min(kMaxGridYZ, nj - c0);
+        CK(ensure_dyn_smem(n_tpl > 1 ? (const void*)fpm_top_score_kernel<true> : (const void*)fpm_top_score_kernel<false>, h->device, smem_ts));
+    const auto score_kernel = n_tpl > 1 ? fpm_top_score_kernel<true> : fpm_top_score_kernel<false>;
+    // bCalMaxByBlock, src/TemplateMatcher.cpp:158-159
+    const FpmLevel& L = h->levels[top];
+    const bool by_block = ((L.w * L.h) / (t.w * t.h) > 500) && h->max_pos > 10;
+    const int mode = by_block ? (h->mfc_compat ? 2 : 1) : 0;    // MFC s_BlockMax differs from the Qt port's (MatchToolDlg.h:109-213)
+    int tile = 8;
+    while ((long long)((maxRW + tile - 1) / tile) * ((maxRH + tile - 1) / tile) > 1024 && tile < 256) tile *= 2;
+    int blk_stride;
+    const int tiles0 = ((maxRW + tile - 1) / tile) * ((maxRH + tile - 1) / tile);
+    if (mode == 1) blk_stride = (maxRW / t.w) * (maxRH / t.h) + 3;
+    else if (mode == 2) blk_stride = std::max((maxRW / (2 * t.w)) * (maxRH / (2 * t.h)) + 2, tiles0);   // an empty MFC table falls back to tiles
+    else blk_stride = tiles0;
+    blk_stride = std::max(blk_stride, 1);
+    if (blk_stride > PK_SUP_MAX * 32) { h->err = "top-layer score map has too many blocks for the peak table"; return FPM_ERR_LIMIT; }
+    CK(h->d_blkv.ensure((size_t)chunk * n_tpl * blk_stride * sizeof(float)));
+    CK(h->d_blkl.ensure((size_t)chunk * n_tpl * blk_stride * sizeof(int)));
+    const double thresh = top_layer_threshold(h, top);
+    const int smem_blocks = peaks_smem_blocks(h, blk_stride);
+    if (smem_blocks < 0) return FPM_ERR_CUDA;
+    for (int c0 = 0; c0 < nj; c0 += chunk) {
+        const int nc = std::min(chunk, nj - c0);
         const int tiles_x = (rpitch + WA_TW - 1) / WA_TW;
         dim3 wgrid(tiles_x * ((p.maxH + WA_TH - 1) / WA_TH), nc);
         KL(K_WARP_TOP, 2.0 * nc * (double)p.maxW * p.maxH,
-           fpm_warp_kernel<<<wgrid, WA_THREADS, 0, h->stream>>>(jobs + c0, 1, h->levels[top],
-                                                                h->d_rot.as<uint8_t>() + (size_t)c0 * rot_stride, rpitch, rot_stride,
+           fpm_warp_kernel<<<wgrid, WA_THREADS, 0, h->stream>>>(jobs + c0, 1, h->levels[top], h->d_rot.as<uint8_t>(), rpitch, rot_stride,
                                                                 h->border, tiles_x, level_vec_ok(h->levels[top]), nullptr, FpmRefineGeom{}));
         dim3 grid((maxRW + TS_TW - 1) / TS_TW, (maxRH + TS_TH - 1) / TS_TH, nc);
         dim3 block(TS_THREADS);
-        KL(K_TOP_SCORE, (double)nc * maxRW * maxRH * t.w * t.h,      // MACs
-           fpm_top_score_kernel<<<grid, block, smem_ts, h->stream>>>(jobs + c0, h->d_rot.as<uint8_t>() + (size_t)c0 * rot_stride, rpitch,
-                                                                     rot_stride, tpl_level_dev(h, top),
-                                                                     h->d_score.as<float>() + (size_t)c0 * score_stride,
-                                                                     spitch, score_stride, top_reject_below(h, top)));
-    }
-    {
-        // bCalMaxByBlock, src/TemplateMatcher.cpp:158-159
-        const FpmLevel& L = h->levels[top];
-        bool by_block = ((L.w * L.h) / (t.w * t.h) > 500) && h->max_pos > 10;
-        int mode = by_block ? (h->mfc_compat ? 2 : 1) : 0;    // MFC s_BlockMax differs from the Qt port's (MatchToolDlg.h:109-213)
-        int tile = 8;
-        while ((long long)((maxRW + tile - 1) / tile) * ((maxRH + tile - 1) / tile) > 1024 && tile < 256) tile *= 2;
-        int blk_stride;
-        const int tiles0 = ((maxRW + tile - 1) / tile) * ((maxRH + tile - 1) / tile);
-        if (mode == 1) blk_stride = (maxRW / t.w) * (maxRH / t.h) + 3;
-        else if (mode == 2) blk_stride = std::max((maxRW / (2 * t.w)) * (maxRH / (2 * t.h)) + 2, tiles0);   // an empty MFC table falls back to tiles
-        else blk_stride = tiles0;
-        blk_stride = std::max(blk_stride, 1);
-        if (blk_stride > PK_SUP_MAX * 32) { h->err = "top-layer score map has too many blocks for the peak table"; return FPM_ERR_LIMIT; }
-        CK(h->d_blkv.ensure((size_t)nj * blk_stride * sizeof(float)));
-        CK(h->d_blkl.ensure((size_t)nj * blk_stride * sizeof(int)));
-        const double thresh = top_layer_threshold(h, top);
-        const int smem_blocks = peaks_smem_blocks(h, blk_stride);
-        if (smem_blocks < 0) return FPM_ERR_CUDA;
-        KL(K_TOP_PEAKS, 4.0 * nj * maxRW * maxRH,
-           fpm_top_peaks_kernel<<<nj, (maxRW * maxRH <= 16384) ? 128 : PK_THREADS, (size_t)smem_blocks * 8, h->stream>>>(
+        KL(K_TOP_SCORE, (double)nc * n_tpl * maxRW * maxRH * t.w * t.h,      // MACs
+           score_kernel<<<grid, block, smem_ts, h->stream>>>(jobs + c0, h->d_rot.as<uint8_t>(), rpitch, rot_stride,
+                                                                     tpl_level_dev(h, top), h->d_score.as<float>(), spitch,
+                                                                     score_stride, top_reject_below(h, top)));
+        KL(K_TOP_PEAKS, 4.0 * nc * n_tpl * maxRW * maxRH,
+           fpm_top_peaks_kernel<<<nc * n_tpl, (maxRW * maxRH <= 16384) ? 128 : PK_THREADS, (size_t)smem_blocks * 8, h->stream>>>(
                jobs, h->d_score.as<float>(), spitch, score_stride, t.w, t.h, mode, tile,
                h->d_blkv.as<float>(), h->d_blkl.as<int>(), blk_stride, thresh, h->max_overlap, max_picks,
-               picks_out, cnt_out, smem_blocks));
+               picks_out, cnt_out, smem_blocks, c0, n_tpl, p.n_ang));
     }
     return FPM_OK;
 }
-
 
 // ---- refinement of a flat candidate list held in d_cand[0] ------------------------------
 // per-layer geometry and workspace of the refinement
@@ -949,7 +1025,8 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
         const int* n_dev = !async ? nullptr : (layer == top - 1 ? counters + CNT_FLAT : counters + CNT_LAYER + layer);
         int* next_cnt = !async ? counters + CNT_NEXT : counters + CNT_LAYER + std::max(layer - 1, 0);
         if (!async) CK(cudaMemsetAsync(counters + CNT_NEXT, 0, sizeof(int), h->stream));
-        const CorrCfg cc = corr_config(t.h);
+        const int n_tpl = std::max((int)h->members.size(), 1);
+        const CorrCfg cc = corr_config(t.h, n_tpl > 1);
         const size_t smem = cc.smem;
         if (smem > 200 * 1024) { h->err = "correlation kernel shared memory limit"; return FPM_ERR_LIMIT; }
         if (smem > 48 * 1024)
@@ -962,7 +1039,7 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
             if (warp_fused)                                 // the warp-fused kernel stages the job matrices of its 42 candidates itself
                 KL(K_PREP, (double)ne * sizeof(FpmWarpJob),
                    fpm_refine_prep_kernel<<<(ne + 127) / 128, 128, 0, h->stream>>>(cands + c0, nc, n_ang, step, L.w, L.h, t.w, t.h,
-                                                                                 h->d_jobs_ref.as<FpmWarpJob>(), n_dev));
+                                                                                 h->d_jobs_ref.as<FpmWarpJob>(), n_dev, n_tpl));
             int raw_epad = 0;                               // 0 = [e][tr][49] row sums, else raw[y][e_pad][64] from the tensor cores
             int raw_tile_evals = 0;                         // evals per 128-row tile of raw (0 = contiguous)
             bool fused = false;                             // numerators + window totals straight from the fused tensor-core kernel
@@ -985,7 +1062,7 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                    fpm_warp_kernel<<<wgrid, WA_THREADS, 0, h->stream>>>(nullptr, n_ang, L,
                                                                         h->d_roi.as<uint8_t>(), rpitch, roi_stride, 0, wtiles_x,
                                                                         level_vec_ok(L), n_dev,
-                                                                        FpmRefineGeom{cands + c0, n_ang, step, L.w, L.h, t.w, t.h}));
+                                                                        FpmRefineGeom{cands + c0, n_ang, step, L.w, L.h, t.w, t.h, n_tpl}));
                 if (go_fused) {
                     int rcm = launch_corr_fused(h, h->d_roi.as<uint8_t>(), rpitch, roi_stride, h->d_tsh.as<uint8_t>() + t.tsh_off, t.bpitch,
                                                 t.w, t.h, ne, h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ang);
@@ -1001,11 +1078,12 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                     KL(K_CORR, (double)ne * FPM_NCELL * (double)t.w * t.h,
                        fpm_corr_rows_kernel<<<cgrid, cc.threads, smem, h->stream>>>(h->d_roi.as<uint8_t>(), rpitch, roi_stride, td, ne,
                                                                                     cc.rb, cc.evals_per_cta, h->d_rowsum.as<int32_t>(),
-                                                                                    h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ang));
+                                                                                    h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ang,
+                                                                                    cands + c0));
                 }
             }
             {
-                auto fin = fpm_refine_finalize_kernel;
+                auto fin = n_tpl > 1 ? fpm_refine_finalize_kernel<true> : fpm_refine_finalize_kernel<false>;
                 KL(K_FINALIZE, (double)ne * ((double)t.h * FPM_NCELL * 4 + 2.0 * (t.h + FPM_ROI_PAD) * FPM_NSHIFT * 4),
                    fin<<<nc, RF_THREADS, 0, h->stream>>>(
                        cands + c0, n_ang, step, raw_epad ? h->d_raw.as<int32_t>() : h->d_rowsum.as<int32_t>(), raw_epad,
@@ -1051,7 +1129,9 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
 }
 
 // ---- final stage: filterWithScore + NMS + conversion, results to host ---------------------
-int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride, fpm_result* out, int cap, int* n_out)
+// n_set > 1: image v of the batch is frame v / n_tpl x member v % n_tpl of the current group, written to the caller's
+// [frame][set index][cap] layout
+int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride, fpm_result* out, int cap, int* n_out, int n_set = 1)
 {
     key_stride = std::max(key_stride, 1);
     int ks = 1;
@@ -1086,12 +1166,14 @@ int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride
     CK(cudaMemcpyAsync(hr, h->d_results.p, (size_t)batch * rcap * sizeof(FpmResultDev), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (check_err && hc[CNT_ERR]) { h->err = "fpm_corr_warp_kernel: source box larger than its staging buffer"; return FPM_ERR_LIMIT; }
+    const int n_tpl = std::max((int)h->members.size(), 1);
     for (int b = 0; b < batch; b++) {
-        n_out[b] = hn[b];
+        const size_t slot = n_set == 1 ? (size_t)b : (size_t)(b / n_tpl) * n_set + h->members[b % n_tpl];
+        n_out[slot] = hn[b];
         int m = std::min(hn[b], cap);
         for (int i = 0; i < m; i++) {
             const FpmResultDev& r = hr[(size_t)b * rcap + i];
-            fpm_result& o = out[(size_t)b * cap + i];
+            fpm_result& o = out[slot * cap + i];
             o.score = r.score; o.angle = r.angle; o.cx = r.cx; o.cy = r.cy;
             o.ltx = r.ltx; o.lty = r.lty; o.rtx = r.rtx; o.rty = r.rty;
             o.rbx = r.rbx; o.rby = r.rby; o.lbx = r.lbx; o.lby = r.lby;
@@ -1147,9 +1229,8 @@ int collect_candidates(fpm_handle* h, int top, int batch, const FpmPickView& pv,
 }
 
 // guards of match(), src/TemplateMatcher.cpp:99-114; returns 1 when the match must return empty
-int match_guards(fpm_handle* h, int w, int hgt)
+int match_guards(const fpm_handle* h, int w, int hgt, int tw, int th)
 {
-    int tw = h->tpl0_w, th = h->tpl0_h;
     if (h->tol_range && (h->tol_r[0] >= h->tol_r[1] || h->tol_r[2] >= h->tol_r[3])) return 1;   // "left value must be smaller"
     if ((tw < w && th > hgt) || (tw > w && th < hgt)) return 1;
     if ((long long)tw * th > (long long)w * hgt) return 1;
@@ -1163,20 +1244,58 @@ int ensure_learned_for_mra(fpm_handle* h)
     return FPM_OK;
 }
 
-// whole match() over a device-resident batch
+// one group's pass over the pyramid of the batch: virtual images v = frame * n_tpl + member
+int match_group(fpm_handle* h, int batch, fpm_result* out, int cap, int* n_out, int n_set)
+{
+    const int top = (int)h->tpl.size() - 1;
+    const int n_tpl = std::max((int)h->members.size(), 1), vbatch = batch * n_tpl;
+    CK(cudaMemsetAsync(h->d_counters.p, 0, CNT_N * sizeof(int), h->stream));
+    int rc = make_top_plan(h, top, batch);
+    if (rc) return rc;
+    const TopPlan& p = h->plan;
+    const int max_picks = h->max_pos + FPM_MATCH_CANDIDATE_NUM;
+    const int njobs = batch * p.n_ang;
+    CK(h->d_picks.ensure((size_t)std::max(njobs * n_tpl, 1) * max_picks * sizeof(FpmPick)));
+    CK(h->d_pickcnt.ensure((size_t)std::max(njobs * n_tpl, 1) * sizeof(int)));
+    rc = run_top(h, top, 0, njobs, h->d_picks.as<FpmPick>(), h->d_pickcnt.as<int>());
+    if (rc) return rc;
+    FpmPickView pv{h->d_picks.as<FpmPick>(), h->d_pickcnt.as<int>(), 0, 0};
+    int n_cands = 0, cand_stride = 0;
+    rc = collect_candidates(h, top, vbatch, pv, p.n_ang, 0, 1, &n_cands, &cand_stride, nullptr);
+    if (rc) return rc;
+    int n_refined = 0;
+    h->ref_out = nullptr; h->ref_cnt = nullptr;
+    rc = run_refine(h, top, n_cands, &n_refined);
+    if (rc) return rc;
+    FpmRefinedView rv{h->d_refined.as<FpmRefined>(), h->d_counters.as<int>() + CNT_REFINED, 0, 1, 0};
+    return run_final(h, vbatch, rv, cand_stride, out, cap, n_out, n_set);
+}
+
+// whole match() over a device-resident batch, for every template of the set: frame b / template t at out + (b * n + t) * cap.
+// The source pyramid (and bitwise_not) is built once, down to the deepest top layer of any group; the groups run one
+// after another on the handle's stream.
 int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt, int stride, size_t frame_stride,
                  fpm_result* out, int cap, int* n_out)
 {
-    for (int b = 0; b < batch; b++) n_out[b] = 0;
+    const int n_set = std::max((int)h->set.size(), 1);
+    for (int b = 0; b < batch * n_set; b++) n_out[b] = 0;
     if (!h->learned) return FPM_OK;                          // :99-101 -> empty
     int rc = ensure_learned_for_mra(h);
     if (rc) return rc;
-    if (match_guards(h, w, hgt)) return FPM_OK;
-    const int top = (int)h->tpl.size() - 1;
+    const size_t n_groups = h->groups.size();
+    std::vector<char> run(n_groups, 0);
+    int max_top = -1;
+    for (size_t g = 0; g < n_groups; g++) {
+        const TplGroup& G = h->groups[g];
+        const bool cur = g == 0;                             // group 0's state is in the handle's fields
+        if (match_guards(h, w, hgt, cur ? h->tpl0_w : G.w0, cur ? h->tpl0_h : G.h0)) continue;
+        run[g] = 1;
+        max_top = std::max(max_top, (int)(cur ? h->tpl.size() : G.tpl.size()) - 1);
+    }
+    if (max_top < 0) return FPM_OK;
     h->cur_batch = batch;
     CK(h->d_counters.ensure(CNT_N * sizeof(int)));
-    CK(h->h_counts.ensure((CNT_N + batch) * sizeof(int)));
-    CK(cudaMemsetAsync(h->d_counters.p, 0, CNT_N * sizeof(int), h->stream));
+    CK(h->h_counts.ensure((CNT_N + (size_t)batch * n_set) * sizeof(int)));
     if (h->bitwise_not) {
         const int ipitch = (int)align_up(w, 128);
         const size_t iimg = (size_t)ipitch * hgt;
@@ -1186,27 +1305,14 @@ int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt,
         CKL();
         d_src = h->d_inv.as<uint8_t>(); stride = ipitch; frame_stride = iimg;
     }
-    rc = build_pyramid(h, d_src, batch, w, hgt, stride, frame_stride, top);
+    rc = build_pyramid(h, d_src, batch, w, hgt, stride, frame_stride, max_top);
     if (rc) return rc;
-    rc = make_top_plan(h, top, batch);
-    if (rc) return rc;
-    const TopPlan& p = h->plan;
-    const int max_picks = h->max_pos + FPM_MATCH_CANDIDATE_NUM;
-    const int njobs = batch * p.n_ang;
-    CK(h->d_picks.ensure((size_t)std::max(njobs, 1) * max_picks * sizeof(FpmPick)));
-    CK(h->d_pickcnt.ensure((size_t)std::max(njobs, 1) * sizeof(int)));
-    rc = run_top(h, top, 0, njobs, h->d_picks.as<FpmPick>(), h->d_pickcnt.as<int>());
-    if (rc) return rc;
-    FpmPickView pv{h->d_picks.as<FpmPick>(), h->d_pickcnt.as<int>(), 0, 0};
-    int n_cands = 0, cand_stride = 0;
-    rc = collect_candidates(h, top, batch, pv, p.n_ang, 0, 1, &n_cands, &cand_stride, nullptr);
-    if (rc) return rc;
-    int n_refined = 0;
-    h->ref_out = nullptr; h->ref_cnt = nullptr;
-    rc = run_refine(h, top, n_cands, &n_refined);
-    if (rc) return rc;
-    FpmRefinedView rv{h->d_refined.as<FpmRefined>(), h->d_counters.as<int>() + CNT_REFINED, 0, 1, 0};
-    return run_final(h, batch, rv, cand_stride, out, cap, n_out);
+    for (size_t g = 0; g < n_groups && rc == FPM_OK; g++) {
+        if (!run[g]) continue;
+        GroupScope scope(h, g);
+        rc = match_group(h, batch, out, cap, n_out, n_set);
+    }
+    return rc;
 }
 
 // ---- angle-sharded latency mode (SURVEY 8e): one frame, nranks GPUs -------------------------------------------
@@ -1274,7 +1380,7 @@ int shard_begin(fpm_handle* h, const uint8_t* src, int w, int hgt, int stride, i
     if (rc) return rc;
     if (!src || w <= 0 || hgt <= 0) return FPM_OK;
     if (stride < w) { h->err = "stride < width"; return FPM_ERR_INVALID; }
-    if (match_guards(h, w, hgt)) return FPM_OK;
+    if (match_guards(h, w, hgt, h->tpl0_w, h->tpl0_h)) return FPM_OK;
     const int N = h->sh_nranks, R = h->sh_rank;
     const uint8_t* d_src = src;
     int pitch = stride;
@@ -1430,6 +1536,8 @@ void fpm_destroy(fpm_handle* h)
                       &h->d_pairs, &h->d_refined, &h->d_rects, &h->d_del, &h->d_idmap, &h->d_results, &h->d_rescnt, &h->d_trace, &h->d_trace_sc,
                       &h->d_dbg[0], &h->d_dbg[1], &h->d_dbg[2], &h->d_dbg[3]};
     for (DevBuf* b : bufs) b->release();
+    for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
+    h->d_tstat.release();
     h->h_counts.release(); h->h_results.release(); h->h_stage.release();
     h->d_jpeg.release();
     h->d_jpeg_scan.release();
@@ -1469,10 +1577,14 @@ int fpm_set_param(fpm_handle* h, int param, double v)
     case FPM_PARAM_SHARD_UPLOAD: h->shard_upload = v != 0; break;
     case FPM_PARAM_ASYNC_DESCENT: h->async_descent = (int)v; break;
     case FPM_PARAM_JPEG_DEVICE_HUFFMAN: h->jpeg_device_huffman = v != 0; break;
-    case FPM_PARAM_TOLERANCE_RANGE: h->tol_range = v != 0; h->plan.valid = false; break;
+    case FPM_PARAM_TOLERANCE_RANGE: h->tol_range = v != 0; break;
     case FPM_PARAM_TOLERANCE1: case FPM_PARAM_TOLERANCE2: case FPM_PARAM_TOLERANCE3: case FPM_PARAM_TOLERANCE4:
-        h->tol_r[param - FPM_PARAM_TOLERANCE1] = v; h->plan.valid = false; break;
+        h->tol_r[param - FPM_PARAM_TOLERANCE1] = v; break;
     default: h->err = "unknown parameter"; return FPM_ERR_INVALID;
+    }
+    if (param == FPM_PARAM_TOLERANCE_RANGE || (param >= FPM_PARAM_TOLERANCE1 && param <= FPM_PARAM_TOLERANCE4)) {
+        h->plan.valid = false;                                 // the angle schedule of every group
+        for (TplGroup& g : h->groups) g.plan.valid = false;
     }
     return FPM_OK;
 }
@@ -1512,24 +1624,58 @@ int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stri
 {
     if (!h) return FPM_ERR_INVALID;
     if (!tpl || width <= 0 || height <= 0 || stride < width) { h->err = "empty template"; return FPM_ERR_INVALID; }   // :47-49
-    h->learned = false;
-    h->tpl0.resize((size_t)width * height);
-    for (int y = 0; y < height; y++) memcpy(h->tpl0.data() + (size_t)y * width, tpl + (size_t)y * stride, width);
-    h->tpl0_w = width; h->tpl0_h = height;
-    h->learn_gen++;
-    return do_learn(h);
+    return fpm_learn_set(h, 1, &tpl, &width, &height, &stride);
 }
+
+int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides)
+{
+    if (!h) return FPM_ERR_INVALID;
+    h->learned = false;
+    h->set.clear();
+    h->learn_gen++;
+    if (n < 1 || !tpls || !widths || !heights || !strides) { h->err = "template set: n < 1 or null arrays"; return FPM_ERR_INVALID; }
+    for (int i = 0; i < n; i++)
+        if (!tpls[i] || widths[i] <= 0 || heights[i] <= 0 || strides[i] < widths[i]) {
+            h->err = "template set: template " + std::to_string(i) + " is empty (null, a size <= 0 or stride < width)";
+            return FPM_ERR_INVALID;
+        }
+    std::vector<SetTpl> set(n);
+    for (int i = 0; i < n; i++) {
+        set[i].w = widths[i]; set[i].h = heights[i];
+        set[i].px.resize((size_t)widths[i] * heights[i]);
+        for (int y = 0; y < heights[i]; y++) memcpy(set[i].px.data() + (size_t)y * widths[i], tpls[i] + (size_t)y * strides[i], widths[i]);
+    }
+    h->set.swap(set);
+    int rc = do_learn(h);
+    if (rc) h->set.clear();
+    return rc;
+}
+
+int fpm_set_size(const fpm_handle* h) { return h && h->learned ? (int)h->set.size() : 0; }
 
 int fpm_is_learned(const fpm_handle* h) { return h && h->learned ? 1 : 0; }
 
 void fpm_clear(fpm_handle* h)
 {
     if (!h) return;
-    h->learned = false; h->tpl.clear(); h->tpl0.clear(); h->has_ur = 0;
+    h->learned = false; h->tpl.clear(); h->set.clear(); h->members.clear(); h->has_ur = 0;
+    for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
+    h->groups.clear();
     h->ur[0] = h->ur[1] = h->ur[2] = h->ur[3] = 0;
 }
 
-// second handle for the concurrent half-batches: same device, parameters and template as h
+namespace {
+// the single-template entry points on a handle that holds a set of more than one: refused, never template 0 alone
+int refuse_set(const fpm_handle* h, const char* fn)
+{
+    if (fpm_set_size(h) <= 1) return FPM_OK;
+    h->err = std::string(fn) + ": the handle holds a set of " + std::to_string(h->set.size()) +
+             " templates (use fpm_match_set_batch / fpm_match_ingested_set_batch)";
+    return FPM_ERR_INVALID;
+}
+}  // namespace
+
+// second handle for the concurrent half-batches: same device, parameters and template set as h
 int ensure_twin(fpm_handle* h)
 {
     if (!h->twin) {
@@ -1543,19 +1689,25 @@ int ensure_twin(fpm_handle* h)
         if (p != FPM_PARAM_TRACE && p != FPM_PARAM_SPLIT_BATCH && fpm_get_param(t, p) != fpm_get_param(h, p))
             fpm_set_param(t, p, fpm_get_param(h, p));
     if (h->twin_gen != h->learn_gen || !t->learned) {
-        int rc = fpm_learn(t, h->tpl0.data(), h->tpl0_w, h->tpl0_h, h->tpl0_w);
+        const int n = (int)h->set.size();
+        std::vector<const uint8_t*> px(n);
+        std::vector<int> ws(n), hs(n);
+        for (int i = 0; i < n; i++) { px[i] = h->set[i].px.data(); ws[i] = h->set[i].w; hs[i] = h->set[i].h; }
+        int rc = fpm_learn_set(t, n, px.data(), ws.data(), hs.data(), ws.data());
         if (rc) { h->err = t->err; return rc; }
         h->twin_gen = h->learn_gen;
     }
     return FPM_OK;
 }
 
-int fpm_match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width, int height, int stride,
-                           size_t frame_stride, fpm_result* out, int cap, int* n)
+namespace {
+// fpm_match_batch_device for the whole set: frame b / template t at out + (b * n_set + t) * cap
+int match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width, int height, int stride,
+                       size_t frame_stride, fpm_result* out, int cap, int* n)
 {
-    if (!h) return FPM_ERR_INVALID;
+    const int n_set = std::max((int)h->set.size(), 1);
     if (!n || batch < 0 || cap < 0 || (cap > 0 && !out)) { h->err = "bad output arguments"; return FPM_ERR_INVALID; }
-    for (int b = 0; b < batch; b++) n[b] = 0;
+    for (int b = 0; b < batch * n_set; b++) n[b] = 0;
     if (!d_src || width <= 0 || height <= 0 || batch == 0) return FPM_OK;       // empty source -> empty result
     if (stride < width) { h->err = "stride < width"; return FPM_ERR_INVALID; }
     CK(cudaSetDevice(h->device));
@@ -1571,8 +1723,8 @@ int fpm_match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int w
         const int b0 = batch / 2;
         int rc2 = FPM_OK;
         std::thread second([&]() {
-            rc2 = fpm_match_batch_device(h->twin, d_src + (size_t)b0 * frame_stride, batch - b0, width, height, stride, frame_stride,
-                                         out + (size_t)b0 * cap, cap, n + b0);
+            rc2 = match_batch_device(h->twin, d_src + (size_t)b0 * frame_stride, batch - b0, width, height, stride, frame_stride,
+                                     out + (size_t)b0 * n_set * cap, cap, n + (size_t)b0 * n_set);
         });
         rc = match_device(h, d_src, b0, width, height, stride, frame_stride, out, cap, n);
         second.join();
@@ -1586,12 +1738,13 @@ int fpm_match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int w
     return rc;
 }
 
-int fpm_match_batch(fpm_handle* h, const uint8_t* src, int batch, int width, int height, int stride, size_t frame_stride,
-                    fpm_result* out, int cap, int* n)
+// fpm_match_batch for the whole set
+int match_batch_host(fpm_handle* h, const uint8_t* src, int batch, int width, int height, int stride, size_t frame_stride,
+                     fpm_result* out, int cap, int* n)
 {
-    if (!h) return FPM_ERR_INVALID;
+    const int n_set = std::max((int)h->set.size(), 1);
     if (!n || batch < 0 || cap < 0 || (cap > 0 && !out)) { h->err = "bad output arguments"; return FPM_ERR_INVALID; }
-    for (int b = 0; b < batch; b++) n[b] = 0;
+    for (int b = 0; b < batch * n_set; b++) n[b] = 0;
     if (!src || width <= 0 || height <= 0 || batch == 0) return FPM_OK;
     if (stride < width) { h->err = "stride < width"; return FPM_ERR_INVALID; }
     CK(cudaSetDevice(h->device));
@@ -1650,7 +1803,7 @@ int fpm_match_batch(fpm_handle* h, const uint8_t* src, int batch, int width, int
         if ((ce = cudaStreamWaitEvent(h->stream, h->ev_copy[k & 1], 0)) != cudaSuccess) return fail_cuda("cudaStreamWaitEvent", ce);
         int b0 = k * chunk, nb = std::min(chunk, batch - b0);
         rc = match_device(h, h->d_src.as<uint8_t>() + (size_t)(k & 1) * buf_bytes, nb, width, height, pitch, img,
-                          out + (size_t)b0 * cap, cap, n + b0);
+                          out + (size_t)b0 * n_set * cap, cap, n + (size_t)b0 * n_set);
         if (rc == FPM_OK && (ce = cudaEventRecord(h->ev_done[k & 1], h->stream)) != cudaSuccess) return fail_cuda("cudaEventRecord", ce);
         prof_collect(h);
     }
@@ -1660,9 +1813,36 @@ int fpm_match_batch(fpm_handle* h, const uint8_t* src, int batch, int width, int
     h->last_ms = std::chrono::duration<double, std::milli>(t1 - t0).count();
     return rc;
 }
+}  // namespace
+
+int fpm_match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width, int height, int stride,
+                           size_t frame_stride, fpm_result* out, int cap, int* n)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_match_batch_device")) return rc;
+    return match_batch_device(h, d_src, batch, width, height, stride, frame_stride, out, cap, n);
+}
+
+int fpm_match_batch(fpm_handle* h, const uint8_t* src, int batch, int width, int height, int stride, size_t frame_stride,
+                    fpm_result* out, int cap, int* n)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_match_batch")) return rc;
+    return match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, n);
+}
+
+int fpm_match_set_batch(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                        size_t frame_stride, fpm_result* out, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (h->trace && fpm_set_size(h) > 1) { h->err = "fpm_match_set_batch: FPM_PARAM_TRACE is not supported for a set of more than one template"; return FPM_ERR_INVALID; }
+    return src_on_device ? match_batch_device(h, src, batch, width, height, stride, frame_stride, out, cap, counts)
+                         : match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, counts);
+}
 
 int fpm_match(fpm_handle* h, const uint8_t* src, int width, int height, int stride, fpm_result* out, int cap, int* n)
 {
+    if (h) if (int rc = refuse_set(h, "fpm_match")) return rc;
     return fpm_match_batch(h, src, 1, width, height, stride, (size_t)stride * (size_t)std::max(height, 0), out, cap, n);
 }
 
@@ -1675,6 +1855,8 @@ int fpm_match_multi(fpm_handle* const* hs, int n_handles, const uint8_t* src, in
     if (!hs || n_handles <= 0 || !src || !out || !counts || cap < 0) return FPM_ERR_INVALID;
     for (int i = 0; i < n_handles; i++)
         if (!hs[i]) return FPM_ERR_INVALID;
+    for (int i = 0; i < n_handles; i++)
+        if (int rc = refuse_set(hs[i], "fpm_match_multi")) return rc;
     for (int i = 0; i < n_handles; i++) counts[i] = 0;
     if (width <= 0 || height <= 0) return FPM_OK;
     if (stride < width) return FPM_ERR_INVALID;
@@ -2492,6 +2674,7 @@ int fpm_ingested_pixels(fpm_handle* h, uint8_t* out)
 int fpm_match_ingested(fpm_handle* h, fpm_result* out, int cap, int* n)
 {
     if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_match_ingested")) return rc;
     if (int rc = ingest_single(h)) return rc;
     return fpm_match_ingested_batch(h, out, cap, n);
 }
@@ -2499,14 +2682,22 @@ int fpm_match_ingested(fpm_handle* h, fpm_result* out, int cap, int* n)
 int fpm_match_ingested_batch(fpm_handle* h, fpm_result* out, int cap, int* counts)
 {
     if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_match_ingested_batch")) return rc;
+    return fpm_match_ingested_set_batch(h, out, cap, counts);
+}
+
+int fpm_match_ingested_set_batch(fpm_handle* h, fpm_result* out, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
     if (h->ingest_count <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
-    return fpm_match_batch_device(h, h->d_ingest.as<uint8_t>(), h->ingest_count, h->ingest_w, h->ingest_h, h->ingest_pitch,
-                                  (size_t)h->ingest_pitch * h->ingest_h, out, cap, counts);
+    return fpm_match_set_batch(h, h->d_ingest.as<uint8_t>(), 1, h->ingest_count, h->ingest_w, h->ingest_h, h->ingest_pitch,
+                               (size_t)h->ingest_pitch * h->ingest_h, out, cap, counts);
 }
 
 int fpm_learn_ingested(fpm_handle* h)
 {
     if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_learn_ingested")) return rc;
     if (int rc = ingest_single(h)) return rc;
     std::vector<uint8_t> px((size_t)h->ingest_w * h->ingest_h);
     int rc = fpm_ingested_pixels(h, px.data());
@@ -2534,11 +2725,16 @@ int fpm_get_user_rect(const fpm_handle* h, int* x, int* y, int* w, int* hgt)
 
 long long fpm_launch_count(const fpm_handle* h) { return h ? h->launches + (h->twin ? h->twin->launches : 0) : 0; }
 
-int fpm_tpl_levels(const fpm_handle* h) { return (h && h->learned) ? (int)h->tpl.size() : 0; }
+int fpm_tpl_levels(const fpm_handle* h)
+{
+    if (h) if (int rc = refuse_set(h, "fpm_tpl_levels")) return rc;
+    return (h && h->learned) ? (int)h->tpl.size() : 0;
+}
 
 int fpm_tpl_level_info(const fpm_handle* h, int level, int* w, int* hgt, double* mean, double* norm, double* inv_area,
                        int* result_equal1)
 {
+    if (h) if (int rc = refuse_set(h, "fpm_tpl_level_info")) return rc;
     if (!h || !h->learned || level < 0 || level >= (int)h->tpl.size()) return FPM_ERR_INVALID;
     const TplLevelHost& t = h->tpl[level];
     if (w) *w = t.w;
@@ -2552,17 +2748,23 @@ int fpm_tpl_level_info(const fpm_handle* h, int level, int* w, int* hgt, double*
 
 int fpm_tpl_level_pixels(const fpm_handle* h, int level, uint8_t* out)
 {
+    if (h) if (int rc = refuse_set(h, "fpm_tpl_level_pixels")) return rc;
     if (!h || !h->learned || level < 0 || level >= (int)h->tpl.size() || !out) return FPM_ERR_INVALID;
     memcpy(out, h->tpl[level].pix.data(), h->tpl[level].pix.size());
     return FPM_OK;
 }
 
-int fpm_tpl_border_color(const fpm_handle* h) { return h ? h->border : 0; }
+int fpm_tpl_border_color(const fpm_handle* h)
+{
+    if (h) if (int rc = refuse_set(h, "fpm_tpl_border_color")) return rc;
+    return h ? h->border : 0;
+}
 
 // ---- stage API (angle-sharded latency mode) -------------------------------------------
 int fpm_stage_num_angles(fpm_handle* h, int width, int height)
 {
     (void)width; (void)height;
+    if (h) if (int rc = refuse_set(h, "fpm_stage_num_angles")) return rc;
     if (!h || !h->learned) return 0;
     if (ensure_learned_for_mra(h)) return 0;
     std::vector<double> a;
@@ -2574,6 +2776,7 @@ int fpm_stage_top(fpm_handle* h, const uint8_t* src, int width, int height, int 
                   double* rows, int cap, int* n)
 {
     if (!h || !n) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_stage_top")) return rc;
     *n = 0;
     if (!h->learned) return FPM_ERR_NOT_LEARNED;
     int rc = ensure_learned_for_mra(h);
@@ -2581,7 +2784,7 @@ int fpm_stage_top(fpm_handle* h, const uint8_t* src, int width, int height, int 
     if (!src || width <= 0 || height <= 0) return FPM_OK;
     CK(cudaSetDevice(h->device));
     h->levels.clear();
-    if (match_guards(h, width, height)) return FPM_OK;
+    if (match_guards(h, width, height, h->tpl0_w, h->tpl0_h)) return FPM_OK;
     const uint8_t* d_src = src;
     int pitch = stride;
     size_t img = (size_t)stride * height;
@@ -2650,6 +2853,7 @@ int fpm_stage_top(fpm_handle* h, const uint8_t* src, int width, int height, int 
 int fpm_stage_sort_candidates(fpm_handle* h, const double* picks, int n, double* cands)
 {
     if (!h || n < 0) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_stage_sort_candidates")) return rc;
     if (h->levels.empty()) { h->err = "fpm_stage_top must run first"; return FPM_ERR_INVALID; }
     std::vector<int> idx(n);
     for (int i = 0; i < n; i++) idx[i] = i;
@@ -2669,6 +2873,7 @@ int fpm_stage_sort_candidates(fpm_handle* h, const double* picks, int n, double*
 int fpm_stage_refine(fpm_handle* h, const double* cands, int n, double* rows, int cap, int* n_out)
 {
     if (!h || !n_out) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_stage_refine")) return rc;
     *n_out = 0;
     if (h->levels.empty()) { h->err = "fpm_stage_top must run first"; return FPM_ERR_INVALID; }
     CK(cudaSetDevice(h->device));
@@ -2713,6 +2918,7 @@ int fpm_stage_refine(fpm_handle* h, const double* cands, int n, double* rows, in
 int fpm_stage_final(fpm_handle* h, const double* refined, int n, fpm_result* out, int cap, int* n_out)
 {
     if (!h || !n_out) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_stage_final")) return rc;
     *n_out = 0;
     if (!h->learned) return FPM_ERR_NOT_LEARNED;
     CK(cudaSetDevice(h->device));
@@ -2797,6 +3003,7 @@ int fpm_match_sharded(fpm_handle* h, const uint8_t* src, int width, int height, 
                       fpm_result* out, int cap, int* n)
 {
     if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_match_sharded")) return rc;
     if (!n || cap < 0 || (cap > 0 && !out)) { h->err = "bad output arguments"; return FPM_ERR_INVALID; }
     *n = 0;
     CK(cudaSetDevice(h->device));
@@ -2821,6 +3028,7 @@ int fpm_match_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* 
     if (!hs || nranks < 1 || !n || cap < 0 || (cap > 0 && !out)) return FPM_ERR_INVALID;
     for (int r = 0; r < nranks; r++) {
         if (!hs[r] || hs[r]->nccl_comm) return FPM_ERR_INVALID;
+        if (int rc = refuse_set(hs[r], "fpm_match_sharded_virtual")) return rc;
         hs[r]->sh_nranks = nranks; hs[r]->sh_rank = r;
         n[r] = 0;
     }
@@ -2926,6 +3134,7 @@ int fpm_dbg_corr_rows(fpm_handle* h, const uint8_t* roi, const uint8_t* tpl, int
     FpmTplLevel td;
     td.ptr = h->d_dbg[1].as<uint8_t>(); td.w = tw; td.h = th; td.pitch = tp;
     td.mean = 0; td.norm = 1; td.inv_area = 1; td.result_equal1 = 0;
+    td.n_tpl = 1; td.tpl_stride = 0; td.stats = nullptr;
     const CorrCfg cc = corr_config(th);
     if (cc.smem > 200 * 1024) { h->err = "correlation kernel shared memory limit"; return FPM_ERR_LIMIT; }
     if (cc.smem > 48 * 1024)
@@ -2934,7 +3143,7 @@ int fpm_dbg_corr_rows(fpm_handle* h, const uint8_t* roi, const uint8_t* tpl, int
     int32_t* dQ = dS + (size_t)(th + FPM_ROI_PAD) * FPM_WSTRIDE;
     dim3 grid(cc.blocks_y_rows, 1);
     fpm_corr_rows_kernel<<<grid, cc.threads, cc.smem, h->stream>>>(h->d_dbg[0].as<uint8_t>(), rpitch, roi_bytes, td, 1, cc.rb,
-                                                                    cc.evals_per_cta, h->d_dbg[2].as<int32_t>(), dS, dQ, nullptr, 1);
+                                                                    cc.evals_per_cta, h->d_dbg[2].as<int32_t>(), dS, dQ, nullptr, 1, nullptr);
     CKL();
     CK(cudaMemcpyAsync(rowsum, h->d_dbg[2].p, (size_t)th * FPM_NCELL * 4, cudaMemcpyDeviceToHost, h->stream));
     // the device records are 8 ints per (eval, row); the caller gets the 7 window sums of each
@@ -3052,6 +3261,7 @@ int fpm_dbg_top_score(fpm_handle* h, const uint8_t* img, int w, int hgt, float* 
 int fpm_dbg_top_score_production(fpm_handle* h, const uint8_t* img, int w, int hgt, float* score, float* reject_below)
 {
     if (!h || !img || !score) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_dbg_top_score_production")) return rc;
     if (!h->learned) return FPM_ERR_NOT_LEARNED;
     CK(cudaSetDevice(h->device));
     const int top = (int)h->tpl.size() - 1;
@@ -3069,9 +3279,9 @@ int fpm_dbg_top_score_production(fpm_handle* h, const uint8_t* img, int w, int h
     CK(cudaMemcpyAsync(h->d_dbg[2].p, &jb, sizeof(jb), cudaMemcpyHostToDevice, h->stream));
     size_t smem = top_score_smem(t.w, t.h);
     if (smem > 200 * 1024) { h->err = "template too large"; return FPM_ERR_LIMIT; }
-    CK(ensure_dyn_smem((const void*)fpm_top_score_kernel, h->device, smem));
+    CK(ensure_dyn_smem((const void*)fpm_top_score_kernel<false>, h->device, smem));
     dim3 grid((RW + TS_TW - 1) / TS_TW, (RH + TS_TH - 1) / TS_TH, 1), block(TS_THREADS);
-    fpm_top_score_kernel<<<grid, block, smem, h->stream>>>(h->d_dbg[2].as<FpmWarpJob>(), h->d_dbg[0].as<uint8_t>(), rp, 0,
+    fpm_top_score_kernel<false><<<grid, block, smem, h->stream>>>(h->d_dbg[2].as<FpmWarpJob>(), h->d_dbg[0].as<uint8_t>(), rp, 0,
                                                            tpl_level_dev(h, top), h->d_dbg[1].as<float>(), sp, 0,
                                                            reject_below ? top_reject_below(h, top) : -INFINITY);
     CKL();
@@ -3109,7 +3319,7 @@ int fpm_dbg_peaks(fpm_handle* h, const float* score, int cols, int rows, int tw,
     if (smem_blocks < 0) return FPM_ERR_CUDA;
     fpm_top_peaks_kernel<<<1, PK_THREADS, (size_t)smem_blocks * 8, h->stream>>>(h->d_dbg[2].as<FpmWarpJob>(), h->d_dbg[0].as<float>(), sp, 0, tw, th,
                                                                               block_mode, tile, bv, bl, blk_stride, thresh, max_overlap,
-                                                                              max_picks, dp, dn, smem_blocks);
+                                                                              max_picks, dp, dn, smem_blocks, 0, 1, 1);
     CKL();
     std::vector<FpmPick> hp(max_picks);
     int hn = 0;

@@ -50,10 +50,11 @@
 #define WA_MAXG 3     // jobs per group
 
 // getRotatedROI matrix of eval j of a candidate (src/TemplateMatcher.cpp:1074-1088), inverted like warpAffine does
-struct FpmRefineGeom { const FpmCand* cands; int n_ang; double angle_step; int lvl_w, lvl_h, tpl_w, tpl_h; };
+// n_tpl: templates of the group (candidate image v reads source frame v / n_tpl)
+struct FpmRefineGeom { const FpmCand* cands; int n_ang; double angle_step; int lvl_w, lvl_h, tpl_w, tpl_h, n_tpl; };
 
 __device__ __forceinline__ FpmWarpJob fpm_refine_job(const FpmCand& c, int j, int n_ang, double angle_step, int lvl_w, int lvl_h,
-                                                     int tpl_w, int tpl_h)
+                                                     int tpl_w, int tpl_h, int n_tpl)
 {
     double angle = (n_ang == 1) ? 0.0 : c.angle + angle_step * (double)(j - 1);
     float ptcx = (float)(lvl_w - 1) / 2.0f, ptcy = (float)(lvl_h - 1) / 2.0f;
@@ -65,7 +66,7 @@ __device__ __forceinline__ FpmWarpJob fpm_refine_job(const FpmCand& c, int j, in
     jb.m[2] -= (double)(rx - 3);
     jb.m[5] -= (double)(ry - 3);
     fpm_invert_affine(jb.m);
-    jb.src_img = c.img;
+    jb.src_img = n_tpl > 1 ? c.img / n_tpl : c.img;
     jb.dw = tpl_w + FPM_ROI_PAD; jb.dh = tpl_h + FPM_ROI_PAD;
     jb.valid = 1;
     return jb;
@@ -113,7 +114,7 @@ fpm_warp_kernel(const FpmWarpJob* __restrict__ jobs_g, int group, FpmLevel src, 
     __shared__ FpmWarpJob jobs_s[WA_MAXG];
     if (threadIdx.x < group)
         jobs_s[threadIdx.x] = geom.cands ? fpm_refine_job(geom.cands[blockIdx.y], threadIdx.x, geom.n_ang, geom.angle_step, geom.lvl_w,
-                                                          geom.lvl_h, geom.tpl_w, geom.tpl_h)
+                                                          geom.lvl_h, geom.tpl_w, geom.tpl_h, geom.n_tpl)
                                          : jobs_g[g0 + threadIdx.x];
     __syncthreads();
     const FpmWarpJob* jobs = jobs_s - g0;              // jobs[g0 + j] below
@@ -355,6 +356,10 @@ __device__ __forceinline__ float fpm_ccoeff_epilogue_top(float numerator, double
 #define TS_TH 16
 #define TS_THREADS 256
 
+// Template groups (tpl.n_tpl > 1): the CTA stages its canvas patch and its row-window sums once and scores the patch
+// against every template of the group in turn; map k of job z is written to score + (z * n_tpl + k) * score_job_stride.
+// GROUP = false (a single template) compiles to the one-template kernel.
+template <bool GROUP>
 __global__ void __launch_bounds__(TS_THREADS)
 fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restrict__ rot, int rpitch,
                      size_t rot_job_stride, FpmTplLevel tpl, float* __restrict__ score, int spitch,
@@ -374,14 +379,17 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
     const int tid = threadIdx.x;
     const uint8_t* __restrict__ r = rot + (size_t)blockIdx.z * rot_job_stride;
     const bool word_ok = ((rpitch & 3) == 0) && ((reinterpret_cast<uintptr_t>(r) & 3) == 0);    // x0 is a multiple of 64
-    for (int i = tid; i < th * nwt; i += TS_THREADS) {
-        int yy = i / nwt, xw = i - yy * nwt;
-        uint32_t v = 0;
+    auto stage_template = [&](const FpmTplLevel& t) {
+        for (int i = tid; i < th * nwt; i += TS_THREADS) {
+            int yy = i / nwt, xw = i - yy * nwt;
+            uint32_t v = 0;
 #pragma unroll
-        for (int k = 0; k < 4; k++)
-            if (4 * xw + k < tw) v |= (uint32_t)tpl.ptr[yy * tpl.pitch + 4 * xw + k] << (8 * k);
-        s_t[i] = v;
-    }
+            for (int k = 0; k < 4; k++)
+                if (4 * xw + k < tw) v |= (uint32_t)t.ptr[yy * t.pitch + 4 * xw + k] << (8 * k);
+            s_t[i] = v;
+        }
+    };
+    stage_template(tpl);
     for (int i = tid; i < ph * pww; i += TS_THREADS) {
         int yy = i / pww, xw = i - yy * pww;
         int gy = y0 + yy;
@@ -403,10 +411,14 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
     const uint32_t tailbm = tail ? (0xffffffffu >> (8 * (4 - tail))) : 0xffffffffu;
     // Row-window sums of the patch, once per CTA: s_rs/s_rq[yy][x] = sum_{j<tw} P[yy][x+j] (^2).  Every score row
     // that covers patch row yy reuses them, so the main loop only multiplies by the template (the zero padding of
-    // the template's last word masks the patch bytes beyond tw there).
+    // the template's last word masks the patch bytes beyond tw there).  The same for every template of a group; not
+    // needed when all of them are flat.
     uint32_t* s_rs = s_t + ((th * nwt + ph * pww + 3) & ~3);   // ph * TS_TW, 16-byte aligned
     uint32_t* s_rq = s_rs + ph * TS_TW;
-    if (!tpl.result_equal1) {
+    bool need_sums = !tpl.result_equal1;
+    if (GROUP)
+        for (int k = 1; k < tpl.n_tpl; k++) need_sums |= !tpl.stats[k].result_equal1;
+    if (need_sums) {
         for (int i = tid; i < ph * (TS_TW / 4); i += TS_THREADS) {
             const int yy = i / (TS_TW / 4), xq = i - yy * (TS_TW / 4);
             const uint32_t* prow = s_p + yy * pww + xq;
@@ -431,66 +443,77 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
     }
     const int tx = tid & 15, ty = tid >> 4;
     const int ox = x0 + 4 * tx, oy = y0 + ty;
-    if (ox >= RW || oy >= RH) return;
-    float* out = score + (size_t)blockIdx.z * score_job_stride + (size_t)oy * spitch + ox;
-    if (tpl.result_equal1) {
-        for (int k = 0; k < 4 && ox + k < RW; k++) out[k] = 1.0f;
-        return;
-    }
-    unsigned long long num[4], wsum[4], wsq[4];
-    if ((long long)tw * th <= 66000) {
-        // every sum is at most 255^2 * w * h < 2^32: plain 32-bit accumulators across all template rows (the 64-bit
-        // adds of the general path cost as many instructions as the dp4a loop itself for a 14x14 template)
-        uint32_t a[4] = {0, 0, 0, 0}, b[4] = {0, 0, 0, 0}, c[4] = {0, 0, 0, 0};
-        for (int yy = 0; yy < th; yy++) {
-            const uint32_t* prow = s_p + (ty + yy) * pww + tx;
-            const uint32_t* trow = s_t + yy * nwt;
-            uint32_t lo = prow[0];
-            for (int xw = 0; xw < nwt; xw++) {
-                const uint32_t hi = prow[xw + 1];
-                const uint32_t t = trow[xw];               // bytes beyond tw are 0 in the staged template
-                a[0] = __dp4a(lo, t, a[0]);
-                a[1] = __dp4a(__funnelshift_r(lo, hi, 8), t, a[1]);
-                a[2] = __dp4a(__funnelshift_r(lo, hi, 16), t, a[2]);
-                a[3] = __dp4a(__funnelshift_r(lo, hi, 24), t, a[3]);
-                lo = hi;
-            }
-            const uint4 rs = *reinterpret_cast<const uint4*>(s_rs + (ty + yy) * TS_TW + 4 * tx);
-            const uint4 rq = *reinterpret_cast<const uint4*>(s_rq + (ty + yy) * TS_TW + 4 * tx);
-            b[0] += rs.x; b[1] += rs.y; b[2] += rs.z; b[3] += rs.w;
-            c[0] += rq.x; c[1] += rq.y; c[2] += rq.z; c[3] += rq.w;
+    const bool live = ox < RW && oy < RH;
+    if (!GROUP && !live) return;
+    const int n_tpl = GROUP ? tpl.n_tpl : 1;
+    for (int kt = 0; kt < n_tpl; kt++) {
+        const FpmTplLevel tk = GROUP ? fpm_tpl_member(tpl, kt) : tpl;
+        if (GROUP && kt > 0) {                                      // every thread is past the previous template's words
+            __syncthreads();
+            stage_template(tk);
+            __syncthreads();
         }
-#pragma unroll
-        for (int k = 0; k < 4; k++) { num[k] = a[k]; wsum[k] = b[k]; wsq[k] = c[k]; }
-    } else {
-#pragma unroll
-        for (int k = 0; k < 4; k++) { num[k] = 0; wsum[k] = 0; wsq[k] = 0; }
-        for (int yy = 0; yy < th; yy++) {
-            const uint32_t* prow = s_p + (ty + yy) * pww + tx;
-            const uint32_t* trow = s_t + yy * nwt;
-            uint32_t a[4] = {0, 0, 0, 0};
-            uint32_t lo = prow[0];
-            for (int xw = 0; xw < nwt; xw++) {
-                const uint32_t hi = prow[xw + 1];
-                const uint32_t t = trow[xw];
-                a[0] = __dp4a(lo, t, a[0]);
-                a[1] = __dp4a(__funnelshift_r(lo, hi, 8), t, a[1]);
-                a[2] = __dp4a(__funnelshift_r(lo, hi, 16), t, a[2]);
-                a[3] = __dp4a(__funnelshift_r(lo, hi, 24), t, a[3]);
-                lo = hi;
-            }
-            const uint4 rs = *reinterpret_cast<const uint4*>(s_rs + (ty + yy) * TS_TW + 4 * tx);
-            const uint4 rq = *reinterpret_cast<const uint4*>(s_rq + (ty + yy) * TS_TW + 4 * tx);
-            num[0] += a[0]; num[1] += a[1]; num[2] += a[2]; num[3] += a[3];   // per-row s32, s64 across rows
-            wsum[0] += rs.x; wsum[1] += rs.y; wsum[2] += rs.z; wsum[3] += rs.w;
-            wsq[0] += rq.x; wsq[1] += rq.y; wsq[2] += rq.z; wsq[3] += rq.w;
+        if (!live) continue;
+        float* out = score + ((size_t)blockIdx.z * n_tpl + kt) * score_job_stride + (size_t)oy * spitch + ox;
+        if (tk.result_equal1) {
+            for (int k = 0; k < 4 && ox + k < RW; k++) out[k] = 1.0f;
+            continue;
         }
+        unsigned long long num[4], wsum[4], wsq[4];
+        if ((long long)tw * th <= 66000) {
+            // every sum is at most 255^2 * w * h < 2^32: plain 32-bit accumulators across all template rows (the 64-bit
+            // adds of the general path cost as many instructions as the dp4a loop itself for a 14x14 template)
+            uint32_t a[4] = {0, 0, 0, 0}, b[4] = {0, 0, 0, 0}, c[4] = {0, 0, 0, 0};
+            for (int yy = 0; yy < th; yy++) {
+                const uint32_t* prow = s_p + (ty + yy) * pww + tx;
+                const uint32_t* trow = s_t + yy * nwt;
+                uint32_t lo = prow[0];
+                for (int xw = 0; xw < nwt; xw++) {
+                    const uint32_t hi = prow[xw + 1];
+                    const uint32_t t = trow[xw];           // bytes beyond tw are 0 in the staged template
+                    a[0] = __dp4a(lo, t, a[0]);
+                    a[1] = __dp4a(__funnelshift_r(lo, hi, 8), t, a[1]);
+                    a[2] = __dp4a(__funnelshift_r(lo, hi, 16), t, a[2]);
+                    a[3] = __dp4a(__funnelshift_r(lo, hi, 24), t, a[3]);
+                    lo = hi;
+                }
+                const uint4 rs = *reinterpret_cast<const uint4*>(s_rs + (ty + yy) * TS_TW + 4 * tx);
+                const uint4 rq = *reinterpret_cast<const uint4*>(s_rq + (ty + yy) * TS_TW + 4 * tx);
+                b[0] += rs.x; b[1] += rs.y; b[2] += rs.z; b[3] += rs.w;
+                c[0] += rq.x; c[1] += rq.y; c[2] += rq.z; c[3] += rq.w;
+            }
+#pragma unroll
+            for (int k = 0; k < 4; k++) { num[k] = a[k]; wsum[k] = b[k]; wsq[k] = c[k]; }
+        } else {
+#pragma unroll
+            for (int k = 0; k < 4; k++) { num[k] = 0; wsum[k] = 0; wsq[k] = 0; }
+            for (int yy = 0; yy < th; yy++) {
+                const uint32_t* prow = s_p + (ty + yy) * pww + tx;
+                const uint32_t* trow = s_t + yy * nwt;
+                uint32_t a[4] = {0, 0, 0, 0};
+                uint32_t lo = prow[0];
+                for (int xw = 0; xw < nwt; xw++) {
+                    const uint32_t hi = prow[xw + 1];
+                    const uint32_t t = trow[xw];
+                    a[0] = __dp4a(lo, t, a[0]);
+                    a[1] = __dp4a(__funnelshift_r(lo, hi, 8), t, a[1]);
+                    a[2] = __dp4a(__funnelshift_r(lo, hi, 16), t, a[2]);
+                    a[3] = __dp4a(__funnelshift_r(lo, hi, 24), t, a[3]);
+                    lo = hi;
+                }
+                const uint4 rs = *reinterpret_cast<const uint4*>(s_rs + (ty + yy) * TS_TW + 4 * tx);
+                const uint4 rq = *reinterpret_cast<const uint4*>(s_rq + (ty + yy) * TS_TW + 4 * tx);
+                num[0] += a[0]; num[1] += a[1]; num[2] += a[2]; num[3] += a[3];   // per-row s32, s64 across rows
+                wsum[0] += rs.x; wsum[1] += rs.y; wsum[2] += rs.z; wsum[3] += rs.w;
+                wsq[0] += rq.x; wsq[1] += rq.y; wsq[2] += rq.z; wsq[3] += rq.w;
+            }
+        }
+        // TM_CCORR result cell is a float32 (cv::matchTemplate output depth), here the rounded exact sum
+        const float inv_tnorm_f = 1.0f / (float)tk.norm;
+        for (int k = 0; k < 4 && ox + k < RW; k++)
+            out[k] = fpm_ccoeff_epilogue_top((float)num[k], (double)wsum[k], (double)wsq[k], tk.mean, tk.norm, tk.inv_area,
+                                             reject_below, inv_tnorm_f);
     }
-    // TM_CCORR result cell is a float32 (cv::matchTemplate output depth), here the rounded exact sum
-    const float inv_tnorm_f = 1.0f / (float)tpl.norm;
-    for (int k = 0; k < 4 && ox + k < RW; k++)
-        out[k] = fpm_ccoeff_epilogue_top((float)num[k], (double)wsum[k], (double)wsq[k], tpl.mean, tpl.norm, tpl.inv_area,
-                                         reject_below, inv_tnorm_f);
 }
 
 // =====================================================================================
@@ -651,21 +674,25 @@ fpm_top_peaks_kernel(const FpmWarpJob* __restrict__ jobs, float* __restrict__ sc
                      size_t score_job_stride, int tw, int th, int mode, int tile,
                      float* __restrict__ blk_val, int* __restrict__ blk_loc, int blk_stride,
                      double thresh, double max_overlap, int max_picks,
-                     FpmPick* __restrict__ picks, int* __restrict__ pick_count, int smem_blocks)
+                     FpmPick* __restrict__ picks, int* __restrict__ pick_count, int smem_blocks, int j0, int n_tpl, int n_ang)
 {
-    const int job = blockIdx.x;
-    const FpmWarpJob& jb = jobs[job];
+    // map blockIdx.x = (canvas j0 + blockIdx.x / n_tpl) x (template blockIdx.x % n_tpl), the score kernel's order; its picks go
+    // to (virtual image, angle) slot job: canvas j = frame * n_ang + angle, virtual image = frame * n_tpl + template
+    const int mi = blockIdx.x;
+    const int wj = j0 + mi / n_tpl;
+    const int job = n_tpl == 1 ? wj : ((wj / n_ang) * n_tpl + mi % n_tpl) * n_ang + wj % n_ang;
+    const FpmWarpJob& jb = jobs[wj];
     const int cols = jb.dw - tw + 1, rows = jb.dh - th + 1;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nthreads = blockDim.x, nwarps = nthreads >> 5;
     if (!jb.valid || cols <= 0 || rows <= 0) { if (tid == 0) pick_count[job] = 0; return; }
-    float* __restrict__ map = score + (size_t)job * score_job_stride;
+    float* __restrict__ map = score + (size_t)mi * score_job_stride;
     const FpmBlockGeom g = fpm_block_geom(mode, cols, rows, tw, th, tile);
     mode = g.mode;                                                // MFC tables that come out empty use the plain search
     // block table: in shared memory when the launch reserved room for it (smem_blocks), else in global scratch
     extern __shared__ float pk_dyn[];
     const bool tbl_smem = g.nblocks <= smem_blocks;
-    float* bval = tbl_smem ? pk_dyn : blk_val + (size_t)job * blk_stride;
-    int* bloc = tbl_smem ? reinterpret_cast<int*>(pk_dyn + smem_blocks) : blk_loc + (size_t)job * blk_stride;
+    float* bval = tbl_smem ? pk_dyn : blk_val + (size_t)mi * blk_stride;
+    int* bloc = tbl_smem ? reinterpret_cast<int*>(pk_dyn + smem_blocks) : blk_loc + (size_t)mi * blk_stride;
     const int regular = g.ncol * g.nrow;
     const int nsup = (g.nblocks + 31) >> 5;
     const FpmFastDiv div_bw = fpm_fastdiv_make(g.bw), div_bh = fpm_fastdiv_make(g.bh);
@@ -952,13 +979,13 @@ fpm_collect_sort_kernel(FpmPickView pv,
 // =====================================================================================
 __global__ void fpm_refine_prep_kernel(const FpmCand* __restrict__ cands, int n_cands, int n_ang,
                                        double angle_step, int lvl_w, int lvl_h, int tpl_w, int tpl_h,
-                                       FpmWarpJob* __restrict__ jobs, const int* __restrict__ n_cands_dev)
+                                       FpmWarpJob* __restrict__ jobs, const int* __restrict__ n_cands_dev, int n_tpl)
 {
     if (n_cands_dev) n_cands = min(n_cands, *n_cands_dev);
     int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n_cands * n_ang) return;
     int ci = e / n_ang, j = e - ci * n_ang;
-    jobs[e] = fpm_refine_job(cands[ci], j, n_ang, angle_step, lvl_w, lvl_h, tpl_w, tpl_h);
+    jobs[e] = fpm_refine_job(cands[ci], j, n_ang, angle_step, lvl_w, lvl_h, tpl_w, tpl_h, n_tpl);
 }
 
 // =====================================================================================
@@ -976,6 +1003,8 @@ __global__ void fpm_refine_prep_kernel(const FpmCand* __restrict__ cands, int n_
 // memory transpose so the global stores are coalesced.
 //   CTA layout: evals_per_cta x rb threads; thread (el, yl) -> eval blockIdx.y*evals_per_cta+el,
 //   row y = blockIdx.x*rb + yl.
+//   Template groups (tpl.n_tpl > 1): the evals of a CTA may belong to different templates (template of eval e =
+//   cands[e / n_ang].img % n_tpl), so every eval stages its own template rows.
 // =====================================================================================
 #define CR_SLAB 32                // template words per slab (128 px)
 #define CR_PW 36                  // slab row pitch in words: 32 + 4 look-ahead; 36 = 4 (mod 32), so a
@@ -992,7 +1021,8 @@ __device__ __forceinline__ uint32_t fpm_u4(const uint4& v, int i) { return i == 
 __global__ void __launch_bounds__(CR_MAX_THREADS)
 fpm_corr_rows_kernel(const uint8_t* __restrict__ roi, int rpitch, size_t roi_stride, FpmTplLevel tpl,
                      int n_evals, int rb, int evals_per_cta, int32_t* __restrict__ rowsum,
-                     int32_t* __restrict__ rowS, int32_t* __restrict__ rowQ, const int* __restrict__ n_evals_dev, int n_ang)
+                     int32_t* __restrict__ rowS, int32_t* __restrict__ rowQ, const int* __restrict__ n_evals_dev, int n_ang,
+                     const FpmCand* __restrict__ cands)
 {
     extern __shared__ __align__(16) uint32_t smem_w[];
     if (n_evals_dev) {                                       // live evals known only on the device (n_ang per candidate)
@@ -1010,7 +1040,8 @@ fpm_corr_rows_kernel(const uint8_t* __restrict__ roi, int rpitch, size_t roi_str
     const bool active = (el < evals_per_cta) && (e < n_evals) && (y < rh);
     const int n_srow = evals_per_cta * rb;                 // staged ROI rows
     const int n_trow = rb + FPM_ROI_PAD;                   // staged template rows: tr = y0-6 .. y0+rb-1
-    const int stage_words = (n_srow + n_trow) * CR_PW;     // one slab buffer: ROI rows then template rows
+    const int n_tblk = tpl.n_tpl > 1 ? evals_per_cta : 1;  // staged templates: one per eval in a group
+    const int stage_words = (n_srow + n_tblk * n_trow) * CR_PW;   // one slab buffer: ROI rows then template rows
     const int nw = (tw + 3) / 4;                           // template words per row
     const int tail = tw & 3;
     const uint32_t tailbm = tail ? (0xffffffffu >> (8 * (4 - tail))) : 0xffffffffu;
@@ -1032,12 +1063,15 @@ fpm_corr_rows_kernel(const uint8_t* __restrict__ roi, int rpitch, size_t roi_str
             const uint8_t* g = ok ? roi + (size_t)re * roi_stride + (size_t)ry * rpitch + xb + 16 * c : roi;
             fpm_cp_async16z(b_s + r * CR_PW + 4 * c, g, ok);
         }
-        for (int i = tid; i < n_trow * 8; i += nthreads) {
-            const int r = i >> 3, c = i & 7;
+        for (int i = tid; i < n_tblk * n_trow * 8; i += nthreads) {
+            const int rr = i >> 3, c = i & 7;
+            const int tb = rr / n_trow, r = rr - tb * n_trow;
             const int tr = y0 - FPM_ROI_PAD + r;
+            const uint8_t* tp = tpl.ptr;
+            if (tpl.n_tpl > 1 && e0 + tb < n_evals) tp += (size_t)(cands[(e0 + tb) / n_ang].img % tpl.n_tpl) * tpl.tpl_stride;
             const bool ok = tr >= 0 && tr < th && xb + 16 * c < tpl.pitch;
-            const uint8_t* g = ok ? tpl.ptr + (size_t)tr * tpl.pitch + xb + 16 * c : tpl.ptr;
-            fpm_cp_async16z(b_t + r * CR_PW + 4 * c, g, ok);
+            const uint8_t* g = ok ? tp + (size_t)tr * tpl.pitch + xb + 16 * c : tpl.ptr;
+            fpm_cp_async16z(b_t + rr * CR_PW + 4 * c, g, ok);
         }
         fpm_cp_async_commit();
     };
@@ -1064,7 +1098,7 @@ fpm_corr_rows_kernel(const uint8_t* __restrict__ roi, int rpitch, size_t roi_str
         __syncthreads();
         if (active) {
             const uint32_t* s_s = smem_w + (size_t)(si & 1) * stage_words;
-            const uint32_t* s_t = s_s + (size_t)n_srow * CR_PW;
+            const uint32_t* s_t = s_s + (size_t)(n_srow + (tpl.n_tpl > 1 ? el * n_trow : 0)) * CR_PW;
             const uint4* srow4 = reinterpret_cast<const uint4*>(s_s + (size_t)tid * CR_PW);
             const uint4* trow4 = reinterpret_cast<const uint4*>(s_t + (size_t)(yl + FPM_ROI_PAD) * CR_PW);   // row tr = y
             const int nx = min(CR_SLAB, nw - xs);
@@ -1256,6 +1290,8 @@ __device__ void fpm_subpix(const double* sc27 /* [theta][y][x] */, double xm, do
 // =====================================================================================
 #define RF_THREADS 192
 
+// GROUP: the candidates are virtual images of a template group (statistics of template img % n_tpl)
+template <bool GROUP>
 __global__ void __launch_bounds__(RF_THREADS, 6)
 fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double angle_step,
                            const int32_t* __restrict__ rowsum, int raw_epad, const int32_t* __restrict__ rowS,
@@ -1269,6 +1305,7 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
 {
     const int ci = blockIdx.x;
     if (n_cands_dev && ci >= *n_cands_dev) return;
+    if (GROUP) tpl = fpm_tpl_member(tpl, cands[ci].img % tpl.n_tpl);    // one candidate per CTA: CTA-uniform statistics
     const int tid = threadIdx.x, j = tid >> 6, cell = tid & 63;
     __shared__ float s_sc[3][FPM_NCELL];
     __shared__ float s_best[3];

@@ -136,6 +136,60 @@ class TemplateMatcher:
         self._check(self._lib.fpm_learn(self._h, t.ctypes.data, t.shape[1], t.shape[0], t.strides[0]))
         return True
 
+    # ---- template sets: n templates in one handle, matched in shared launches (fpm_learn_set) ----
+    def learnPatternSet(self, templates) -> bool:
+        """n templates (2-D uint8 arrays) replace the pattern; all use this matcher's parameters."""
+        ts = [_as_u8_2d(t) for t in templates]
+        n = len(ts)
+        self._tpl_keepalive = ts
+        ptrs = (C.c_void_p * max(n, 1))(*[t.ctypes.data for t in ts])
+        ws = (C.c_int * max(n, 1))(*[t.shape[1] for t in ts])
+        hs = (C.c_int * max(n, 1))(*[t.shape[0] for t in ts])
+        st = (C.c_int * max(n, 1))(*[t.strides[0] for t in ts])
+        self._check(self._lib.fpm_learn_set(self._h, n, ptrs, ws, hs, st))
+        return True
+
+    def patternSetSize(self) -> int: return int(self._lib.fpm_set_size(self._h))
+
+    def _set_results(self, res, counts, B, T):
+        cap = self.result_capacity
+        return [[_convert(res[(b * T + t) * cap:(b * T + t + 1) * cap], min(counts[b * T + t], cap)) for t in range(T)]
+                for b in range(B)]
+
+    def matchSetBatchRaw(self, ptr: int, B: int, W: int, H: int, stride: int, frame_stride: int, on_device: bool,
+                         res=None, counts=None):
+        """Pointer-level set match: returns (results ctypes array [B][T][cap], counts [B][T])."""
+        cap, T = self.result_capacity, max(self.patternSetSize(), 1)
+        if res is None:
+            res = (L.fpm_result * (cap * B * T))()
+        if counts is None:
+            counts = (C.c_int * (B * T))()
+        self._check(self._lib.fpm_match_set_batch(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride, res, cap,
+                                                  counts))
+        return res, counts
+
+    def matchSetBatch(self, frames: np.ndarray) -> List[List[List[SingleTargetMatch]]]:
+        """frames: [B, H, W] uint8 in host memory -> [frame][template][results]."""
+        f = np.asarray(frames)
+        if f.ndim != 3 or f.dtype != np.uint8 or f.strides[2] != 1:
+            raise FpmError("frames must be a [B,H,W] uint8 array with unit pixel stride")
+        B, H, W = f.shape
+        T = max(self.patternSetSize(), 1)
+        res, counts = self.matchSetBatchRaw(f.ctypes.data, B, W, H, f.strides[1], f.strides[0], False)
+        return self._set_results(res, counts, B, T)
+
+    def matchSet(self, sourceImage) -> List[List[SingleTargetMatch]]:
+        """one host image -> [template][results]"""
+        return self.matchSetBatch(_as_u8_2d(sourceImage)[None])[0]
+
+    def matchIngestedSetBatch(self) -> List[List[List[SingleTargetMatch]]]:
+        """the frames of the last ingest x the set: [frame][template][results]"""
+        B, T, cap = self.ingestedCount(), max(self.patternSetSize(), 1), self.result_capacity
+        res = (L.fpm_result * (cap * max(B, 1) * T))()
+        counts = (C.c_int * (max(B, 1) * T))()
+        self._check(self._lib.fpm_match_ingested_set_batch(self._h, res, cap, counts))
+        return self._set_results(res, counts, B, T)
+
     # ---- match (src/TemplateMatcher.cpp:97-437) ----
     def match(self, sourceImage) -> List[SingleTargetMatch]:
         if sourceImage is None or np.asarray(sourceImage).size == 0:
@@ -589,27 +643,45 @@ def ocr_assemble(centres, labels, line_tol: float = 10.0) -> str:
 
 class GlyphReader:
     """One learned TemplateMatcher per glyph; read(image) = the upstream OCR loop: match every glyph, collect the
-    centres with their letter, assemble lines."""
+    centres with their letter, assemble lines.  readBatch(frames) reads many frames with one handle holding all glyphs as
+    a template set (created on first use)."""
 
     def __init__(self, templates: dict, device: int = 0, result_capacity: int = 256, **params):
         self.letters = [ch for ch in OCR_LETTERS if ch in templates] + sorted(k for k in templates if k not in OCR_LETTERS)
+        self._templates = [templates[ch] for ch in self.letters]
+        self._device, self._capacity, self._params = device, result_capacity, params
+        self._set_matcher = None
         self.matchers = []
         for ch in self.letters:
-            m = TemplateMatcher(device, result_capacity=result_capacity)
-            for k, v in params.items():
-                {"max_pos": m.setMaxPositions, "max_overlap": m.setMaxOverlap, "score": m.setScore,
-                 "tolerance_angle": m.setToleranceAngle, "min_reduce_area": m.setMinReduceArea, "use_simd": m.setUseSIMD,
-                 "sub_pixel": m.setSubPixelEstimation}[k](v)
+            m = self._new_matcher()
             if not m.learnPattern(templates[ch]):
                 raise FpmError("learnPattern failed for glyph %r" % ch)
             self.matchers.append(m)
 
-    def read(self, sourceImage, line_tol: float = 10.0):
-        """Returns (text, {letter: [SingleTargetMatch, ...]})."""
-        per = match_multi(self.matchers, sourceImage)
+    def _new_matcher(self):
+        m = TemplateMatcher(self._device, result_capacity=self._capacity)
+        for k, v in self._params.items():
+            {"max_pos": m.setMaxPositions, "max_overlap": m.setMaxOverlap, "score": m.setScore,
+             "tolerance_angle": m.setToleranceAngle, "min_reduce_area": m.setMinReduceArea, "use_simd": m.setUseSIMD,
+             "sub_pixel": m.setSubPixelEstimation}[k](v)
+        return m
+
+    def _assemble(self, per, line_tol):
         centres, labels = [], []
         for ch, res in zip(self.letters, per):
             for r in res:
                 centres.append(r.ptCenter)
                 labels.append(ch)
         return ocr_assemble(centres, labels, line_tol), dict(zip(self.letters, per))
+
+    def readBatch(self, frames, line_tol: float = 10.0):
+        """frames: [B, H, W] uint8 (or a list of equally sized images) -> [(text, {letter: results})] per frame."""
+        if self._set_matcher is None:
+            self._set_matcher = self._new_matcher()
+            self._set_matcher.learnPatternSet(self._templates)
+        f = np.ascontiguousarray(np.stack([_as_u8_2d(x) for x in frames]) if isinstance(frames, (list, tuple)) else frames, np.uint8)
+        return [self._assemble(per, line_tol) for per in self._set_matcher.matchSetBatch(f)]
+
+    def read(self, sourceImage, line_tol: float = 10.0):
+        """Returns (text, {letter: [SingleTargetMatch, ...]})."""
+        return self._assemble(match_multi(self.matchers, sourceImage), line_tol)

@@ -94,6 +94,24 @@ double fpm_get_param(const fpm_handle* h, int param);
 
 /* learnPattern (src/TemplateMatcher.cpp:45-95).  tpl: host pointer, u8, `stride` bytes per row. */
 int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stride);
+/* Template sets (the upstream OCR loop, MatchTool/MatchToolDlg.cpp:718-770: one LoadDst + Match per glyph): n templates
+ * (template i: tpls[i], widths[i] x heights[i], strides[i] bytes per row) replace the handle's pattern, all with the handle's
+ * parameters.  FPM_ERR_INVALID (the message names the index) for n < 1, null pointers or an empty template; the handle then
+ * holds none.  fpm_learn is a set of one.  Templates of one level-0 size and border colour form a group that shares every
+ * launch of the pipeline (the template is a kernel dimension); groups run one after another.  There is no NMS across templates.
+ * A handle holding more than one template refuses every single-template entry point with FPM_ERR_INVALID and a message:
+ * fpm_match*, fpm_match_ingested*, fpm_learn_ingested, fpm_match_multi, fpm_match_sharded*, fpm_stage_*, fpm_tpl_* (and
+ * fpm_match_set_batch with FPM_PARAM_TRACE on).  FPM_PARAM_MIN_REDUCE_AREA changed after learning re-learns the whole set. */
+int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides);
+int fpm_set_size(const fpm_handle* h);              /* 0 = nothing learned, 1 after fpm_learn */
+/* batch frames (HOST memory, or device memory with src_on_device = 1; frame i at src + i*frame_stride) x the set: frame b /
+ * template t at out + (b*n + t)*cap, its total in counts[b*n + t].  For every (b, t) exactly the list a handle holding only
+ * template t returns for frame b through fpm_match_batch_device.  Host frames use the chunked H2D pipeline of fpm_match_batch. */
+int fpm_match_set_batch(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                        size_t frame_stride, fpm_result* out, int cap, int* counts);
+/* the frames left by the last ingest (fpm_ingest_jpeg_batch etc.) x the set */
+int fpm_match_ingested_set_batch(fpm_handle* h, fpm_result* out, int cap, int* counts);
+
 /* isPatternLearned / clearPattern (include/TemplateMatcher.h:43-46). */
 int fpm_is_learned(const fpm_handle* h);
 void fpm_clear(fpm_handle* h);
@@ -114,7 +132,8 @@ int fpm_match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int w
 
 /* Multi-template matching (SURVEY 8f rank 3; the upstream "NCC-based OCR" loop, MatchTool/MatchToolDlg.cpp:727-750:
  * one LoadDst + Match per glyph template): the same HOST image matched by n_handles learned handles of one
- * device, concurrently.  out holds n_handles*cap records (handle i at out + i*cap), counts n_handles totals. */
+ * device, concurrently.  out holds n_handles*cap records (handle i at out + i*cap), counts n_handles totals.
+ * Handles may differ in parameters; templates with one set of parameters are better served by fpm_learn_set. */
 int fpm_match_multi(fpm_handle* const* hs, int n_handles, const uint8_t* src, int width, int height, int stride,
                     fpm_result* out, int cap, int* counts);
 /* Text assembly of that loop (MatchToolDlg.cpp:752-771): centres + one label each -> lines (sorted by y, split where
