@@ -39,6 +39,8 @@ SIGNATURES = {
     "fpm_set_size": (_i, [_vp]),
     "fpm_match_set_batch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _vp, _i, _vp]),
     "fpm_match_ingested_set_batch": (_i, [_vp, _vp, _i, _vp]),
+    "fpm_match_set_batch_merged": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _d, _vp, _vp, _i, _vp, _vp]),
+    "fpm_match_ingested_set_batch_merged": (_i, [_vp, _d, _vp, _vp, _i, _vp, _vp]),
     "fpm_is_learned": (_i, [_vp]),
     "fpm_clear": (None, [_vp]),
     "fpm_match": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _pi]),

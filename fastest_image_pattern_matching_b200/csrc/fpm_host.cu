@@ -204,6 +204,8 @@ struct fpm_handle {
     std::vector<SetTpl> set;       // the learned templates (fpm_learn: one), kept for re-learning when MinReduceArea changes
     std::vector<TplGroup> groups;  // their groups; groups[0]'s state is in the fields below (see TplGroup)
     DevBuf d_tstat;                // FpmTplStat of every (group, level, member)
+    DevBuf d_members;              // the members of every group, group after group (merged set results: output rows)
+    DevBuf d_mlists, d_merged;     // merged set results: per-template lists of a sub-batch, the merge's outputs
     std::vector<int> members;      // current group: its set indices
     int tpl0_w = 0, tpl0_h = 0;    // current group: level-0 size
     std::vector<TplLevelHost> tpl;
@@ -273,13 +275,14 @@ namespace {
 // CNT_LAYER + l: candidates entering pyramid layer l (descent without host round trips)
 enum { CNT_FLAT = 0, CNT_NEXT = 1, CNT_REFINED = 2, CNT_TOTAL = 3, CNT_ERR = 4, CNT_LAYER = 8, CNT_N = 8 + FPM_MAX_LEVELS };
 enum { K_PYRDOWN = 0, K_WARP_TOP, K_TOP_SCORE, K_TOP_PEAKS, K_COLLECT, K_PREP, K_WARP_ROI, K_CORR, K_FINALIZE, K_FINAL, K_CORR_MMA, K_CORR_FUSED, K_CORR_WARP,
-       K_JPEG_UPLOAD, K_JPEG_UNSTUFF, K_JPEG_PASSES, K_JPEG_SCAN, K_JPEG_WRITE, K_JPEG_IDCT, K_COUNT };
+       K_JPEG_UPLOAD, K_JPEG_UNSTUFF, K_JPEG_PASSES, K_JPEG_SCAN, K_JPEG_WRITE, K_JPEG_IDCT, K_SET_MERGE, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"fpm_pyrdown_kernel", "fpm_warp_kernel(top)", "fpm_top_score_kernel", "fpm_top_peaks_kernel",
                                            "fpm_collect_sort_kernel", "fpm_refine_prep_kernel", "fpm_warp_kernel(roi)",
                                            "fpm_corr_rows_kernel", "fpm_refine_finalize_kernel", "fpm_final_kernel",
                                            "fpm_corr_mma_kernel", "fpm_corr_fused_kernel", "fpm_corr_warp_kernel",
                                            "jpeg_upload(H2D copy)", "fpm_jpeg_unstuff_count/write_kernel", "fpm_jpeg_cold/sync_kernel(passes)",
-                                           "fpm_jpeg_block_tile/dc_tile/offsets_kernel(scans)", "fpm_jpeg_write_kernel", "fpm_ingest_jpeg_idct_kernel"};
+                                           "fpm_jpeg_block_tile/dc_tile/offsets_kernel(scans)", "fpm_jpeg_write_kernel", "fpm_ingest_jpeg_idct_kernel",
+                                           "fpm_set_merge_kernel"};
 static_assert(K_COUNT <= 24, "profile arrays");
 
 cudaEvent_t prof_event(fpm_handle* h)
@@ -729,6 +732,10 @@ int do_learn(fpm_handle* h)
             }
     CK(h->d_tstat.ensure(n_stat * sizeof(FpmTplStat)));
     CK(cudaMemcpy(h->d_tstat.p, stats.data(), n_stat * sizeof(FpmTplStat), cudaMemcpyHostToDevice));
+    std::vector<int> members;
+    for (const TplGroup& G : gs) members.insert(members.end(), G.members.begin(), G.members.end());
+    CK(h->d_members.ensure(members.size() * sizeof(int)));
+    CK(cudaMemcpy(h->d_members.p, members.data(), members.size() * sizeof(int), cudaMemcpyHostToDevice));
     // group 0 goes into the handle's fields (its plan buffers stay the handle's), the others wait in groups[1..]
     TplGroup& G0 = gs[0];
     h->tpl.swap(G0.tpl); h->members.swap(G0.members);
@@ -1128,10 +1135,23 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
     return FPM_OK;
 }
 
+// merged set results of one sub-batch (fpm_match_set_batch_merged): every group's fpm_final_kernel leaves its lists on the
+// device, frame b / set index t at lists + (b * n_set + t) * lcap with its count at counts[b * n_set + t], for
+// fpm_set_merge_kernel
+struct MergeDev {
+    FpmResultDev* lists = nullptr;
+    int* counts = nullptr;
+    int lcap = 0;
+    int ocap = 0;                  // merged records per frame in d_merged: min(cap, n_set * lcap), a merged list never exceeds its inputs
+    const int* rows = nullptr;     // the current group's members (d_members)
+    int* err = nullptr;            // the current group's slot for CNT_ERR (read back with the merged results)
+};
+
 // ---- final stage: filterWithScore + NMS + conversion, results to host ---------------------
 // n_set > 1: image v of the batch is frame v / n_tpl x member v % n_tpl of the current group, written to the caller's
-// [frame][set index][cap] layout
-int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride, fpm_result* out, int cap, int* n_out, int n_set = 1)
+// [frame][set index][cap] layout, or (md) to the device lists of the merge
+int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride, fpm_result* out, int cap, int* n_out, int n_set = 1,
+              const MergeDev* md = nullptr)
 {
     key_stride = std::max(key_stride, 1);
     int ks = 1;
@@ -1143,9 +1163,12 @@ int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride
     const int pair_cap = std::min(ks, 512);                 // all-pairs NMS matrix for up to 512 survivors per frame
     CK(h->d_pairs.ensure((size_t)batch * pair_cap * pair_cap));
     const int rcap = std::max(cap, 1);
-    CK(h->d_results.ensure((size_t)batch * rcap * sizeof(FpmResultDev)));
-    CK(h->d_rescnt.ensure((size_t)batch * sizeof(int)));
-    CK(h->h_results.ensure((size_t)batch * rcap * sizeof(FpmResultDev) + (size_t)batch * sizeof(int)));
+    if (!md) {
+        CK(h->d_results.ensure((size_t)batch * rcap * sizeof(FpmResultDev)));
+        CK(h->d_rescnt.ensure((size_t)batch * sizeof(int)));
+        CK(h->h_results.ensure((size_t)batch * rcap * sizeof(FpmResultDev) + (size_t)batch * sizeof(int)));
+    }
+    const int n_tpl = std::max((int)h->members.size(), 1);
     // NMS rectangle size: pyramid[iStopLayer] * (iStopLayer == 0 ? 1 : 2)  (src/TemplateMatcher.cpp:376-377)
     const int stop_l = std::min(h->stop_layer1 ? 1 : 0, (int)h->tpl.size() - 1);
     const int nms_w = h->tpl[stop_l].w * (h->stop_layer1 ? 2 : 1), nms_h = h->tpl[stop_l].h * (h->stop_layer1 ? 2 : 1);
@@ -1155,7 +1178,15 @@ int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride
                                                              h->d_keys.as<unsigned long long>(), ks, h->d_rects.as<FpmRRect>(),
                                                              h->d_del.as<int>(), h->d_idmap.as<int>(),
                                                              h->d_pairs.as<unsigned char>(), pair_cap, h->mfc_compat, h->max_pos,
-                                                             h->d_results.as<FpmResultDev>(), rcap, h->d_rescnt.as<int>()));
+                                                             md ? md->lists : h->d_results.as<FpmResultDev>(),
+                                                             md ? md->lcap : rcap, md ? md->counts : h->d_rescnt.as<int>(),
+                                                             md ? md->rows : nullptr, n_tpl, n_set));
+    if (md) {                                                 // no copy, no synchronise: the merge reads the lists
+        if (h->err_check_pending)
+            CK(cudaMemcpyAsync(md->err, h->d_counters.as<int>() + CNT_ERR, sizeof(int), cudaMemcpyDeviceToDevice, h->stream));
+        h->err_check_pending = false;
+        return FPM_OK;
+    }
     FpmResultDev* hr = h->h_results.as<FpmResultDev>();
     int* hn = reinterpret_cast<int*>(hr + (size_t)batch * rcap);
     int* hc = h->h_counts.as<int>();
@@ -1166,7 +1197,6 @@ int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride
     CK(cudaMemcpyAsync(hr, h->d_results.p, (size_t)batch * rcap * sizeof(FpmResultDev), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     if (check_err && hc[CNT_ERR]) { h->err = "fpm_corr_warp_kernel: source box larger than its staging buffer"; return FPM_ERR_LIMIT; }
-    const int n_tpl = std::max((int)h->members.size(), 1);
     for (int b = 0; b < batch; b++) {
         const size_t slot = n_set == 1 ? (size_t)b : (size_t)(b / n_tpl) * n_set + h->members[b % n_tpl];
         n_out[slot] = hn[b];
@@ -1245,7 +1275,7 @@ int ensure_learned_for_mra(fpm_handle* h)
 }
 
 // one group's pass over the pyramid of the batch: virtual images v = frame * n_tpl + member
-int match_group(fpm_handle* h, int batch, fpm_result* out, int cap, int* n_out, int n_set)
+int match_group(fpm_handle* h, int batch, fpm_result* out, int cap, int* n_out, int n_set, const MergeDev* md)
 {
     const int top = (int)h->tpl.size() - 1;
     const int n_tpl = std::max((int)h->members.size(), 1), vbatch = batch * n_tpl;
@@ -1268,17 +1298,93 @@ int match_group(fpm_handle* h, int batch, fpm_result* out, int cap, int* n_out, 
     rc = run_refine(h, top, n_cands, &n_refined);
     if (rc) return rc;
     FpmRefinedView rv{h->d_refined.as<FpmRefined>(), h->d_counters.as<int>() + CNT_REFINED, 0, 1, 0};
-    return run_final(h, vbatch, rv, cand_stride, out, cap, n_out, n_set);
+    return run_final(h, vbatch, rv, cand_stride, out, cap, n_out, n_set, md);
 }
 
-// whole match() over a device-resident batch, for every template of the set: frame b / template t at out + (b * n + t) * cap.
+// merged set results (fpm_match_set_batch_merged): the caller's outputs besides out / counts, which then hold one list and
+// one count per frame
+struct SetMerge {
+    double max_overlap;
+    int* labels;                   // [frame][cap]
+    int* set_counts;               // [frame][n_set], or nullptr
+    SetMerge shifted(int frames, int cap, int n_set) const
+    {
+        return SetMerge{max_overlap, labels + (size_t)frames * cap, set_counts ? set_counts + (size_t)frames * n_set : nullptr};
+    }
+};
+
+// d_merged, read back in one copy: int counts[batch] | int set_counts[batch][n_set] | int labels[batch][ocap] |
+// int err[n_groups] (CNT_ERR of each group) | FpmResultDev records[batch][ocap] at a 256-byte aligned offset
+struct MergedLayout {
+    size_t set_counts, labels, err;   // int offsets
+    size_t header_bytes, rec_off, bytes;
+    MergedLayout(int batch, int n_set, int ocap, int n_groups)
+    {
+        set_counts = (size_t)batch;
+        labels = set_counts + (size_t)batch * n_set;
+        err = labels + (size_t)batch * ocap;
+        header_bytes = (err + n_groups) * sizeof(int);
+        rec_off = align_up(header_bytes, 256);
+        bytes = rec_off + (size_t)batch * ocap * sizeof(FpmResultDev);
+    }
+};
+
+// fpm_set_merge_kernel over the lists the groups left in d_mlists, then ONE read-back of everything (merged counts, the
+// per-template totals, labels, CNT_ERR slots, records) and one synchronise
+int run_set_merge(fpm_handle* h, int batch, int n_set, int n_groups, const MergeDev& md, const SetMerge* mg, fpm_result* out,
+                  int cap, int* n_out)
+{
+    const int ocap = md.ocap;
+    const MergedLayout lay(batch, n_set, ocap, n_groups);
+    int ks = 1;
+    while (ks < n_set * md.lcap) ks <<= 1;
+    CK(h->d_keys.ensure((size_t)batch * ks * sizeof(unsigned long long)));
+    CK(h->d_rects.ensure((size_t)batch * ks * sizeof(FpmRRect)));
+    CK(h->d_del.ensure((size_t)batch * ks * sizeof(int)));
+    CK(h->d_idmap.ensure((size_t)batch * ks * sizeof(int)));
+    int* d_counts = h->d_merged.as<int>();
+    int* d_labels = d_counts + lay.labels;
+    FpmResultDev* d_rec = reinterpret_cast<FpmResultDev*>(h->d_merged.as<char>() + lay.rec_off);
+    KL(K_SET_MERGE, (double)batch * n_set * md.lcap,
+       fpm_set_merge_kernel<<<batch, FN_THREADS, 0, h->stream>>>(md.lists, md.counts, n_set, md.lcap, mg->max_overlap,
+                                                                  h->d_keys.as<unsigned long long>(), ks, h->d_rects.as<FpmRRect>(),
+                                                                  h->d_del.as<int>(), h->d_idmap.as<int>(), d_rec, d_labels, ocap,
+                                                                  d_counts));
+    CK(h->h_results.ensure(lay.bytes));
+    CK(cudaMemcpyAsync(h->h_results.p, h->d_merged.p, lay.bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const int* hh = h->h_results.as<int>();
+    const int* h_labels = hh + lay.labels;
+    for (int g = 0; g < n_groups; g++)
+        if (hh[lay.err + g]) { h->err = "fpm_corr_warp_kernel: source box larger than its staging buffer"; return FPM_ERR_LIMIT; }
+    const FpmResultDev* h_rec = reinterpret_cast<const FpmResultDev*>(h->h_results.as<char>() + lay.rec_off);
+    for (int b = 0; b < batch; b++) {
+        n_out[b] = hh[b];
+        if (mg->set_counts)
+            for (int t = 0; t < n_set; t++) mg->set_counts[(size_t)b * n_set + t] = hh[lay.set_counts + (size_t)b * n_set + t];
+        const int m = std::min(hh[b], cap);
+        for (int i = 0; i < m; i++) {
+            const FpmResultDev& r = h_rec[(size_t)b * ocap + i];
+            fpm_result& o = out[(size_t)b * cap + i];
+            o.score = r.score; o.angle = r.angle; o.cx = r.cx; o.cy = r.cy;
+            o.ltx = r.ltx; o.lty = r.lty; o.rtx = r.rtx; o.rty = r.rty;
+            o.rbx = r.rbx; o.rby = r.rby; o.lbx = r.lbx; o.lby = r.lby;
+            mg->labels[(size_t)b * cap + i] = h_labels[(size_t)b * ocap + i];
+        }
+    }
+    return FPM_OK;
+}
+
+// whole match() over a device-resident batch, for every template of the set: frame b / template t at out + (b * n + t) * cap,
+// or (mg) the merged list of frame b at out + b * cap.
 // The source pyramid (and bitwise_not) is built once, down to the deepest top layer of any group; the groups run one
 // after another on the handle's stream.
 int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt, int stride, size_t frame_stride,
-                 fpm_result* out, int cap, int* n_out)
+                 fpm_result* out, int cap, int* n_out, const SetMerge* mg = nullptr)
 {
     const int n_set = std::max((int)h->set.size(), 1);
-    for (int b = 0; b < batch * n_set; b++) n_out[b] = 0;
+    for (int b = 0; b < batch * (mg ? 1 : n_set); b++) n_out[b] = 0;
+    if (mg && mg->set_counts) std::fill(mg->set_counts, mg->set_counts + (size_t)batch * n_set, 0);
     if (!h->learned) return FPM_OK;                          // :99-101 -> empty
     int rc = ensure_learned_for_mra(h);
     if (rc) return rc;
@@ -1307,11 +1413,39 @@ int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt,
     }
     rc = build_pyramid(h, d_src, batch, w, hgt, stride, frame_stride, max_top);
     if (rc) return rc;
+    MergeDev md;
+    if (mg) {
+        // list capacity: a group's list of a frame never exceeds its candidate list, n_angles * (MaxPos + 5) entries
+        int longest = 0;
+        for (size_t g = 0; g < n_groups; g++) {
+            if (!run[g]) continue;
+            GroupScope scope(h, g);
+            if ((rc = make_top_plan(h, (int)h->tpl.size() - 1, batch))) return rc;
+            longest = std::max(longest, h->plan.n_ang * (h->max_pos + FPM_MATCH_CANDIDATE_NUM));
+        }
+        md.lcap = std::min(cap, longest);
+        if ((long long)n_set * md.lcap >= (1ll << 30)) { h->err = "merged set results: n_set * list capacity too large"; return FPM_ERR_LIMIT; }
+        md.ocap = std::min(cap, n_set * md.lcap);
+        const MergedLayout lay(batch, n_set, md.ocap, (int)n_groups);
+        CK(h->d_mlists.ensure((size_t)batch * n_set * std::max(md.lcap, 1) * sizeof(FpmResultDev)));
+        CK(h->d_merged.ensure(lay.bytes));
+        CK(cudaMemsetAsync(h->d_merged.p, 0, lay.header_bytes, h->stream));   // the totals of groups that do not run, the CNT_ERR slots
+        md.lists = h->d_mlists.as<FpmResultDev>();
+        md.counts = h->d_merged.as<int>() + lay.set_counts;
+        md.err = h->d_merged.as<int>() + lay.err;
+    }
+    int* err_slots = md.err;
+    size_t member_off = 0;
     for (size_t g = 0; g < n_groups && rc == FPM_OK; g++) {
+        const size_t n_members = g == 0 ? h->members.size() : h->groups[g].members.size();
+        md.rows = h->d_members.as<int>() + member_off;
+        md.err = err_slots ? err_slots + g : nullptr;
+        member_off += n_members;
         if (!run[g]) continue;
         GroupScope scope(h, g);
-        rc = match_group(h, batch, out, cap, n_out, n_set);
+        rc = match_group(h, batch, out, cap, n_out, n_set, mg ? &md : nullptr);
     }
+    if (rc == FPM_OK && mg) rc = run_set_merge(h, batch, n_set, (int)n_groups, md, mg, out, cap, n_out);
     return rc;
 }
 
@@ -1534,7 +1668,7 @@ void fpm_destroy(fpm_handle* h)
                       &h->d_jobs_top, &h->d_angles, &h->d_ftx, &h->d_fty, &h->d_off, &h->d_keys, &h->d_cand[0], &h->d_cand[1],
                       &h->d_candcnt, &h->d_toppt, &h->d_counters, &h->d_jobs_ref, &h->d_roi, &h->d_rowsum, &h->d_rowS, &h->d_rowQ,
                       &h->d_pairs, &h->d_refined, &h->d_rects, &h->d_del, &h->d_idmap, &h->d_results, &h->d_rescnt, &h->d_trace, &h->d_trace_sc,
-                      &h->d_dbg[0], &h->d_dbg[1], &h->d_dbg[2], &h->d_dbg[3]};
+                      &h->d_dbg[0], &h->d_dbg[1], &h->d_dbg[2], &h->d_dbg[3], &h->d_members, &h->d_mlists, &h->d_merged};
     for (DevBuf* b : bufs) b->release();
     for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
     h->d_tstat.release();
@@ -1701,13 +1835,14 @@ int ensure_twin(fpm_handle* h)
 }
 
 namespace {
-// fpm_match_batch_device for the whole set: frame b / template t at out + (b * n_set + t) * cap
+// fpm_match_batch_device for the whole set: frame b / template t at out + (b * n_set + t) * cap, or (mg) frame b's merged
+// list at out + b * cap
 int match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width, int height, int stride,
-                       size_t frame_stride, fpm_result* out, int cap, int* n)
+                       size_t frame_stride, fpm_result* out, int cap, int* n, const SetMerge* mg = nullptr)
 {
-    const int n_set = std::max((int)h->set.size(), 1);
+    const int n_set = std::max((int)h->set.size(), 1), n_rows = mg ? 1 : n_set;
     if (!n || batch < 0 || cap < 0 || (cap > 0 && !out)) { h->err = "bad output arguments"; return FPM_ERR_INVALID; }
-    for (int b = 0; b < batch * n_set; b++) n[b] = 0;
+    for (int b = 0; b < batch * n_rows; b++) n[b] = 0;
     if (!d_src || width <= 0 || height <= 0 || batch == 0) return FPM_OK;       // empty source -> empty result
     if (stride < width) { h->err = "stride < width"; return FPM_ERR_INVALID; }
     CK(cudaSetDevice(h->device));
@@ -1722,15 +1857,16 @@ int match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width
         if (rc) return rc;
         const int b0 = batch / 2;
         int rc2 = FPM_OK;
+        const SetMerge mg2 = mg ? mg->shifted(b0, cap, n_set) : SetMerge{};
         std::thread second([&]() {
             rc2 = match_batch_device(h->twin, d_src + (size_t)b0 * frame_stride, batch - b0, width, height, stride, frame_stride,
-                                     out + (size_t)b0 * n_set * cap, cap, n + (size_t)b0 * n_set);
+                                     out + (size_t)b0 * n_rows * cap, cap, n + (size_t)b0 * n_rows, mg ? &mg2 : nullptr);
         });
-        rc = match_device(h, d_src, b0, width, height, stride, frame_stride, out, cap, n);
+        rc = match_device(h, d_src, b0, width, height, stride, frame_stride, out, cap, n, mg);
         second.join();
         if (rc == FPM_OK && rc2 != FPM_OK) { rc = rc2; h->err = h->twin->err; }
     } else {
-        rc = match_device(h, d_src, batch, width, height, stride, frame_stride, out, cap, n);
+        rc = match_device(h, d_src, batch, width, height, stride, frame_stride, out, cap, n, mg);
     }
     prof_collect(h);
     auto t1 = std::chrono::high_resolution_clock::now();
@@ -1738,13 +1874,13 @@ int match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width
     return rc;
 }
 
-// fpm_match_batch for the whole set
+// fpm_match_batch for the whole set (mg: merged, as in match_batch_device)
 int match_batch_host(fpm_handle* h, const uint8_t* src, int batch, int width, int height, int stride, size_t frame_stride,
-                     fpm_result* out, int cap, int* n)
+                     fpm_result* out, int cap, int* n, const SetMerge* mg = nullptr)
 {
-    const int n_set = std::max((int)h->set.size(), 1);
+    const int n_set = std::max((int)h->set.size(), 1), n_rows = mg ? 1 : n_set;
     if (!n || batch < 0 || cap < 0 || (cap > 0 && !out)) { h->err = "bad output arguments"; return FPM_ERR_INVALID; }
-    for (int b = 0; b < batch * n_set; b++) n[b] = 0;
+    for (int b = 0; b < batch * n_rows; b++) n[b] = 0;
     if (!src || width <= 0 || height <= 0 || batch == 0) return FPM_OK;
     if (stride < width) { h->err = "stride < width"; return FPM_ERR_INVALID; }
     CK(cudaSetDevice(h->device));
@@ -1802,8 +1938,9 @@ int match_batch_host(fpm_handle* h, const uint8_t* src, int batch, int width, in
         if (k + 1 < nchunks && (ce = enqueue_copy(k + 1)) != cudaSuccess) return fail_cuda("host->device copy", ce);
         if ((ce = cudaStreamWaitEvent(h->stream, h->ev_copy[k & 1], 0)) != cudaSuccess) return fail_cuda("cudaStreamWaitEvent", ce);
         int b0 = k * chunk, nb = std::min(chunk, batch - b0);
+        const SetMerge mgk = mg ? mg->shifted(b0, cap, n_set) : SetMerge{};
         rc = match_device(h, h->d_src.as<uint8_t>() + (size_t)(k & 1) * buf_bytes, nb, width, height, pitch, img,
-                          out + (size_t)b0 * n_set * cap, cap, n + (size_t)b0 * n_set);
+                          out + (size_t)b0 * n_rows * cap, cap, n + (size_t)b0 * n_rows, mg ? &mgk : nullptr);
         if (rc == FPM_OK && (ce = cudaEventRecord(h->ev_done[k & 1], h->stream)) != cudaSuccess) return fail_cuda("cudaEventRecord", ce);
         prof_collect(h);
     }
@@ -1838,6 +1975,20 @@ int fpm_match_set_batch(fpm_handle* h, const uint8_t* src, int src_on_device, in
     if (h->trace && fpm_set_size(h) > 1) { h->err = "fpm_match_set_batch: FPM_PARAM_TRACE is not supported for a set of more than one template"; return FPM_ERR_INVALID; }
     return src_on_device ? match_batch_device(h, src, batch, width, height, stride, frame_stride, out, cap, counts)
                          : match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, counts);
+}
+
+int fpm_match_set_batch_merged(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                               size_t frame_stride, double max_overlap, fpm_result* out, int* labels, int cap, int* counts,
+                               int* set_counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (h->trace && fpm_set_size(h) > 1) { h->err = "fpm_match_set_batch_merged: FPM_PARAM_TRACE is not supported for a set of more than one template"; return FPM_ERR_INVALID; }
+    if (!std::isfinite(max_overlap)) { h->err = "fpm_match_set_batch_merged: max_overlap must be finite"; return FPM_ERR_INVALID; }
+    if (cap > 0 && !labels) { h->err = "fpm_match_set_batch_merged: labels is NULL while cap > 0"; return FPM_ERR_INVALID; }
+    if (set_counts && batch > 0) std::fill(set_counts, set_counts + (size_t)batch * std::max(fpm_set_size(h), 1), 0);
+    const SetMerge mg{max_overlap, labels, set_counts};
+    return src_on_device ? match_batch_device(h, src, batch, width, height, stride, frame_stride, out, cap, counts, &mg)
+                         : match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, counts, &mg);
 }
 
 int fpm_match(fpm_handle* h, const uint8_t* src, int width, int height, int stride, fpm_result* out, int cap, int* n)
@@ -2692,6 +2843,15 @@ int fpm_match_ingested_set_batch(fpm_handle* h, fpm_result* out, int cap, int* c
     if (h->ingest_count <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
     return fpm_match_set_batch(h, h->d_ingest.as<uint8_t>(), 1, h->ingest_count, h->ingest_w, h->ingest_h, h->ingest_pitch,
                                (size_t)h->ingest_pitch * h->ingest_h, out, cap, counts);
+}
+
+int fpm_match_ingested_set_batch_merged(fpm_handle* h, double max_overlap, fpm_result* out, int* labels, int cap, int* counts,
+                                        int* set_counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (h->ingest_count <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
+    return fpm_match_set_batch_merged(h, h->d_ingest.as<uint8_t>(), 1, h->ingest_count, h->ingest_w, h->ingest_h, h->ingest_pitch,
+                                      (size_t)h->ingest_pitch * h->ingest_h, max_overlap, out, labels, cap, counts, set_counts);
 }
 
 int fpm_learn_ingested(fpm_handle* h)

@@ -1714,15 +1714,88 @@ __device__ __forceinline__ bool fpm_refined_valid(const FpmRefinedView& v, int i
     return k < *reinterpret_cast<const int*>(blk + (size_t)v.seg_cap * sizeof(FpmRefined));
 }
 
+struct FpmNoGroup { __device__ __forceinline__ int operator()(int) const { return -1; } };
+
+// Greedy rotated-rectangle NMS of one CTA over rects[0, m), sorted by score descending: entry k is dropped when an earlier
+// kept entry i gives fpm_rrect_overlap_decision(rects[i], rects[k], max_overlap) (the ratio over the kept rectangle's area);
+// entries of one group (group(i) >= 0, the same for both) are never decided against each other.  bits (m <= FN_PAIR_MAX): the kept entries are left as bit words,
+// s_kept[w] with s_base[w] survivors before word w and s_base[FN_PAIR_MAX / 32] survivors in all; otherwise del[k] = 1 marks
+// the dropped entries (del[0, m) zero on entry).  Ends with the CTA synchronised.
+template <class Group>
+__device__ __forceinline__ void fpm_greedy_nms(const FpmRRect* __restrict__ rects, int* __restrict__ del, int m, bool bits,
+                                               double max_overlap, Group group, unsigned* s_bits, unsigned* s_kept, int* s_base)
+{
+    const int tid = threadIdx.x;
+    // Small sets: all pair decisions are evaluated in parallel first (the geometry is the expensive,
+    // latency-bound part), then the greedy pass only reads the byte matrix.
+    if (bits) {
+        // Pair decisions as bit rows in shared memory (row i, bit k = "k must go if i stays"): a warp per row, one
+        // ballot per 32 columns.  The greedy pass is then a chain of register / shared-memory operations in ONE warp
+        // (lane l keeps the deletion bits of survivors 32 l .. 32 l + 31) instead of a chain of global-memory round trips.
+        const int nw = (m + 31) >> 5;
+        const int lane = tid & 31;
+        for (int i = tid >> 5; i < m; i += FN_THREADS / 32) {
+            const FpmRRect ri = rects[i];
+            const int gi = group(i);
+            for (int j = 0; j < nw; j++) {
+                bool hit = false;
+                const int k = 32 * j + lane;
+                if (k > i && k < m) {
+                    const FpmRRect rk = rects[k];
+                    hit = !(gi >= 0 && group(k) == gi) && !fpm_rrect_far(ri, rk) && fpm_rrect_overlap_decision(ri, rk, max_overlap, nullptr, nullptr);
+                }
+                const unsigned w = __ballot_sync(0xffffffffu, hit);
+                if (lane == 0) s_bits[i * (FN_PAIR_MAX / 32) + j] = w;
+            }
+        }
+        __syncthreads();
+        if (tid < 32) {
+            unsigned dw = 0;
+            for (int i = 0; i < m - 1; i++) {
+                const unsigned wi = __shfl_sync(0xffffffffu, dw, i >> 5);
+                if (!((wi >> (i & 31)) & 1u) && lane < nw) dw |= s_bits[i * (FN_PAIR_MAX / 32) + lane];
+            }
+            // survivors and their ranks straight from the bit words: exclusive prefix of the per-word counts
+            const int left = m - 32 * lane;
+            const unsigned valid = lane < nw ? (left >= 32 ? 0xffffffffu : ((1u << left) - 1u)) : 0u;
+            const unsigned kept = ~dw & valid;
+            int incl = __popc(kept);
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const int t = __shfl_up_sync(0xffffffffu, incl, o);
+                if (lane >= o) incl += t;
+            }
+            if (lane < FN_PAIR_MAX / 32) { s_kept[lane] = kept; s_base[lane] = incl - __popc(kept); }
+            if (lane == 31) s_base[FN_PAIR_MAX / 32] = incl;          // total survivors
+        }
+        __syncthreads();
+    } else {
+        for (int i = 0; i < m - 1; i++) {
+            if (!del[i]) {
+                const FpmRRect ri = rects[i];
+                const int gi = group(i);
+                for (int k = i + 1 + tid; k < m; k += FN_THREADS)
+                    if (!del[k] && !(gi >= 0 && group(k) == gi) && !fpm_rrect_far(ri, rects[k]) &&
+                        fpm_rrect_overlap_decision(ri, rects[k], max_overlap, nullptr, nullptr))
+                        del[k] = 1;
+            }
+            __syncthreads();
+        }
+    }
+}
+
 __global__ void __launch_bounds__(FN_THREADS)
 fpm_final_kernel(FpmRefinedView rv,
                  double score_thresh, double max_overlap, int nms_w, int nms_h, int tpl_w, int tpl_h,
                  unsigned long long* __restrict__ key_scratch, int key_stride,
                  FpmRRect* __restrict__ rect_scratch, int* __restrict__ del_scratch,
                  int* __restrict__ idmap_scratch, unsigned char* __restrict__ pair_scratch, int pair_cap,
-                 int mfc_compat, int max_pos, FpmResultDev* __restrict__ results, int result_cap, int* __restrict__ result_count)
+                 int mfc_compat, int max_pos, FpmResultDev* __restrict__ results, int result_cap, int* __restrict__ result_count,
+                 const int* __restrict__ row_members, int n_tpl, int n_set)
 {
     const int img = blockIdx.x, tid = threadIdx.x;
+    // output row of the image: itself, or (row_members: a group of a template set) frame img / n_tpl x set index
+    const int row = row_members ? (img / n_tpl) * n_set + row_members[img % n_tpl] : img;
     const int n_total = fpm_refined_slots(rv);
     // sort keys in shared memory when the per-frame capacity allows (a bitonic sort in global memory pays one L2 round
     // trip per stage)
@@ -1735,7 +1808,6 @@ fpm_final_kernel(FpmRefinedView rv,
     __shared__ unsigned s_bits[FN_PAIR_MAX * (FN_PAIR_MAX / 32)];     // 32 KB: pair-decision bit rows of the NMS
     __shared__ unsigned s_kept[FN_PAIR_MAX / 32];
     __shared__ int s_base[FN_PAIR_MAX / 32 + 1];
-    bool bit_path = false;
     if (tid == 0) s_n = 0;
     __syncthreads();
     for (int i = tid; i < n_total; i += FN_THREADS)
@@ -1771,61 +1843,8 @@ fpm_final_kernel(FpmRefinedView rv,
     }
     __syncthreads();
     // filterWithRotatedRect: scores are sorted descending so the later index always loses.
-    // Small sets: all pair decisions are evaluated in parallel first (the geometry is the expensive,
-    // latency-bound part), then the greedy pass only reads the byte matrix.
-    if (m <= pair_cap && m <= FN_PAIR_MAX) {
-        // Pair decisions as bit rows in shared memory (row i, bit k = "k must go if i stays"): a warp per row, one
-        // ballot per 32 columns.  The greedy pass is then a chain of register / shared-memory operations in ONE warp
-        // (lane l keeps the deletion bits of survivors 32 l .. 32 l + 31) instead of a chain of global-memory round trips.
-        const int nw = (m + 31) >> 5;
-        const int lane = tid & 31;
-        for (int i = tid >> 5; i < m; i += FN_THREADS / 32) {
-            const FpmRRect ri = rects[i];
-            for (int j = 0; j < nw; j++) {
-                bool hit = false;
-                const int k = 32 * j + lane;
-                if (k > i && k < m) {
-                    const FpmRRect rk = rects[k];
-                    hit = !fpm_rrect_far(ri, rk) && fpm_rrect_overlap_decision(ri, rk, max_overlap, nullptr, nullptr);
-                }
-                const unsigned w = __ballot_sync(0xffffffffu, hit);
-                if (lane == 0) s_bits[i * (FN_PAIR_MAX / 32) + j] = w;
-            }
-        }
-        __syncthreads();
-        if (tid < 32) {
-            unsigned dw = 0;
-            for (int i = 0; i < m - 1; i++) {
-                const unsigned wi = __shfl_sync(0xffffffffu, dw, i >> 5);
-                if (!((wi >> (i & 31)) & 1u) && lane < nw) dw |= s_bits[i * (FN_PAIR_MAX / 32) + lane];
-            }
-            // survivors and their ranks straight from the bit words: exclusive prefix of the per-word counts
-            const int left = m - 32 * lane;
-            const unsigned valid = lane < nw ? (left >= 32 ? 0xffffffffu : ((1u << left) - 1u)) : 0u;
-            const unsigned kept = ~dw & valid;
-            int incl = __popc(kept);
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const int t = __shfl_up_sync(0xffffffffu, incl, o);
-                if (lane >= o) incl += t;
-            }
-            if (lane < FN_PAIR_MAX / 32) { s_kept[lane] = kept; s_base[lane] = incl - __popc(kept); }
-            if (lane == 31) s_base[FN_PAIR_MAX / 32] = incl;          // total survivors
-        }
-        bit_path = true;
-        __syncthreads();
-    } else {
-        for (int i = 0; i < m - 1; i++) {
-            if (!del[i]) {
-                const FpmRRect ri = rects[i];
-                for (int k = i + 1 + tid; k < m; k += FN_THREADS)
-                    if (!del[k] && !fpm_rrect_far(ri, rects[k]) &&
-                        fpm_rrect_overlap_decision(ri, rects[k], max_overlap, nullptr, nullptr))
-                        del[k] = 1;
-            }
-            __syncthreads();
-        }
-    }
+    const bool bit_path = m <= pair_cap && m <= FN_PAIR_MAX;
+    fpm_greedy_nms(rects, del, m, bit_path, max_overlap, FpmNoGroup(), s_bits, s_kept, s_base);
     // survivor ranks (from the bit words, or by one thread on the large-set path: idmap is free again and holds
     // the rank of record i, or -1), conversion by all threads
     if (!bit_path) {
@@ -1836,12 +1855,12 @@ fpm_final_kernel(FpmRefinedView rv,
                 idmap[i] = keep ? cnt : -1;
                 if (keep) cnt++;
             }
-            result_count[img] = cnt;
+            result_count[row] = cnt;
         }
         __syncthreads();
     } else if (tid == 0) {
         const int total = s_base[FN_PAIR_MAX / 32];
-        result_count[img] = (mfc_compat && total > max_pos) ? max_pos : total;
+        result_count[row] = (mfc_compat && total > max_pos) ? max_pos : total;
     }
     for (int i = tid; i < m; i += FN_THREADS) {
         int rank;
@@ -1880,6 +1899,100 @@ fpm_final_kernel(FpmRefinedView rv,
             if (ang > 180) ang -= 360;
             o.angle = ang;
         }
-        results[(size_t)img * result_cap + rank] = o;
+        results[(size_t)row * result_cap + rank] = o;
     }
+}
+
+// =====================================================================================
+// K10  template sets, merged results: one CTA per frame b merges the frame's n_set per-template lists (template t: the
+// first min(counts[b*n_set + t], lcap) records of lists + (b*n_set + t)*lcap) into one list.  Order: score descending,
+// ties to the lower template, then the lower position (the sort key's low word t*lcap + i).  Greedy NMS across
+// templates only (pairs of one template were decided by its own NMS): rectangles from three corners of the records.
+// The kept records go to out[b*out_cap + k] unchanged, their set index to out_labels, their number to out_count[b].
+// =====================================================================================
+struct FpmLabelOf {
+    const int* lab;
+    __device__ __forceinline__ int operator()(int i) const { return lab[i]; }
+};
+
+// one frame of fpm_set_merge_kernel, m entries; inlined once with keys in shared and once in global memory, so that every
+// key access has a known address space
+__device__ __forceinline__ void fpm_set_merge_frame(unsigned long long* __restrict__ keys, int m, const FpmResultDev* __restrict__ fl,
+                                                    const int* __restrict__ fc, int n_set, int lcap, double max_overlap,
+                                                    FpmRRect* __restrict__ rects, int* __restrict__ del, int* __restrict__ lab,
+                                                    unsigned* s_bits, unsigned* s_kept, int* s_base, FpmResultDev* __restrict__ out,
+                                                    int* __restrict__ out_labels, int out_cap, int* __restrict__ out_count)
+{
+    const int tid = threadIdx.x;
+    int n_pad = 1;
+    while (n_pad < m) n_pad <<= 1;
+    for (int t = 0, off = 0; t < n_set; t++) {
+        const int take = min(fc[t], lcap);
+        for (int i = tid; i < take; i += FN_THREADS) {
+            const uint32_t e = (uint32_t)(t * lcap + i);
+            keys[off + i] = ((unsigned long long)fpm_desc_key((float)fl[e].score) << 32) | e;
+        }
+        off += take;
+    }
+    for (int i = m + tid; i < n_pad; i += FN_THREADS) keys[i] = ~0ull;
+    __syncthreads();
+    fpm_bitonic_sort(keys, n_pad, tid, FN_THREADS);
+    for (int i = tid; i < m; i += FN_THREADS) {
+        const uint32_t e = (uint32_t)keys[i];
+        const FpmResultDev& r = fl[e];
+        rects[i] = fpm_rrect_from3((float)r.ltx, (float)r.lty, (float)r.rtx, (float)r.rty, (float)r.rbx, (float)r.rby);
+        lab[i] = (int)(e / (uint32_t)lcap);
+        del[i] = 0;
+    }
+    __syncthreads();
+    const bool bits = m <= FN_PAIR_MAX;
+    fpm_greedy_nms(rects, del, m, bits, max_overlap, FpmLabelOf{lab}, s_bits, s_kept, s_base);
+    if (!bits) {
+        if (tid == 0) {                                         // del[i] becomes the rank of entry i, or -1
+            int cnt = 0;
+            for (int i = 0; i < m; i++) del[i] = del[i] ? -1 : cnt++;
+            *out_count = cnt;
+        }
+        __syncthreads();
+    } else if (tid == 0) {
+        *out_count = s_base[FN_PAIR_MAX / 32];
+    }
+    for (int i = tid; i < m; i += FN_THREADS) {
+        int rank;
+        if (bits) {
+            const unsigned kw = s_kept[i >> 5];
+            rank = ((kw >> (i & 31)) & 1u) ? s_base[i >> 5] + __popc(kw & ((1u << (i & 31)) - 1u)) : -1;
+        } else {
+            rank = del[i];
+        }
+        if (rank < 0 || rank >= out_cap) continue;
+        out[rank] = fl[(uint32_t)keys[i]];
+        out_labels[rank] = lab[i];
+    }
+}
+
+__global__ void __launch_bounds__(FN_THREADS)
+fpm_set_merge_kernel(const FpmResultDev* __restrict__ lists, const int* __restrict__ counts, int n_set, int lcap, double max_overlap,
+                     unsigned long long* __restrict__ key_scratch, int key_stride, FpmRRect* __restrict__ rect_scratch,
+                     int* __restrict__ del_scratch, int* __restrict__ lab_scratch,
+                     FpmResultDev* __restrict__ out, int* __restrict__ out_labels, int out_cap, int* __restrict__ out_count)
+{
+    const int b = blockIdx.x;
+    __shared__ unsigned long long s_keys[FN_KEYS_SMEM];
+    __shared__ unsigned s_bits[FN_PAIR_MAX * (FN_PAIR_MAX / 32)];
+    __shared__ unsigned s_kept[FN_PAIR_MAX / 32];
+    __shared__ int s_base[FN_PAIR_MAX / 32 + 1];
+    const FpmResultDev* fl = lists + (size_t)b * n_set * lcap;
+    const int* fc = counts + (size_t)b * n_set;
+    int m = 0;
+    for (int t = 0; t < n_set; t++) m += min(fc[t], lcap);
+    FpmRRect* rects = rect_scratch + (size_t)b * key_stride;
+    int* del = del_scratch + (size_t)b * key_stride;
+    int* lab = lab_scratch + (size_t)b * key_stride;
+    if (m <= FN_KEYS_SMEM)
+        fpm_set_merge_frame(s_keys, m, fl, fc, n_set, lcap, max_overlap, rects, del, lab, s_bits, s_kept, s_base,
+                            out + (size_t)b * out_cap, out_labels + (size_t)b * out_cap, out_cap, out_count + b);
+    else
+        fpm_set_merge_frame(key_scratch + (size_t)b * key_stride, m, fl, fc, n_set, lcap, max_overlap, rects, del, lab, s_bits,
+                            s_kept, s_base, out + (size_t)b * out_cap, out_labels + (size_t)b * out_cap, out_cap, out_count + b);
 }

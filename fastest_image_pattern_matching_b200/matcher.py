@@ -190,6 +190,55 @@ class TemplateMatcher:
         self._check(self._lib.fpm_match_ingested_set_batch(self._h, res, cap, counts))
         return self._set_results(res, counts, B, T)
 
+    # ---- merged set results: one labelled list per frame, rotated-rectangle NMS across templates ----
+    def _merged_results(self, res, labels, counts, B):
+        cap = self.result_capacity
+        out = []
+        for b in range(B):
+            m = min(counts[b], cap)
+            out.append(list(zip(labels[b * cap:b * cap + m], _convert(res[b * cap:(b + 1) * cap], m))))
+        return out
+
+    def matchSetBatchMergedRaw(self, ptr: int, B: int, W: int, H: int, stride: int, frame_stride: int, on_device: bool,
+                               max_overlap: float, res=None, labels=None, counts=None, set_counts=None):
+        """Pointer-level merged set match (fpm_match_set_batch_merged): returns (results ctypes array [B][cap], labels [B][cap],
+        counts [B], set_counts [B][T]: the per-template totals)."""
+        cap, T = self.result_capacity, max(self.patternSetSize(), 1)
+        if res is None:
+            res = (L.fpm_result * (cap * B))()
+        if labels is None:
+            labels = (C.c_int * (cap * B))()
+        if counts is None:
+            counts = (C.c_int * B)()
+        if set_counts is None:
+            set_counts = (C.c_int * (B * T))()
+        self._check(self._lib.fpm_match_set_batch_merged(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride,
+                                                         float(max_overlap), res, labels, cap, counts, set_counts))
+        return res, labels, counts, set_counts
+
+    def matchSetBatchMerged(self, frames: np.ndarray, max_overlap: float) -> List[List[Tuple[int, SingleTargetMatch]]]:
+        """frames: [B, H, W] uint8 in host memory -> per frame one list of (set index, result), score descending, after NMS
+        across templates with the overlap threshold max_overlap (the per-template lists keep MaxOverlap)."""
+        f = np.asarray(frames)
+        if f.ndim != 3 or f.dtype != np.uint8 or f.strides[2] != 1:
+            raise FpmError("frames must be a [B,H,W] uint8 array with unit pixel stride")
+        B, H, W = f.shape
+        res, labels, counts, _ = self.matchSetBatchMergedRaw(f.ctypes.data, B, W, H, f.strides[1], f.strides[0], False, max_overlap)
+        return self._merged_results(res, labels, counts, B)
+
+    def matchSetMerged(self, sourceImage, max_overlap: float) -> List[Tuple[int, SingleTargetMatch]]:
+        """one host image -> [(set index, result)]"""
+        return self.matchSetBatchMerged(_as_u8_2d(sourceImage)[None], max_overlap)[0]
+
+    def matchIngestedSetBatchMerged(self, max_overlap: float) -> List[List[Tuple[int, SingleTargetMatch]]]:
+        """the frames of the last ingest x the set, merged: [frame][(set index, result)]"""
+        B, T, cap = self.ingestedCount(), max(self.patternSetSize(), 1), self.result_capacity
+        res = (L.fpm_result * (cap * max(B, 1)))()
+        labels = (C.c_int * (cap * max(B, 1)))()
+        counts = (C.c_int * max(B, 1))()
+        self._check(self._lib.fpm_match_ingested_set_batch_merged(self._h, float(max_overlap), res, labels, cap, counts, None))
+        return self._merged_results(res, labels, counts, B)
+
     # ---- match (src/TemplateMatcher.cpp:97-437) ----
     def match(self, sourceImage) -> List[SingleTargetMatch]:
         if sourceImage is None or np.asarray(sourceImage).size == 0:
@@ -674,13 +723,24 @@ class GlyphReader:
                 labels.append(ch)
         return ocr_assemble(centres, labels, line_tol), dict(zip(self.letters, per))
 
-    def readBatch(self, frames, line_tol: float = 10.0):
-        """frames: [B, H, W] uint8 (or a list of equally sized images) -> [(text, {letter: results})] per frame."""
+    def readBatch(self, frames, line_tol: float = 10.0, merge_overlap: Optional[float] = None):
+        """frames: [B, H, W] uint8 (or a list of equally sized images) -> [(text, {letter: results})] per frame.
+        merge_overlap: None reads every glyph's own list; a float merges the glyphs' lists of a frame with NMS across
+        glyphs at that overlap threshold (similar glyphs that hit the same cell, O/0/Q or 8/B, keep only the best) and
+        {letter: results} holds the survivors."""
         if self._set_matcher is None:
             self._set_matcher = self._new_matcher()
             self._set_matcher.learnPatternSet(self._templates)
         f = np.ascontiguousarray(np.stack([_as_u8_2d(x) for x in frames]) if isinstance(frames, (list, tuple)) else frames, np.uint8)
-        return [self._assemble(per, line_tol) for per in self._set_matcher.matchSetBatch(f)]
+        if merge_overlap is None:
+            return [self._assemble(per, line_tol) for per in self._set_matcher.matchSetBatch(f)]
+        out = []
+        for merged in self._set_matcher.matchSetBatchMerged(f, merge_overlap):
+            per = [[] for _ in self.letters]
+            for t, r in merged:
+                per[t].append(r)
+            out.append(self._assemble(per, line_tol))
+        return out
 
     def read(self, sourceImage, line_tol: float = 10.0):
         """Returns (text, {letter: [SingleTargetMatch, ...]})."""

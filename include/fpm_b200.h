@@ -111,6 +111,22 @@ int fpm_match_set_batch(fpm_handle* h, const uint8_t* src, int src_on_device, in
                         size_t frame_stride, fpm_result* out, int cap, int* counts);
 /* the frames left by the last ingest (fpm_ingest_jpeg_batch etc.) x the set */
 int fpm_match_ingested_set_batch(fpm_handle* h, fpm_result* out, int cap, int* counts);
+/* The same match with one labelled list per frame: the n lists L(b, t) fpm_match_set_batch writes for frame b with the same
+ * cap (their first min(count, cap) records) merged by score descending (ties: lower set index t, then lower position in
+ * L(b, t)) and greedy rotated-rectangle NMS across templates: an entry of template t is dropped when an earlier kept entry of
+ * a template t' != t overlaps it by more than max_overlap of the kept rectangle's area, or contains it (the rectangles come
+ * from the records' lt, rt and rb corners).  Entries of one template never suppress each other: a set of one merges to its
+ * own list.  max_overlap is this call's own threshold (any finite value; FPM_PARAM_MAX_OVERLAP stays the per-template one).
+ * Frame b's kept records, bit-identical to the per-template ones, go to out + b*cap and their set index to labels + b*cap
+ * (the first min(counts[b], cap)); counts[b] is their total.  set_counts (NULL: not written) gets the per-template totals
+ * fpm_match_set_batch reports, [b*n + t], so a caller can tell when cap cut an input list.  labels may be NULL only when
+ * cap = 0.  Refusals as fpm_match_set_batch's, and FPM_ERR_INVALID for a NaN or infinite max_overlap. */
+int fpm_match_set_batch_merged(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                               size_t frame_stride, double max_overlap, fpm_result* out, int* labels, int cap, int* counts,
+                               int* set_counts);
+/* the frames left by the last ingest x the set, merged as in fpm_match_set_batch_merged */
+int fpm_match_ingested_set_batch_merged(fpm_handle* h, double max_overlap, fpm_result* out, int* labels, int cap, int* counts,
+                                        int* set_counts);
 
 /* isPatternLearned / clearPattern (include/TemplateMatcher.h:43-46). */
 int fpm_is_learned(const fpm_handle* h);

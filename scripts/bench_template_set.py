@@ -2,10 +2,13 @@
   m12_read     one M12 read (36 glyphs on M12_D_Test): fpm_match_set_batch of one frame vs fpm_match_multi (p50, launches)
   m12_frames   64 seeded M12-like frames (shifted, noised), host-pinned and device-resident: one set call vs a loop of
                fpm_match_multi over the frames (images/s)
+  m12_merged   the same 64 frames at Score 0.7, device-resident and pinned: fpm_match_set_batch_merged (NMS across the glyphs
+               at overlap 0.3) vs fpm_match_set_batch (images/s), and the fpm_set_merge_kernel time of one profiled call
   rot128       8 templates of 128x128 at +-180 deg on 64 frames of 2048x1536 (device-resident): one set call (dp4a refinement)
                vs one handle per template (tensor cores where they apply)
 Every timing is a host clock around calls that end in a device synchronise, after warm-up.  Results of the two arms are
-checked equal.  Writes one JSON file (default profiles/template_set_b200.json) with the card name and power limit.
+checked equal; the merged lists of the first and last frame are checked against the host reference of the merge
+(tests/test_gpu_set_merge.py).  Writes one JSON file (default profiles/template_set_b200.json) with the card name and power limit.
     python scripts/bench_template_set.py [--out PATH] [--reps 20]"""
 import argparse
 import json
@@ -23,6 +26,7 @@ import fpm_workloads as synth  # noqa: E402
 from oracle import oracle as O  # noqa: E402
 from fastest_image_pattern_matching_b200 import TemplateMatcher, match_multi  # noqa: E402
 from tests.helpers import configure  # noqa: E402
+from tests.test_gpu_set_merge import merge_reference  # noqa: E402
 
 
 def card():
@@ -106,6 +110,29 @@ def main():
     ms = alternate(arms, max(3, a.reps // 4))
     out["m12_frames"] = {k + "_images_per_s": round(B / (float(np.median(v)) / 1e3), 1) for k, v in ms.items()}
     out["m12_frames"]["batch"] = B
+
+    # ---- merged set results: the same frames at Score 0.7, where similar glyphs hit the same character cells
+    s7 = configure(TemplateMatcher(0, result_capacity=256), dict(case["params"], score=0.7))
+    s7.learnPatternSet(glyphs)
+    rs7 = s7.matchSetBatchRaw(dev.data_ptr(), B, W, H, W, H * W, True)
+    rm7 = s7.matchSetBatchMergedRaw(dev.data_ptr(), B, W, H, W, H * W, True, 0.3)
+    T, cap = len(glyphs), 256
+    for b in (0, B - 1):                                     # the merged lists against the host reference of the merge
+        lists = [[rs7[0][(b * T + t) * cap + i] for i in range(min(rs7[1][b * T + t], cap))] for t in range(T)]
+        want = [(t, bytes(r)) for t, r in merge_reference(lists, 0.3)]
+        assert rm7[2][b] == len(want)
+        assert [(rm7[1][b * cap + k], bytes(rm7[0][b * cap + k])) for k in range(min(rm7[2][b], cap))] == want[:cap]
+    arms = {"set_device": lambda: s7.matchSetBatchRaw(dev.data_ptr(), B, W, H, W, H * W, True, *rs7),
+            "merged_device": lambda: s7.matchSetBatchMergedRaw(dev.data_ptr(), B, W, H, W, H * W, True, 0.3, *rm7),
+            "set_pinned": lambda: s7.matchSetBatchRaw(pinned.data_ptr(), B, W, H, W, H * W, False, *rs7),
+            "merged_pinned": lambda: s7.matchSetBatchMergedRaw(pinned.data_ptr(), B, W, H, W, H * W, False, 0.3, *rm7)}
+    ms = alternate(arms, a.reps)
+    out["m12_merged"] = {k + "_images_per_s": round(B / (float(np.median(v)) / 1e3), 1) for k, v in ms.items()}
+    out["m12_merged"].update(batch=B, score=0.7, merge_overlap=0.3, per_template_hits=int(sum(rs7[1])), merged_hits=int(sum(rm7[2])))
+    s7.setProfile(True); s7.profileReset()
+    s7.matchSetBatchMergedRaw(dev.data_ptr(), B, W, H, W, H * W, True, 0.3, *rm7)
+    out["m12_merged"]["merged_profile_ms"] = {k: round(v[0], 4) for k, v in s7.profile().items() if v[0] > 0}
+    s7.close()
     for m in singles:
         m.close()
 
