@@ -89,6 +89,10 @@ SIGNATURES = {
     "fpm_comm_destroy": (None, [_vp]),
     "fpm_match_sharded": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _pi]),
     "fpm_match_sharded_virtual": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _vp]),
+    "fpm_match_set_sharded": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _i, _vp]),
+    "fpm_match_set_sharded_merged": (_i, [_vp, _vp, _i, _i, _i, _i, _d, _vp, _vp, _i, _vp, _vp]),
+    "fpm_match_set_sharded_virtual": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _vp]),
+    "fpm_match_set_sharded_merged_virtual": (_i, [_vp, _i, _vp, _i, _i, _i, _d, _vp, _vp, _i, _vp, _vp]),
     "fpm_shard_angle_range": (_i, [_i, _i, _i, _pi, _pi]),
     "fpm_collective_count": (C.c_longlong, [_vp]),
     "fpm_dbg_pyrdown": (_i, [_vp, _vp, _i, _i, _i, _vp]),

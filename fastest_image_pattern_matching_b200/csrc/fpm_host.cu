@@ -228,7 +228,16 @@ struct fpm_handle {
     DevBuf d_gpicks, d_grefined;   // allgather buffers: one fixed-size block per rank, consumed in place by the kernels
     FpmRefined* ref_out = nullptr; // where run_refine appends (null: d_refined / counters[CNT_REFINED])
     int* ref_cnt = nullptr;
-    struct ShardState { int top = 0, chunk = 0, n_all = 0, n_local = 0, seg_cap = 0, empty = 1; size_t pick_blk = 0, ref_blk = 0; } sh;
+    // one call's layout of the rank blocks, the same on every rank: block = picks of every group that runs
+    // [group][template][chunk angle][MaxPos+5], then their counts [group][template][chunk angle]; refined block = one
+    // segment { FpmRefined[seg_cap]; int count; int pad } per group
+    struct ShardGroup { int chunk = 0, n_tpl = 0, seg_cap = 0, n_local = 0, key_stride = 1; size_t pick_off = 0, cnt_off = 0, ref_off = 0; };
+    struct ShardState {
+        int empty = 1;
+        size_t pick_blk = 0, cnt_off = 0, n_cnt = 0, ref_blk = 0;   // cnt_off: bytes to the counts; n_cnt: ints of counts
+        std::vector<char> run;
+        std::vector<ShardGroup> g;
+    } sh;
     std::vector<FpmLevel> levels; // source pyramid of the current batch
     const std::vector<FpmLevel>* shared_levels = nullptr;   // fpm_match_multi: the pyramid built once by the first handle
     TopPlan plan;
@@ -867,9 +876,10 @@ float top_reject_below(const fpm_handle* h, int top)
 // ---- top-layer sweep: warp + score + peaks for jobs [j0, j0 + nj) of the plan's (frame, angle) list -----
 // Each (frame, angle) canvas is warped once and scored against every template of the group.  picks go to
 // picks_out[slot][max_picks], counts to cnt_out[slot]: slot = job - j0 for one template, (frame * n_tpl + template) *
-// n_angles + angle for a group (whole sweeps only).  The sweep runs in chunks of canvases whose n_tpl score maps each fit
-// FPM_PARAM_WORKSPACE_MB and whose jobs fit gridDim.y / gridDim.z.
-int run_top(fpm_handle* h, int top, int j0, int nj, FpmPick* picks_out, int* cnt_out)
+// row_angles + angle for a group, with row_angles = the whole schedule (0) for whole sweeps and the chunk for the
+// angle-sharded sweep of one frame (jobs [j0, j0 + nj), nj <= row_angles).  The sweep runs in chunks of canvases whose n_tpl
+// score maps each fit FPM_PARAM_WORKSPACE_MB and whose jobs fit gridDim.y / gridDim.z.
+int run_top(fpm_handle* h, int top, int j0, int nj, FpmPick* picks_out, int* cnt_out, int row_angles = 0)
 {
     TopPlan& p = h->plan;
     const int max_picks = h->max_pos + FPM_MATCH_CANDIDATE_NUM;
@@ -928,7 +938,7 @@ int run_top(fpm_handle* h, int top, int j0, int nj, FpmPick* picks_out, int* cnt
            fpm_top_peaks_kernel<<<nc * n_tpl, (maxRW * maxRH <= 16384) ? 128 : PK_THREADS, (size_t)smem_blocks * 8, h->stream>>>(
                jobs, h->d_score.as<float>(), spitch, score_stride, t.w, t.h, mode, tile,
                h->d_blkv.as<float>(), h->d_blkl.as<int>(), blk_stride, thresh, h->max_overlap, max_picks,
-               picks_out, cnt_out, smem_blocks, c0, n_tpl, p.n_ang));
+               picks_out, cnt_out, smem_blocks, c0, n_tpl, row_angles ? row_angles : p.n_ang));
     }
     return FPM_OK;
 }
@@ -1213,9 +1223,10 @@ int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride
 }
 
 // candidate list: gather the picks of all angles, std::sort by score (:214), un-rotation (:265-266).  Leaves this
-// rank's candidates (all of them when shard_n == 1) in d_cand[0]; *n_all (optional) = size of the global list of image 0.
+// rank's candidates (all of them when shard_n == 1) in d_cand[0] and, unless n_cands is null (the angle-sharded mode knows
+// its counts from the gathered pick counts), reads their number back.
 int collect_candidates(fpm_handle* h, int top, int batch, const FpmPickView& pv, int n_angles, int shard_rank, int shard_n,
-                       int* n_cands, int* cand_stride_out, int* n_all)
+                       int* n_cands, int* cand_stride_out)
 {
     const int max_picks = h->max_pos + FPM_MATCH_CANDIDATE_NUM;
     const int cand_stride = std::max(n_angles * max_picks, 1);
@@ -1240,14 +1251,14 @@ int collect_candidates(fpm_handle* h, int top, int batch, const FpmPickView& pv,
                h->d_ftx.as<float>(), h->d_fty.as<float>(), (L.w - 1) / 2.0f, (L.h - 1) / 2.0f,
                h->d_keys.as<unsigned long long>(), n_pad, use_smem, h->d_off.as<int>(), h->d_cand[0].as<FpmCand>(),
                counters + CNT_FLAT, h->trace ? h->d_toppt.as<float>() : nullptr, cand_stride,
-               n_all ? counters + CNT_TOTAL : h->d_candcnt.as<int>(), 0, shard_rank, shard_n));
+               h->d_candcnt.as<int>(), 0, shard_rank, shard_n));
     }
+    if (!n_cands) return FPM_OK;
     int* hc = h->h_counts.as<int>();
     CK(cudaMemcpyAsync(hc, h->d_counters.p, CNT_N * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     *n_cands = hc[CNT_FLAT];
-    if (n_all) *n_all = hc[CNT_TOTAL];
-    if (h->trace && !n_all) {
+    if (h->trace) {
         std::vector<float> tp((size_t)cand_stride * 4);
         int n0 = 0;
         CK(cudaMemcpy(&n0, h->d_candcnt.p, sizeof(int), cudaMemcpyDeviceToHost));
@@ -1291,7 +1302,7 @@ int match_group(fpm_handle* h, int batch, fpm_result* out, int cap, int* n_out, 
     if (rc) return rc;
     FpmPickView pv{h->d_picks.as<FpmPick>(), h->d_pickcnt.as<int>(), 0, 0};
     int n_cands = 0, cand_stride = 0;
-    rc = collect_candidates(h, top, vbatch, pv, p.n_ang, 0, 1, &n_cands, &cand_stride, nullptr);
+    rc = collect_candidates(h, top, vbatch, pv, p.n_ang, 0, 1, &n_cands, &cand_stride);
     if (rc) return rc;
     int n_refined = 0;
     h->ref_out = nullptr; h->ref_cnt = nullptr;
@@ -1375,6 +1386,47 @@ int run_set_merge(fpm_handle* h, int batch, int n_set, int n_groups, const Merge
     return FPM_OK;
 }
 
+// run[g] = 1 for the groups the size guards let run on a w x hgt source; returns the deepest top layer among them (-1: none)
+int runnable_groups(const fpm_handle* h, int w, int hgt, std::vector<char>& run)
+{
+    const size_t n_groups = h->groups.size();
+    run.assign(n_groups, 0);
+    int max_top = -1;
+    for (size_t g = 0; g < n_groups; g++) {
+        const TplGroup& G = h->groups[g];
+        const bool cur = g == 0;                             // group 0's state is in the handle's fields
+        if (match_guards(h, w, hgt, cur ? h->tpl0_w : G.w0, cur ? h->tpl0_h : G.h0)) continue;
+        run[g] = 1;
+        max_top = std::max(max_top, (int)(cur ? h->tpl.size() : G.tpl.size()) - 1);
+    }
+    return max_top;
+}
+
+// device lists of the merge for the groups that run (run[g]) over `batch` frames, header zeroed on the stream
+int merge_setup(fpm_handle* h, int batch, int cap, int n_set, const std::vector<char>& run, MergeDev* md)
+{
+    // list capacity: a group's list of a frame never exceeds its candidate list, n_angles * (MaxPos + 5) entries
+    const size_t n_groups = h->groups.size();
+    int longest = 0;
+    for (size_t g = 0; g < n_groups; g++) {
+        if (!run[g]) continue;
+        GroupScope scope(h, g);
+        if (int rc = make_top_plan(h, (int)h->tpl.size() - 1, batch)) return rc;
+        longest = std::max(longest, h->plan.n_ang * (h->max_pos + FPM_MATCH_CANDIDATE_NUM));
+    }
+    md->lcap = std::min(cap, longest);
+    if ((long long)n_set * md->lcap >= (1ll << 30)) { h->err = "merged set results: n_set * list capacity too large"; return FPM_ERR_LIMIT; }
+    md->ocap = std::min(cap, n_set * md->lcap);
+    const MergedLayout lay(batch, n_set, md->ocap, (int)n_groups);
+    CK(h->d_mlists.ensure((size_t)batch * n_set * std::max(md->lcap, 1) * sizeof(FpmResultDev)));
+    CK(h->d_merged.ensure(lay.bytes));
+    CK(cudaMemsetAsync(h->d_merged.p, 0, lay.header_bytes, h->stream));   // the totals of groups that do not run, the CNT_ERR slots
+    md->lists = h->d_mlists.as<FpmResultDev>();
+    md->counts = h->d_merged.as<int>() + lay.set_counts;
+    md->err = h->d_merged.as<int>() + lay.err;
+    return FPM_OK;
+}
+
 // whole match() over a device-resident batch, for every template of the set: frame b / template t at out + (b * n + t) * cap,
 // or (mg) the merged list of frame b at out + b * cap.
 // The source pyramid (and bitwise_not) is built once, down to the deepest top layer of any group; the groups run one
@@ -1389,15 +1441,8 @@ int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt,
     int rc = ensure_learned_for_mra(h);
     if (rc) return rc;
     const size_t n_groups = h->groups.size();
-    std::vector<char> run(n_groups, 0);
-    int max_top = -1;
-    for (size_t g = 0; g < n_groups; g++) {
-        const TplGroup& G = h->groups[g];
-        const bool cur = g == 0;                             // group 0's state is in the handle's fields
-        if (match_guards(h, w, hgt, cur ? h->tpl0_w : G.w0, cur ? h->tpl0_h : G.h0)) continue;
-        run[g] = 1;
-        max_top = std::max(max_top, (int)(cur ? h->tpl.size() : G.tpl.size()) - 1);
-    }
+    std::vector<char> run;
+    const int max_top = runnable_groups(h, w, hgt, run);
     if (max_top < 0) return FPM_OK;
     h->cur_batch = batch;
     CK(h->d_counters.ensure(CNT_N * sizeof(int)));
@@ -1414,26 +1459,7 @@ int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt,
     rc = build_pyramid(h, d_src, batch, w, hgt, stride, frame_stride, max_top);
     if (rc) return rc;
     MergeDev md;
-    if (mg) {
-        // list capacity: a group's list of a frame never exceeds its candidate list, n_angles * (MaxPos + 5) entries
-        int longest = 0;
-        for (size_t g = 0; g < n_groups; g++) {
-            if (!run[g]) continue;
-            GroupScope scope(h, g);
-            if ((rc = make_top_plan(h, (int)h->tpl.size() - 1, batch))) return rc;
-            longest = std::max(longest, h->plan.n_ang * (h->max_pos + FPM_MATCH_CANDIDATE_NUM));
-        }
-        md.lcap = std::min(cap, longest);
-        if ((long long)n_set * md.lcap >= (1ll << 30)) { h->err = "merged set results: n_set * list capacity too large"; return FPM_ERR_LIMIT; }
-        md.ocap = std::min(cap, n_set * md.lcap);
-        const MergedLayout lay(batch, n_set, md.ocap, (int)n_groups);
-        CK(h->d_mlists.ensure((size_t)batch * n_set * std::max(md.lcap, 1) * sizeof(FpmResultDev)));
-        CK(h->d_merged.ensure(lay.bytes));
-        CK(cudaMemsetAsync(h->d_merged.p, 0, lay.header_bytes, h->stream));   // the totals of groups that do not run, the CNT_ERR slots
-        md.lists = h->d_mlists.as<FpmResultDev>();
-        md.counts = h->d_merged.as<int>() + lay.set_counts;
-        md.err = h->d_merged.as<int>() + lay.err;
-    }
+    if (mg && (rc = merge_setup(h, batch, cap, n_set, run, &md))) return rc;
     int* err_slots = md.err;
     size_t member_off = 0;
     for (size_t g = 0; g < n_groups && rc == FPM_OK; g++) {
@@ -1504,8 +1530,12 @@ int shard_allgather(fpm_handle* h, void* buf, size_t bytes)
 // contiguous chunk of the angle schedule per rank: rank r sweeps [r*chunk, min(A, (r+1)*chunk))
 inline int shard_chunk(int n_angles, int nranks) { return std::max(1, (n_angles + nranks - 1) / nranks); }
 
-// phase 1: source on the device (uploaded in 1/N row slices + allgather when it comes from the host), pyramid,
-// top-layer sweep of this rank's angles into its block of the gather buffer
+// candidates of a global list of n entries that rank R of N refines (candidate k -> rank k mod N)
+inline int shard_share(int n, int R, int N) { return n > R ? (n - R + N - 1) / N : 0; }
+
+// phase 1: source on the device (uploaded in 1/N row slices + allgather when it comes from the host), pyramid down to the
+// deepest top layer of the groups that run, then for every such group the top-layer sweep of this rank's chunk of its angle
+// schedule for all its templates, into the group's place in this rank's block of the gather buffer
 int shard_begin(fpm_handle* h, const uint8_t* src, int w, int hgt, int stride, int src_on_device)
 {
     h->sh = fpm_handle::ShardState();
@@ -1514,7 +1544,9 @@ int shard_begin(fpm_handle* h, const uint8_t* src, int w, int hgt, int stride, i
     if (rc) return rc;
     if (!src || w <= 0 || hgt <= 0) return FPM_OK;
     if (stride < w) { h->err = "stride < width"; return FPM_ERR_INVALID; }
-    if (match_guards(h, w, hgt, h->tpl0_w, h->tpl0_h)) return FPM_OK;
+    std::vector<char> run;
+    const int max_top = runnable_groups(h, w, hgt, run);
+    if (max_top < 0) return FPM_OK;
     const int N = h->sh_nranks, R = h->sh_rank;
     const uint8_t* d_src = src;
     int pitch = stride;
@@ -1541,7 +1573,6 @@ int shard_begin(fpm_handle* h, const uint8_t* src, int w, int hgt, int stride, i
         }
         d_src = h->d_src.as<uint8_t>();
     }
-    const int top = (int)h->tpl.size() - 1;
     h->cur_batch = 1;
     CK(h->d_counters.ensure(CNT_N * sizeof(int)));
     CK(h->h_counts.ensure((CNT_N + 1) * sizeof(int)));
@@ -1555,22 +1586,43 @@ int shard_begin(fpm_handle* h, const uint8_t* src, int w, int hgt, int stride, i
         CKL();
         d_src = h->d_inv.as<uint8_t>(); pitch = ipitch; img = iimg;
     }
-    rc = build_pyramid(h, d_src, 1, w, hgt, pitch, img, top);
+    rc = build_pyramid(h, d_src, 1, w, hgt, pitch, img, max_top);
     if (rc) return rc;
-    rc = make_top_plan(h, top, 1);
-    if (rc) return rc;
-    const TopPlan& p = h->plan;
+    // the block layout, from the plans (the same on every rank)
+    fpm_handle::ShardState& S = h->sh;
     const int max_picks = h->max_pos + FPM_MATCH_CANDIDATE_NUM;
-    const int chunk = shard_chunk(p.n_ang, N);
-    const size_t blk = align_up((size_t)chunk * max_picks * sizeof(FpmPick) + (size_t)chunk * sizeof(int), 16);
-    CK(h->d_gpicks.ensure(blk * N));
-    uint8_t* mine = h->d_gpicks.as<uint8_t>() + (size_t)R * blk;
-    int* cnt = reinterpret_cast<int*>(mine + (size_t)chunk * max_picks * sizeof(FpmPick));
-    CK(cudaMemsetAsync(cnt, 0, (size_t)chunk * sizeof(int), h->stream));      // angles past the schedule's end stay empty
-    const int a0 = std::min(p.n_ang, R * chunk), a1 = std::min(p.n_ang, a0 + chunk);
-    rc = run_top(h, top, a0, a1 - a0, reinterpret_cast<FpmPick*>(mine), cnt);
-    if (rc) return rc;
-    h->sh.top = top; h->sh.chunk = chunk; h->sh.pick_blk = blk; h->sh.empty = 0;
+    const size_t n_groups = h->groups.size();
+    S.g.assign(n_groups, fpm_handle::ShardGroup());
+    size_t pick_bytes = 0, n_cnt = 0;
+    for (size_t g = 0; g < n_groups; g++) {
+        if (!run[g]) continue;
+        GroupScope scope(h, g);
+        if ((rc = make_top_plan(h, (int)h->tpl.size() - 1, 1))) return rc;
+        fpm_handle::ShardGroup& sg = S.g[g];
+        sg.n_tpl = std::max((int)h->members.size(), 1);
+        sg.chunk = shard_chunk(h->plan.n_ang, N);
+        sg.pick_off = pick_bytes;
+        sg.cnt_off = n_cnt;
+        pick_bytes += (size_t)sg.n_tpl * sg.chunk * max_picks * sizeof(FpmPick);
+        n_cnt += (size_t)sg.n_tpl * sg.chunk;
+    }
+    S.cnt_off = pick_bytes; S.n_cnt = n_cnt;
+    S.pick_blk = align_up(pick_bytes + n_cnt * sizeof(int), 16);
+    CK(h->d_gpicks.ensure(S.pick_blk * N));
+    uint8_t* mine = h->d_gpicks.as<uint8_t>() + (size_t)R * S.pick_blk;
+    int* cnt = reinterpret_cast<int*>(mine + S.cnt_off);
+    CK(cudaMemsetAsync(cnt, 0, n_cnt * sizeof(int), h->stream));   // angles past a schedule's end stay empty
+    for (size_t g = 0; g < n_groups; g++) {
+        if (!run[g]) continue;
+        GroupScope scope(h, g);
+        const fpm_handle::ShardGroup& sg = S.g[g];
+        const int n_ang = h->plan.n_ang;
+        const int a0 = std::min(n_ang, R * sg.chunk), a1 = std::min(n_ang, a0 + sg.chunk);
+        rc = run_top(h, (int)h->tpl.size() - 1, a0, a1 - a0, reinterpret_cast<FpmPick*>(mine + sg.pick_off), cnt + sg.cnt_off, sg.chunk);
+        if (rc) return rc;
+    }
+    S.run.swap(run);
+    S.empty = 0;
     return FPM_OK;
 }
 
@@ -1580,26 +1632,61 @@ int shard_exchange_picks(fpm_handle* h)
     return shard_allgather(h, h->d_gpicks.p, h->sh.pick_blk);
 }
 
-// phase 2: identical global candidate list on every rank, this rank's share refined into its block of the second buffer
+// phase 2: one read-back of the gathered pick counts gives every rank the global list size of every (group, template) and
+// so the layout of the refined blocks; per group, every rank sorts the identical global lists in place and refines its share
+// into the group's segment of its refined block
 int shard_mid(fpm_handle* h)
 {
     if (h->sh.empty) return FPM_OK;
-    const int N = h->sh_nranks, R = h->sh_rank, top = h->sh.top;
-    FpmPickView pv{h->d_gpicks.as<FpmPick>(), nullptr, h->sh.chunk, h->sh.pick_blk};
-    int n_local = 0, cand_stride = 0, n_all = 0;
-    int rc = collect_candidates(h, top, 1, pv, h->sh.chunk * N, R, N, &n_local, &cand_stride, &n_all);
-    if (rc) return rc;
-    const int seg_cap = std::max(1, (n_all + N - 1) / N);
-    const size_t blk = align_up((size_t)seg_cap * sizeof(FpmRefined) + 8, 16);
-    CK(h->d_grefined.ensure(blk * N));
-    uint8_t* mine = h->d_grefined.as<uint8_t>() + (size_t)R * blk;
-    h->ref_out = reinterpret_cast<FpmRefined*>(mine);
-    h->ref_cnt = reinterpret_cast<int*>(mine + (size_t)seg_cap * sizeof(FpmRefined));
-    int n_refined = 0;
-    rc = run_refine(h, top, n_local, &n_refined);
-    h->ref_out = nullptr; h->ref_cnt = nullptr;
-    if (rc) return rc;
-    h->sh.n_all = n_all; h->sh.n_local = n_local; h->sh.seg_cap = seg_cap; h->sh.ref_blk = blk;
+    fpm_handle::ShardState& S = h->sh;
+    const int N = h->sh_nranks, R = h->sh_rank;
+    const size_t cnt_bytes = S.n_cnt * sizeof(int);
+    CK(h->h_counts.ensure(std::max(cnt_bytes * N, (CNT_N + 1) * sizeof(int))));
+    if (cnt_bytes)
+        CK(cudaMemcpy2DAsync(h->h_counts.p, cnt_bytes, h->d_gpicks.as<uint8_t>() + S.cnt_off, S.pick_blk, cnt_bytes, N,
+                             cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    const int* hc = h->h_counts.as<int>();
+    const size_t n_groups = S.g.size();
+    size_t ref_bytes = 0;
+    for (size_t g = 0; g < n_groups; g++) {
+        if (!S.run[g]) continue;
+        fpm_handle::ShardGroup& sg = S.g[g];
+        int seg = 0;
+        for (int t = 0; t < sg.n_tpl; t++) {
+            int n = 0;
+            for (int r = 0; r < N; r++)
+                for (int l = 0; l < sg.chunk; l++) n += hc[(size_t)r * S.n_cnt + sg.cnt_off + (size_t)t * sg.chunk + l];
+            sg.n_local += shard_share(n, R, N);
+            seg += (n + N - 1) / N;                          // the largest share any rank gets of this list
+            sg.key_stride = std::max(sg.key_stride, n);
+        }
+        sg.seg_cap = std::max(1, seg);
+        sg.ref_off = ref_bytes;
+        ref_bytes += align_up((size_t)sg.seg_cap * sizeof(FpmRefined) + 8, 16);
+    }
+    S.ref_blk = std::max<size_t>(ref_bytes, 16);
+    CK(h->d_grefined.ensure(S.ref_blk * N));
+    uint8_t* base = h->d_gpicks.as<uint8_t>();
+    uint8_t* mine = h->d_grefined.as<uint8_t>() + (size_t)R * S.ref_blk;
+    for (size_t g = 0; g < n_groups; g++) {
+        if (!S.run[g]) continue;
+        GroupScope scope(h, g);
+        const fpm_handle::ShardGroup& sg = S.g[g];
+        const int top = (int)h->tpl.size() - 1;
+        CK(cudaMemsetAsync(h->d_counters.as<int>() + CNT_FLAT, 0, sizeof(int), h->stream));
+        const FpmPickView pv{reinterpret_cast<const FpmPick*>(base + sg.pick_off), reinterpret_cast<const int*>(base + S.cnt_off) + sg.cnt_off,
+                             sg.chunk, S.pick_blk};
+        int cand_stride = 0;
+        int rc = collect_candidates(h, top, sg.n_tpl, pv, sg.chunk * N, R, N, nullptr, &cand_stride);
+        if (rc) return rc;
+        h->ref_out = reinterpret_cast<FpmRefined*>(mine + sg.ref_off);
+        h->ref_cnt = reinterpret_cast<int*>(mine + sg.ref_off + (size_t)sg.seg_cap * sizeof(FpmRefined));
+        int n_refined = 0;
+        rc = run_refine(h, top, sg.n_local, &n_refined);
+        h->ref_out = nullptr; h->ref_cnt = nullptr;
+        if (rc) return rc;
+    }
     return FPM_OK;
 }
 
@@ -1609,13 +1696,89 @@ int shard_exchange_refined(fpm_handle* h)
     return shard_allgather(h, h->d_grefined.p, h->sh.ref_blk);
 }
 
-// phase 3: replicated filterWithScore + NMS + conversion straight from the gathered blocks
-int shard_end(fpm_handle* h, fpm_result* out, int cap, int* n)
+// phase 3: per group, the replicated filterWithScore + NMS + conversion straight from the gathered blocks, to the caller's
+// [template][cap] lists or (mg) the device lists of the merge, then one merge launch
+int shard_end(fpm_handle* h, fpm_result* out, int cap, int* n_out, const SetMerge* mg)
 {
-    *n = 0;
-    if (h->sh.empty) return FPM_OK;
-    FpmRefinedView rv{h->d_grefined.as<FpmRefined>(), nullptr, h->sh.seg_cap, h->sh_nranks, h->sh.ref_blk};
-    return run_final(h, 1, rv, std::max(h->sh.n_all, 1), out, cap, n);
+    const fpm_handle::ShardState& S = h->sh;
+    if (S.empty) return FPM_OK;
+    const int n_set = std::max((int)h->set.size(), 1);
+    const size_t n_groups = S.g.size();
+    MergeDev md;
+    if (mg) if (int rc = merge_setup(h, 1, cap, n_set, S.run, &md)) return rc;
+    int* err_slots = md.err;
+    size_t member_off = 0;
+    for (size_t g = 0; g < n_groups; g++) {
+        const size_t n_members = g == 0 ? h->members.size() : h->groups[g].members.size();
+        md.rows = h->d_members.as<int>() + member_off;
+        md.err = err_slots ? err_slots + g : nullptr;
+        member_off += n_members;
+        if (!S.run[g]) continue;
+        GroupScope scope(h, g);
+        const fpm_handle::ShardGroup& sg = S.g[g];
+        const FpmRefinedView rv{reinterpret_cast<const FpmRefined*>(h->d_grefined.as<uint8_t>() + sg.ref_off), nullptr, sg.seg_cap,
+                                h->sh_nranks, S.ref_blk};
+        if (int rc = run_final(h, sg.n_tpl, rv, sg.key_stride, out, cap, n_out, n_set, mg ? &md : nullptr)) return rc;
+    }
+    return mg ? run_set_merge(h, 1, n_set, (int)n_groups, md, mg, out, cap, n_out) : FPM_OK;
+}
+
+// one frame against the whole set across the communicator's ranks (fpm_match_set_sharded*): every rank gets the lists
+// fpm_match_set_batch (mg: fpm_match_set_batch_merged) returns for the frame on one GPU
+int match_set_sharded(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device, fpm_result* out,
+                      int cap, int* n, const SetMerge* mg)
+{
+    CK(cudaSetDevice(h->device));
+    auto t0 = std::chrono::high_resolution_clock::now();
+    int rc = shard_begin(h, src, width, height, stride, src_on_device);
+    if (!rc) rc = shard_exchange_picks(h);
+    if (!rc) rc = shard_mid(h);
+    if (!rc) rc = shard_exchange_refined(h);
+    if (!rc) rc = shard_end(h, out, cap, n, mg);
+    prof_collect(h);
+    if (rc) cudaStreamSynchronize(h->stream);
+    h->last_ms = std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count();
+    return rc;
+}
+
+// The same pipeline with `nranks` handles of ONE device playing the ranks and the two exchanges done as device-to-device
+// block copies: exercises the partitioning and the in-place consumption of the gathered buffers where only one GPU (and no
+// NCCL peer) is available.  Rank r's lists go to out + r * n_rows * cap and n + r * n_rows (n_rows = 1 merged, else the set
+// size); mg[r] is rank r's merge.  count_exchanges: every exchange round adds one to each handle's collective count.
+int match_set_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
+                              fpm_result* out, int cap, int* n, int n_rows, const SetMerge* mg, bool count_exchanges)
+{
+    for (int r = 0; r < nranks; r++) { hs[r]->sh_nranks = nranks; hs[r]->sh_rank = r; }
+    auto exchange = [&](DevBuf fpm_handle::*buf, size_t fpm_handle::ShardState::*blk) -> int {
+        for (int r = 0; r < nranks; r++) {
+            fpm_handle* h = hs[r];
+            CK(cudaStreamSynchronize(h->stream));
+        }
+        for (int q = 0; q < nranks; q++) {
+            fpm_handle* h = hs[q];
+            if (h->sh.empty) continue;
+            const size_t b = h->sh.*blk;
+            for (int r = 0; r < nranks; r++)
+                if (r != q && !hs[r]->sh.empty)
+                    CK(cudaMemcpyAsync((h->*buf).as<uint8_t>() + (size_t)r * b, (hs[r]->*buf).as<uint8_t>() + (size_t)r * b, b,
+                                       cudaMemcpyDeviceToDevice, h->stream));
+            if (count_exchanges) h->collectives++;
+        }
+        return FPM_OK;
+    };
+    int rc = FPM_OK;
+    for (int r = 0; r < nranks && !rc; r++) { cudaSetDevice(hs[r]->device); rc = shard_begin(hs[r], src, width, height, stride, 0); }
+    if (!rc) rc = exchange(&fpm_handle::d_gpicks, &fpm_handle::ShardState::pick_blk);
+    for (int r = 0; r < nranks && !rc; r++) rc = shard_mid(hs[r]);
+    if (!rc) rc = exchange(&fpm_handle::d_grefined, &fpm_handle::ShardState::ref_blk);
+    for (int r = 0; r < nranks && !rc; r++)
+        rc = shard_end(hs[r], out + (size_t)r * n_rows * cap, cap, n + (size_t)r * n_rows, mg ? mg + r : nullptr);
+    for (int r = 0; r < nranks; r++) {
+        prof_collect(hs[r]);
+        if (rc) cudaStreamSynchronize(hs[r]->stream);
+        hs[r]->sh_nranks = 1; hs[r]->sh_rank = 0;
+    }
+    return rc;
 }
 
 }  // namespace
@@ -3159,6 +3322,52 @@ int fpm_shard_angle_range(int n_angles, int nranks, int rank, int* a0, int* a1)
 
 long long fpm_collective_count(const fpm_handle* h) { return h ? h->collectives : 0; }
 
+namespace {
+// refusals shared by the whole-set sharded calls (fpm_match_set_batch's, plus a missing communicator)
+int check_set_sharded(fpm_handle* h, const char* fn, int cap, const void* out, const int* n)
+{
+    if (h->trace && fpm_set_size(h) > 1) {
+        h->err = std::string(fn) + ": FPM_PARAM_TRACE is not supported for a set of more than one template";
+        return FPM_ERR_INVALID;
+    }
+    if (!n || cap < 0 || (cap > 0 && !out)) { h->err = std::string(fn) + ": bad output arguments"; return FPM_ERR_INVALID; }
+    if (h->sh_nranks > 1 && !h->nccl_comm) {
+        h->err = std::string(fn) + ": " + std::to_string(h->sh_nranks) + " ranks without a communicator (fpm_comm_init / fpm_comm_attach)";
+        return FPM_ERR_INVALID;
+    }
+    return FPM_OK;
+}
+
+int check_merge_args(fpm_handle* h, const char* fn, double max_overlap, int cap, const int* labels)
+{
+    if (!std::isfinite(max_overlap)) { h->err = std::string(fn) + ": max_overlap must be finite"; return FPM_ERR_INVALID; }
+    if (cap > 0 && !labels) { h->err = std::string(fn) + ": labels is NULL while cap > 0"; return FPM_ERR_INVALID; }
+    return FPM_OK;
+}
+
+// refusals of the virtual-rank drivers: every handle present, none with a communicator, one set size on all of them
+int check_virtual(fpm_handle* const* hs, int nranks, const char* fn, bool whole_set)
+{
+    if (!hs || nranks < 1) return FPM_ERR_INVALID;
+    for (int r = 0; r < nranks; r++)
+        if (!hs[r]) return FPM_ERR_INVALID;
+    auto refuse = [&](const std::string& msg) {
+        for (int r = 0; r < nranks; r++) hs[r]->err = std::string(fn) + ": " + msg;
+        return FPM_ERR_INVALID;
+    };
+    for (int r = 0; r < nranks; r++) {
+        if (hs[r]->nccl_comm) return whole_set ? refuse("the handle of rank " + std::to_string(r) + " has a communicator") : FPM_ERR_INVALID;
+        if (!whole_set) {
+            if (int rc = refuse_set(hs[r], fn)) return rc;
+        } else if (fpm_set_size(hs[r]) != fpm_set_size(hs[0])) {
+            return refuse("rank " + std::to_string(r) + " holds a set of " + std::to_string(fpm_set_size(hs[r])) + " templates, rank 0 one of " +
+                          std::to_string(fpm_set_size(hs[0])));
+        }
+    }
+    return FPM_OK;
+}
+}  // namespace
+
 int fpm_match_sharded(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
                       fpm_result* out, int cap, int* n)
 {
@@ -3166,58 +3375,67 @@ int fpm_match_sharded(fpm_handle* h, const uint8_t* src, int width, int height, 
     if (int rc = refuse_set(h, "fpm_match_sharded")) return rc;
     if (!n || cap < 0 || (cap > 0 && !out)) { h->err = "bad output arguments"; return FPM_ERR_INVALID; }
     *n = 0;
-    CK(cudaSetDevice(h->device));
-    auto t0 = std::chrono::high_resolution_clock::now();
-    int rc = shard_begin(h, src, width, height, stride, src_on_device);
-    if (!rc) rc = shard_exchange_picks(h);
-    if (!rc) rc = shard_mid(h);
-    if (!rc) rc = shard_exchange_refined(h);
-    if (!rc) rc = shard_end(h, out, cap, n);
-    prof_collect(h);
-    if (rc) cudaStreamSynchronize(h->stream);
-    h->last_ms = std::chrono::duration<double, std::milli>(std::chrono::high_resolution_clock::now() - t0).count();
-    return rc;
+    return match_set_sharded(h, src, width, height, stride, src_on_device, out, cap, n, nullptr);
 }
 
-// The same pipeline with `nranks` handles of ONE device playing the ranks and the two exchanges done as device-to-device
-// block copies: exercises the partitioning and the in-place consumption of the gathered buffers where only one GPU
-// (and no NCCL peer) is available.  Every rank's result list is returned (rank r at out + r*cap, n[r]).
+// rank r's result list at out + r*cap, n[r]; the block copies are not counted as collectives
 int fpm_match_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
                               fpm_result* out, int cap, int* n)
 {
-    if (!hs || nranks < 1 || !n || cap < 0 || (cap > 0 && !out)) return FPM_ERR_INVALID;
+    if (!n || cap < 0 || (cap > 0 && !out)) return FPM_ERR_INVALID;
+    if (int rc = check_virtual(hs, nranks, "fpm_match_sharded_virtual", false)) return rc;
+    for (int r = 0; r < nranks; r++) n[r] = 0;
+    return match_set_sharded_virtual(hs, nranks, src, width, height, stride, out, cap, n, 1, nullptr, false);
+}
+
+int fpm_match_set_sharded(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                          fpm_result* out, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (int rc = check_set_sharded(h, "fpm_match_set_sharded", cap, out, counts)) return rc;
+    std::fill(counts, counts + std::max(fpm_set_size(h), 1), 0);
+    return match_set_sharded(h, src, width, height, stride, src_on_device, out, cap, counts, nullptr);
+}
+
+int fpm_match_set_sharded_merged(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                                 double max_overlap, fpm_result* out, int* labels, int cap, int* count, int* set_counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (int rc = check_set_sharded(h, "fpm_match_set_sharded_merged", cap, out, count)) return rc;
+    if (int rc = check_merge_args(h, "fpm_match_set_sharded_merged", max_overlap, cap, labels)) return rc;
+    *count = 0;
+    if (set_counts) std::fill(set_counts, set_counts + std::max(fpm_set_size(h), 1), 0);
+    const SetMerge mg{max_overlap, labels, set_counts};
+    return match_set_sharded(h, src, width, height, stride, src_on_device, out, cap, count, &mg);
+}
+
+int fpm_match_set_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
+                                  fpm_result* out, int cap, int* counts)
+{
+    if (int rc = check_virtual(hs, nranks, "fpm_match_set_sharded_virtual", true)) return rc;
+    for (int r = 0; r < nranks; r++)
+        if (int rc = check_set_sharded(hs[r], "fpm_match_set_sharded_virtual", cap, out, counts)) return rc;
+    const int n_set = std::max(fpm_set_size(hs[0]), 1);
+    std::fill(counts, counts + (size_t)nranks * n_set, 0);
+    return match_set_sharded_virtual(hs, nranks, src, width, height, stride, out, cap, counts, n_set, nullptr, true);
+}
+
+int fpm_match_set_sharded_merged_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height,
+                                         int stride, double max_overlap, fpm_result* out, int* labels, int cap, int* count,
+                                         int* set_counts)
+{
+    if (int rc = check_virtual(hs, nranks, "fpm_match_set_sharded_merged_virtual", true)) return rc;
     for (int r = 0; r < nranks; r++) {
-        if (!hs[r] || hs[r]->nccl_comm) return FPM_ERR_INVALID;
-        if (int rc = refuse_set(hs[r], "fpm_match_sharded_virtual")) return rc;
-        hs[r]->sh_nranks = nranks; hs[r]->sh_rank = r;
-        n[r] = 0;
+        if (int rc = check_set_sharded(hs[r], "fpm_match_set_sharded_merged_virtual", cap, out, count)) return rc;
+        if (int rc = check_merge_args(hs[r], "fpm_match_set_sharded_merged_virtual", max_overlap, cap, labels)) return rc;
     }
-    auto exchange = [&](DevBuf fpm_handle::*buf, size_t fpm_handle::ShardState::*blk) -> int {
-        for (int r = 0; r < nranks; r++) {
-            fpm_handle* h = hs[r];
-            CK(cudaStreamSynchronize(h->stream));
-        }
-        for (int q = 0; q < nranks; q++) {
-            fpm_handle* h = hs[q];
-            if (h->sh.empty) continue;
-            const size_t b = h->sh.*blk;
-            for (int r = 0; r < nranks; r++)
-                if (r != q && !hs[r]->sh.empty)
-                    CK(cudaMemcpyAsync((h->*buf).as<uint8_t>() + (size_t)r * b, (hs[r]->*buf).as<uint8_t>() + (size_t)r * b, b,
-                                       cudaMemcpyDeviceToDevice, h->stream));
-        }
-        return FPM_OK;
-    };
-    int rc = FPM_OK;
-    auto restore = [&]() { for (int r = 0; r < nranks; r++) { hs[r]->sh_nranks = 1; hs[r]->sh_rank = 0; } };
-    for (int r = 0; r < nranks && !rc; r++) { cudaSetDevice(hs[r]->device); rc = shard_begin(hs[r], src, width, height, stride, 0); }
-    if (!rc) rc = exchange(&fpm_handle::d_gpicks, &fpm_handle::ShardState::pick_blk);
-    for (int r = 0; r < nranks && !rc; r++) rc = shard_mid(hs[r]);
-    if (!rc) rc = exchange(&fpm_handle::d_grefined, &fpm_handle::ShardState::ref_blk);
-    for (int r = 0; r < nranks && !rc; r++) rc = shard_end(hs[r], out + (size_t)r * cap, cap, n + r);
-    for (int r = 0; r < nranks; r++) prof_collect(hs[r]);
-    restore();
-    return rc;
+    const int n_set = std::max(fpm_set_size(hs[0]), 1);
+    std::fill(count, count + nranks, 0);
+    if (set_counts) std::fill(set_counts, set_counts + (size_t)nranks * n_set, 0);
+    std::vector<SetMerge> mg(nranks);
+    for (int r = 0; r < nranks; r++)
+        mg[r] = SetMerge{max_overlap, labels ? labels + (size_t)r * cap : nullptr, set_counts ? set_counts + (size_t)r * n_set : nullptr};
+    return match_set_sharded_virtual(hs, nranks, src, width, height, stride, out, cap, count, 1, mg.data(), true);
 }
 
 // ---- stage kernels for parity tests ----------------------------------------------------

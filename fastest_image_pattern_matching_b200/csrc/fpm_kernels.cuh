@@ -677,7 +677,9 @@ fpm_top_peaks_kernel(const FpmWarpJob* __restrict__ jobs, float* __restrict__ sc
                      FpmPick* __restrict__ picks, int* __restrict__ pick_count, int smem_blocks, int j0, int n_tpl, int n_ang)
 {
     // map blockIdx.x = (canvas j0 + blockIdx.x / n_tpl) x (template blockIdx.x % n_tpl), the score kernel's order; its picks go
-    // to (virtual image, angle) slot job: canvas j = frame * n_ang + angle, virtual image = frame * n_tpl + template
+    // to (virtual image, angle) slot job: canvas j = frame * n_ang + angle, virtual image = frame * n_tpl + template.  The
+    // angle-sharded sweep of one frame passes its chunk of the schedule as n_ang (jobs relative to the chunk's first angle), so
+    // the picks land in its rank block as [template][chunk angle]
     const int mi = blockIdx.x;
     const int wj = j0 + mi / n_tpl;
     const int job = n_tpl == 1 ? wj : ((wj / n_ang) * n_tpl + mi % n_tpl) * n_ang + wj % n_ang;
@@ -866,12 +868,13 @@ __device__ __forceinline__ uint32_t fpm_desc_key(float f)
 #define CS_MAX_SMEM_ANGLES 1024     // angle sweeps up to this size keep their pick-count prefix in shared memory
 
 // Where the picks of (image, angle) live.  Contiguous: picks[(img*n_angles + a)*max_picks], count[img*n_angles + a].
-// Segmented (angle-sharded mode, one image): the buffer is the result of an allgather of one fixed-size block per
-// rank, block r = { FpmPick[seg_angles][max_picks]; int count[seg_angles] } holding angles [r*seg_angles, (r+1)*seg_angles)
-// of the schedule, so the gathered buffer is consumed in place.
+// Segmented (angle-sharded mode, one frame, images = the templates of a group): the buffer is the result of an allgather
+// of one fixed-size block per rank; rank r swept angles [r*seg_angles, (r+1)*seg_angles) of the schedule, and in its block
+// the group's picks of (img, local angle l) sit at picks[(img*seg_angles + l)*max_picks] and their count at
+// count[img*seg_angles + l], both pointers shifted by r*seg_stride bytes.  The gathered buffer is consumed in place.
 struct FpmPickView {
-    const FpmPick* picks;
-    const int* count;
+    const FpmPick* picks;       // segmented: the group's picks in rank block 0
+    const int* count;           // segmented: the group's counts in rank block 0
     int seg_angles;             // 0 = contiguous
     size_t seg_stride;          // bytes per rank block
 };
@@ -879,14 +882,14 @@ __device__ __forceinline__ const FpmPick* fpm_pick_row(const FpmPickView& v, int
 {
     if (v.seg_angles == 0) return v.picks + ((size_t)img * n_angles + a) * max_picks;
     const int r = a / v.seg_angles, l = a - r * v.seg_angles;
-    return reinterpret_cast<const FpmPick*>(reinterpret_cast<const char*>(v.picks) + (size_t)r * v.seg_stride) + (size_t)l * max_picks;
+    return reinterpret_cast<const FpmPick*>(reinterpret_cast<const char*>(v.picks) + (size_t)r * v.seg_stride) +
+           ((size_t)img * v.seg_angles + l) * max_picks;
 }
 __device__ __forceinline__ int fpm_pick_count(const FpmPickView& v, int img, int n_angles, int max_picks, int a)
 {
     if (v.seg_angles == 0) return v.count[img * n_angles + a];
     const int r = a / v.seg_angles, l = a - r * v.seg_angles;
-    const char* blk = reinterpret_cast<const char*>(v.picks) + (size_t)r * v.seg_stride;
-    return reinterpret_cast<const int*>(blk + (size_t)v.seg_angles * max_picks * sizeof(FpmPick))[l];
+    return reinterpret_cast<const int*>(reinterpret_cast<const char*>(v.count) + (size_t)r * v.seg_stride)[img * v.seg_angles + l];
 }
 
 // shard_n > 1 (angle-sharded mode): every rank sorts the identical global list and keeps candidates
@@ -1691,7 +1694,8 @@ __device__ __forceinline__ bool fpm_rrect_far(const FpmRRect& a, const FpmRRect&
 }
 
 // Refined records of a call.  Contiguous: recs[0 .. *count).  Segmented (angle-sharded mode): the allgathered buffer of
-// one block per rank, block r = { FpmRefined[seg_cap]; int count; int pad }, consumed in place.
+// one block per rank, consumed in place; recs points at the group's segment { FpmRefined[seg_cap]; int count; int pad } in
+// rank block 0, and rank r's segment is seg_stride bytes further per rank.
 struct FpmRefinedView {
     const FpmRefined* recs;
     const int* count;

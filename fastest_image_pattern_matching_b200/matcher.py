@@ -557,6 +557,31 @@ class TemplateMatcher:
         self._check(self._lib.fpm_match_sharded(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0, res, cap, C.byref(n)))
         return _convert(res, min(n.value, cap))
 
+    def matchSetSharded(self, sourceImage=None, ptr=None, shape=None, stride=None, on_device=False) -> List[List[SingleTargetMatch]]:
+        """collective, the whole template set against one frame (fpm_match_set_sharded): every rank passes the SAME frame and
+        receives the same [template][results] lists, equal to matchSet on one GPU"""
+        cap, T = self.result_capacity, max(self.patternSetSize(), 1)
+        res, counts = (L.fpm_result * (cap * T))(), (C.c_int * T)()
+        if ptr is None:
+            s = _as_u8_2d(sourceImage)
+            ptr, shape, stride = s.ctypes.data, s.shape, s.strides[0]
+        self._check(self._lib.fpm_match_set_sharded(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0, res, cap, counts))
+        return self._set_results(res, counts, 1, T)[0]
+
+    def matchSetShardedMerged(self, sourceImage=None, max_overlap: Optional[float] = None, ptr=None, shape=None, stride=None,
+                              on_device=False) -> List[Tuple[int, SingleTargetMatch]]:
+        """collective, merged as matchSetMerged (fpm_match_set_sharded_merged): [(set index, result)] on every rank"""
+        if max_overlap is None:
+            raise FpmError("matchSetShardedMerged needs max_overlap")
+        cap, T = self.result_capacity, max(self.patternSetSize(), 1)
+        res, labels, count, set_counts = (L.fpm_result * cap)(), (C.c_int * cap)(), (C.c_int * 1)(), (C.c_int * T)()
+        if ptr is None:
+            s = _as_u8_2d(sourceImage)
+            ptr, shape, stride = s.ctypes.data, s.shape, s.strides[0]
+        self._check(self._lib.fpm_match_set_sharded_merged(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0,
+                                                           float(max_overlap), res, labels, cap, count, set_counts))
+        return self._merged_results(res, labels, count, 1)[0]
+
     # ---- angle-sharded stage API ----
     def stageNumAngles(self, W, H) -> int: return self._lib.fpm_stage_num_angles(self._h, W, H)
 
@@ -649,6 +674,34 @@ def match_sharded_virtual(matchers, sourceImage):
         errs = [lib.fpm_last_error(m._h).decode() for m in matchers]
         raise FpmError("fpm_match_sharded_virtual error %d: %s" % (rc, "; ".join(e for e in errs if e)))
     return [_convert(res[i * cap:(i + 1) * cap], min(counts[i], cap)) for i in range(n)]
+
+
+def match_set_sharded_virtual(matchers, sourceImage, max_overlap=None):
+    """fpm_match_set_sharded_virtual: the whole template set against one frame, angle-sharded over the given handles of ONE
+    device as the ranks.  Returns one result per rank (they must all be equal): [template][results], or with max_overlap
+    the merged [(set index, result)] list (fpm_match_set_sharded_merged_virtual)."""
+    s = _as_u8_2d(sourceImage)
+    lib = matchers[0]._lib
+    n = len(matchers)
+    cap = min(m.result_capacity for m in matchers)
+    T = max(matchers[0].patternSetSize(), 1)
+    hs = (C.c_void_p * n)(*[m._h for m in matchers])
+    if max_overlap is None:
+        res, counts = (L.fpm_result * (cap * n * T))(), (C.c_int * (n * T))()
+        rc = lib.fpm_match_set_sharded_virtual(hs, n, s.ctypes.data, s.shape[1], s.shape[0], s.strides[0], res, cap, counts)
+    else:
+        res, labels, counts, set_counts = (L.fpm_result * (cap * n))(), (C.c_int * (cap * n))(), (C.c_int * n)(), (C.c_int * (n * T))()
+        rc = lib.fpm_match_set_sharded_merged_virtual(hs, n, s.ctypes.data, s.shape[1], s.shape[0], s.strides[0], float(max_overlap),
+                                                      res, labels, cap, counts, set_counts)
+    if rc != 0:
+        errs = [lib.fpm_last_error(m._h).decode() for m in matchers]
+        raise FpmError("fpm_match_set_sharded%s_virtual error %d: %s" % ("" if max_overlap is None else "_merged", rc,
+                                                                         "; ".join(e for e in errs if e)))
+    if max_overlap is None:
+        return [[_convert(res[(r * T + t) * cap:(r * T + t + 1) * cap], min(counts[r * T + t], cap)) for t in range(T)]
+                for r in range(n)]
+    return [list(zip(labels[r * cap:r * cap + min(counts[r], cap)], _convert(res[r * cap:(r + 1) * cap], min(counts[r], cap))))
+            for r in range(n)]
 
 
 # ---- multi-template matching ("NCC-based OCR", MatchTool/MatchToolDlg.cpp:718-770) --------------------------

@@ -101,7 +101,7 @@ int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stri
  * launch of the pipeline (the template is a kernel dimension); groups run one after another.  There is no NMS across templates.
  * A handle holding more than one template refuses every single-template entry point with FPM_ERR_INVALID and a message:
  * fpm_match*, fpm_match_ingested*, fpm_learn_ingested, fpm_match_multi, fpm_match_sharded*, fpm_stage_*, fpm_tpl_* (and
- * fpm_match_set_batch with FPM_PARAM_TRACE on).  FPM_PARAM_MIN_REDUCE_AREA changed after learning re-learns the whole set. */
+ * fpm_match_set_batch with FPM_PARAM_TRACE on).  fpm_match_set_sharded* run a set in the angle-sharded mode.  FPM_PARAM_MIN_REDUCE_AREA changed after learning re-learns the whole set. */
 int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides);
 int fpm_set_size(const fpm_handle* h);              /* 0 = nothing learned, 1 after fpm_learn */
 /* batch frames (HOST memory, or device memory with src_on_device = 1; frame i at src + i*frame_stride) x the set: frame b /
@@ -261,6 +261,30 @@ int fpm_match_sharded(fpm_handle* h, const uint8_t* src, int width, int height, 
                       fpm_result* out, int cap, int* n);
 int fpm_match_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
                               fpm_result* out /* nranks*cap */, int cap, int* n /* nranks */);
+/* ---- template sets in the angle-sharded latency mode: one frame against the whole set across the ranks ----
+ * fpm_match_set_sharded: collective; src is this rank's copy of the SAME frame (host, or device with src_on_device = 1).
+ *   Template t's list goes to out + t*cap and its total to counts[t] (n = fpm_set_size).  On every rank the lists are
+ *   bit-identical to what fpm_match_set_batch returns for the frame on one GPU (batch of 1, same cap).  Every group of the set
+ *   sweeps this rank's chunk of its angle schedule (fpm_shard_angle_range) for all its templates, and the call issues the
+ *   collectives of a one-template call however many groups the set has: two allgathers, plus one when a host frame is uploaded
+ *   in slices (FPM_PARAM_SHARD_UPLOAD).  Refuses (FPM_ERR_INVALID, with a message) what fpm_match_set_batch refuses, and more
+ *   than one rank without a communicator.  A handle with nothing learned returns empty lists.
+ * fpm_match_set_sharded_merged: the same, merged as fpm_match_set_batch_merged does for one frame: one labelled list at out /
+ *   labels, its total in *count, the per-template totals in set_counts (NULL: not written).  Also refuses a NaN or infinite
+ *   max_overlap, and NULL labels while cap > 0.
+ * The _virtual calls: nranks handles of ONE device play the ranks (none may have a communicator, all hold sets of one size);
+ *   the exchanges are device-to-device block copies, each round counted as one collective in fpm_collective_count of every
+ *   handle.  Rank r's lists go to out + r*n*cap and counts + r*n; merged, to out + r*cap, labels + r*cap, count[r] and
+ *   set_counts + r*n. */
+int fpm_match_set_sharded(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                          fpm_result* out, int cap, int* counts);
+int fpm_match_set_sharded_merged(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                                 double max_overlap, fpm_result* out, int* labels, int cap, int* count, int* set_counts);
+int fpm_match_set_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
+                                  fpm_result* out, int cap, int* counts);
+int fpm_match_set_sharded_merged_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height,
+                                         int stride, double max_overlap, fpm_result* out, int* labels, int cap, int* count,
+                                         int* set_counts);
 /* contiguous chunk [a0, a1) of an n_angles schedule swept by `rank` (host arithmetic, no device needed) */
 int fpm_shard_angle_range(int n_angles, int nranks, int rank, int* a0, int* a1);
 /* number of NCCL collectives issued by this handle since creation */
