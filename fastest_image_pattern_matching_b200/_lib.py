@@ -36,6 +36,7 @@ SIGNATURES = {
     "fpm_get_param": (_d, [_vp, _i]),
     "fpm_learn": (_i, [_vp, _vp, _i, _i, _i]),
     "fpm_learn_set": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
+    "fpm_learn_masked": (_i, [_vp, _vp, _i, _i, _i, _vp, _i]),
     "fpm_set_size": (_i, [_vp]),
     "fpm_match_set_batch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _vp, _i, _vp]),
     "fpm_match_ingested_set_batch": (_i, [_vp, _vp, _i, _vp]),
@@ -76,6 +77,7 @@ SIGNATURES = {
     "fpm_tpl_levels": (_i, [_vp]),
     "fpm_tpl_level_info": (_i, [_vp, _i, _pi, _pi, _pd, _pd, _pd, _pi]),
     "fpm_tpl_level_pixels": (_i, [_vp, _i, _vp]),
+    "fpm_tpl_level_mask": (_i, [_vp, _i, _vp]),
     "fpm_tpl_border_color": (_i, [_vp]),
     "fpm_stage_num_angles": (_i, [_vp, _i, _i]),
     "fpm_stage_top": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _i, _vp, _i, _pi]),

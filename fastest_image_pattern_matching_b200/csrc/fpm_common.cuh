@@ -44,6 +44,10 @@ struct FpmTplLevel {
     int n_tpl;              // templates in the group (1: a single template, stats unused)
     size_t tpl_stride;
     const FpmTplStat* stats;
+    // masked template (fpm_learn_masked): the kept pixels of row y are the column ranges [b, e) of
+    // mrun[mrow[y] .. mrow[y + 1]); the pixels at ptr are already multiplied by the mask.  null: every pixel is kept.
+    const int* mrow;
+    const int2* mrun;
 };
 
 // template k of a group level

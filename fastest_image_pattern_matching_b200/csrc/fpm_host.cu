@@ -138,6 +138,11 @@ struct TplLevelHost {
     std::vector<uint8_t> pix;    // w*h
     size_t tpl_stride = 0;       // template groups: bytes from one member's level to the next one's
     size_t stat_off = 0;         // template groups: index of member 0's FpmTplStat of this level in d_tstat
+    // masked template: M_L as 0/1 bytes (w*h), its kept count, and where its run table starts in d_mruns
+    // (h + 1 int offsets, then the int2 runs); empty mask = every pixel kept
+    std::vector<uint8_t> mask;
+    long long n_kept = 0;
+    size_t run_off = 0, run_data_off = 0;
 };
 
 struct TopPlan {                  // cached per (source size, parameters); always the WHOLE angle schedule
@@ -202,6 +207,8 @@ struct fpm_handle {
     int learned_mra = -1;
     int border = 0;
     std::vector<SetTpl> set;       // the learned templates (fpm_learn: one), kept for re-learning when MinReduceArea changes
+    std::vector<uint8_t> mask0;    // fpm_learn_masked: the level-0 mask of set[0] as 0/1 bytes (empty: unmasked)
+    DevBuf d_mruns, d_mpyr, d_mwS, d_mwQ;   // masked template: run tables, mask pyramid at learn time, refinement window sums
     std::vector<TplGroup> groups;  // their groups; groups[0]'s state is in the fields below (see TplGroup)
     DevBuf d_tstat;                // FpmTplStat of every (group, level, member)
     DevBuf d_members;              // the members of every group, group after group (merged set results: output rows)
@@ -284,14 +291,15 @@ namespace {
 // CNT_LAYER + l: candidates entering pyramid layer l (descent without host round trips)
 enum { CNT_FLAT = 0, CNT_NEXT = 1, CNT_REFINED = 2, CNT_TOTAL = 3, CNT_ERR = 4, CNT_LAYER = 8, CNT_N = 8 + FPM_MAX_LEVELS };
 enum { K_PYRDOWN = 0, K_WARP_TOP, K_TOP_SCORE, K_TOP_PEAKS, K_COLLECT, K_PREP, K_WARP_ROI, K_CORR, K_FINALIZE, K_FINAL, K_CORR_MMA, K_CORR_FUSED, K_CORR_WARP,
-       K_JPEG_UPLOAD, K_JPEG_UNSTUFF, K_JPEG_PASSES, K_JPEG_SCAN, K_JPEG_WRITE, K_JPEG_IDCT, K_SET_MERGE, K_COUNT };
+       K_JPEG_UPLOAD, K_JPEG_UNSTUFF, K_JPEG_PASSES, K_JPEG_SCAN, K_JPEG_WRITE, K_JPEG_IDCT, K_SET_MERGE, K_TOP_SCORE_MASKED,
+       K_MASK_WINDOW, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"fpm_pyrdown_kernel", "fpm_warp_kernel(top)", "fpm_top_score_kernel", "fpm_top_peaks_kernel",
                                            "fpm_collect_sort_kernel", "fpm_refine_prep_kernel", "fpm_warp_kernel(roi)",
                                            "fpm_corr_rows_kernel", "fpm_refine_finalize_kernel", "fpm_final_kernel",
                                            "fpm_corr_mma_kernel", "fpm_corr_fused_kernel", "fpm_corr_warp_kernel",
                                            "jpeg_upload(H2D copy)", "fpm_jpeg_unstuff_count/write_kernel", "fpm_jpeg_cold/sync_kernel(passes)",
                                            "fpm_jpeg_block_tile/dc_tile/offsets_kernel(scans)", "fpm_jpeg_write_kernel", "fpm_ingest_jpeg_idct_kernel",
-                                           "fpm_set_merge_kernel"};
+                                           "fpm_set_merge_kernel", "fpm_top_score_kernel(masked)", "fpm_mask_window_kernel"};
 static_assert(K_COUNT <= 24, "profile arrays");
 
 cudaEvent_t prof_event(fpm_handle* h)
@@ -350,6 +358,8 @@ FpmTplLevel tpl_level_dev(const fpm_handle* h, int l)
     d.n_tpl = std::max((int)h->members.size(), 1);
     d.tpl_stride = t.tpl_stride;
     d.stats = d.n_tpl > 1 ? h->d_tstat.as<FpmTplStat>() + t.stat_off : nullptr;
+    d.mrow = t.mask.empty() ? nullptr : reinterpret_cast<const int*>(h->d_mruns.as<uint8_t>() + t.run_off);
+    d.mrun = t.mask.empty() ? nullptr : reinterpret_cast<const int2*>(h->d_mruns.as<uint8_t>() + t.run_data_off);
     return d;
 }
 
@@ -438,10 +448,11 @@ CorrCfg corr_config(int tpl_h, bool per_eval_tpl = false)
     return c;
 }
 
-inline size_t top_score_smem(int tw, int th)
+// masked: row prefix sums of TS_TW + tw entries in place of the TS_TW row-window sums
+inline size_t top_score_smem(int tw, int th, bool masked = false)
 {
-    size_t nwt = (tw + 3) / 4, pww = TS_TW / 4 + nwt + 1;
-    return 4 * ((size_t)th * nwt + (size_t)(TS_TH + th - 1) * (pww + 2 * TS_TW)) + 16;   // template, patch, row-window sums
+    size_t nwt = (tw + 3) / 4, pww = TS_TW / 4 + nwt + 1, rs_w = masked ? TS_TW + tw : TS_TW;
+    return 4 * ((size_t)th * nwt + (size_t)(TS_TH + th - 1) * (pww + 2 * rs_w)) + 16;   // template, patch, row-window sums
 }
 
 inline int level_vec_ok(const FpmLevel& L)
@@ -612,9 +623,11 @@ bool fw_box_fits(int vec)
     return worst[vec] <= FW_BOX_BYTES;
 }
 
+// A masked template takes the mode-1 route: its window sums are computed from the ROI patches in HBM, which this kernel
+// never writes.
 bool corr_warp_usable(const fpm_handle* h, int tw, int n_ang, const FpmLevel& L)
 {
-    if (h->use_tc != 6 || h->members.size() > 1) return false;   // opt-in: bit-identical, less DRAM traffic, but slower than warp + MMA today
+    if (h->use_tc != 6 || h->members.size() > 1 || !h->mask0.empty()) return false;   // opt-in: bit-identical, less DRAM traffic, but slower than warp + MMA today
     if (n_ang != 3 || tw < 64 || !get_encode_tiled()) return false;
     return level_copy_vec(L) >= 4 && fw_box_fits(4);       // the box is staged with 4-byte copies
 }
@@ -643,6 +656,24 @@ int launch_corr_warp(fpm_handle* h, const FpmLevel& L, const FpmWarpJob* jobs, c
     return FPM_OK;
 }
 
+// masked template: the 49 window sums of every eval, int64 [e][49] in d_mwS / d_mwQ, from the ROI patches in d_roi
+int launch_mask_window(fpm_handle* h, int rpitch, size_t roi_stride, const FpmTplLevel& td, int ne, const int* n_cands_dev, int n_ang)
+{
+    const int pstride = (int)align_up(td.w + FPM_ROI_PAD + 1, 4);                 // prefix entries of one ROI row
+    const size_t per_warp = 2 * sizeof(uint32_t) * (size_t)pstride;
+    if (per_warp > 200 * 1024) { h->err = "masked template too wide for the window-sum kernel"; return FPM_ERR_LIMIT; }
+    const int warps = (int)std::min<size_t>(MW_MAX_WARPS, std::max<size_t>(1, 64 * 1024 / per_warp));   // <= 64 KB per CTA
+    const size_t smem = warps * per_warp;
+    CK(ensure_dyn_smem((const void*)fpm_mask_window_kernel, h->device, smem));
+    CK(h->d_mwS.ensure((size_t)ne * FPM_NCELL * sizeof(long long)));
+    CK(h->d_mwQ.ensure((size_t)ne * FPM_NCELL * sizeof(long long)));
+    // algorithmic work: one pass over the ROI patch (bytes)
+    KL(K_MASK_WINDOW, (double)ne * (td.w + FPM_ROI_PAD) * (td.h + FPM_ROI_PAD),
+       fpm_mask_window_kernel<<<ne, warps * 32, smem, h->stream>>>(h->d_roi.as<uint8_t>(), rpitch, roi_stride, td, ne, pstride,
+                                                                   h->d_mwS.as<long long>(), h->d_mwQ.as<long long>(), n_cands_dev, n_ang));
+    return FPM_OK;
+}
+
 // ---- learnPattern, src/TemplateMatcher.cpp:45-95, for every template of the set ---------------------
 // Device layout: group by group and level by level, the members of a group level back to back (a set of one: today's
 // single-template layout).  Each group's template pyramids are built by one pyramid chain over its members.
@@ -653,11 +684,13 @@ int do_learn(fpm_handle* h)
     for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
     h->groups.clear();
     std::vector<TplGroup> gs;
+    const bool masked = !h->mask0.empty();                        // fpm_learn_masked: a set of one
     for (int i = 0; i < (int)h->set.size(); i++) {
         const SetTpl& st = h->set[i];
-        unsigned long long S = 0;
-        for (uint8_t v : st.px) S += v;
-        const int border = ((double)S / ((double)st.h * st.w)) < 128 ? 255 : 0;     // iBorderColor (:58-59)
+        unsigned long long S = 0, N = 0;
+        for (size_t k = 0; k < st.px.size(); k++)
+            if (!masked || h->mask0[k]) { S += st.px[k]; N++; }
+        const int border = ((double)S / (double)N) < 128 ? 255 : 0;     // iBorderColor (:58-59), over the kept pixels
         size_t g = 0;
         while (g < gs.size() && !(gs[g].w0 == st.w && gs[g].h0 == st.h && gs[g].border == border)) g++;
         if (g == gs.size()) { gs.emplace_back(); gs[g].w0 = st.w; gs[g].h0 = st.h; gs[g].border = border; }
@@ -700,14 +733,32 @@ int do_learn(fpm_handle* h)
         int rc = launch_pyramid_chain(h, lv, top, T);
         if (rc) return rc;
     }
-    CK(h->d_tsh.ensure(toff));
-    for (const TplGroup& G : gs) {
-        if (G.members.size() != 1) continue;
-        for (const TplLevelHost& t : G.tpl) {
-            dim3 g((t.bpitch + 127) / 128, t.h, 8);
-            fpm_shift_template_kernel<<<g, 128, 0, h->stream>>>(h->d_tpl.as<uint8_t>() + t.dev_off, t.w, t.h, t.pitch,
-                                                                h->d_tsh.as<uint8_t>() + t.tsh_off, t.bpitch);
-            CKL();
+    // mask pyramid: M_{L+1} = (pyrDown(255 * M_L) >= 128), one level per launch of the pyramid kernel
+    std::vector<std::vector<uint8_t>> mk;
+    if (masked) {
+        const std::vector<TplLevelHost>& tl = gs[0].tpl;
+        mk.assign(tl.size(), std::vector<uint8_t>());
+        mk[0] = h->mask0;
+        CK(h->d_mpyr.ensure(off));
+        uint8_t* mb = h->d_mpyr.as<uint8_t>();
+        for (size_t l = 1; l < tl.size(); l++) {
+            const TplLevelHost &a = tl[l - 1], &b = tl[l];
+            std::vector<uint8_t> up(mk[l - 1].size()), dn((size_t)b.w * b.h);
+            for (size_t i = 0; i < up.size(); i++) up[i] = mk[l - 1][i] ? 255 : 0;
+            CK(cudaMemcpy2DAsync(mb + a.dev_off, a.pitch, up.data(), a.w, a.w, a.h, cudaMemcpyHostToDevice, h->stream));
+            int rc = launch_pyrdown(h, FpmLevel{mb + a.dev_off, a.w, a.h, a.pitch, 0}, FpmLevel{mb + b.dev_off, b.w, b.h, b.pitch, 0},
+                                    nullptr, 1);
+            if (rc) return rc;
+            CK(cudaMemcpy2DAsync(dn.data(), b.w, mb + b.dev_off, b.pitch, b.w, b.h, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaStreamSynchronize(h->stream));
+            size_t n = 0;
+            for (uint8_t& v : dn) { v = v >= 128 ? 1 : 0; n += v; }
+            if (n == 0) {
+                h->err = "fpm_learn_masked: the mask keeps no pixel at pyramid level " + std::to_string(l) + " (" + std::to_string(b.w) +
+                         "x" + std::to_string(b.h) + "); enlarge the kept region or lower FPM_PARAM_MIN_REDUCE_AREA";
+                return FPM_ERR_INVALID;
+            }
+            mk[l].swap(dn);
         }
     }
     std::vector<uint8_t> all(off);
@@ -715,19 +766,24 @@ int do_learn(fpm_handle* h)
     CK(cudaStreamSynchronize(h->stream));
     std::vector<FpmTplStat> stats(n_stat);
     for (TplGroup& G : gs)
-        for (TplLevelHost& t : G.tpl)
+        for (size_t l = 0; l < G.tpl.size(); l++)
             for (size_t k = 0; k < G.members.size(); k++) {
+                TplLevelHost& t = G.tpl[l];
                 const uint8_t* base = all.data() + t.dev_off + k * t.tpl_stride;
-                unsigned long long S = 0, Q = 0;
+                const uint8_t* m = masked ? mk[l].data() : nullptr;
+                unsigned long long S = 0, Q = 0, n = 0;
                 for (int y = 0; y < t.h; y++)
-                    for (int x = 0; x < t.w; x++) { const unsigned v = base[(size_t)y * t.pitch + x]; S += v; Q += (unsigned long long)v * v; }
-                double N = (double)t.h * t.w;
+                    for (int x = 0; x < t.w; x++) {
+                        if (m && !m[(size_t)y * t.w + x]) continue;
+                        const unsigned v = base[(size_t)y * t.pitch + x]; S += v; Q += (unsigned long long)v * v; n++;
+                    }
+                double N = (double)n;                              // the kept pixels (all of them without a mask)
                 // cv::meanStdDev (u8): scale = 1/N; mean = S*scale; var = max(Q*scale - mean^2, 0); sdv = sqrt(var)
                 double scale = 1.0 / N;
                 double mean = (double)S * scale;
                 double var = std::max((double)Q * scale - mean * mean, 0.0);
                 double sdv = sqrt(var);
-                double invArea = 1.0 / ((double)t.h * t.w);
+                double invArea = 1.0 / N;
                 double templNorm = sdv * sdv;                       // :74
                 const int equal1 = templNorm < DBL_EPSILON ? 1 : 0; // :77
                 templNorm = sqrt(templNorm);                        // :85
@@ -739,6 +795,45 @@ int do_learn(fpm_handle* h)
                     for (int y = 0; y < t.h; y++) memcpy(t.pix.data() + (size_t)y * t.w, base + (size_t)y * t.pitch, t.w);
                 }
             }
+    if (masked) {
+        // the correlation kernels see M_L * T_L; the window sums walk the runs of kept pixels of every row
+        std::vector<uint8_t> runs;
+        std::vector<uint8_t> tm(off, 0);
+        for (size_t l = 0; l < gs[0].tpl.size(); l++) {
+            TplLevelHost& t = gs[0].tpl[l];
+            t.mask = mk[l];
+            t.n_kept = 0;
+            std::vector<int> rows(1, 0), rr;
+            for (int y = 0; y < t.h; y++) {
+                const uint8_t* m = t.mask.data() + (size_t)y * t.w;
+                for (int x = 0; x < t.w; x++) {
+                    tm[t.dev_off + (size_t)y * t.pitch + x] = m[x] ? t.pix[(size_t)y * t.w + x] : 0;
+                    t.n_kept += m[x];
+                    if (m[x] && (x == 0 || !m[x - 1])) rr.push_back(x);
+                    if (m[x] && (x == t.w - 1 || !m[x + 1])) rr.push_back(x + 1);
+                }
+                rows.push_back((int)rr.size() / 2);
+            }
+            t.run_off = align_up(runs.size(), 16);
+            t.run_data_off = align_up(t.run_off + rows.size() * sizeof(int), 16);
+            runs.resize(t.run_data_off + rr.size() * sizeof(int));
+            memcpy(runs.data() + t.run_off, rows.data(), rows.size() * sizeof(int));
+            memcpy(runs.data() + t.run_data_off, rr.data(), rr.size() * sizeof(int));
+        }
+        CK(cudaMemcpy(h->d_tpl.p, tm.data(), off, cudaMemcpyHostToDevice));
+        CK(h->d_mruns.ensure(runs.size()));
+        CK(cudaMemcpy(h->d_mruns.p, runs.data(), runs.size(), cudaMemcpyHostToDevice));
+    }
+    CK(h->d_tsh.ensure(toff));
+    for (const TplGroup& G : gs) {
+        if (G.members.size() != 1) continue;
+        for (const TplLevelHost& t : G.tpl) {
+            dim3 g((t.bpitch + 127) / 128, t.h, 8);
+            fpm_shift_template_kernel<<<g, 128, 0, h->stream>>>(h->d_tpl.as<uint8_t>() + t.dev_off, t.w, t.h, t.pitch,
+                                                                h->d_tsh.as<uint8_t>() + t.tsh_off, t.bpitch);
+            CKL();
+        }
+    }
     CK(h->d_tstat.ensure(n_stat * sizeof(FpmTplStat)));
     CK(cudaMemcpy(h->d_tstat.p, stats.data(), n_stat * sizeof(FpmTplStat), cudaMemcpyHostToDevice));
     std::vector<int> members;
@@ -898,11 +993,11 @@ int run_top(fpm_handle* h, int top, int j0, int nj, FpmPick* picks_out, int* cnt
                                              std::max<size_t>(1, budget / ((size_t)n_tpl * score_stride * sizeof(float)))});
     CK(h->d_rot.ensure(rot_stride * chunk));
     CK(h->d_score.ensure(score_stride * chunk * n_tpl * sizeof(float)));
-    const size_t smem_ts = top_score_smem(t.w, t.h);
+    const bool masked = !t.mask.empty();
+    const size_t smem_ts = top_score_smem(t.w, t.h, masked);
     if (smem_ts > 200 * 1024) { h->err = "top-layer template too large for the score kernel"; return FPM_ERR_LIMIT; }
-    if (smem_ts > 48 * 1024)
-        CK(ensure_dyn_smem(n_tpl > 1 ? (const void*)fpm_top_score_kernel<true> : (const void*)fpm_top_score_kernel<false>, h->device, smem_ts));
-    const auto score_kernel = n_tpl > 1 ? fpm_top_score_kernel<true> : fpm_top_score_kernel<false>;
+    const auto score_kernel = n_tpl > 1 ? fpm_top_score_kernel<true> : (masked ? fpm_top_score_kernel<false, true> : fpm_top_score_kernel<false>);
+    if (smem_ts > 48 * 1024) CK(ensure_dyn_smem((const void*)score_kernel, h->device, smem_ts));
     // bCalMaxByBlock, src/TemplateMatcher.cpp:158-159
     const FpmLevel& L = h->levels[top];
     const bool by_block = ((L.w * L.h) / (t.w * t.h) > 500) && h->max_pos > 10;
@@ -930,7 +1025,7 @@ int run_top(fpm_handle* h, int top, int j0, int nj, FpmPick* picks_out, int* cnt
                                                                 h->border, tiles_x, level_vec_ok(h->levels[top]), nullptr, FpmRefineGeom{}));
         dim3 grid((maxRW + TS_TW - 1) / TS_TW, (maxRH + TS_TH - 1) / TS_TH, nc);
         dim3 block(TS_THREADS);
-        KL(K_TOP_SCORE, (double)nc * n_tpl * maxRW * maxRH * t.w * t.h,      // MACs
+        KL(masked ? K_TOP_SCORE_MASKED : K_TOP_SCORE, (double)nc * n_tpl * maxRW * maxRH * t.w * t.h,      // MACs
            score_kernel<<<grid, block, smem_ts, h->stream>>>(jobs + c0, h->d_rot.as<uint8_t>(), rpitch, rot_stride,
                                                                      tpl_level_dev(h, top), h->d_score.as<float>(), spitch,
                                                                      score_stride, top_reject_below(h, top)));
@@ -964,6 +1059,7 @@ RefineLayer refine_layer(const fpm_handle* h, int layer, int n_ang)
     if (mma_usable(h, t.w) || mma_narrow_fused(h, t.w))
         r.per_eval += std::max((size_t)(t.h + FPM_ROI_PAD) * MM_N * 4, (size_t)MM_N * 4 + 2 * FPM_NSHIFT * 8);
     if (!mma_usable(h, t.w)) r.per_eval += (size_t)t.h * FPM_NCELL * 4;
+    if (!t.mask.empty()) r.per_eval += 2 * FPM_NCELL * sizeof(long long);   // masked window sums
     return r;
 }
 
@@ -1099,6 +1195,11 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                                                                                     cands + c0));
                 }
             }
+            const bool masked = td.mrun && !t.equal1;
+            if (masked) {
+                int rcm = launch_mask_window(h, rpitch, roi_stride, td, ne, n_dev, n_ang);
+                if (rcm) return rcm;
+            }
             {
                 auto fin = n_tpl > 1 ? fpm_refine_finalize_kernel<true> : fpm_refine_finalize_kernel<false>;
                 KL(K_FINALIZE, (double)ne * ((double)t.h * FPM_NCELL * 4 + 2.0 * (t.h + FPM_ROI_PAD) * FPM_NSHIFT * 4),
@@ -1110,7 +1211,8 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                        next_cnt, ref_out, ref_cnt,
                        h->trace ? h->d_trace.as<FpmEvalTrace>() + (size_t)c0 * n_ang : nullptr,
                        h->trace ? h->d_trace_sc.as<float>() + (size_t)c0 * n_ang * FPM_NCELL : nullptr,
-                       fused ? h->d_numer.as<float>() : nullptr, h->d_totS.as<long long>(), h->d_totQ.as<long long>(), raw_tile_evals, n_dev));
+                       fused ? h->d_numer.as<float>() : nullptr, (masked ? h->d_mwS : h->d_totS).as<long long>(),
+                       (masked ? h->d_mwQ : h->d_totQ).as<long long>(), raw_tile_evals, n_dev));
             }
             if (h->trace && !warp_fused)                    // this wave's ROI patches, before the next wave overwrites them
                 CK(cudaMemcpyAsync(h->tr_rois[layer].px.data() + (size_t)c0 * n_ang * roi_stride, h->d_roi.p, (size_t)ne * roi_stride,
@@ -1924,11 +2026,14 @@ int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stri
     return fpm_learn_set(h, 1, &tpl, &width, &height, &stride);
 }
 
-int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides)
+namespace {
+// fpm_learn_set, with the 0/1 level-0 mask of a masked template (n == 1) or an empty one
+int learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides,
+              std::vector<uint8_t> mask)
 {
-    if (!h) return FPM_ERR_INVALID;
     h->learned = false;
     h->set.clear();
+    h->mask0.clear();
     h->learn_gen++;
     if (n < 1 || !tpls || !widths || !heights || !strides) { h->err = "template set: n < 1 or null arrays"; return FPM_ERR_INVALID; }
     for (int i = 0; i < n; i++)
@@ -1943,9 +2048,40 @@ int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* w
         for (int y = 0; y < heights[i]; y++) memcpy(set[i].px.data() + (size_t)y * widths[i], tpls[i] + (size_t)y * strides[i], widths[i]);
     }
     h->set.swap(set);
+    h->mask0.swap(mask);
     int rc = do_learn(h);
-    if (rc) h->set.clear();
+    if (rc) { h->set.clear(); h->mask0.clear(); }
     return rc;
+}
+}  // namespace
+
+int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides)
+{
+    if (!h) return FPM_ERR_INVALID;
+    return learn_set(h, n, tpls, widths, heights, strides, std::vector<uint8_t>());
+}
+
+int fpm_learn_masked(fpm_handle* h, const uint8_t* tpl, int width, int height, int stride, const uint8_t* mask, int mask_stride)
+{
+    if (!h) return FPM_ERR_INVALID;
+    const char* why = nullptr;
+    if (!tpl || width <= 0 || height <= 0 || stride < width) why = "empty template";
+    else if (!mask) why = "fpm_learn_masked: null mask";
+    else if (mask_stride < width) why = "fpm_learn_masked: mask stride smaller than the template width";
+    std::vector<uint8_t> m;
+    if (!why) {
+        m.resize((size_t)width * height);
+        size_t kept = 0;
+        for (int y = 0; y < height; y++)
+            for (int x = 0; x < width; x++) kept += m[(size_t)y * width + x] = mask[(size_t)y * mask_stride + x] ? 1 : 0;
+        if (!kept) why = "fpm_learn_masked: the mask keeps no pixel";
+    }
+    if (why) {
+        h->learned = false; h->set.clear(); h->mask0.clear(); h->learn_gen++;
+        h->err = why;
+        return FPM_ERR_INVALID;
+    }
+    return learn_set(h, 1, &tpl, &width, &height, &stride, std::move(m));
 }
 
 int fpm_set_size(const fpm_handle* h) { return h && h->learned ? (int)h->set.size() : 0; }
@@ -1955,7 +2091,7 @@ int fpm_is_learned(const fpm_handle* h) { return h && h->learned ? 1 : 0; }
 void fpm_clear(fpm_handle* h)
 {
     if (!h) return;
-    h->learned = false; h->tpl.clear(); h->set.clear(); h->members.clear(); h->has_ur = 0;
+    h->learned = false; h->tpl.clear(); h->set.clear(); h->mask0.clear(); h->members.clear(); h->has_ur = 0;
     for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
     h->groups.clear();
     h->ur[0] = h->ur[1] = h->ur[2] = h->ur[3] = 0;
@@ -1990,7 +2126,7 @@ int ensure_twin(fpm_handle* h)
         std::vector<const uint8_t*> px(n);
         std::vector<int> ws(n), hs(n);
         for (int i = 0; i < n; i++) { px[i] = h->set[i].px.data(); ws[i] = h->set[i].w; hs[i] = h->set[i].h; }
-        int rc = fpm_learn_set(t, n, px.data(), ws.data(), hs.data(), ws.data());
+        int rc = learn_set(t, n, px.data(), ws.data(), hs.data(), ws.data(), h->mask0);
         if (rc) { h->err = t->err; return rc; }
         h->twin_gen = h->learn_gen;
     }
@@ -3069,6 +3205,19 @@ int fpm_tpl_level_info(const fpm_handle* h, int level, int* w, int* hgt, double*
     return FPM_OK;
 }
 
+int fpm_tpl_level_mask(const fpm_handle* h, int level, uint8_t* out)
+{
+    if (h) if (int rc = refuse_set(h, "fpm_tpl_level_mask")) return rc;
+    if (!h || !h->learned || level < 0 || level >= (int)h->tpl.size()) return FPM_ERR_INVALID;
+    const TplLevelHost& t = h->tpl[level];
+    const size_t n = (size_t)t.w * t.h;
+    if (out) {
+        if (t.mask.empty()) memset(out, 1, n);
+        else memcpy(out, t.mask.data(), n);
+    }
+    return t.mask.empty() ? (int)n : (int)t.n_kept;
+}
+
 int fpm_tpl_level_pixels(const fpm_handle* h, int level, uint8_t* out)
 {
     if (h) if (int rc = refuse_set(h, "fpm_tpl_level_pixels")) return rc;
@@ -3512,7 +3661,7 @@ int fpm_dbg_corr_rows(fpm_handle* h, const uint8_t* roi, const uint8_t* tpl, int
     FpmTplLevel td;
     td.ptr = h->d_dbg[1].as<uint8_t>(); td.w = tw; td.h = th; td.pitch = tp;
     td.mean = 0; td.norm = 1; td.inv_area = 1; td.result_equal1 = 0;
-    td.n_tpl = 1; td.tpl_stride = 0; td.stats = nullptr;
+    td.n_tpl = 1; td.tpl_stride = 0; td.stats = nullptr; td.mrow = nullptr; td.mrun = nullptr;
     const CorrCfg cc = corr_config(th);
     if (cc.smem > 200 * 1024) { h->err = "correlation kernel shared memory limit"; return FPM_ERR_LIMIT; }
     if (cc.smem > 48 * 1024)
@@ -3655,11 +3804,13 @@ int fpm_dbg_top_score_production(fpm_handle* h, const uint8_t* img, int w, int h
     jb.dw = w; jb.dh = hgt; jb.valid = 1;
     CK(cudaMemcpy2DAsync(h->d_dbg[0].p, rp, img, w, w, hgt, cudaMemcpyHostToDevice, h->stream));
     CK(cudaMemcpyAsync(h->d_dbg[2].p, &jb, sizeof(jb), cudaMemcpyHostToDevice, h->stream));
-    size_t smem = top_score_smem(t.w, t.h);
+    const bool masked = !t.mask.empty();
+    size_t smem = top_score_smem(t.w, t.h, masked);
     if (smem > 200 * 1024) { h->err = "template too large"; return FPM_ERR_LIMIT; }
-    CK(ensure_dyn_smem((const void*)fpm_top_score_kernel<false>, h->device, smem));
+    const auto kern = masked ? fpm_top_score_kernel<false, true> : fpm_top_score_kernel<false>;
+    CK(ensure_dyn_smem((const void*)kern, h->device, smem));
     dim3 grid((RW + TS_TW - 1) / TS_TW, (RH + TS_TH - 1) / TS_TH, 1), block(TS_THREADS);
-    fpm_top_score_kernel<false><<<grid, block, smem, h->stream>>>(h->d_dbg[2].as<FpmWarpJob>(), h->d_dbg[0].as<uint8_t>(), rp, 0,
+    kern<<<grid, block, smem, h->stream>>>(h->d_dbg[2].as<FpmWarpJob>(), h->d_dbg[0].as<uint8_t>(), rp, 0,
                                                            tpl_level_dev(h, top), h->d_dbg[1].as<float>(), sp, 0,
                                                            reject_below ? top_reject_below(h, top) : -INFINITY);
     CKL();

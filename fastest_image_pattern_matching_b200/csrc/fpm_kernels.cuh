@@ -359,7 +359,11 @@ __device__ __forceinline__ float fpm_ccoeff_epilogue_top(float numerator, double
 // Template groups (tpl.n_tpl > 1): the CTA stages its canvas patch and its row-window sums once and scores the patch
 // against every template of the group in turn; map k of job z is written to score + (z * n_tpl + k) * score_job_stride.
 // GROUP = false (a single template) compiles to the one-template kernel.
-template <bool GROUP>
+// MASKED (a single masked template, tpl.mrun set): the window sums run over the kept pixels only.  Instead of one row-window
+// sum per patch row the CTA keeps row prefix sums of the patch and of its squares, ph x (TS_TW + tw) each, and every score adds
+// P[x + e] - P[x + b] over the runs [b, e) of each template row: exact integers, the same ones a full mask gives through the
+// row-window sums.
+template <bool GROUP, bool MASKED = false>
 __global__ void __launch_bounds__(TS_THREADS)
 fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restrict__ rot, int rpitch,
                      size_t rot_job_stride, FpmTplLevel tpl, float* __restrict__ score, int spitch,
@@ -413,12 +417,42 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
     // that covers patch row yy reuses them, so the main loop only multiplies by the template (the zero padding of
     // the template's last word masks the patch bytes beyond tw there).  The same for every template of a group; not
     // needed when all of them are flat.
-    uint32_t* s_rs = s_t + ((th * nwt + ph * pww + 3) & ~3);   // ph * TS_TW, 16-byte aligned
-    uint32_t* s_rq = s_rs + ph * TS_TW;
+    const int rs_w = MASKED ? TS_TW + tw : TS_TW;              // prefix entries P[0 .. TS_TW + tw - 1] per patch row when MASKED
+    uint32_t* s_rs = s_t + ((th * nwt + ph * pww + 3) & ~3);   // ph * rs_w, 16-byte aligned
+    uint32_t* s_rq = s_rs + ph * rs_w;
     bool need_sums = !tpl.result_equal1;
     if (GROUP)
         for (int k = 1; k < tpl.n_tpl; k++) need_sums |= !tpl.stats[k].result_equal1;
-    if (need_sums) {
+    if (MASKED && need_sums) {
+        // one warp per patch row: each lane takes a word (4 pixels), an inclusive warp scan of the word sums gives the
+        // prefix in front of every word; P[x] = sum of the pixels left of column x
+        const int warp = tid >> 5, lane = tid & 31;
+        for (int yy = warp; yy < ph; yy += TS_THREADS / 32) {
+            uint32_t cs = 0, cq = 0;
+            for (int w0 = 0; 4 * w0 < rs_w; w0 += 32) {
+                const int xw = w0 + lane;
+                const uint32_t v = xw < pww ? s_p[yy * pww + xw] : 0u;
+                const uint32_t b0 = v & 255u, b1 = (v >> 8) & 255u, b2 = (v >> 16) & 255u, b3 = v >> 24;
+                const uint32_t ws = b0 + b1 + b2 + b3, wq = b0 * b0 + b1 * b1 + b2 * b2 + b3 * b3;
+                uint32_t is = ws, iq = wq;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const uint32_t us = __shfl_up_sync(0xffffffffu, is, o), uq = __shfl_up_sync(0xffffffffu, iq, o);
+                    if (lane >= o) { is += us; iq += uq; }
+                }
+                uint32_t ps = cs + is - ws, pq = cq + iq - wq;
+#pragma unroll
+                for (int k = 0; k < 4; k++) {
+                    if (4 * xw + k < rs_w) { s_rs[yy * rs_w + 4 * xw + k] = ps; s_rq[yy * rs_w + 4 * xw + k] = pq; }
+                    const uint32_t bk = (v >> (8 * k)) & 255u;
+                    ps += bk; pq += bk * bk;
+                }
+                cs += __shfl_sync(0xffffffffu, is, 31);
+                cq += __shfl_sync(0xffffffffu, iq, 31);
+            }
+        }
+        __syncthreads();
+    } else if (need_sums) {
         for (int i = tid; i < ph * (TS_TW / 4); i += TS_THREADS) {
             const int yy = i / (TS_TW / 4), xq = i - yy * (TS_TW / 4);
             const uint32_t* prow = s_p + yy * pww + xq;
@@ -444,6 +478,24 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
     const int tx = tid & 15, ty = tid >> 4;
     const int ox = x0 + 4 * tx, oy = y0 + ty;
     const bool live = ox < RW && oy < RH;
+    // window sum / square sum of the 4 scores' windows in template row yy
+    auto window_rows = [&](int yy, uint4& rs, uint4& rq) {
+        const uint32_t* ps = s_rs + (ty + yy) * rs_w + 4 * tx;
+        const uint32_t* pq = s_rq + (ty + yy) * rs_w + 4 * tx;
+        if (!MASKED) {
+            rs = *reinterpret_cast<const uint4*>(ps);
+            rq = *reinterpret_cast<const uint4*>(pq);
+            return;
+        }
+        rs = make_uint4(0, 0, 0, 0); rq = make_uint4(0, 0, 0, 0);
+        for (int k = __ldg(tpl.mrow + yy), ke = __ldg(tpl.mrow + yy + 1); k < ke; k++) {
+            const int2 be = __ldg(tpl.mrun + k);
+            rs.x += ps[be.y] - ps[be.x]; rs.y += ps[be.y + 1] - ps[be.x + 1];
+            rs.z += ps[be.y + 2] - ps[be.x + 2]; rs.w += ps[be.y + 3] - ps[be.x + 3];
+            rq.x += pq[be.y] - pq[be.x]; rq.y += pq[be.y + 1] - pq[be.x + 1];
+            rq.z += pq[be.y + 2] - pq[be.x + 2]; rq.w += pq[be.y + 3] - pq[be.x + 3];
+        }
+    };
     if (!GROUP && !live) return;
     const int n_tpl = GROUP ? tpl.n_tpl : 1;
     for (int kt = 0; kt < n_tpl; kt++) {
@@ -477,8 +529,8 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
                     a[3] = __dp4a(__funnelshift_r(lo, hi, 24), t, a[3]);
                     lo = hi;
                 }
-                const uint4 rs = *reinterpret_cast<const uint4*>(s_rs + (ty + yy) * TS_TW + 4 * tx);
-                const uint4 rq = *reinterpret_cast<const uint4*>(s_rq + (ty + yy) * TS_TW + 4 * tx);
+                uint4 rs, rq;
+                window_rows(yy, rs, rq);
                 b[0] += rs.x; b[1] += rs.y; b[2] += rs.z; b[3] += rs.w;
                 c[0] += rq.x; c[1] += rq.y; c[2] += rq.z; c[3] += rq.w;
             }
@@ -501,8 +553,8 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
                     a[3] = __dp4a(__funnelshift_r(lo, hi, 24), t, a[3]);
                     lo = hi;
                 }
-                const uint4 rs = *reinterpret_cast<const uint4*>(s_rs + (ty + yy) * TS_TW + 4 * tx);
-                const uint4 rq = *reinterpret_cast<const uint4*>(s_rq + (ty + yy) * TS_TW + 4 * tx);
+                uint4 rs, rq;
+                window_rows(yy, rs, rq);
                 num[0] += a[0]; num[1] += a[1]; num[2] += a[2]; num[3] += a[3];   // per-row s32, s64 across rows
                 wsum[0] += rs.x; wsum[1] += rs.y; wsum[2] += rs.z; wsum[3] += rs.w;
                 wsq[0] += rq.x; wsq[1] += rq.y; wsq[2] += rq.z; wsq[3] += rq.w;
@@ -1285,6 +1337,87 @@ __device__ void fpm_subpix(const double* sc27 /* [theta][y][x] */, double xm, do
 }
 
 // =====================================================================================
+// masked refinement window sums (fpm_learn_masked): for every eval and every cell (r, c) of its 7x7 patch the exact sums
+// of the ROI pixels and of their squares under the KEPT template pixels, t = sum M*S and t2 = sum M*S^2, as int64
+// [eval][49] for fpm_refine_finalize_kernel.  One CTA per eval, one warp per ROI row at a time (rows y = warp, warp + nw,
+// ...), no block-wide barrier until the end: the warp turns its row into prefix sums P[x] (the pixels left of column x;
+// u32 is exact, (tw + 6) * 255^2 < 2^32) with one scan of the lanes' 4-pixel words, then each lane adds
+// P[c + e] - P[c + b] over the runs [b, e) of template row y - r for its items of the 98 (cell, sum or square) totals,
+// which it keeps in registers across its rows.  The warps' totals meet in shared memory at the end.  About 49 * (sum of
+// runs) adds per eval against the 49 * w * h MACs of the numerator; a full mask gives the same integers as the row-window
+// sums of the unmasked path.
+// =====================================================================================
+#define MW_MAX_WARPS 8
+
+__global__ void __launch_bounds__(MW_MAX_WARPS * 32)
+fpm_mask_window_kernel(const uint8_t* __restrict__ roi, int rpitch, size_t roi_stride, FpmTplLevel tpl, int ne, int pstride,
+                       long long* __restrict__ totS, long long* __restrict__ totQ, const int* __restrict__ n_cands_dev, int n_ang)
+{
+    extern __shared__ __align__(16) uint32_t s_pre[];        // per warp: pstride pixel prefix sums, then pstride square ones
+    __shared__ unsigned long long s_tot[2 * FPM_NCELL];
+    const int e = blockIdx.x;
+    if (e >= ne || (n_cands_dev && e >= *n_cands_dev * n_ang)) return;
+    const int th = tpl.h, rw = tpl.w + FPM_ROI_PAD, rh = th + FPM_ROI_PAD, pl = rw + 1;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nw = blockDim.x >> 5;
+    for (int i = tid; i < 2 * FPM_NCELL; i += blockDim.x) s_tot[i] = 0;
+    uint32_t* s_ps = s_pre + (size_t)warp * 2 * pstride;
+    uint32_t* s_pq = s_ps + pstride;
+    const uint8_t* __restrict__ base = roi + (size_t)e * roi_stride;
+    long long acc[4] = {0, 0, 0, 0};                         // items j = lane + 32 k: j < 49 pixel sums of cell j, else squares
+    for (int y = warp; y < rh; y += nw) {
+        const uint32_t* row = reinterpret_cast<const uint32_t*>(base + (size_t)y * rpitch);   // rpitch % 16 == 0
+        uint32_t cs = 0, cq = 0;
+        for (int w0 = 0; 4 * w0 < pl; w0 += 32) {
+            const int xw = w0 + lane;
+            uint32_t v = 4 * xw < rw ? __ldg(row + xw) : 0u;
+            if (4 * xw < rw && 4 * xw + 4 > rw) v &= 0xffffffffu >> (8 * (4 * xw + 4 - rw));
+            const uint32_t b0 = v & 255u, b1 = (v >> 8) & 255u, b2 = (v >> 16) & 255u, b3 = v >> 24;
+            const uint32_t ws = b0 + b1 + b2 + b3, wq = b0 * b0 + b1 * b1 + b2 * b2 + b3 * b3;
+            uint32_t is = ws, iq = wq;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const uint32_t us = __shfl_up_sync(0xffffffffu, is, o), uq = __shfl_up_sync(0xffffffffu, iq, o);
+                if (lane >= o) { is += us; iq += uq; }
+            }
+            const uint32_t ps = cs + is - ws, pq = cq + iq - wq;  // in front of this word
+            if (4 * xw < pl) {                                    // pstride % 4 == 0: the word's 4 entries fit
+                *reinterpret_cast<uint4*>(s_ps + 4 * xw) = make_uint4(ps, ps + b0, ps + b0 + b1, ps + b0 + b1 + b2);
+                *reinterpret_cast<uint4*>(s_pq + 4 * xw) = make_uint4(pq, pq + b0 * b0, pq + b0 * b0 + b1 * b1,
+                                                                      pq + b0 * b0 + b1 * b1 + b2 * b2);
+            }
+            cs += __shfl_sync(0xffffffffu, is, 31);
+            cq += __shfl_sync(0xffffffffu, iq, 31);
+        }
+        __syncwarp();
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const int j = lane + 32 * k;
+            if (j >= 2 * FPM_NCELL) continue;
+            const int cell = j < FPM_NCELL ? j : j - FPM_NCELL;
+            const int r = cell / FPM_NSHIFT, c = cell - r * FPM_NSHIFT, tr = y - r;   // template row over ROI row y in window (r, c)
+            if (tr < 0 || tr >= th) continue;
+            const uint32_t* p = (j < FPM_NCELL ? s_ps : s_pq) + c;
+            uint32_t s = 0;
+            for (int q = __ldg(tpl.mrow + tr), qe = __ldg(tpl.mrow + tr + 1); q < qe; q++) {
+                const int2 be = __ldg(tpl.mrun + q);
+                s += p[be.y] - p[be.x];
+            }
+            acc[k] += s;
+        }
+        __syncwarp();                                        // the next row overwrites this warp's prefix sums
+    }
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < 4; k++) {
+        const int j = lane + 32 * k;
+        if (j < 2 * FPM_NCELL && acc[k]) atomicAdd(&s_tot[j], (unsigned long long)acc[k]);
+    }
+    __syncthreads();
+    for (int i = tid; i < 2 * FPM_NCELL; i += blockDim.x)
+        (i < FPM_NCELL ? totS[(size_t)e * FPM_NCELL + i] : totQ[(size_t)e * FPM_NCELL + i - FPM_NCELL]) = (long long)s_tot[i];
+}
+
+// =====================================================================================
 // refine_finalize: one CTA per candidate, 64 threads per angle.
 //   numerator  = float32 chain over template rows of the exact s32 row sums (reference order,
 //                src/TemplateMatcher.cpp:505-508) or exact s64 total when use_chain == 0
@@ -1321,7 +1454,9 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
     // all th + 6 ROI rows minus the r rows above and the 6 - r rows below it.  The totals are gathered by all 64 threads of
     // the eval (every thread a strided share of the rows, 14 loads per row in flight) instead of a 2*th-load serial loop
     // per cell, which was most of this kernel's time at single-frame latency.
-    const bool coop_window = !tpl.result_equal1 && !numer;
+    // A masked template (tpl.mrun set) takes its 49 window sums per eval from totS / totQ [e][49] (fpm_mask_window_kernel).
+    const bool masked = tpl.mrun != nullptr;
+    const bool coop_window = !tpl.result_equal1 && !numer && !masked;
     if (coop_window) {
         if (tid < 3 * FPM_NSHIFT) { s_totS[tid / FPM_NSHIFT][tid % FPM_NSHIFT] = 0; s_totQ[tid / FPM_NSHIFT][tid % FPM_NSHIFT] = 0; }
         __syncthreads();
@@ -1378,12 +1513,17 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
             // fused tensor-core kernel: the float chain is already folded (column 8c + 7 - r), the window sums are
             // the totals over all ROI rows minus the r rows above and the 6 - r rows below the window
             const float numf = numer[(size_t)e * 64 + c * 8 + (7 - r)];
-            const int rh = th + FPM_ROI_PAD;
-            long long ws = totS[(size_t)e * FPM_NSHIFT + c], wq = totQ[(size_t)e * FPM_NSHIFT + c];
-            const int32_t* ps = rowS + (size_t)e * rh * FPM_WSTRIDE + c;
-            const int32_t* pq = rowQ + (size_t)e * rh * FPM_WSTRIDE + c;
-            for (int y = 0; y < r; y++) { ws -= ps[(size_t)y * FPM_WSTRIDE]; wq -= pq[(size_t)y * FPM_WSTRIDE]; }
-            for (int y = r + th; y < rh; y++) { ws -= ps[(size_t)y * FPM_WSTRIDE]; wq -= pq[(size_t)y * FPM_WSTRIDE]; }
+            long long ws, wq;
+            if (masked) {
+                ws = totS[(size_t)e * FPM_NCELL + cell]; wq = totQ[(size_t)e * FPM_NCELL + cell];
+            } else {
+                const int rh = th + FPM_ROI_PAD;
+                ws = totS[(size_t)e * FPM_NSHIFT + c]; wq = totQ[(size_t)e * FPM_NSHIFT + c];
+                const int32_t* ps = rowS + (size_t)e * rh * FPM_WSTRIDE + c;
+                const int32_t* pq = rowQ + (size_t)e * rh * FPM_WSTRIDE + c;
+                for (int y = 0; y < r; y++) { ws -= ps[(size_t)y * FPM_WSTRIDE]; wq -= pq[(size_t)y * FPM_WSTRIDE]; }
+                for (int y = r + th; y < rh; y++) { ws -= ps[(size_t)y * FPM_WSTRIDE]; wq -= pq[(size_t)y * FPM_WSTRIDE]; }
+            }
             sc = fpm_ccoeff_epilogue(numf, (double)ws, (double)wq, tpl.mean, tpl.norm, tpl.inv_area);
         } else {
             // row sums either as [e][tr][49] (dp4a kernel) or as raw[y][e_pad][64] with y = tr + r and
@@ -1426,9 +1566,14 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
                 for (int tr = 0; tr < th; tr++) acc += rs[(size_t)tr * rstride];
                 numf = (float)acc;
             }
-            long long ws = (long long)s_totS[j][c], wq = (long long)s_totQ[j][c];
-            for (int y = 0; y < r; y++) { ws -= s_edgeS[j][y][c]; wq -= s_edgeQ[j][y][c]; }
-            for (int y = r; y < FPM_ROI_PAD; y++) { ws -= s_edgeS[j][FPM_ROI_PAD + y][c]; wq -= s_edgeQ[j][FPM_ROI_PAD + y][c]; }   // ROI rows th + r .. th + 5
+            long long ws, wq;
+            if (masked) {
+                ws = totS[(size_t)e * FPM_NCELL + cell]; wq = totQ[(size_t)e * FPM_NCELL + cell];
+            } else {
+                ws = (long long)s_totS[j][c]; wq = (long long)s_totQ[j][c];
+                for (int y = 0; y < r; y++) { ws -= s_edgeS[j][y][c]; wq -= s_edgeQ[j][y][c]; }
+                for (int y = r; y < FPM_ROI_PAD; y++) { ws -= s_edgeS[j][FPM_ROI_PAD + y][c]; wq -= s_edgeQ[j][FPM_ROI_PAD + y][c]; }   // ROI rows th + r .. th + 5
+            }
             sc = fpm_ccoeff_epilogue(numf, (double)ws, (double)wq, tpl.mean, tpl.norm, tpl.inv_area);
         }
         s_sc[j][cell] = sc;

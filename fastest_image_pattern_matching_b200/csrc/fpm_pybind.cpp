@@ -42,10 +42,15 @@ PYBIND11_MODULE(fpm_b200_pybind, m)
         .def("clearPattern", &fpm::TemplateMatcher::clearPattern)
         .def("hasUserDefinedRect", &fpm::TemplateMatcher::hasUserDefinedRect)
         .def("learnPattern",
-             [](fpm::TemplateMatcher& self, Img t) {
+             [](fpm::TemplateMatcher& self, Img t, py::object mask) {
                  if (t.ndim() != 2 || t.size() == 0) return false;
-                 return self.learnPattern(t.data(), (int)t.shape(1), (int)t.shape(0), (int)t.strides(0));
-             })
+                 if (mask.is_none()) return self.learnPattern(t.data(), (int)t.shape(1), (int)t.shape(0), (int)t.strides(0));
+                 Img m = mask.cast<Img>();
+                 if (m.ndim() != 2 || m.shape(0) != t.shape(0) || m.shape(1) != t.shape(1))
+                     throw std::invalid_argument("mask must be a 2-D array of the template's shape");
+                 return self.learnPattern(t.data(), (int)t.shape(1), (int)t.shape(0), (int)t.strides(0), m.data(), (int)m.strides(0));
+             },
+             py::arg("tpl"), py::arg("mask") = py::none())
         .def("match", [](fpm::TemplateMatcher& self, Img s) {
             if (s.ndim() != 2 || s.size() == 0) return std::vector<fpm::SingleTargetMatch>();
             const unsigned char* p = s.data();

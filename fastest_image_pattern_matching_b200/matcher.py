@@ -128,12 +128,21 @@ class TemplateMatcher:
     def launchCount(self) -> int: return int(self._lib.fpm_launch_count(self._h))
 
     # ---- learnPattern (src/TemplateMatcher.cpp:45-95) ----
-    def learnPattern(self, templateImage) -> bool:
+    def learnPattern(self, templateImage, mask=None) -> bool:
+        """mask (optional): a 2-D array of the template's shape, nonzero = kept pixel; the masked pixels do not count
+        (fpm_learn_masked).  Without a mask the whole rectangle is matched."""
         if templateImage is None or np.asarray(templateImage).size == 0:
             return False
         t = _as_u8_2d(templateImage)
         self._tpl_keepalive = t
-        self._check(self._lib.fpm_learn(self._h, t.ctypes.data, t.shape[1], t.shape[0], t.strides[0]))
+        if mask is None:
+            self._check(self._lib.fpm_learn(self._h, t.ctypes.data, t.shape[1], t.shape[0], t.strides[0]))
+            return True
+        m = np.ascontiguousarray(np.asarray(mask) != 0, dtype=np.uint8)
+        if m.shape != t.shape:
+            raise ValueError(f"mask shape {m.shape} differs from the template's {t.shape}")
+        self._check(self._lib.fpm_learn_masked(self._h, t.ctypes.data, t.shape[1], t.shape[0], t.strides[0],
+                                               m.ctypes.data, m.strides[0]))
         return True
 
     # ---- template sets: n templates in one handle, matched in shared launches (fpm_learn_set) ----
@@ -388,8 +397,11 @@ class TemplateMatcher:
                                                      C.byref(inv), C.byref(eq)))
             pix = np.empty((h.value, w.value), np.uint8)
             self._check(self._lib.fpm_tpl_level_pixels(self._h, l, pix.ctypes.data))
+            mask = np.empty((h.value, w.value), np.uint8)
+            n_kept = self._lib.fpm_tpl_level_mask(self._h, l, mask.ctypes.data)
+            self._check(min(n_kept, 0))
             out.append(dict(w=w.value, h=h.value, mean=mean.value, norm=norm.value, inv_area=inv.value,
-                            result_equal1=bool(eq.value), pixels=pix))
+                            result_equal1=bool(eq.value), pixels=pix, mask=mask, n_kept=n_kept))
         return out
 
     def borderColor(self) -> int: return self._lib.fpm_tpl_border_color(self._h)

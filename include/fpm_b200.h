@@ -104,6 +104,18 @@ int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stri
  * fpm_match_set_batch with FPM_PARAM_TRACE on).  fpm_match_set_sharded* run a set in the angle-sharded mode.  FPM_PARAM_MIN_REDUCE_AREA changed after learning re-learns the whole set. */
 int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides);
 int fpm_set_size(const fpm_handle* h);              /* 0 = nothing learned, 1 after fpm_learn */
+/* Masked template (a don't-care mask, like cv::matchTemplate(..., mask) with TM_CCOEFF_NORMED): mask is u8 of the template's
+ * size, `mask_stride` bytes per row, a nonzero byte keeps the pixel.  M_0 = (mask != 0); M_{L+1} = (pyrDown(255 * M_L) >= 128).
+ * The template pyramid T_L is built from the whole template as fpm_learn builds it.  Every level's mean / norm / inv_area come
+ * from the exact sums over the kept pixels (n_L = sum M_L, inv_area = 1 / n_L), the border colour from the kept mean of level 0.
+ * At every placement the numerator is the one of the template M_L * T_L and the window sums t, t2 run over the kept pixels only;
+ * rectangles, corners, NMS and sub-pixel fitting use the template rectangle.  A full mask gives bit for bit fpm_learn's results.
+ * Works on every single-template entry point (not in sets).  FPM_PARAM_TENSOR_CORES = 6 takes the mode-1 route on a masked
+ * handle (its window sums need the ROI patches in memory).  FPM_ERR_INVALID with a message for a null mask, a mask that keeps no
+ * pixel, or one that keeps none at some pyramid level (the message names it); the handle then holds no template.
+ * fpm_learn, fpm_learn_set and fpm_learn_ingested learn unmasked templates; a FPM_PARAM_MIN_REDUCE_AREA change re-learns with
+ * the mask. */
+int fpm_learn_masked(fpm_handle* h, const uint8_t* tpl, int width, int height, int stride, const uint8_t* mask, int mask_stride);
 /* batch frames (HOST memory, or device memory with src_on_device = 1; frame i at src + i*frame_stride) x the set: frame b /
  * template t at out + (b*n + t)*cap, its total in counts[b*n + t].  For every (b, t) exactly the list a handle holding only
  * template t returns for frame b through fpm_match_batch_device.  Host frames use the chunked H2D pipeline of fpm_match_batch. */
@@ -222,6 +234,8 @@ int fpm_tpl_levels(const fpm_handle* h);                 /* pyramid size (top la
 int fpm_tpl_level_info(const fpm_handle* h, int level, int* w, int* hgt, double* mean, double* norm,
                        double* inv_area, int* result_equal1);
 int fpm_tpl_level_pixels(const fpm_handle* h, int level, uint8_t* out /* w*h */);
+/* M_L of a masked template as 0/1 bytes (out may be NULL); returns n_L, its kept count.  Unmasked: all ones, w*h. */
+int fpm_tpl_level_mask(const fpm_handle* h, int level, uint8_t* out /* w*h */);
 int fpm_tpl_border_color(const fpm_handle* h);
 
 /* ---- angle-sharded (multi-GPU latency mode) stage API; records are plain doubles ----

@@ -67,6 +67,12 @@ public:
         if (!tpl || w <= 0 || h <= 0) return false;                       // src/TemplateMatcher.cpp:47-49
         return fpm_learn(h_, tpl, w, h, stride) == FPM_OK;
     }
+    // masked template: `mask` (same size, `mask_stride` bytes per row), nonzero = kept; false when fpm_learn_masked refuses it
+    bool learnPattern(const unsigned char* tpl, int w, int h, int stride, const unsigned char* mask, int mask_stride)
+    {
+        if (!tpl || w <= 0 || h <= 0) return false;
+        return fpm_learn_masked(h_, tpl, w, h, stride, mask, mask_stride) == FPM_OK;
+    }
     std::vector<SingleTargetMatch> match(const unsigned char* src, int w, int h, int stride)
     {
         std::vector<SingleTargetMatch> out;
@@ -90,6 +96,12 @@ public:
     {
         if (t.empty() || t.type() != CV_8UC1) return false;
         return learnPattern(t.data, t.cols, t.rows, (int)t.step);
+    }
+    bool learnPattern(const cv::Mat& t, const cv::Mat& mask)
+    {
+        if (mask.empty()) return learnPattern(t);
+        if (t.empty() || t.type() != CV_8UC1 || mask.type() != CV_8UC1 || mask.size() != t.size()) return false;
+        return learnPattern(t.data, t.cols, t.rows, (int)t.step, mask.data, (int)mask.step);
     }
     std::vector<SingleTargetMatch> match(const cv::Mat& s)
     {
