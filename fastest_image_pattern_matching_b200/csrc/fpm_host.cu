@@ -3806,7 +3806,7 @@ int fpm_dbg_top_score_production(fpm_handle* h, const uint8_t* img, int w, int h
     CK(cudaMemcpyAsync(h->d_dbg[2].p, &jb, sizeof(jb), cudaMemcpyHostToDevice, h->stream));
     const bool masked = !t.mask.empty();
     size_t smem = top_score_smem(t.w, t.h, masked);
-    if (smem > 200 * 1024) { h->err = "template too large"; return FPM_ERR_LIMIT; }
+    if (smem > 200 * 1024) { h->err = "top-layer template too large for the score kernel"; return FPM_ERR_LIMIT; }
     const auto kern = masked ? fpm_top_score_kernel<false, true> : fpm_top_score_kernel<false>;
     CK(ensure_dyn_smem((const void*)kern, h->device, smem));
     dim3 grid((RW + TS_TW - 1) / TS_TW, (RH + TS_TH - 1) / TS_TH, 1), block(TS_THREADS);

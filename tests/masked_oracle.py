@@ -66,10 +66,13 @@ def masked_window_sums(src, m):
     pq[:, 1:] = np.cumsum(s * s, axis=1)
     t = np.zeros((R, C), np.int64)
     t2 = np.zeros((R, C), np.int64)
+    cols = np.arange(C)
     for i, runs in enumerate(mask_runs(m)):
-        for b, e in runs:
-            t += ps[i:i + R, e:e + C] - ps[i:i + R, b:b + C]
-            t2 += pq[i:i + R, e:e + C] - pq[i:i + R, b:b + C]
+        if not runs:
+            continue
+        b, e = (np.asarray(v)[:, None] + cols for v in zip(*runs))     # [run][c]: all runs of the row in one gather
+        t += (ps[i:i + R, e] - ps[i:i + R, b]).sum(axis=1)
+        t2 += (pq[i:i + R, e] - pq[i:i + R, b]).sum(axis=1)
     return t, t2
 
 
@@ -188,3 +191,69 @@ def corner_cut_mask(w, h):
 
 
 MASKS = {"disc": disc_mask, "ring": ring_mask, "holed": holed_mask, "blob": blob_mask, "corner_cut": corner_cut_mask}
+
+
+def ccoeff_branches_masked(src, td, m, result, layer):
+    """ccoeff_branches with the masked window sums: which epilogue branch every cell takes (oracle.BRANCH_*)"""
+    if td.result_equal1[layer]:
+        return np.full(result.shape, O.BRANCH_EQUAL1, np.int8)
+    num, den = ccoeff_num_den_masked(src, td, m, result, layer)
+    absn = np.abs(num)
+    return np.where(den == 0, O.BRANCH_FLAT, np.where(absn < den, O.BRANCH_QUOTIENT,
+                    np.where(absn < den * 1.125, O.BRANCH_CLAMP, O.BRANCH_ZERO))).astype(np.int8)
+
+
+# ---------------- edge masks: the run-table cases the blobs above never produce ----------------
+# Thin structures vanish down the pyramid (M_{L+1} = pyrDown(255 M_L) >= 128), so each of these keeps a solid part that is
+# grown until every level of the deepest pyramid the tests use (MinReduceArea 64) keeps 4 pixels (one kept pixel is a
+# flat template, which scores 1 everywhere).
+EDGE_MIN_DST = 8
+
+
+def _survives(m):
+    top = O.get_top_layer(m.shape[1], m.shape[0], EDGE_MIN_DST)
+    return all(l.sum() >= 4 for l in mask_pyramid(m, top))
+
+
+def comb_mask(w, h):
+    """many runs per row: columns x % 4 != 3 (runs of 3), and every third row single pixels x % 2 == 0 (runs of 1)"""
+    xx = np.arange(w)[None, :]
+    yy = np.arange(h)[:, None]
+    return np.where(yy % 3 == 1, xx % 2 == 0, xx % 4 != 3).astype(np.uint8)
+
+
+def banded_mask(w, h):
+    """whole empty rows: bands of 6 empty rows (empty rows at level 1 too) between bands of kept rows, under the fewest
+    kept first rows that keep every level non-empty"""
+    yy = np.arange(h)
+    for k in range(4, h + 1):
+        m = np.repeat(((yy < k) | (yy % 12 < 4) | (yy % 12 >= 10))[:, None], w, axis=1).astype(np.uint8)
+        if _survives(m):
+            return m
+    return np.ones((h, w), np.uint8)
+
+
+def frame_mask(w, h):
+    """runs at x = 0 and x = w: a frame whose sides are as thin as the pyramid allows, its middle rows two runs each"""
+    for k in range(1, max(w, h)):
+        m = np.ones((h, w), np.uint8)
+        m[k:h - k, k:w - k] = 0
+        if _survives(m):
+            return m
+    return np.ones((h, w), np.uint8)
+
+
+def sparse_mask(w, h):
+    """a sparse lattice of single pixels, plus the smallest centred block that keeps every pyramid level non-empty"""
+    m = np.zeros((h, w), np.uint8)
+    m[1::4, ::5] = 1
+    for s in range(1, max(w, h)):
+        b = m.copy()
+        y0, x0 = max(h // 2 - s // 2, 0), max(w // 2 - s, 0)
+        b[y0:y0 + s, x0:x0 + 2 * s] = 1
+        if _survives(b):
+            return b
+    return np.ones((h, w), np.uint8)
+
+
+EDGE_MASKS = {"comb": comb_mask, "banded": banded_mask, "frame": frame_mask, "sparse": sparse_mask}

@@ -10,7 +10,8 @@ import pytest
 import fpm_workloads as synth
 from oracle import oracle as O
 from tests.helpers import configure
-from tests.masked_oracle import MASKS, MaskedOracleMatcher, disc_mask, mask_pyramid, masked_level_stats
+from tests.masked_oracle import (EDGE_MASKS, MASKS, MaskedOracleMatcher, disc_mask, mask_pyramid, mask_runs,
+                                 masked_level_stats)
 
 
 def _pyrdown_numpy(a):
@@ -80,9 +81,20 @@ def _compare_cv(src, tpl, m, got):
 @pytest.mark.parametrize("mask_name", sorted(MASKS))
 @pytest.mark.parametrize("seed", [0, 1])
 def test_masked_scores_match_cv2(mask_name, seed):
+    _masked_scores_match_cv2(MASKS[mask_name], seed)
+
+
+@pytest.mark.parametrize("mask_name", sorted(EDGE_MASKS))
+@pytest.mark.parametrize("seed", [0, 1])
+def test_edge_masked_scores_match_cv2(mask_name, seed):
+    """comb, banded, frame and sparse masks: many runs, runs of one pixel, empty rows, runs at both edges"""
+    _masked_scores_match_cv2(EDGE_MASKS[mask_name], seed)
+
+
+def _masked_scores_match_cv2(mask_fn, seed):
     rng = np.random.default_rng(100 + seed)
     tpl = _template(37, 29, 200 + seed)
-    m = MASKS[mask_name](37, 29)
+    m = mask_fn(37, 29)
     om = MaskedOracleMatcher()
     om.min_reduce_area = 64
     assert om.learn_pattern(tpl, m)
@@ -93,6 +105,9 @@ def test_masked_scores_match_cv2(mask_name, seed):
         s = src if layer == 0 else cv2.resize(src, (max(t.shape[1] + 8, src.shape[1] >> layer), max(t.shape[0] + 8, src.shape[0] >> layer)))
         for use_simd in (True, False):           # refinement numerator (float row chain) and top-layer numerator (exact)
             got = om._match_template(s, layer, use_simd).copy()
+            if om.td.result_equal1[layer]:       # a flat kept template (a frame's one-pixel top level): cv2 divides by 0
+                assert (got == 1).all()
+                continue
             _compare_cv(s, t, ml, got)
 
 
@@ -154,3 +169,29 @@ def test_refusals():
     with pytest.raises(ValueError, match="level 1"):
         om.learn_pattern(tpl, one)
     assert masked_level_stats(tpl, np.ones_like(tpl))[4] == tpl.size
+
+
+# the shapes the GPU cell tests refine (tests/test_gpu_refine_cells.py SYNTH) and the wide masked templates
+EDGE_SHAPES = [(120, 10, 64), (123, 36, 64), (65, 44, 64), (63, 40, 64), (122, 30, 256), (128, 60, 64), (30, 60, 64),
+               (40, 32, 64), (64, 48, 256), (60, 44, 256), (5000, 64, 10000), (6400, 64, 10000)]
+
+
+@pytest.mark.parametrize("mask_name", sorted(EDGE_MASKS))
+def test_edge_masks_have_their_run_table_cases(mask_name):
+    """each edge mask learns at every shape (no level empty) and has at level 0 or 1 (both refined when the pyramid has
+    three levels) the case it is named for, checked on the level masks and not on the level-0 drawing"""
+    for (w, h, mra) in EDGE_SHAPES:
+        m0 = EDGE_MASKS[mask_name](w, h)
+        om = MaskedOracleMatcher()
+        om.min_reduce_area = mra
+        assert om.learn_pattern(np.zeros((h, w), np.uint8), m0)
+        runs = [mask_runs(ml) for ml in om.masks]
+        if mask_name == "comb":
+            assert max(len(r) for r in runs[0]) >= 8 and any(e - b == 1 for r in runs[0] for b, e in r), (w, h)
+        elif mask_name == "banded":
+            assert len(om.masks) > 2 and any(not r for r in runs[1]), (w, h)
+        elif mask_name == "frame":
+            for ml, lr in zip(om.masks[:2], runs[:2]):
+                assert any(len(r) >= 2 and r[0][0] == 0 and r[-1][1] == ml.shape[1] for r in lr), (w, h)
+        else:
+            assert m0.mean() < 1 / 3 and any(e - b == 1 for r in runs[0] for b, e in r), (w, h)
