@@ -37,6 +37,7 @@ SIGNATURES = {
     "fpm_learn": (_i, [_vp, _vp, _i, _i, _i]),
     "fpm_learn_set": (_i, [_vp, _i, _vp, _vp, _vp, _vp]),
     "fpm_learn_masked": (_i, [_vp, _vp, _i, _i, _i, _vp, _i]),
+    "fpm_learn_set_masked": (_i, [_vp, _i, _vp, _vp, _vp, _vp, _vp, _vp]),
     "fpm_set_size": (_i, [_vp]),
     "fpm_match_set_batch": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _vp, _i, _vp]),
     "fpm_match_ingested_set_batch": (_i, [_vp, _vp, _i, _vp]),

@@ -44,8 +44,9 @@ struct FpmTplLevel {
     int n_tpl;              // templates in the group (1: a single template, stats unused)
     size_t tpl_stride;
     const FpmTplStat* stats;
-    // masked template (fpm_learn_masked): the kept pixels of row y are the column ranges [b, e) of
-    // mrun[mrow[y] .. mrow[y + 1]); the pixels at ptr are already multiplied by the mask.  null: every pixel is kept.
+    // masked template or group: the kept pixels of row y of template k are the column ranges [b, e) of
+    // mrun[mrow[k * (h + 1) + y] .. mrow[k * (h + 1) + y + 1]) (fpm_tpl_member moves mrow to template k's h + 1 offsets);
+    // the pixels at ptr are already multiplied by the mask.  null: every pixel is kept.
     const int* mrow;
     const int2* mrun;
 };
@@ -57,6 +58,7 @@ FPM_HD FpmTplLevel fpm_tpl_member(FpmTplLevel t, int k)
         t.ptr += (size_t)k * t.tpl_stride;
         const FpmTplStat s = t.stats[k];
         t.mean = s.mean; t.norm = s.norm; t.inv_area = s.inv_area; t.result_equal1 = s.result_equal1;
+        if (t.mrow) t.mrow += (size_t)k * (t.h + 1);
     }
     return t;
 }

@@ -138,8 +138,9 @@ struct TplLevelHost {
     std::vector<uint8_t> pix;    // w*h
     size_t tpl_stride = 0;       // template groups: bytes from one member's level to the next one's
     size_t stat_off = 0;         // template groups: index of member 0's FpmTplStat of this level in d_tstat
-    // masked template: M_L as 0/1 bytes (w*h), its kept count, and where its run table starts in d_mruns
-    // (h + 1 int offsets, then the int2 runs); empty mask = every pixel kept
+    bool all_flat = false;       // every member's result_equal1 is set
+    // masked group: member 0's M_L as 0/1 bytes (w*h) and its kept count, and where the level's run table starts in d_mruns
+    // (n_tpl x (h + 1) int offsets, member k's at k * (h + 1), then the int2 runs of all members); empty mask = unmasked group
     std::vector<uint8_t> mask;
     long long n_kept = 0;
     size_t run_off = 0, run_data_off = 0;
@@ -155,7 +156,7 @@ struct TopPlan {                  // cached per (source size, parameters); alway
     bool valid = false;
 };
 
-// Templates of a set with the same level-0 size and border colour: they share the top layer, the angle schedule, the
+// Templates of a set with the same level-0 size, border colour and masked-ness: they share the top layer, the angle schedule, the
 // canvases, the ROI sizes and the NMS rectangle, and run through the pipeline together as virtual images
 // v = frame * n + member.  The group being matched lives in the handle's fields (tpl, border, tpl0_w/h, members, plan,
 // d_jobs_top, d_angles, d_ftx, d_fty); group 0 is there at rest, the others are swapped in for their pass.
@@ -163,12 +164,13 @@ struct TplGroup {
     std::vector<int> members;      // set indices, ascending
     std::vector<TplLevelHost> tpl; // levels (statistics and pixels of members[0])
     int border = 0, w0 = 0, h0 = 0;
+    bool masked = false;           // its members carry masks (a group is all masked or all unmasked)
     TopPlan plan;
     DevBuf d_jobs_top, d_angles, d_ftx, d_fty;
     void release() { d_jobs_top.release(); d_angles.release(); d_ftx.release(); d_fty.release(); }
 };
 
-struct SetTpl { std::vector<uint8_t> px; int w = 0, h = 0; };
+struct SetTpl { std::vector<uint8_t> px, mask; int w = 0, h = 0; };   // mask: 0/1 bytes (w*h), empty = unmasked
 
 }  // namespace
 
@@ -207,8 +209,8 @@ struct fpm_handle {
     int learned_mra = -1;
     int border = 0;
     std::vector<SetTpl> set;       // the learned templates (fpm_learn: one), kept for re-learning when MinReduceArea changes
-    std::vector<uint8_t> mask0;    // fpm_learn_masked: the level-0 mask of set[0] as 0/1 bytes (empty: unmasked)
-    DevBuf d_mruns, d_mpyr, d_mwS, d_mwQ;   // masked template: run tables, mask pyramid at learn time, refinement window sums
+    bool masked_set = false;       // learned by fpm_learn_set_masked: learn refusals name the template index
+    DevBuf d_mruns, d_mpyr, d_mwS, d_mwQ;   // masked templates: run tables, mask pyramids at learn time, refinement window sums
     std::vector<TplGroup> groups;  // their groups; groups[0]'s state is in the fields below (see TplGroup)
     DevBuf d_tstat;                // FpmTplStat of every (group, level, member)
     DevBuf d_members;              // the members of every group, group after group (merged set results: output rows)
@@ -627,7 +629,7 @@ bool fw_box_fits(int vec)
 // never writes.
 bool corr_warp_usable(const fpm_handle* h, int tw, int n_ang, const FpmLevel& L)
 {
-    if (h->use_tc != 6 || h->members.size() > 1 || !h->mask0.empty()) return false;   // opt-in: bit-identical, less DRAM traffic, but slower than warp + MMA today
+    if (h->use_tc != 6 || h->members.size() > 1 || !h->tpl[0].mask.empty()) return false;   // opt-in: bit-identical, less DRAM traffic, but slower than warp + MMA today
     if (n_ang != 3 || tw < 64 || !get_encode_tiled()) return false;
     return level_copy_vec(L) >= 4 && fw_box_fits(4);       // the box is staged with 4-byte copies
 }
@@ -656,8 +658,10 @@ int launch_corr_warp(fpm_handle* h, const FpmLevel& L, const FpmWarpJob* jobs, c
     return FPM_OK;
 }
 
-// masked template: the 49 window sums of every eval, int64 [e][49] in d_mwS / d_mwQ, from the ROI patches in d_roi
-int launch_mask_window(fpm_handle* h, int rpitch, size_t roi_stride, const FpmTplLevel& td, int ne, const int* n_cands_dev, int n_ang)
+// masked group: the 49 window sums of every eval, int64 [e][49] in d_mwS / d_mwQ, from the ROI patches in d_roi (eval e of
+// candidate cands[e / n_ang], whose template is cands[e / n_ang].img % td.n_tpl)
+int launch_mask_window(fpm_handle* h, int rpitch, size_t roi_stride, const FpmTplLevel& td, int ne, const int* n_cands_dev, int n_ang,
+                       const FpmCand* cands)
 {
     const int pstride = (int)align_up(td.w + FPM_ROI_PAD + 1, 4);                 // prefix entries of one ROI row
     const size_t per_warp = 2 * sizeof(uint32_t) * (size_t)pstride;
@@ -670,7 +674,8 @@ int launch_mask_window(fpm_handle* h, int rpitch, size_t roi_stride, const FpmTp
     // algorithmic work: one pass over the ROI patch (bytes)
     KL(K_MASK_WINDOW, (double)ne * (td.w + FPM_ROI_PAD) * (td.h + FPM_ROI_PAD),
        fpm_mask_window_kernel<<<ne, warps * 32, smem, h->stream>>>(h->d_roi.as<uint8_t>(), rpitch, roi_stride, td, ne, pstride,
-                                                                   h->d_mwS.as<long long>(), h->d_mwQ.as<long long>(), n_cands_dev, n_ang));
+                                                                   h->d_mwS.as<long long>(), h->d_mwQ.as<long long>(), n_cands_dev, n_ang,
+                                                                   cands));
     return FPM_OK;
 }
 
@@ -684,16 +689,17 @@ int do_learn(fpm_handle* h)
     for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
     h->groups.clear();
     std::vector<TplGroup> gs;
-    const bool masked = !h->mask0.empty();                        // fpm_learn_masked: a set of one
+    // masked and unmasked templates never share a group: unmasked groups keep the kernels without run walks
     for (int i = 0; i < (int)h->set.size(); i++) {
         const SetTpl& st = h->set[i];
+        const bool masked = !st.mask.empty();
         unsigned long long S = 0, N = 0;
         for (size_t k = 0; k < st.px.size(); k++)
-            if (!masked || h->mask0[k]) { S += st.px[k]; N++; }
+            if (!masked || st.mask[k]) { S += st.px[k]; N++; }
         const int border = ((double)S / (double)N) < 128 ? 255 : 0;     // iBorderColor (:58-59), over the kept pixels
         size_t g = 0;
-        while (g < gs.size() && !(gs[g].w0 == st.w && gs[g].h0 == st.h && gs[g].border == border)) g++;
-        if (g == gs.size()) { gs.emplace_back(); gs[g].w0 = st.w; gs[g].h0 = st.h; gs[g].border = border; }
+        while (g < gs.size() && !(gs[g].w0 == st.w && gs[g].h0 == st.h && gs[g].border == border && gs[g].masked == masked)) g++;
+        if (g == gs.size()) { gs.emplace_back(); gs[g].w0 = st.w; gs[g].h0 = st.h; gs[g].border = border; gs[g].masked = masked; }
         gs[g].members.push_back(i);
     }
     size_t off = 0, toff = 0, n_stat = 0;
@@ -733,44 +739,57 @@ int do_learn(fpm_handle* h)
         int rc = launch_pyramid_chain(h, lv, top, T);
         if (rc) return rc;
     }
-    // mask pyramid: M_{L+1} = (pyrDown(255 * M_L) >= 128), one level per launch of the pyramid kernel
-    std::vector<std::vector<uint8_t>> mk;
-    if (masked) {
-        const std::vector<TplLevelHost>& tl = gs[0].tpl;
-        mk.assign(tl.size(), std::vector<uint8_t>());
-        mk[0] = h->mask0;
+    // mask pyramids of the masked groups: M_{L+1} = (pyrDown(255 * M_L) >= 128), per level one launch of the pyramid kernel
+    // over the group's members (at k * tpl_stride, as their templates) and one read-back.  mk[g][l]: the members' M_l, w*h each.
+    std::vector<std::vector<std::vector<uint8_t>>> mk(gs.size());
+    for (size_t gi = 0; gi < gs.size(); gi++) {
+        const TplGroup& G = gs[gi];
+        if (!G.masked) continue;
+        const std::vector<TplLevelHost>& tl = G.tpl;
+        const int T = (int)G.members.size();
+        mk[gi].assign(tl.size(), std::vector<uint8_t>());
+        for (int k = 0; k < T; k++) mk[gi][0].insert(mk[gi][0].end(), h->set[G.members[k]].mask.begin(), h->set[G.members[k]].mask.end());
         CK(h->d_mpyr.ensure(off));
         uint8_t* mb = h->d_mpyr.as<uint8_t>();
         for (size_t l = 1; l < tl.size(); l++) {
             const TplLevelHost &a = tl[l - 1], &b = tl[l];
-            std::vector<uint8_t> up(mk[l - 1].size()), dn((size_t)b.w * b.h);
-            for (size_t i = 0; i < up.size(); i++) up[i] = mk[l - 1][i] ? 255 : 0;
-            CK(cudaMemcpy2DAsync(mb + a.dev_off, a.pitch, up.data(), a.w, a.w, a.h, cudaMemcpyHostToDevice, h->stream));
-            int rc = launch_pyrdown(h, FpmLevel{mb + a.dev_off, a.w, a.h, a.pitch, 0}, FpmLevel{mb + b.dev_off, b.w, b.h, b.pitch, 0},
-                                    nullptr, 1);
+            const size_t na = (size_t)a.w * a.h, nb = (size_t)b.w * b.h;
+            std::vector<uint8_t> up(a.tpl_stride * T, 0), dn(b.tpl_stride * T);
+            for (int k = 0; k < T; k++)
+                for (int y = 0; y < a.h; y++)
+                    for (int x = 0; x < a.w; x++) up[k * a.tpl_stride + (size_t)y * a.pitch + x] = mk[gi][l - 1][k * na + (size_t)y * a.w + x] ? 255 : 0;
+            CK(cudaMemcpyAsync(mb + a.dev_off, up.data(), up.size(), cudaMemcpyHostToDevice, h->stream));
+            int rc = launch_pyrdown(h, FpmLevel{mb + a.dev_off, a.w, a.h, a.pitch, a.tpl_stride},
+                                    FpmLevel{mb + b.dev_off, b.w, b.h, b.pitch, b.tpl_stride}, nullptr, T);
             if (rc) return rc;
-            CK(cudaMemcpy2DAsync(dn.data(), b.w, mb + b.dev_off, b.pitch, b.w, b.h, cudaMemcpyDeviceToHost, h->stream));
+            CK(cudaMemcpyAsync(dn.data(), mb + b.dev_off, dn.size(), cudaMemcpyDeviceToHost, h->stream));
             CK(cudaStreamSynchronize(h->stream));
-            size_t n = 0;
-            for (uint8_t& v : dn) { v = v >= 128 ? 1 : 0; n += v; }
-            if (n == 0) {
-                h->err = "fpm_learn_masked: the mask keeps no pixel at pyramid level " + std::to_string(l) + " (" + std::to_string(b.w) +
-                         "x" + std::to_string(b.h) + "); enlarge the kept region or lower FPM_PARAM_MIN_REDUCE_AREA";
-                return FPM_ERR_INVALID;
+            std::vector<uint8_t>& m = mk[gi][l];
+            m.resize(nb * T);
+            for (int k = 0; k < T; k++) {
+                size_t n = 0;
+                for (int y = 0; y < b.h; y++)
+                    for (int x = 0; x < b.w; x++) n += m[k * nb + (size_t)y * b.w + x] = dn[k * b.tpl_stride + (size_t)y * b.pitch + x] >= 128 ? 1 : 0;
+                if (n == 0) {
+                    const std::string lv = " keeps no pixel at pyramid level " + std::to_string(l) + " (" + std::to_string(b.w) + "x" +
+                                           std::to_string(b.h) + "); enlarge the kept region or lower FPM_PARAM_MIN_REDUCE_AREA";
+                    h->err = h->masked_set ? "fpm_learn_set_masked: the mask of template " + std::to_string(G.members[k]) + lv
+                                           : "fpm_learn_masked: the mask" + lv;
+                    return FPM_ERR_INVALID;
+                }
             }
-            mk[l].swap(dn);
         }
     }
     std::vector<uint8_t> all(off);
     CK(cudaMemcpyAsync(all.data(), h->d_tpl.p, off, cudaMemcpyDeviceToHost, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     std::vector<FpmTplStat> stats(n_stat);
-    for (TplGroup& G : gs)
-        for (size_t l = 0; l < G.tpl.size(); l++)
-            for (size_t k = 0; k < G.members.size(); k++) {
-                TplLevelHost& t = G.tpl[l];
+    for (size_t gi = 0; gi < gs.size(); gi++)
+        for (size_t l = 0; l < gs[gi].tpl.size(); l++)
+            for (size_t k = 0; k < gs[gi].members.size(); k++) {
+                TplLevelHost& t = gs[gi].tpl[l];
                 const uint8_t* base = all.data() + t.dev_off + k * t.tpl_stride;
-                const uint8_t* m = masked ? mk[l].data() : nullptr;
+                const uint8_t* m = gs[gi].masked ? mk[gi][l].data() + k * t.w * t.h : nullptr;
                 unsigned long long S = 0, Q = 0, n = 0;
                 for (int y = 0; y < t.h; y++)
                     for (int x = 0; x < t.w; x++) {
@@ -789,30 +808,37 @@ int do_learn(fpm_handle* h)
                 templNorm = sqrt(templNorm);                        // :85
                 templNorm /= sqrt(invArea);                         // :86
                 stats[t.stat_off + k] = FpmTplStat{mean, templNorm, invArea, equal1};
+                t.all_flat = (k == 0 || t.all_flat) && equal1;
                 if (k == 0) {
                     t.mean = mean; t.norm = templNorm; t.inv_area = invArea; t.equal1 = equal1;
                     t.pix.resize((size_t)t.w * t.h);
                     for (int y = 0; y < t.h; y++) memcpy(t.pix.data() + (size_t)y * t.w, base + (size_t)y * t.pitch, t.w);
                 }
             }
-    if (masked) {
-        // the correlation kernels see M_L * T_L; the window sums walk the runs of kept pixels of every row
-        std::vector<uint8_t> runs;
-        std::vector<uint8_t> tm(off, 0);
-        for (size_t l = 0; l < gs[0].tpl.size(); l++) {
-            TplLevelHost& t = gs[0].tpl[l];
-            t.mask = mk[l];
+    // masked groups: the correlation kernels see M_L * T_L of every member; the window sums walk the runs of kept pixels of
+    // every row of the member's own mask
+    std::vector<uint8_t> runs;
+    for (size_t gi = 0; gi < gs.size(); gi++) {
+        if (!gs[gi].masked) continue;
+        for (size_t l = 0; l < gs[gi].tpl.size(); l++) {
+            TplLevelHost& t = gs[gi].tpl[l];
+            const size_t n = (size_t)t.w * t.h;
+            t.mask.assign(mk[gi][l].begin(), mk[gi][l].begin() + n);
             t.n_kept = 0;
             std::vector<int> rows(1, 0), rr;
-            for (int y = 0; y < t.h; y++) {
-                const uint8_t* m = t.mask.data() + (size_t)y * t.w;
-                for (int x = 0; x < t.w; x++) {
-                    tm[t.dev_off + (size_t)y * t.pitch + x] = m[x] ? t.pix[(size_t)y * t.w + x] : 0;
-                    t.n_kept += m[x];
-                    if (m[x] && (x == 0 || !m[x - 1])) rr.push_back(x);
-                    if (m[x] && (x == t.w - 1 || !m[x + 1])) rr.push_back(x + 1);
+            for (size_t k = 0; k < gs[gi].members.size(); k++) {
+                if (k) rows.push_back(rows.back());                // member k's h + 1 offsets start where member k - 1's end
+                for (int y = 0; y < t.h; y++) {
+                    const uint8_t* m = mk[gi][l].data() + k * n + (size_t)y * t.w;
+                    uint8_t* px = all.data() + t.dev_off + k * t.tpl_stride + (size_t)y * t.pitch;
+                    for (int x = 0; x < t.w; x++) {
+                        if (!m[x]) px[x] = 0;
+                        if (k == 0) t.n_kept += m[x];
+                        if (m[x] && (x == 0 || !m[x - 1])) rr.push_back(x);
+                        if (m[x] && (x == t.w - 1 || !m[x + 1])) rr.push_back(x + 1);
+                    }
+                    rows.push_back((int)rr.size() / 2);
                 }
-                rows.push_back((int)rr.size() / 2);
             }
             t.run_off = align_up(runs.size(), 16);
             t.run_data_off = align_up(t.run_off + rows.size() * sizeof(int), 16);
@@ -820,7 +846,9 @@ int do_learn(fpm_handle* h)
             memcpy(runs.data() + t.run_off, rows.data(), rows.size() * sizeof(int));
             memcpy(runs.data() + t.run_data_off, rr.data(), rr.size() * sizeof(int));
         }
-        CK(cudaMemcpy(h->d_tpl.p, tm.data(), off, cudaMemcpyHostToDevice));
+    }
+    if (!runs.empty()) {
+        CK(cudaMemcpy(h->d_tpl.p, all.data(), off, cudaMemcpyHostToDevice));
         CK(h->d_mruns.ensure(runs.size()));
         CK(cudaMemcpy(h->d_mruns.p, runs.data(), runs.size(), cudaMemcpyHostToDevice));
     }
@@ -996,7 +1024,8 @@ int run_top(fpm_handle* h, int top, int j0, int nj, FpmPick* picks_out, int* cnt
     const bool masked = !t.mask.empty();
     const size_t smem_ts = top_score_smem(t.w, t.h, masked);
     if (smem_ts > 200 * 1024) { h->err = "top-layer template too large for the score kernel"; return FPM_ERR_LIMIT; }
-    const auto score_kernel = n_tpl > 1 ? fpm_top_score_kernel<true> : (masked ? fpm_top_score_kernel<false, true> : fpm_top_score_kernel<false>);
+    const auto score_kernel = n_tpl > 1 ? (masked ? fpm_top_score_kernel<true, true> : fpm_top_score_kernel<true>)
+                                        : (masked ? fpm_top_score_kernel<false, true> : fpm_top_score_kernel<false>);
     if (smem_ts > 48 * 1024) CK(ensure_dyn_smem((const void*)score_kernel, h->device, smem_ts));
     // bCalMaxByBlock, src/TemplateMatcher.cpp:158-159
     const FpmLevel& L = h->levels[top];
@@ -1195,9 +1224,9 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                                                                                     cands + c0));
                 }
             }
-            const bool masked = td.mrun && !t.equal1;
+            const bool masked = td.mrun && !t.all_flat;      // finalize reads the sums of the members that are not flat
             if (masked) {
-                int rcm = launch_mask_window(h, rpitch, roi_stride, td, ne, n_dev, n_ang);
+                int rcm = launch_mask_window(h, rpitch, roi_stride, td, ne, n_dev, n_ang, cands + c0);
                 if (rcm) return rcm;
             }
             {
@@ -2027,13 +2056,13 @@ int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stri
 }
 
 namespace {
-// fpm_learn_set, with the 0/1 level-0 mask of a masked template (n == 1) or an empty one
+// fpm_learn_set, with the 0/1 level-0 mask of every template (empty: unmasked) or none (masks empty: all unmasked);
+// masked_set: refusals name the template index (fpm_learn_set_masked)
 int learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides,
-              std::vector<uint8_t> mask)
+              std::vector<std::vector<uint8_t>> masks, bool masked_set)
 {
     h->learned = false;
     h->set.clear();
-    h->mask0.clear();
     h->learn_gen++;
     if (n < 1 || !tpls || !widths || !heights || !strides) { h->err = "template set: n < 1 or null arrays"; return FPM_ERR_INVALID; }
     for (int i = 0; i < n; i++)
@@ -2046,19 +2075,55 @@ int learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* width
         set[i].w = widths[i]; set[i].h = heights[i];
         set[i].px.resize((size_t)widths[i] * heights[i]);
         for (int y = 0; y < heights[i]; y++) memcpy(set[i].px.data() + (size_t)y * widths[i], tpls[i] + (size_t)y * strides[i], widths[i]);
+        if (!masks.empty()) set[i].mask.swap(masks[i]);
     }
     h->set.swap(set);
-    h->mask0.swap(mask);
+    h->masked_set = masked_set;
     int rc = do_learn(h);
-    if (rc) { h->set.clear(); h->mask0.clear(); }
+    if (rc) h->set.clear();
     return rc;
+}
+
+// the 0/1 copy of a caller's mask (w x h, mask_stride bytes per row) and its kept count
+size_t copy_mask(const uint8_t* mask, int mask_stride, int w, int hgt, std::vector<uint8_t>& m)
+{
+    m.resize((size_t)w * hgt);
+    size_t kept = 0;
+    for (int y = 0; y < hgt; y++)
+        for (int x = 0; x < w; x++) kept += m[(size_t)y * w + x] = mask[(size_t)y * mask_stride + x] ? 1 : 0;
+    return kept;
+}
+
+int refuse_learn(fpm_handle* h, const std::string& why)
+{
+    h->learned = false; h->set.clear(); h->learn_gen++;
+    h->err = why;
+    return FPM_ERR_INVALID;
 }
 }  // namespace
 
 int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides)
 {
     if (!h) return FPM_ERR_INVALID;
-    return learn_set(h, n, tpls, widths, heights, strides, std::vector<uint8_t>());
+    return learn_set(h, n, tpls, widths, heights, strides, {}, false);
+}
+
+int fpm_learn_set_masked(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights,
+                         const int* strides, const uint8_t* const* masks, const int* mask_strides)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (!masks) return learn_set(h, n, tpls, widths, heights, strides, {}, false);
+    if (!mask_strides) return refuse_learn(h, "fpm_learn_set_masked: null mask_strides with masks");
+    if (n < 1 || !tpls || !widths || !heights || !strides) return learn_set(h, n, tpls, widths, heights, strides, {}, true);
+    std::vector<std::vector<uint8_t>> ms(n);
+    for (int i = 0; i < n; i++) {
+        if (!masks[i]) continue;
+        if (!tpls[i] || widths[i] <= 0 || heights[i] <= 0 || strides[i] < widths[i]) break;   // learn_set names the empty template
+        const std::string ti = "fpm_learn_set_masked: template " + std::to_string(i);
+        if (mask_strides[i] < widths[i]) return refuse_learn(h, ti + ": mask stride smaller than the template width");
+        if (!copy_mask(masks[i], mask_strides[i], widths[i], heights[i], ms[i])) return refuse_learn(h, ti + ": the mask keeps no pixel");
+    }
+    return learn_set(h, n, tpls, widths, heights, strides, std::move(ms), true);
 }
 
 int fpm_learn_masked(fpm_handle* h, const uint8_t* tpl, int width, int height, int stride, const uint8_t* mask, int mask_stride)
@@ -2068,20 +2133,10 @@ int fpm_learn_masked(fpm_handle* h, const uint8_t* tpl, int width, int height, i
     if (!tpl || width <= 0 || height <= 0 || stride < width) why = "empty template";
     else if (!mask) why = "fpm_learn_masked: null mask";
     else if (mask_stride < width) why = "fpm_learn_masked: mask stride smaller than the template width";
-    std::vector<uint8_t> m;
-    if (!why) {
-        m.resize((size_t)width * height);
-        size_t kept = 0;
-        for (int y = 0; y < height; y++)
-            for (int x = 0; x < width; x++) kept += m[(size_t)y * width + x] = mask[(size_t)y * mask_stride + x] ? 1 : 0;
-        if (!kept) why = "fpm_learn_masked: the mask keeps no pixel";
-    }
-    if (why) {
-        h->learned = false; h->set.clear(); h->mask0.clear(); h->learn_gen++;
-        h->err = why;
-        return FPM_ERR_INVALID;
-    }
-    return learn_set(h, 1, &tpl, &width, &height, &stride, std::move(m));
+    std::vector<std::vector<uint8_t>> m(1);
+    if (!why && !copy_mask(mask, mask_stride, width, height, m[0])) why = "fpm_learn_masked: the mask keeps no pixel";
+    if (why) return refuse_learn(h, why);
+    return learn_set(h, 1, &tpl, &width, &height, &stride, std::move(m), false);
 }
 
 int fpm_set_size(const fpm_handle* h) { return h && h->learned ? (int)h->set.size() : 0; }
@@ -2091,7 +2146,7 @@ int fpm_is_learned(const fpm_handle* h) { return h && h->learned ? 1 : 0; }
 void fpm_clear(fpm_handle* h)
 {
     if (!h) return;
-    h->learned = false; h->tpl.clear(); h->set.clear(); h->mask0.clear(); h->members.clear(); h->has_ur = 0;
+    h->learned = false; h->tpl.clear(); h->set.clear(); h->members.clear(); h->has_ur = 0;
     for (size_t g = 1; g < h->groups.size(); g++) h->groups[g].release();
     h->groups.clear();
     h->ur[0] = h->ur[1] = h->ur[2] = h->ur[3] = 0;
@@ -2125,8 +2180,9 @@ int ensure_twin(fpm_handle* h)
         const int n = (int)h->set.size();
         std::vector<const uint8_t*> px(n);
         std::vector<int> ws(n), hs(n);
-        for (int i = 0; i < n; i++) { px[i] = h->set[i].px.data(); ws[i] = h->set[i].w; hs[i] = h->set[i].h; }
-        int rc = learn_set(t, n, px.data(), ws.data(), hs.data(), ws.data(), h->mask0);
+        std::vector<std::vector<uint8_t>> ms(n);
+        for (int i = 0; i < n; i++) { px[i] = h->set[i].px.data(); ws[i] = h->set[i].w; hs[i] = h->set[i].h; ms[i] = h->set[i].mask; }
+        int rc = learn_set(t, n, px.data(), ws.data(), hs.data(), ws.data(), std::move(ms), h->masked_set);
         if (rc) { h->err = t->err; return rc; }
         h->twin_gen = h->learn_gen;
     }

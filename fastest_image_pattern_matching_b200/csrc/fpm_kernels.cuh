@@ -359,10 +359,10 @@ __device__ __forceinline__ float fpm_ccoeff_epilogue_top(float numerator, double
 // Template groups (tpl.n_tpl > 1): the CTA stages its canvas patch and its row-window sums once and scores the patch
 // against every template of the group in turn; map k of job z is written to score + (z * n_tpl + k) * score_job_stride.
 // GROUP = false (a single template) compiles to the one-template kernel.
-// MASKED (a single masked template, tpl.mrun set): the window sums run over the kept pixels only.  Instead of one row-window
+// MASKED (a masked template or group, tpl.mrun set): the window sums run over the kept pixels only.  Instead of one row-window
 // sum per patch row the CTA keeps row prefix sums of the patch and of its squares, ph x (TS_TW + tw) each, and every score adds
-// P[x + e] - P[x + b] over the runs [b, e) of each template row: exact integers, the same ones a full mask gives through the
-// row-window sums.
+// P[x + e] - P[x + b] over the runs [b, e) of each row of the scored template's own mask: exact integers, the same ones a full
+// mask gives through the row-window sums.  The prefix sums do not depend on the template: a group builds them once.
 template <bool GROUP, bool MASKED = false>
 __global__ void __launch_bounds__(TS_THREADS)
 fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restrict__ rot, int rpitch,
@@ -478,8 +478,8 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
     const int tx = tid & 15, ty = tid >> 4;
     const int ox = x0 + 4 * tx, oy = y0 + ty;
     const bool live = ox < RW && oy < RH;
-    // window sum / square sum of the 4 scores' windows in template row yy
-    auto window_rows = [&](int yy, uint4& rs, uint4& rq) {
+    // window sum / square sum of the 4 scores' windows in row yy of template t
+    auto window_rows = [&](const FpmTplLevel& t, int yy, uint4& rs, uint4& rq) {
         const uint32_t* ps = s_rs + (ty + yy) * rs_w + 4 * tx;
         const uint32_t* pq = s_rq + (ty + yy) * rs_w + 4 * tx;
         if (!MASKED) {
@@ -488,8 +488,8 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
             return;
         }
         rs = make_uint4(0, 0, 0, 0); rq = make_uint4(0, 0, 0, 0);
-        for (int k = __ldg(tpl.mrow + yy), ke = __ldg(tpl.mrow + yy + 1); k < ke; k++) {
-            const int2 be = __ldg(tpl.mrun + k);
+        for (int k = __ldg(t.mrow + yy), ke = __ldg(t.mrow + yy + 1); k < ke; k++) {
+            const int2 be = __ldg(t.mrun + k);
             rs.x += ps[be.y] - ps[be.x]; rs.y += ps[be.y + 1] - ps[be.x + 1];
             rs.z += ps[be.y + 2] - ps[be.x + 2]; rs.w += ps[be.y + 3] - ps[be.x + 3];
             rq.x += pq[be.y] - pq[be.x]; rq.y += pq[be.y + 1] - pq[be.x + 1];
@@ -530,7 +530,7 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
                     lo = hi;
                 }
                 uint4 rs, rq;
-                window_rows(yy, rs, rq);
+                window_rows(tk, yy, rs, rq);
                 b[0] += rs.x; b[1] += rs.y; b[2] += rs.z; b[3] += rs.w;
                 c[0] += rq.x; c[1] += rq.y; c[2] += rq.z; c[3] += rq.w;
             }
@@ -554,7 +554,7 @@ fpm_top_score_kernel(const FpmWarpJob* __restrict__ jobs, const uint8_t* __restr
                     lo = hi;
                 }
                 uint4 rs, rq;
-                window_rows(yy, rs, rq);
+                window_rows(tk, yy, rs, rq);
                 num[0] += a[0]; num[1] += a[1]; num[2] += a[2]; num[3] += a[3];   // per-row s32, s64 across rows
                 wsum[0] += rs.x; wsum[1] += rs.y; wsum[2] += rs.z; wsum[3] += rs.w;
                 wsq[0] += rq.x; wsq[1] += rq.y; wsq[2] += rq.z; wsq[3] += rq.w;
@@ -1337,7 +1337,7 @@ __device__ void fpm_subpix(const double* sc27 /* [theta][y][x] */, double xm, do
 }
 
 // =====================================================================================
-// masked refinement window sums (fpm_learn_masked): for every eval and every cell (r, c) of its 7x7 patch the exact sums
+// masked refinement window sums (masked templates and groups): for every eval and every cell (r, c) of its 7x7 patch the exact sums
 // of the ROI pixels and of their squares under the KEPT template pixels, t = sum M*S and t2 = sum M*S^2, as int64
 // [eval][49] for fpm_refine_finalize_kernel.  One CTA per eval, one warp per ROI row at a time (rows y = warp, warp + nw,
 // ...), no block-wide barrier until the end: the warp turns its row into prefix sums P[x] (the pixels left of column x;
@@ -1351,12 +1351,17 @@ __device__ void fpm_subpix(const double* sc27 /* [theta][y][x] */, double xm, do
 
 __global__ void __launch_bounds__(MW_MAX_WARPS * 32)
 fpm_mask_window_kernel(const uint8_t* __restrict__ roi, int rpitch, size_t roi_stride, FpmTplLevel tpl, int ne, int pstride,
-                       long long* __restrict__ totS, long long* __restrict__ totQ, const int* __restrict__ n_cands_dev, int n_ang)
+                       long long* __restrict__ totS, long long* __restrict__ totQ, const int* __restrict__ n_cands_dev, int n_ang,
+                       const FpmCand* __restrict__ cands)
 {
     extern __shared__ __align__(16) uint32_t s_pre[];        // per warp: pstride pixel prefix sums, then pstride square ones
     __shared__ unsigned long long s_tot[2 * FPM_NCELL];
     const int e = blockIdx.x;
     if (e >= ne || (n_cands_dev && e >= *n_cands_dev * n_ang)) return;
+    if (tpl.n_tpl > 1) {                                     // a group: the eval's own template (CTA-uniform)
+        tpl = fpm_tpl_member(tpl, cands[e / n_ang].img % tpl.n_tpl);
+        if (tpl.result_equal1) return;                       // finalize scores a flat template 1 without its sums
+    }
     const int th = tpl.h, rw = tpl.w + FPM_ROI_PAD, rh = th + FPM_ROI_PAD, pl = rw + 1;
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nw = blockDim.x >> 5;
     for (int i = tid; i < 2 * FPM_NCELL; i += blockDim.x) s_tot[i] = 0;

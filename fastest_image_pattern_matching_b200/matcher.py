@@ -146,16 +146,32 @@ class TemplateMatcher:
         return True
 
     # ---- template sets: n templates in one handle, matched in shared launches (fpm_learn_set) ----
-    def learnPatternSet(self, templates) -> bool:
-        """n templates (2-D uint8 arrays) replace the pattern; all use this matcher's parameters."""
+    def learnPatternSet(self, templates, masks=None) -> bool:
+        """n templates (2-D uint8 arrays) replace the pattern; all use this matcher's parameters.  masks (optional): a list
+        of n entries, each None (unmasked) or an array of its template's shape, nonzero = kept (fpm_learn_set_masked)."""
         ts = [_as_u8_2d(t) for t in templates]
         n = len(ts)
-        self._tpl_keepalive = ts
         ptrs = (C.c_void_p * max(n, 1))(*[t.ctypes.data for t in ts])
         ws = (C.c_int * max(n, 1))(*[t.shape[1] for t in ts])
         hs = (C.c_int * max(n, 1))(*[t.shape[0] for t in ts])
         st = (C.c_int * max(n, 1))(*[t.strides[0] for t in ts])
-        self._check(self._lib.fpm_learn_set(self._h, n, ptrs, ws, hs, st))
+        if masks is None:
+            self._tpl_keepalive = ts
+            self._check(self._lib.fpm_learn_set(self._h, n, ptrs, ws, hs, st))
+            return True
+        if len(masks) != n:
+            raise ValueError(f"{len(masks)} masks for {n} templates")
+        ms = []
+        for i, (t, m) in enumerate(zip(ts, masks)):
+            if m is not None:
+                m = np.ascontiguousarray(np.asarray(m) != 0, dtype=np.uint8)
+                if m.shape != t.shape:
+                    raise ValueError(f"mask {i}: shape {m.shape} differs from the template's {t.shape}")
+            ms.append(m)
+        self._tpl_keepalive = (ts, ms)
+        mp = (C.c_void_p * max(n, 1))(*[None if m is None else m.ctypes.data for m in ms])
+        mst = (C.c_int * max(n, 1))(*[0 if m is None else m.strides[0] for m in ms])
+        self._check(self._lib.fpm_learn_set_masked(self._h, n, ptrs, ws, hs, st, mp, mst))
         return True
 
     def patternSetSize(self) -> int: return int(self._lib.fpm_set_size(self._h))
@@ -758,17 +774,23 @@ def ocr_assemble(centres, labels, line_tol: float = 10.0) -> str:
 class GlyphReader:
     """One learned TemplateMatcher per glyph; read(image) = the upstream OCR loop: match every glyph, collect the
     centres with their letter, assemble lines.  readBatch(frames) reads many frames with one handle holding all glyphs as
-    a template set (created on first use)."""
+    a template set (created on first use).  masks (optional): {letter: mask} for glyphs matched under a don't-care mask,
+    e.g. their strokes; glyphs without an entry are unmasked."""
 
-    def __init__(self, templates: dict, device: int = 0, result_capacity: int = 256, **params):
+    def __init__(self, templates: dict, masks: Optional[dict] = None, device: int = 0, result_capacity: int = 256, **params):
         self.letters = [ch for ch in OCR_LETTERS if ch in templates] + sorted(k for k in templates if k not in OCR_LETTERS)
         self._templates = [templates[ch] for ch in self.letters]
+        masks = masks or {}
+        unknown = sorted(set(masks) - set(templates))
+        if unknown:
+            raise ValueError(f"masks for glyphs without a template: {unknown}")
+        self._masks = [masks.get(ch) for ch in self.letters]
         self._device, self._capacity, self._params = device, result_capacity, params
         self._set_matcher = None
         self.matchers = []
-        for ch in self.letters:
+        for ch, mk in zip(self.letters, self._masks):
             m = self._new_matcher()
-            if not m.learnPattern(templates[ch]):
+            if not m.learnPattern(templates[ch], mk):
                 raise FpmError("learnPattern failed for glyph %r" % ch)
             self.matchers.append(m)
 
@@ -795,7 +817,7 @@ class GlyphReader:
         {letter: results} holds the survivors."""
         if self._set_matcher is None:
             self._set_matcher = self._new_matcher()
-            self._set_matcher.learnPatternSet(self._templates)
+            self._set_matcher.learnPatternSet(self._templates, self._masks if any(m is not None for m in self._masks) else None)
         f = np.ascontiguousarray(np.stack([_as_u8_2d(x) for x in frames]) if isinstance(frames, (list, tuple)) else frames, np.uint8)
         if merge_overlap is None:
             return [self._assemble(per, line_tol) for per in self._set_matcher.matchSetBatch(f)]

@@ -97,12 +97,21 @@ int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stri
 /* Template sets (the upstream OCR loop, MatchTool/MatchToolDlg.cpp:718-770: one LoadDst + Match per glyph): n templates
  * (template i: tpls[i], widths[i] x heights[i], strides[i] bytes per row) replace the handle's pattern, all with the handle's
  * parameters.  FPM_ERR_INVALID (the message names the index) for n < 1, null pointers or an empty template; the handle then
- * holds none.  fpm_learn is a set of one.  Templates of one level-0 size and border colour form a group that shares every
- * launch of the pipeline (the template is a kernel dimension); groups run one after another.  There is no NMS across templates.
+ * holds none.  fpm_learn is a set of one.  Templates of one level-0 size, border colour and masked-ness (fpm_learn_set_masked)
+ * form a group that shares every launch of the pipeline (the template is a kernel dimension); groups run one after another.
+ * There is no NMS across templates.
  * A handle holding more than one template refuses every single-template entry point with FPM_ERR_INVALID and a message:
  * fpm_match*, fpm_match_ingested*, fpm_learn_ingested, fpm_match_multi, fpm_match_sharded*, fpm_stage_*, fpm_tpl_* (and
  * fpm_match_set_batch with FPM_PARAM_TRACE on).  fpm_match_set_sharded* run a set in the angle-sharded mode.  FPM_PARAM_MIN_REDUCE_AREA changed after learning re-learns the whole set. */
 int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides);
+/* fpm_learn_set with a don't-care mask per template: masks[i] (u8, template i's size, mask_strides[i] bytes per row,
+ * nonzero = kept) or NULL for an unmasked member; masks == NULL is fpm_learn_set.  Each masked member is learned exactly as
+ * fpm_learn_masked learns it, and every set entry point returns for it the lists of a handle holding only that template.
+ * Masked and unmasked members never share a group.  FPM_ERR_INVALID (the message names the template index, and the level
+ * for the last case) for mask_strides == NULL with masks, mask_strides[i] < widths[i], a mask that keeps no pixel, or one that
+ * keeps none at some pyramid level; the handle then holds none.  A FPM_PARAM_MIN_REDUCE_AREA change re-learns with the masks. */
+int fpm_learn_set_masked(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights,
+                         const int* strides, const uint8_t* const* masks, const int* mask_strides);
 int fpm_set_size(const fpm_handle* h);              /* 0 = nothing learned, 1 after fpm_learn */
 /* Masked template (a don't-care mask, like cv::matchTemplate(..., mask) with TM_CCOEFF_NORMED): mask is u8 of the template's
  * size, `mask_stride` bytes per row, a nonzero byte keeps the pixel.  M_0 = (mask != 0); M_{L+1} = (pyrDown(255 * M_L) >= 128).
@@ -110,8 +119,8 @@ int fpm_set_size(const fpm_handle* h);              /* 0 = nothing learned, 1 af
  * from the exact sums over the kept pixels (n_L = sum M_L, inv_area = 1 / n_L), the border colour from the kept mean of level 0.
  * At every placement the numerator is the one of the template M_L * T_L and the window sums t, t2 run over the kept pixels only;
  * rectangles, corners, NMS and sub-pixel fitting use the template rectangle.  A full mask gives bit for bit fpm_learn's results.
- * Works on every single-template entry point (not in sets).  FPM_PARAM_TENSOR_CORES = 6 takes the mode-1 route on a masked
- * handle (its window sums need the ROI patches in memory).  FPM_ERR_INVALID with a message for a null mask, a mask that keeps no
+ * Works on every single-template entry point; fpm_learn_set_masked learns masked templates into a set.
+ * FPM_PARAM_TENSOR_CORES = 6 takes the mode-1 route on a masked handle (its window sums need the ROI patches in memory).  FPM_ERR_INVALID with a message for a null mask, a mask that keeps no
  * pixel, or one that keeps none at some pyramid level (the message names it); the handle then holds no template.
  * fpm_learn, fpm_learn_set and fpm_learn_ingested learn unmasked templates; a FPM_PARAM_MIN_REDUCE_AREA change re-learns with
  * the mask. */
