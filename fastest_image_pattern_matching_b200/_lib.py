@@ -21,7 +21,7 @@ class fpm_result(C.Structure):
 PARAM_MAX_POSITIONS, PARAM_MAX_OVERLAP, PARAM_SCORE, PARAM_TOLERANCE_ANGLE, PARAM_MIN_REDUCE_AREA, \
     PARAM_USE_SIMD, PARAM_SUBPIXEL, PARAM_TRACE, PARAM_WORKSPACE_MB, PARAM_PROFILE, PARAM_H2D_CHUNK, PARAM_TENSOR_CORES, PARAM_MFC_COMPAT, PARAM_STOP_LAYER1, PARAM_BITWISE_NOT, PARAM_TOLERANCE_RANGE, \
     PARAM_TOLERANCE1, PARAM_TOLERANCE2, PARAM_TOLERANCE3, PARAM_TOLERANCE4, PARAM_SPLIT_BATCH, PARAM_SHARD_UPLOAD, PARAM_ASYNC_DESCENT, \
-    PARAM_JPEG_DEVICE_HUFFMAN, PARAM_JPEG_PASSES = range(25)
+    PARAM_JPEG_DEVICE_HUFFMAN, PARAM_JPEG_PASSES, PARAM_SCALE_MIN, PARAM_SCALE_MAX = range(27)
 
 _vp, _i, _d, _sz = C.c_void_p, C.c_int, C.c_double, C.c_size_t
 _pi, _pd = C.POINTER(C.c_int), C.POINTER(C.c_double)
@@ -62,6 +62,8 @@ SIGNATURES = {
     "fpm_ingested_count": (_i, [_vp]),
     "fpm_ingested_frame_pixels": (_i, [_vp, _i, _vp]),
     "fpm_match_ingested_batch": (_i, [_vp, _vp, _i, _vp]),
+    "fpm_match_scaled": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _vp, _vp, _i, _vp]),
+    "fpm_match_ingested_scaled": (_i, [_vp, _vp, _vp, _i, _vp]),
     "fpm_dbg_jpeg_luma_parallel_batch": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _i]),
     "fpm_dbg_jpeg_unstuff": (_i, [_vp, _sz, _i, _vp, _sz, _vp, _i, _vp, _pi, _pi]),
     "fpm_match_batch_device": (_i, [_vp, _vp, _i, _i, _i, _i, _sz, _vp, _i, _vp]),

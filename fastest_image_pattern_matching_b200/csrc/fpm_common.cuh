@@ -78,6 +78,7 @@ struct FpmCand {
     float ptx, pty;         // top layer: pt ; refinement: ptLT (cv::Point2f)
     int img;                // image index in the batch (virtual image of a template group)
     int id;                 // rank in the score-sorted top-layer list of its image
+    double scale;           // match scale s: the source is resampled by 1/s (FPM_PARAM_SCALE_MIN / MAX; 1 = unscaled)
 };
 
 // Refined target before NMS
@@ -85,6 +86,7 @@ struct FpmRefined {
     double angle, score;
     double ptx, pty;        // cv::Point2d pt
     int img, id;
+    double scale;           // match scale of the record (FpmCand::scale)
 };
 
 // per-eval record written by refine_finalize for tracing (parity ladder T6)
@@ -139,12 +141,22 @@ FPM_HD void fpm_pt_rotate(float px, float py, float ox, float oy, double ang, fl
     *ry = (float)dY;
 }
 
-// cv::getRotationMatrix2D(center, angle, 1) followed by the inversion cv::warpAffine applies
+// Scale-tolerant matching: p -> c + k * (p - c), evaluated in double and stored as float.  k = s maps a point of a source
+// resampled by 1/s back to the source, k = 1/s maps a source point into the resampled source.  Callers skip it at s == 1,
+// which keeps the unscaled float path bit for bit.
+FPM_HD void fpm_scale_about(float px, float py, float cx, float cy, double k, float* rx, float* ry)
+{
+    *rx = (float)((double)cx + k * ((double)px - (double)cx));
+    *ry = (float)((double)cy + k * ((double)py - (double)cy));
+}
+
+// cv::getRotationMatrix2D(center, angle, scale) followed by the inversion cv::warpAffine applies
 // when WARP_INVERSE_MAP is not set (OpenCV imgproc imgwarp.cpp; model pinned in SURVEY 8c).
-FPM_HD void fpm_rotation_matrix(float cx, float cy, double angle_deg, double* m)
+// alpha = cos * scale, beta = sin * scale as OpenCV computes them, so scale 1 gives the unscaled matrix bit for bit.
+FPM_HD void fpm_rotation_matrix(float cx, float cy, double angle_deg, double* m, double scale = 1.0)
 {
     double a = angle_deg * (FPM_PI / 180);
-    double alpha = cos(a), beta = sin(a);
+    double alpha = cos(a) * scale, beta = sin(a) * scale;
     m[0] = alpha; m[1] = beta;  m[2] = (1 - alpha) * (double)cx - beta * (double)cy;
     m[3] = -beta; m[4] = alpha; m[5] = beta * (double)cx + (1 - alpha) * (double)cy;
 }

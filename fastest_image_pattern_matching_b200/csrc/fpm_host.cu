@@ -148,11 +148,13 @@ struct TplLevelHost {
 
 struct TopPlan {                  // cached per (source size, parameters); always the WHOLE angle schedule
     int sw = 0, sh = 0, top = -1, batch = 0;
-    double tol = -1;
-    std::vector<double> angles;   // full schedule
-    std::vector<float> ftx, fty;  // canvas translation per angle
+    double tol = -1, scale_min = 0, scale_max = 0;
+    // pose slots k * n_angles + a of scale k and angle a (scale-major; one scale: slot == angle)
+    std::vector<double> angles;   // angle per slot: the full angle schedule once per scale
+    std::vector<double> scales;   // scale per slot
+    std::vector<float> ftx, fty;  // canvas translation per slot
     int maxW = 0, maxH = 0;
-    int n_ang = 0;                // angles.size()
+    int n_ang = 0;                // slots: angles.size()
     bool valid = false;
 };
 
@@ -195,6 +197,7 @@ struct fpm_handle {
     unsigned learn_gen = 0, twin_gen = 0;
     int stop_layer1 = 0, bitwise_not = 0, tol_range = 0;   // MFC-only modes (MatchTool/MatchToolDlg.cpp:788-816, :936)
     double tol_r[4] = {0, 0, 0, 0};
+    double scale_min = 1.0, scale_max = 1.0;   // FPM_PARAM_SCALE_MIN / MAX: the match scale range
     int mfc_compat = 0;            // 1: MFC result convention (angle sign/wrap, TargetNum truncation, double corners)
     int async_descent = -1;        // FPM_PARAM_ASYNC_DESCENT: -1 auto (batches < 8 frames), 0 never, 1 always
     int jpeg_device_huffman = 1;   // FPM_PARAM_JPEG_DEVICE_HUFFMAN
@@ -225,7 +228,7 @@ struct fpm_handle {
     int ur[4] = {0, 0, 0, 0};
     int has_ur = 0;
     // workspace
-    DevBuf d_src, d_pyr, d_rot, d_score, d_blkv, d_blkl, d_picks, d_pickcnt, d_jobs_top, d_angles, d_ftx, d_fty;
+    DevBuf d_src, d_pyr, d_rot, d_score, d_blkv, d_blkl, d_picks, d_pickcnt, d_jobs_top, d_angles, d_ftx, d_fty, d_scales;
     DevBuf d_off, d_keys, d_cand[2], d_candcnt, d_toppt, d_counters, d_jobs_ref, d_roi, d_rowsum, d_rowS, d_rowQ;
     DevBuf d_pairs, d_refined, d_rects, d_del, d_idmap, d_results, d_rescnt, d_trace, d_trace_sc, d_dbg[4];
     PinnedBuf h_counts, h_results, h_stage;
@@ -236,6 +239,10 @@ struct fpm_handle {
     int shard_upload = 1;          // FPM_PARAM_SHARD_UPLOAD: host frame uploaded as 1/N row slices + NVLink allgather
     DevBuf d_gpicks, d_grefined;   // allgather buffers: one fixed-size block per rank, consumed in place by the kernels
     FpmRefined* ref_out = nullptr; // where run_refine appends (null: d_refined / counters[CNT_REFINED])
+    // fpm_match_scaled: run_final writes the scale of the record written at out_base[i] to scales_out[i] (out_base: the caller's
+    // whole output array, so chunks, split halves and their twin handle all index it the same way)
+    double* scales_out = nullptr;
+    const fpm_result* scales_base = nullptr;
     int* ref_cnt = nullptr;
     // one call's layout of the rank blocks, the same on every rank: block = picks of every group that runs
     // [group][template][chunk angle][MaxPos+5], then their counts [group][template][chunk angle]; refined block = one
@@ -630,6 +637,7 @@ bool fw_box_fits(int vec)
 bool corr_warp_usable(const fpm_handle* h, int tw, int n_ang, const FpmLevel& L)
 {
     if (h->use_tc != 6 || h->members.size() > 1 || !h->tpl[0].mask.empty()) return false;   // opt-in: bit-identical, less DRAM traffic, but slower than warp + MMA today
+    if (h->scale_min != 1.0 || h->scale_max != 1.0) return false;   // scaled ROIs: source boxes this kernel's staging is not sized for
     if (n_ang != 3 || tw < 64 || !get_encode_tiled()) return false;
     return level_copy_vec(L) >= 4 && fw_box_fits(4);       // the box is staged with 4-byte copies
 }
@@ -935,28 +943,51 @@ void angle_schedule(const fpm_handle* h, int top, std::vector<double>& angles)
     }
 }
 
+// Scale schedule of the range [lo, hi] for a top template level of w x h: {lo} when lo == hi, else n geometric steps of at most
+// 1 + ds, ds = 2 / max(w, h) (the template's far edge moves by about 2 px, like the angle step atan(2 / max(w, h))), ending
+// exactly at hi
+void scale_schedule(double lo, double hi, int w, int h, std::vector<double>& out)
+{
+    out.clear();
+    if (lo == hi) { out.push_back(lo); return; }
+    const double ds = 2.0 / std::max(w, h), r = log(hi / lo);
+    const int n = (int)ceil(r / log1p(ds)) + 1;
+    for (int k = 0; k < n - 1; k++) out.push_back(lo * exp(k * r / (n - 1)));
+    out.push_back(hi);
+}
+
 // The plan always covers the whole schedule (a few dozen doubles per angle); a partial sweep (stage API, angle-sharded
 // mode) runs a sub-range of its job list, so a cached plan can never truncate a later full sweep.
 int make_top_plan(fpm_handle* h, int top, int batch)
 {
     const FpmLevel& L = h->levels[top];
     TopPlan& p = h->plan;
-    if (p.valid && p.sw == L.w && p.sh == L.h && p.top == top && p.batch == batch && p.tol == h->tol_angle)
+    if (p.valid && p.sw == L.w && p.sh == L.h && p.top == top && p.batch == batch && p.tol == h->tol_angle &&
+        p.scale_min == h->scale_min && p.scale_max == h->scale_max)
         return FPM_OK;
     p.valid = false;
-    angle_schedule(h, top, p.angles);
-    p.sw = L.w; p.sh = L.h; p.top = top; p.batch = batch; p.tol = h->tol_angle;
-    p.n_ang = (int)p.angles.size();
     const TplLevelHost& t = h->tpl[top];
+    std::vector<double> ang1, sc;
+    angle_schedule(h, top, ang1);
+    scale_schedule(h->scale_min, h->scale_max, t.w, t.h, sc);
+    p.angles.clear(); p.scales.clear();
+    for (double s : sc)
+        for (double a : ang1) { p.angles.push_back(a); p.scales.push_back(s); }
+    p.sw = L.w; p.sh = L.h; p.top = top; p.batch = batch; p.tol = h->tol_angle; p.scale_min = h->scale_min; p.scale_max = h->scale_max;
+    p.n_ang = (int)p.angles.size();
     float cx = (L.w - 1) / 2.0f, cy = (L.h - 1) / 2.0f;
     std::vector<FpmWarpJob> jobs((size_t)batch * std::max(p.n_ang, 1));
     p.ftx.assign(p.n_ang, 0.f); p.fty.assign(p.n_ang, 0.f);
     p.maxW = p.maxH = 1;
     for (int a = 0; a < p.n_ang; a++) {
+        // scale s: the canvas resamples the level by 1/s around its centre (getRotationMatrix2D(c, angle, 1/s)) and is sized for
+        // the resampled level, cvRound(w / s) x cvRound(h / s)
+        const double s = p.scales[a];
+        const int rsw = s == 1.0 ? L.w : (int)lrint(L.w / s), rsh = s == 1.0 ? L.h : (int)lrint(L.h / s);
         FpmWarpJob jb;
-        fpm_rotation_matrix(cx, cy, p.angles[a], jb.m);
+        fpm_rotation_matrix(cx, cy, p.angles[a], jb.m, 1.0 / s);
         int bw, bh;
-        best_rotation_size(L.w, L.h, t.w, t.h, p.angles[a], &bw, &bh);
+        best_rotation_size(rsw, rsh, t.w, t.h, p.angles[a], &bw, &bh);
         float fTx = (bw - 1) / 2.0f - cx, fTy = (bh - 1) / 2.0f - cy;
         jb.m[2] += (double)fTx; jb.m[5] += (double)fTy;
         fpm_invert_affine(jb.m);
@@ -970,6 +1001,8 @@ int make_top_plan(fpm_handle* h, int top, int batch)
         CK(cudaMemcpyAsync(h->d_jobs_top.p, jobs.data(), jobs.size() * sizeof(FpmWarpJob), cudaMemcpyHostToDevice, h->stream));
         CK(h->d_angles.ensure(p.n_ang * sizeof(double)));
         CK(cudaMemcpyAsync(h->d_angles.p, p.angles.data(), p.n_ang * sizeof(double), cudaMemcpyHostToDevice, h->stream));
+        CK(h->d_scales.ensure(p.n_ang * sizeof(double)));
+        CK(cudaMemcpyAsync(h->d_scales.p, p.scales.data(), p.n_ang * sizeof(double), cudaMemcpyHostToDevice, h->stream));
         CK(h->d_ftx.ensure(p.n_ang * sizeof(float)));
         CK(h->d_fty.ensure(p.n_ang * sizeof(float)));
         CK(cudaMemcpyAsync(h->d_ftx.p, p.ftx.data(), p.n_ang * sizeof(float), cudaMemcpyHostToDevice, h->stream));
@@ -1120,6 +1153,8 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
         return FPM_OK;
     }
     const int n_ang = (!h->tol_range && h->tol_angle < FPM_VISION_TOLERANCE) ? 1 : 3;
+    // a scale range refines the scale too: evals k * n_ang + j over the scales s / (1 + ds_L), s, s * (1 + ds_L)
+    const int n_sc = h->scale_min != h->scale_max ? 3 : 1, n_ev = n_sc * n_ang;
     CK(h->d_cand[1].ensure((size_t)n_cands * sizeof(FpmCand)));
     int cur = 0, n = n_cands;
     double layer_score[FPM_MAX_LEVELS + 1];
@@ -1132,9 +1167,9 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
     }
     const size_t budget = (size_t)(h->workspace_mb * 1024.0 * 1024.0);
     // the descent without host round trips needs every layer to fit one workspace wave at the top-layer count
-    bool async = !h->trace && n_cands <= 65535 && (h->async_descent == 1 || (h->async_descent < 0 && h->cur_batch < 8));
+    bool async = !h->trace && n_cands * n_sc <= 65535 && (h->async_descent == 1 || (h->async_descent < 0 && h->cur_batch < 8));
     for (int layer = top - 1; layer >= stop && async; layer--)
-        if (refine_layer(h, layer, n_ang).per_eval * n_ang * (size_t)n_cands > budget) async = false;
+        if (refine_layer(h, layer, n_ang).per_eval * n_ev * (size_t)n_cands > budget) async = false;
     if (async) CK(cudaMemsetAsync(counters + CNT_LAYER, 0, FPM_MAX_LEVELS * sizeof(int), h->stream));
     for (int layer = top - 1; layer >= stop && n > 0; layer--) {
         const TplLevelHost& t = h->tpl[layer];
@@ -1144,24 +1179,25 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
         const int rpitch = rl.rpitch;
         const size_t roi_stride = rl.roi_stride;
         const bool warp_fused = rl.warp_fused;
-        int wave_cands = (int)std::max<size_t>(1, budget / (rl.per_eval * n_ang));
+        const double scale_step = 2.0 / std::max(t.w, t.h);
+        int wave_cands = (int)std::max<size_t>(1, budget / (rl.per_eval * n_ev));
         wave_cands = std::min(wave_cands, n);
-        wave_cands = std::min(wave_cands, 65535);             // one candidate per gridDim.y slot of the ROI warp
-        const int wave_evals = wave_cands * n_ang;
+        wave_cands = std::min(wave_cands, 65535 / n_sc);      // one (candidate, scale) per gridDim.y slot of the ROI warp
+        const int wave_evals = wave_cands * n_ev;
         CK(h->d_jobs_ref.ensure((size_t)wave_evals * sizeof(FpmWarpJob)));
         if (!warp_fused) CK(h->d_roi.ensure(roi_stride * wave_evals));
         if (!mma_usable(h, t.w)) CK(h->d_rowsum.ensure((size_t)wave_evals * t.h * FPM_NCELL * 4));
         CK(h->d_rowS.ensure((size_t)wave_evals * (t.h + FPM_ROI_PAD) * FPM_WSTRIDE * 4));
         CK(h->d_rowQ.ensure((size_t)wave_evals * (t.h + FPM_ROI_PAD) * FPM_WSTRIDE * 4));
         if (h->trace) {
-            CK(h->d_trace.ensure((size_t)n * n_ang * sizeof(FpmEvalTrace)));
-            CK(cudaMemsetAsync(h->d_trace.p, 0, (size_t)n * n_ang * sizeof(FpmEvalTrace), h->stream));
+            CK(h->d_trace.ensure((size_t)n * n_ev * sizeof(FpmEvalTrace)));
+            CK(cudaMemsetAsync(h->d_trace.p, 0, (size_t)n * n_ev * sizeof(FpmEvalTrace), h->stream));
             // all-ones bytes are NaN: a score cell the finalize kernel does not write cannot pass for a result
-            CK(h->d_trace_sc.ensure((size_t)n * n_ang * FPM_NCELL * sizeof(float)));
-            CK(cudaMemsetAsync(h->d_trace_sc.p, 0xff, (size_t)n * n_ang * FPM_NCELL * sizeof(float), h->stream));
+            CK(h->d_trace_sc.ensure((size_t)n * n_ev * FPM_NCELL * sizeof(float)));
+            CK(cudaMemsetAsync(h->d_trace_sc.p, 0xff, (size_t)n * n_ev * FPM_NCELL * sizeof(float), h->stream));
             fpm_handle::TraceRois& tr = h->tr_rois[layer];
             tr.w = t.w + FPM_ROI_PAD; tr.h = t.h + FPM_ROI_PAD; tr.pitch = rpitch;
-            tr.px.assign(warp_fused ? 0 : (size_t)n * n_ang * roi_stride, 0);
+            tr.px.assign(warp_fused ? 0 : (size_t)n * n_ev * roi_stride, 0);
         }
         // live candidates of this layer / where the survivors are counted
         const int* n_dev = !async ? nullptr : (layer == top - 1 ? counters + CNT_FLAT : counters + CNT_LAYER + layer);
@@ -1177,7 +1213,7 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
         const FpmCand* cands = h->d_cand[cur].as<FpmCand>();
         for (int c0 = 0; c0 < n; c0 += wave_cands) {
             const int nc = std::min(wave_cands, n - c0);
-            const int ne = nc * n_ang;
+            const int ne = nc * n_ev;
             if (warp_fused)                                 // the warp-fused kernel stages the job matrices of its 42 candidates itself
                 KL(K_PREP, (double)ne * sizeof(FpmWarpJob),
                    fpm_refine_prep_kernel<<<(ne + 127) / 128, 128, 0, h->stream>>>(cands + c0, nc, n_ang, step, L.w, L.h, t.w, t.h,
@@ -1193,7 +1229,7 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                 raw_tile_evals = FW_TILE_EVALS;
             } else {
                 const int wtiles_x = (rpitch + WA_TW - 1) / WA_TW;
-                dim3 wgrid(wtiles_x * ((t.h + FPM_ROI_PAD + WA_TH - 1) / WA_TH), nc);      // one CTA = one tile of the n_ang ROIs of a candidate
+                dim3 wgrid(wtiles_x * ((t.h + FPM_ROI_PAD + WA_TH - 1) / WA_TH), nc * n_sc);   // one CTA = one tile of the n_ang ROIs of a (candidate, scale)
                 // algorithmic bytes: 1 B gathered + 1 B written per ROI pixel (SURVEY 8d)
                 // which correlation kernel will read the patches (the one-CTA-per-128-evals kernel only pays for many LIVE evals:
                 // never with an upper-bound count)
@@ -1204,15 +1240,15 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                    fpm_warp_kernel<<<wgrid, WA_THREADS, 0, h->stream>>>(nullptr, n_ang, L,
                                                                         h->d_roi.as<uint8_t>(), rpitch, roi_stride, 0, wtiles_x,
                                                                         level_vec_ok(L), n_dev,
-                                                                        FpmRefineGeom{cands + c0, n_ang, step, L.w, L.h, t.w, t.h, n_tpl}));
+                                                                        FpmRefineGeom{cands + c0, n_ang, n_sc, step, scale_step, L.w, L.h, t.w, t.h, n_tpl}));
                 if (go_fused) {
                     int rcm = launch_corr_fused(h, h->d_roi.as<uint8_t>(), rpitch, roi_stride, h->d_tsh.as<uint8_t>() + t.tsh_off, t.bpitch,
-                                                t.w, t.h, ne, h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ang);
+                                                t.w, t.h, ne, h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ev);
                     if (rcm) return rcm;
                     fused = true;
                 } else if (mma_usable(h, t.w)) {
                     int rcm = launch_corr_mma(h, h->d_roi.as<uint8_t>(), rpitch, roi_stride, h->d_tsh.as<uint8_t>() + t.tsh_off, t.bpitch,
-                                              t.w, t.h, ne, &raw_epad, h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ang);
+                                              t.w, t.h, ne, &raw_epad, h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ev);
                     if (rcm) return rcm;
                 } else {
                     dim3 cgrid(cc.blocks_y_rows, (ne + cc.evals_per_cta - 1) / cc.evals_per_cta);
@@ -1220,13 +1256,13 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                     KL(K_CORR, (double)ne * FPM_NCELL * (double)t.w * t.h,
                        fpm_corr_rows_kernel<<<cgrid, cc.threads, smem, h->stream>>>(h->d_roi.as<uint8_t>(), rpitch, roi_stride, td, ne,
                                                                                     cc.rb, cc.evals_per_cta, h->d_rowsum.as<int32_t>(),
-                                                                                    h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ang,
+                                                                                    h->d_rowS.as<int32_t>(), h->d_rowQ.as<int32_t>(), n_dev, n_ev,
                                                                                     cands + c0));
                 }
             }
             const bool masked = td.mrun && !t.all_flat;      // finalize reads the sums of the members that are not flat
             if (masked) {
-                int rcm = launch_mask_window(h, rpitch, roi_stride, td, ne, n_dev, n_ang, cands + c0);
+                int rcm = launch_mask_window(h, rpitch, roi_stride, td, ne, n_dev, n_ev, cands + c0);
                 if (rcm) return rcm;
             }
             {
@@ -1238,13 +1274,13 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
                        L.h, layer_score[layer], h->use_simd, layer == stop ? 1 : 0, stop ? 2 : 1, (h->subpixel && layer == 0) ? 1 : 0,
                        h->d_cand[cur ^ 1].as<FpmCand>(),
                        next_cnt, ref_out, ref_cnt,
-                       h->trace ? h->d_trace.as<FpmEvalTrace>() + (size_t)c0 * n_ang : nullptr,
-                       h->trace ? h->d_trace_sc.as<float>() + (size_t)c0 * n_ang * FPM_NCELL : nullptr,
+                       h->trace ? h->d_trace.as<FpmEvalTrace>() + (size_t)c0 * n_ev : nullptr,
+                       h->trace ? h->d_trace_sc.as<float>() + (size_t)c0 * n_ev * FPM_NCELL : nullptr,
                        fused ? h->d_numer.as<float>() : nullptr, (masked ? h->d_mwS : h->d_totS).as<long long>(),
-                       (masked ? h->d_mwQ : h->d_totQ).as<long long>(), raw_tile_evals, n_dev));
+                       (masked ? h->d_mwQ : h->d_totQ).as<long long>(), raw_tile_evals, n_dev, n_sc, scale_step));
             }
             if (h->trace && !warp_fused)                    // this wave's ROI patches, before the next wave overwrites them
-                CK(cudaMemcpyAsync(h->tr_rois[layer].px.data() + (size_t)c0 * n_ang * roi_stride, h->d_roi.p, (size_t)ne * roi_stride,
+                CK(cudaMemcpyAsync(h->tr_rois[layer].px.data() + (size_t)c0 * n_ev * roi_stride, h->d_roi.p, (size_t)ne * roi_stride,
                                    cudaMemcpyDeviceToHost, h->stream));
         }
         cur ^= 1;
@@ -1253,19 +1289,19 @@ int run_refine(fpm_handle* h, int top, int n_cands, int* n_refined_out)
         CK(cudaStreamSynchronize(h->stream));
         if (h->trace) {
             const FpmCand* cands_done = h->d_cand[cur ^ 1].as<FpmCand>();
-            std::vector<FpmEvalTrace> tr((size_t)n * n_ang);
+            std::vector<FpmEvalTrace> tr((size_t)n * n_ev);
             std::vector<FpmCand> cc2(n);
             CK(cudaMemcpy(tr.data(), h->d_trace.p, tr.size() * sizeof(FpmEvalTrace), cudaMemcpyDeviceToHost));
             CK(cudaMemcpy(cc2.data(), cands_done, cc2.size() * sizeof(FpmCand), cudaMemcpyDeviceToHost));
             std::vector<double>& rows = h->tr_evals[layer];
             for (int i = 0; i < n; i++)
-                for (int j = 0; j < n_ang; j++) {
-                    const FpmEvalTrace& e = tr[(size_t)i * n_ang + j];
+                for (int j = 0; j < n_ev; j++) {
+                    const FpmEvalTrace& e = tr[(size_t)i * n_ev + j];
                     rows.push_back(cc2[i].id); rows.push_back(e.angle); rows.push_back(e.score);
                     rows.push_back(e.locx); rows.push_back(e.locy);
                 }
             std::vector<float>& sc = h->tr_scores[layer];
-            sc.resize((size_t)n * n_ang * FPM_NCELL);
+            sc.resize((size_t)n * n_ev * FPM_NCELL);
             CK(cudaMemcpy(sc.data(), h->d_trace_sc.p, sc.size() * sizeof(float), cudaMemcpyDeviceToHost));
         }
         if (hc[CNT_ERR]) { h->err = "fpm_corr_warp_kernel: source box larger than its staging buffer"; return FPM_ERR_LIMIT; }
@@ -1345,6 +1381,7 @@ int run_final(fpm_handle* h, int batch, const FpmRefinedView& rv, int key_stride
         for (int i = 0; i < m; i++) {
             const FpmResultDev& r = hr[(size_t)b * rcap + i];
             fpm_result& o = out[slot * cap + i];
+            if (h->scales_out) h->scales_out[&o - h->scales_base] = r.scale;
             o.score = r.score; o.angle = r.angle; o.cx = r.cx; o.cy = r.cy;
             o.ltx = r.ltx; o.lty = r.lty; o.rtx = r.rtx; o.rty = r.rty;
             o.rbx = r.rbx; o.rby = r.rby; o.lbx = r.lbx; o.lby = r.lby;
@@ -1382,7 +1419,8 @@ int collect_candidates(fpm_handle* h, int top, int batch, const FpmPickView& pv,
                h->d_ftx.as<float>(), h->d_fty.as<float>(), (L.w - 1) / 2.0f, (L.h - 1) / 2.0f,
                h->d_keys.as<unsigned long long>(), n_pad, use_smem, h->d_off.as<int>(), h->d_cand[0].as<FpmCand>(),
                counters + CNT_FLAT, h->trace ? h->d_toppt.as<float>() : nullptr, cand_stride,
-               h->d_candcnt.as<int>(), 0, shard_rank, shard_n));
+               h->d_candcnt.as<int>(), 0, shard_rank, shard_n,
+               (h->scale_min == 1.0 && h->scale_max == 1.0) ? nullptr : h->d_scales.as<double>()));
     }
     if (!n_cands) return FPM_OK;
     int* hc = h->h_counts.as<int>();
@@ -1558,6 +1596,22 @@ int merge_setup(fpm_handle* h, int batch, int cap, int n_set, const std::vector<
     return FPM_OK;
 }
 
+// The match scale range (FPM_PARAM_SCALE_MIN / MAX), checked at match time because the two setters may run in either order:
+// min <= max, and [1, 1] on the calls that do not carry a scale (scaled_ok = false: template sets of more than one template, the
+// angle-sharded calls, fpm_stage_*).
+int refuse_scale(const fpm_handle* h, const char* fn, bool scaled_ok)
+{
+    if (h->scale_min == 1.0 && h->scale_max == 1.0) return FPM_OK;
+    if (h->scale_min > h->scale_max)
+        h->err = std::string(fn) + ": FPM_PARAM_SCALE_MIN (" + std::to_string(h->scale_min) + ") > FPM_PARAM_SCALE_MAX (" +
+                 std::to_string(h->scale_max) + ")";
+    else if (!scaled_ok)
+        h->err = std::string(fn) + ": this call matches at scale 1 only (set FPM_PARAM_SCALE_MIN = FPM_PARAM_SCALE_MAX = 1)";
+    else
+        return FPM_OK;
+    return FPM_ERR_INVALID;
+}
+
 // whole match() over a device-resident batch, for every template of the set: frame b / template t at out + (b * n + t) * cap,
 // or (mg) the merged list of frame b at out + b * cap.
 // The source pyramid (and bitwise_not) is built once, down to the deepest top layer of any group; the groups run one
@@ -1569,7 +1623,10 @@ int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt,
     for (int b = 0; b < batch * (mg ? 1 : n_set); b++) n_out[b] = 0;
     if (mg && mg->set_counts) std::fill(mg->set_counts, mg->set_counts + (size_t)batch * n_set, 0);
     if (!h->learned) return FPM_OK;                          // :99-101 -> empty
-    int rc = ensure_learned_for_mra(h);
+    const bool is_set = fpm_set_size(h) > 1;
+    int rc = refuse_scale(h, is_set ? "fpm_match_set_batch" : "fpm_match", !is_set);
+    if (rc) return rc;
+    rc = ensure_learned_for_mra(h);
     if (rc) return rc;
     const size_t n_groups = h->groups.size();
     std::vector<char> run;
@@ -2008,6 +2065,14 @@ int fpm_set_param(fpm_handle* h, int param, double v)
     case FPM_PARAM_TOLERANCE_RANGE: h->tol_range = v != 0; break;
     case FPM_PARAM_TOLERANCE1: case FPM_PARAM_TOLERANCE2: case FPM_PARAM_TOLERANCE3: case FPM_PARAM_TOLERANCE4:
         h->tol_r[param - FPM_PARAM_TOLERANCE1] = v; break;
+    case FPM_PARAM_SCALE_MIN: case FPM_PARAM_SCALE_MAX:
+        // beyond 2 the bilinear resampling (no prefilter) aliases; below 0.5 the top-layer canvases grow by 4x or more
+        if (!std::isfinite(v) || v < 0.5 || v > 2.0) {
+            h->err = std::string(param == FPM_PARAM_SCALE_MIN ? "FPM_PARAM_SCALE_MIN" : "FPM_PARAM_SCALE_MAX") + " must lie in [0.5, 2], got " +
+                     std::to_string(v);
+            return FPM_ERR_INVALID;
+        }
+        (param == FPM_PARAM_SCALE_MIN ? h->scale_min : h->scale_max) = v; break;
     default: h->err = "unknown parameter"; return FPM_ERR_INVALID;
     }
     if (param == FPM_PARAM_TOLERANCE_RANGE || (param >= FPM_PARAM_TOLERANCE1 && param <= FPM_PARAM_TOLERANCE4)) {
@@ -2044,6 +2109,8 @@ double fpm_get_param(const fpm_handle* h, int param)
     case FPM_PARAM_TOLERANCE_RANGE: return h->tol_range;
     case FPM_PARAM_TOLERANCE1: case FPM_PARAM_TOLERANCE2: case FPM_PARAM_TOLERANCE3: case FPM_PARAM_TOLERANCE4:
         return h->tol_r[param - FPM_PARAM_TOLERANCE1];
+    case FPM_PARAM_SCALE_MIN: return h->scale_min;
+    case FPM_PARAM_SCALE_MAX: return h->scale_max;
     default: return 0;
     }
 }
@@ -2210,6 +2277,7 @@ int match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width
         // the other half's kernels fill the device.
         rc = ensure_twin(h);
         if (rc) return rc;
+        h->twin->scales_out = h->scales_out; h->twin->scales_base = h->scales_base;
         const int b0 = batch / 2;
         int rc2 = FPM_OK;
         const SetMerge mg2 = mg ? mg->shifted(b0, cap, n_set) : SetMerge{};
@@ -3177,6 +3245,37 @@ int fpm_ingested_pixels(fpm_handle* h, uint8_t* out)
     return fpm_ingested_frame_pixels(h, 0, out);
 }
 
+namespace {
+// fpm_match_scaled / fpm_match_ingested_scaled: the scale of every record written during the call goes to scales
+struct ScalesOut {
+    fpm_handle* h;
+    ScalesOut(fpm_handle* hh, fpm_result* out, double* scales) : h(hh) { h->scales_out = scales; h->scales_base = out; }
+    ~ScalesOut()
+    {
+        h->scales_out = nullptr; h->scales_base = nullptr;
+        if (h->twin) { h->twin->scales_out = nullptr; h->twin->scales_base = nullptr; }
+    }
+};
+}  // namespace
+
+int fpm_match_scaled(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                     size_t frame_stride, fpm_result* out, double* scales, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_match_scaled")) return rc;
+    ScalesOut so(h, out, scales);
+    return src_on_device ? match_batch_device(h, src, batch, width, height, stride, frame_stride, out, cap, counts)
+                         : match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, counts);
+}
+
+int fpm_match_ingested_scaled(fpm_handle* h, fpm_result* out, double* scales, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    if (int rc = refuse_set(h, "fpm_match_ingested_scaled")) return rc;
+    ScalesOut so(h, out, scales);
+    return fpm_match_ingested_set_batch(h, out, cap, counts);
+}
+
 int fpm_match_ingested(fpm_handle* h, fpm_result* out, int cap, int* n)
 {
     if (!h) return FPM_ERR_INVALID;
@@ -3305,6 +3404,7 @@ int fpm_stage_top(fpm_handle* h, const uint8_t* src, int width, int height, int 
 {
     if (!h || !n) return FPM_ERR_INVALID;
     if (int rc = refuse_set(h, "fpm_stage_top")) return rc;
+    if (int rc = refuse_scale(h, "fpm_stage_top", false)) return rc;
     *n = 0;
     if (!h->learned) return FPM_ERR_NOT_LEARNED;
     int rc = ensure_learned_for_mra(h);
@@ -3382,6 +3482,7 @@ int fpm_stage_sort_candidates(fpm_handle* h, const double* picks, int n, double*
 {
     if (!h || n < 0) return FPM_ERR_INVALID;
     if (int rc = refuse_set(h, "fpm_stage_sort_candidates")) return rc;
+    if (int rc = refuse_scale(h, "fpm_stage_sort_candidates", false)) return rc;
     if (h->levels.empty()) { h->err = "fpm_stage_top must run first"; return FPM_ERR_INVALID; }
     std::vector<int> idx(n);
     for (int i = 0; i < n; i++) idx[i] = i;
@@ -3402,6 +3503,7 @@ int fpm_stage_refine(fpm_handle* h, const double* cands, int n, double* rows, in
 {
     if (!h || !n_out) return FPM_ERR_INVALID;
     if (int rc = refuse_set(h, "fpm_stage_refine")) return rc;
+    if (int rc = refuse_scale(h, "fpm_stage_refine", false)) return rc;
     *n_out = 0;
     if (h->levels.empty()) { h->err = "fpm_stage_top must run first"; return FPM_ERR_INVALID; }
     CK(cudaSetDevice(h->device));
@@ -3410,7 +3512,7 @@ int fpm_stage_refine(fpm_handle* h, const double* cands, int n, double* rows, in
     for (int i = 0; i < n; i++) {
         const double* c = cands + (size_t)i * 5;
         cc[i].id = (int)c[0]; cc[i].ptx = (float)c[1]; cc[i].pty = (float)c[2]; cc[i].score = c[3]; cc[i].angle = c[4];
-        cc[i].img = 0;
+        cc[i].img = 0; cc[i].scale = 1.0;
     }
     CK(h->d_cand[0].ensure(cc.size() * sizeof(FpmCand)));
     CK(cudaMemcpyAsync(h->d_cand[0].p, cc.data(), cc.size() * sizeof(FpmCand), cudaMemcpyHostToDevice, h->stream));
@@ -3447,6 +3549,7 @@ int fpm_stage_final(fpm_handle* h, const double* refined, int n, fpm_result* out
 {
     if (!h || !n_out) return FPM_ERR_INVALID;
     if (int rc = refuse_set(h, "fpm_stage_final")) return rc;
+    if (int rc = refuse_scale(h, "fpm_stage_final", false)) return rc;
     *n_out = 0;
     if (!h->learned) return FPM_ERR_NOT_LEARNED;
     CK(cudaSetDevice(h->device));
@@ -3454,7 +3557,7 @@ int fpm_stage_final(fpm_handle* h, const double* refined, int n, fpm_result* out
     int max_id = 0;
     for (int i = 0; i < n; i++) {
         const double* r = refined + (size_t)i * 5;
-        rr[i].id = (int)r[0]; rr[i].ptx = r[1]; rr[i].pty = r[2]; rr[i].score = r[3]; rr[i].angle = r[4]; rr[i].img = 0;
+        rr[i].id = (int)r[0]; rr[i].ptx = r[1]; rr[i].pty = r[2]; rr[i].score = r[3]; rr[i].angle = r[4]; rr[i].img = 0; rr[i].scale = 1.0;
         max_id = std::max(max_id, rr[i].id);
     }
     CK(h->d_counters.ensure(CNT_N * sizeof(int)));
@@ -3531,6 +3634,7 @@ namespace {
 // refusals shared by the whole-set sharded calls (fpm_match_set_batch's, plus a missing communicator)
 int check_set_sharded(fpm_handle* h, const char* fn, int cap, const void* out, const int* n)
 {
+    if (int rc = refuse_scale(h, fn, false)) return rc;
     if (h->trace && fpm_set_size(h) > 1) {
         h->err = std::string(fn) + ": FPM_PARAM_TRACE is not supported for a set of more than one template";
         return FPM_ERR_INVALID;
@@ -3560,6 +3664,8 @@ int check_virtual(fpm_handle* const* hs, int nranks, const char* fn, bool whole_
         for (int r = 0; r < nranks; r++) hs[r]->err = std::string(fn) + ": " + msg;
         return FPM_ERR_INVALID;
     };
+    for (int r = 0; r < nranks; r++)
+        if (int rc = refuse_scale(hs[r], fn, false)) return rc;
     for (int r = 0; r < nranks; r++) {
         if (hs[r]->nccl_comm) return whole_set ? refuse("the handle of rank " + std::to_string(r) + " has a communicator") : FPM_ERR_INVALID;
         if (!whole_set) {
@@ -3578,6 +3684,7 @@ int fpm_match_sharded(fpm_handle* h, const uint8_t* src, int width, int height, 
 {
     if (!h) return FPM_ERR_INVALID;
     if (int rc = refuse_set(h, "fpm_match_sharded")) return rc;
+    if (int rc = refuse_scale(h, "fpm_match_sharded", false)) return rc;
     if (!n || cap < 0 || (cap > 0 && !out)) { h->err = "bad output arguments"; return FPM_ERR_INVALID; }
     *n = 0;
     return match_set_sharded(h, src, width, height, stride, src_on_device, out, cap, n, nullptr);

@@ -51,18 +51,30 @@
 
 // getRotatedROI matrix of eval j of a candidate (src/TemplateMatcher.cpp:1074-1088), inverted like warpAffine does
 // n_tpl: templates of the group (candidate image v reads source frame v / n_tpl)
-struct FpmRefineGeom { const FpmCand* cands; int n_ang; double angle_step; int lvl_w, lvl_h, tpl_w, tpl_h, n_tpl; };
+// Scale-tolerant matching: eval e = k * n_ang + j of a candidate of scale s has angle index j and scale
+// fpm_eval_scale(s, k, n_sc, scale_step): {s / (1 + ds), s, s * (1 + ds)} when a scale range is matched (n_sc == 3), {s}
+// otherwise.  At a scale s != 1 the source is resampled by 1/s around the level centre c: matrix getRotationMatrix2D(c, angle,
+// 1/s), and the anchor becomes c + (1/s) * (rotated anchor - c).
+struct FpmRefineGeom { const FpmCand* cands; int n_ang, n_sc; double angle_step, scale_step; int lvl_w, lvl_h, tpl_w, tpl_h, n_tpl; };
 
-__device__ __forceinline__ FpmWarpJob fpm_refine_job(const FpmCand& c, int j, int n_ang, double angle_step, int lvl_w, int lvl_h,
-                                                     int tpl_w, int tpl_h, int n_tpl)
+FPM_HD double fpm_eval_scale(double s, int k, int n_sc, double ds)
 {
+    return n_sc == 1 ? s : (k == 0 ? s / (1 + ds) : (k == 1 ? s : s * (1 + ds)));
+}
+
+__device__ __forceinline__ FpmWarpJob fpm_refine_job(const FpmCand& c, int e, int n_ang, int n_sc, double angle_step, double scale_step,
+                                                     int lvl_w, int lvl_h, int tpl_w, int tpl_h, int n_tpl)
+{
+    const int k = e / n_ang, j = e - k * n_ang;
+    const double scale = fpm_eval_scale(c.scale, k, n_sc, scale_step);
     double angle = (n_ang == 1) ? 0.0 : c.angle + angle_step * (double)(j - 1);
     float ptcx = (float)(lvl_w - 1) / 2.0f, ptcy = (float)(lvl_h - 1) / 2.0f;
     float ltx = c.ptx * 2, lty = c.pty * 2;
     float rx, ry;
     fpm_pt_rotate(ltx, lty, ptcx, ptcy, angle * FPM_D2R, &rx, &ry);
+    if (scale != 1.0) fpm_scale_about(rx, ry, ptcx, ptcy, 1.0 / scale, &rx, &ry);
     FpmWarpJob jb;
-    fpm_rotation_matrix(ptcx, ptcy, angle, jb.m);
+    fpm_rotation_matrix(ptcx, ptcy, angle, jb.m, 1.0 / scale);
     jb.m[2] -= (double)(rx - 3);
     jb.m[5] -= (double)(ry - 3);
     fpm_invert_affine(jb.m);
@@ -107,13 +119,15 @@ fpm_warp_kernel(const FpmWarpJob* __restrict__ jobs_g, int group, FpmLevel src, 
 {
     // n_groups_dev (optional): number of live job groups, known only on the device (descent without a host round trip per layer:
     // the grid covers an upper bound, the surplus CTAs leave at once)
-    if (n_groups_dev && (int)blockIdx.y >= *n_groups_dev) return;
+    // refinement: blockIdx.y = candidate * n_sc + scale index k, the n_ang ROIs of one scale share a staged box
+    if (n_groups_dev && (int)blockIdx.y >= *n_groups_dev * (geom.cands ? geom.n_sc : 1)) return;
     const int g0 = blockIdx.y * group;
     // jobs: given (top-layer sweep, tests), or the ROI matrices of candidate blockIdx.y computed here from its record
     // (geom.cands != null: one launch less per pyramid layer than a separate preparation kernel)
     __shared__ FpmWarpJob jobs_s[WA_MAXG];
     if (threadIdx.x < group)
-        jobs_s[threadIdx.x] = geom.cands ? fpm_refine_job(geom.cands[blockIdx.y], threadIdx.x, geom.n_ang, geom.angle_step, geom.lvl_w,
+        jobs_s[threadIdx.x] = geom.cands ? fpm_refine_job(geom.cands[blockIdx.y / geom.n_sc], (blockIdx.y % geom.n_sc) * geom.n_ang + threadIdx.x,
+                                                          geom.n_ang, geom.n_sc, geom.angle_step, geom.scale_step, geom.lvl_w,
                                                           geom.lvl_h, geom.tpl_w, geom.tpl_h, geom.n_tpl)
                                          : jobs_g[g0 + threadIdx.x];
     __syncthreads();
@@ -955,8 +969,12 @@ fpm_collect_sort_kernel(FpmPickView pv,
                         int* __restrict__ off_scratch,
                         FpmCand* __restrict__ cands_flat, int* __restrict__ flat_counter,
                         float* __restrict__ top_pt, int cand_stride,
-                        int* __restrict__ cand_count, int angle_idx_base, int shard_rank, int shard_n)
+                        int* __restrict__ cand_count, int angle_idx_base, int shard_rank, int shard_n,
+                        const double* __restrict__ scales)
 {
+    // pose slot a = scale index * n_angles_of_the_schedule + angle index (angles[a], scales[a]; scales null: every slot at scale 1).
+    // At scale s != 1 the canvas resampled the level by 1/s around the centre: a pick maps back by centre + s * (p - centre)
+    // before the un-rotation
     extern __shared__ unsigned long long s_keys[];
     const int img = blockIdx.x, tid = threadIdx.x;
     __shared__ int s_n, s_base;
@@ -1016,8 +1034,11 @@ fpm_collect_sort_kernel(FpmPickView pv,
             c.angle = angles[a];
             c.score = (double)p.v;
             c.img = img; c.id = i;
+            c.scale = scales ? scales[a] : 1.0;
             double dRAngle = -c.angle * FPM_D2R;
-            fpm_pt_rotate(ptx, pty, centre_x, centre_y, dRAngle, &c.ptx, &c.pty);
+            float qx = ptx, qy = pty;
+            if (c.scale != 1.0) fpm_scale_about(ptx, pty, centre_x, centre_y, c.scale, &qx, &qy);
+            fpm_pt_rotate(qx, qy, centre_x, centre_y, dRAngle, &c.ptx, &c.pty);
             cands_flat[base + i / shard_n] = c;
         }
         if (top_pt) {
@@ -1040,7 +1061,7 @@ __global__ void fpm_refine_prep_kernel(const FpmCand* __restrict__ cands, int n_
     int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n_cands * n_ang) return;
     int ci = e / n_ang, j = e - ci * n_ang;
-    jobs[e] = fpm_refine_job(cands[ci], j, n_ang, angle_step, lvl_w, lvl_h, tpl_w, tpl_h, n_tpl);
+    jobs[e] = fpm_refine_job(cands[ci], j, n_ang, 1, angle_step, 0.0, lvl_w, lvl_h, tpl_w, tpl_h, n_tpl);
 }
 
 // =====================================================================================
@@ -1430,6 +1451,7 @@ fpm_mask_window_kernel(const uint8_t* __restrict__ roi, int rpitch, size_t roi_s
 //   best of the 3 angles, layer threshold, pose update (src/TemplateMatcher.cpp:331-367)
 // =====================================================================================
 #define RF_THREADS 192
+#define RF_MAXEV 9         // evals per candidate: 3 angles x 3 scales
 
 // GROUP: the candidates are virtual images of a template group (statistics of template img % n_tpl)
 template <bool GROUP>
@@ -1442,18 +1464,21 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
                            FpmRefined* __restrict__ refined, int* __restrict__ refined_count,
                            FpmEvalTrace* __restrict__ trace, float* __restrict__ trace_scores,
                            const float* __restrict__ numer, const long long* __restrict__ totS,
-                           const long long* __restrict__ totQ, int raw_tile_evals, const int* __restrict__ n_cands_dev)
+                           const long long* __restrict__ totQ, int raw_tile_evals, const int* __restrict__ n_cands_dev,
+                           int n_sc, double scale_step)
 {
     const int ci = blockIdx.x;
     if (n_cands_dev && ci >= *n_cands_dev) return;
     if (GROUP) tpl = fpm_tpl_member(tpl, cands[ci].img % tpl.n_tpl);    // one candidate per CTA: CTA-uniform statistics
-    const int tid = threadIdx.x, j = tid >> 6, cell = tid & 63;
-    __shared__ float s_sc[3][FPM_NCELL];
-    __shared__ float s_best[3];
-    __shared__ int s_loc[3];
+    // n_ev = n_sc * n_ang evals per candidate (eval k * n_ang + j: scale index k, angle index j); the 64-thread eval slots
+    // j0 = 0, 1, 2 take the evals j0, j0 + 3, j0 + 6
+    const int tid = threadIdx.x, j0 = tid >> 6, cell = tid & 63, n_ev = n_sc * n_ang;
+    __shared__ float s_sc[RF_MAXEV][FPM_NCELL];
+    __shared__ float s_best[RF_MAXEV];
+    __shared__ int s_loc[RF_MAXEV];
     __shared__ double s_scratch[27 + 270 + 100 + 100 + 270];
-    __shared__ unsigned long long s_totS[3][FPM_NSHIFT], s_totQ[3][FPM_NSHIFT];      // sums over ALL ROI rows per shift
-    __shared__ int s_edgeS[3][2 * FPM_ROI_PAD][FPM_NSHIFT], s_edgeQ[3][2 * FPM_ROI_PAD][FPM_NSHIFT];   // rows 0..5 and th..th+5
+    __shared__ unsigned long long s_totS[RF_MAXEV][FPM_NSHIFT], s_totQ[RF_MAXEV][FPM_NSHIFT];      // sums over ALL ROI rows per shift
+    __shared__ int s_edgeS[RF_MAXEV][2 * FPM_ROI_PAD][FPM_NSHIFT], s_edgeQ[RF_MAXEV][2 * FPM_ROI_PAD][FPM_NSHIFT];   // rows 0..5 and th..th+5
     const int th = tpl.h;
     // Window sums of CCOEFF_Denominator.  The 49 windows of an eval share their rows: window (r, c) = total of column c over
     // all th + 6 ROI rows minus the r rows above and the 6 - r rows below it.  The totals are gathered by all 64 threads of
@@ -1463,10 +1488,10 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
     const bool masked = tpl.mrun != nullptr;
     const bool coop_window = !tpl.result_equal1 && !numer && !masked;
     if (coop_window) {
-        if (tid < 3 * FPM_NSHIFT) { s_totS[tid / FPM_NSHIFT][tid % FPM_NSHIFT] = 0; s_totQ[tid / FPM_NSHIFT][tid % FPM_NSHIFT] = 0; }
+        for (int i = tid; i < n_ev * FPM_NSHIFT; i += RF_THREADS) { s_totS[i / FPM_NSHIFT][i % FPM_NSHIFT] = 0; s_totQ[i / FPM_NSHIFT][i % FPM_NSHIFT] = 0; }
         __syncthreads();
-        if (j < n_ang) {
-            const int e = ci * n_ang + j;
+        for (int j = j0; j < n_ev; j += 3) {
+            const int e = ci * n_ev + j;
             const int rh = th + FPM_ROI_PAD;
             const int32_t* ps = rowS + (size_t)e * rh * FPM_WSTRIDE;
             const int32_t* pq = rowQ + (size_t)e * rh * FPM_WSTRIDE;
@@ -1508,8 +1533,8 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
         }
         __syncthreads();
     }
-    if (j < n_ang && cell < FPM_NCELL) {
-        const int e = ci * n_ang + j;
+    for (int j = j0; j < n_ev && cell < FPM_NCELL; j += 3) {
+        const int e = ci * n_ev + j;
         const int r = cell / FPM_NSHIFT, c = cell - r * FPM_NSHIFT;
         float sc;
         if (tpl.result_equal1) {
@@ -1585,7 +1610,7 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
         if (trace_scores) trace_scores[(size_t)e * FPM_NCELL + cell] = sc;
     }
     __syncthreads();
-    if (j < n_ang && cell == 0) {
+    for (int j = j0; j < n_ev && cell == 0; j += 3) {
         float best = s_sc[j][0]; int loc = 0;
         for (int i = 1; i < FPM_NCELL; i++) if (s_sc[j][i] > best) { best = s_sc[j][i]; loc = i; }
         s_best[j] = best; s_loc[j] = loc;
@@ -1594,29 +1619,32 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
     if (tid != 0) return;
     const FpmCand c = cands[ci];
     int bi = 0; double big = -1;
-    for (int k = 0; k < n_ang; k++) {
-        double ang = (n_ang == 1) ? 0.0 : c.angle + angle_step * (double)(k - 1);
+    for (int k = 0; k < n_ev; k++) {                                   // the first strict maximum in eval order
+        const int ja = k % n_ang;
+        double ang = (n_ang == 1) ? 0.0 : c.angle + angle_step * (double)(ja - 1);
         if ((double)s_best[k] > big) { bi = k; big = (double)s_best[k]; }
         if (trace) {
             FpmEvalTrace t; t.angle = ang; t.score = s_best[k]; t.locx = s_loc[k] % FPM_NSHIFT; t.locy = s_loc[k] / FPM_NSHIFT;
-            trace[ci * n_ang + k] = t;
+            trace[ci * n_ev + k] = t;
         }
     }
     if ((double)s_best[bi] < layer_score) return;                      // :331-332
-    double new_angle = (n_ang == 1) ? 0.0 : c.angle + angle_step * (double)(bi - 1);
+    const int bj = bi % n_ang, b0 = bi - bj;                           // angle index of the best eval, first eval of its scale
+    const double scale = fpm_eval_scale(c.scale, bi / n_ang, n_sc, scale_step);
+    double new_angle = (n_ang == 1) ? 0.0 : c.angle + angle_step * (double)(bj - 1);
     int lx = s_loc[bi] % FPM_NSHIFT, ly = s_loc[bi] / FPM_NSHIFT;
     double ptx = (double)lx, pty = (double)ly;
     bool on_border = (lx == 0 || ly == 0 || lx == FPM_NSHIFT - 1 || ly == FPM_NSHIFT - 1);
-    if (subpixel && is_last && !on_border && bi == 1 && n_ang == 3) {    // :334-344
+    if (subpixel && is_last && !on_border && bj == 1 && n_ang == 3) {    // :334-344 (the three angle evals of the best scale)
         // neighbours of the other two angles are taken around THEIR OWN maxima (vecResult, :323-328);
         // an angle whose maximum sits on the border leaves vecResult unset in the reference -> 0 here
         double* sc27 = s_scratch;
         for (int t = 0; t < 3; t++) {
-            int tx = s_loc[t] % FPM_NSHIFT, ty = s_loc[t] / FPM_NSHIFT;
+            int tx = s_loc[b0 + t] % FPM_NSHIFT, ty = s_loc[b0 + t] / FPM_NSHIFT;
             bool tb = (tx == 0 || ty == 0 || tx == FPM_NSHIFT - 1 || ty == FPM_NSHIFT - 1);
             for (int y = -1; y <= 1; y++)
                 for (int x = -1; x <= 1; x++)
-                    sc27[t * 9 + (y + 1) * 3 + (x + 1)] = tb ? 0.0 : (double)s_sc[t][(ty + y) * FPM_NSHIFT + tx + x];
+                    sc27[t * 9 + (y + 1) * 3 + (x + 1)] = tb ? 0.0 : (double)s_sc[b0 + t][(ty + y) * FPM_NSHIFT + tx + x];
         }
         double nx, ny, na;
         fpm_subpix(sc27, ptx, pty, new_angle, angle_step, &nx, &ny, &na, s_scratch + 27);
@@ -1626,19 +1654,22 @@ fpm_refine_finalize_kernel(const FpmCand* __restrict__ cands, int n_ang, double 
     float ltx = c.ptx * 2, lty = c.pty * 2;
     float padx, pady;
     fpm_pt_rotate(ltx, lty, ptcx, ptcy, new_angle * FPM_D2R, &padx, &pady);      // :350
+    if (scale != 1.0) fpm_scale_about(padx, pady, ptcx, ptcy, 1.0 / scale, &padx, &pady);   // the ROI's anchor (fpm_refine_job)
     padx = padx - 3.0f; pady = pady - 3.0f;
     float qx = (float)(ptx + (double)padx), qy = (float)(pty + (double)pady);    // :351
+    if (scale != 1.0) fpm_scale_about(qx, qy, ptcx, ptcy, scale, &qx, &qy);
     float rx, ry;
     fpm_pt_rotate(qx, qy, ptcx, ptcy, -new_angle * FPM_D2R, &rx, &ry);           // :353
     if (is_last) {
         FpmRefined o;
         o.angle = new_angle; o.score = (double)s_best[bi];
         o.ptx = (double)(rx * (float)out_scale); o.pty = (double)(ry * (float)out_scale);   // pt * (iStopLayer == 0 ? 1 : 2), :357
-        o.img = c.img; o.id = c.id;
+        o.img = c.img; o.id = c.id; o.scale = scale;
         refined[atomicAdd(refined_count, 1)] = o;
     } else {
         FpmCand o = c;
         o.angle = new_angle;
+        o.scale = scale;
         o.score = (double)s_best[bi];
         o.ptx = rx; o.pty = ry;
         next[atomicAdd(next_count, 1)] = o;
@@ -1805,7 +1836,7 @@ __global__ void fpm_cands_to_refined_kernel(const FpmCand* __restrict__ cands, i
     float k = (top == 0) ? 1.0f : 2.0f;
     o.angle = c.angle; o.score = c.score;
     o.ptx = (double)(c.ptx * k); o.pty = (double)(c.pty * k);
-    o.img = c.img; o.id = c.id;
+    o.img = c.img; o.id = c.id; o.scale = c.scale;
     refined[i] = o;
     if (i == 0) *refined_count = n;
 }
@@ -1816,13 +1847,17 @@ __global__ void fpm_cands_to_refined_kernel(const FpmCand* __restrict__ cands, i
 // =====================================================================================
 struct FpmResultDev {
     double score, angle, cx, cy, ltx, lty, rtx, rty, rbx, rby, lbx, lby;
+    double scale;           // match scale of the target (fpm_match_scaled)
 };
 
-__device__ __forceinline__ void fpm_corners(double ptx, double pty, double angle, int w, int h, float* lt,
+// wd, hd: the rectangle's size, the template's times the match scale (exact integers at scale 1), narrowed to float here like
+// the reference's float corner math
+__device__ __forceinline__ void fpm_corners(double ptx, double pty, double angle, double wd, double hd, float* lt,
                                             float* rt, float* lb, float* rb)
 {
     double dRAngle = -angle * FPM_D2R;
     float c = (float)cos(dRAngle), s = (float)sin(dRAngle);
+    const float w = (float)wd, h = (float)hd;
     lt[0] = (float)ptx; lt[1] = (float)pty;
     rt[0] = lt[0] + w * c; rt[1] = lt[1] - w * s;
     lb[0] = lt[0] + h * s; lb[1] = lt[1] + h * c;
@@ -1940,7 +1975,7 @@ __device__ __forceinline__ void fpm_greedy_nms(const FpmRRect* __restrict__ rect
 
 __global__ void __launch_bounds__(FN_THREADS)
 fpm_final_kernel(FpmRefinedView rv,
-                 double score_thresh, double max_overlap, int nms_w, int nms_h, int tpl_w, int tpl_h,
+                 double score_thresh, double max_overlap, double nms_w, double nms_h, double tpl_w, double tpl_h,
                  unsigned long long* __restrict__ key_scratch, int key_stride,
                  FpmRRect* __restrict__ rect_scratch, int* __restrict__ del_scratch,
                  int* __restrict__ idmap_scratch, unsigned char* __restrict__ pair_scratch, int pair_cap,
@@ -1991,7 +2026,7 @@ fpm_final_kernel(FpmRefinedView rv,
     for (int i = tid; i < m; i += FN_THREADS) {
         const FpmRefined& r = fpm_refined_at(rv, (int)(uint32_t)(keys[i] & 0xffffffffu));
         float lt[2], rt[2], lb[2], rb[2];
-        fpm_corners(r.ptx, r.pty, r.angle, nms_w, nms_h, lt, rt, lb, rb);
+        fpm_corners(r.ptx, r.pty, r.angle, nms_w * r.scale, nms_h * r.scale, lt, rt, lb, rb);   // the scaled rectangle
         rects[i] = fpm_rrect_from3(lt[0], lt[1], rt[0], rt[1], rb[0], rb[1]);
         del[i] = 0;
     }
@@ -2029,10 +2064,12 @@ fpm_final_kernel(FpmRefinedView rv,
         const FpmRefined& r = fpm_refined_at(rv, (int)(uint32_t)(keys[i] & 0xffffffffu));
         FpmResultDev o;
         o.score = r.score;
+        o.scale = r.scale;
+        const double tw = tpl_w * r.scale, th = tpl_h * r.scale;
         if (!mfc_compat) {
             // Qt TemplateMatcher conversion (src/TemplateMatcher.cpp:407-432): float corner math
             float lt[2], rt[2], lb[2], rb[2];
-            fpm_corners(r.ptx, r.pty, r.angle, tpl_w, tpl_h, lt, rt, lb, rb);
+            fpm_corners(r.ptx, r.pty, r.angle, tw, th, lt, rt, lb, rb);
             o.angle = r.angle;
             o.cx = (double)((lt[0] + rt[0] + lb[0] + rb[0]) / 4.0f);
             o.cy = (double)((lt[1] + rt[1] + lb[1] + rb[1]) / 4.0f);
@@ -2043,9 +2080,9 @@ fpm_final_kernel(FpmRefinedView rv,
             // angle negated and wrapped to [-180, 180]
             const double a = -r.angle * FPM_D2R, c = cos(a), sn = sin(a);
             o.ltx = r.ptx; o.lty = r.pty;
-            o.rtx = o.ltx + tpl_w * c; o.rty = o.lty - tpl_w * sn;
-            o.lbx = o.ltx + tpl_h * sn; o.lby = o.lty + tpl_h * c;
-            o.rbx = o.rtx + tpl_h * sn; o.rby = o.rty + tpl_h * c;
+            o.rtx = o.ltx + tw * c; o.rty = o.lty - tw * sn;
+            o.lbx = o.ltx + th * sn; o.lby = o.lty + th * c;
+            o.rbx = o.rtx + th * sn; o.rby = o.rty + th * c;
             o.cx = (o.ltx + o.rtx + o.rbx + o.lbx) / 4;
             o.cy = (o.lty + o.rty + o.rby + o.lby) / 4;
             double ang = -r.angle;

@@ -20,7 +20,8 @@ PYBIND11_MODULE(fpm_b200_pybind, m)
         .def_property_readonly("ptLB", [](const fpm::SingleTargetMatch& r) { return py::make_tuple(r.ptLB.x, r.ptLB.y); })
         .def_property_readonly("ptCenter", [](const fpm::SingleTargetMatch& r) { return py::make_tuple(r.ptCenter.x, r.ptCenter.y); })
         .def_readonly("dMatchedAngle", &fpm::SingleTargetMatch::dMatchedAngle)
-        .def_readonly("dMatchScore", &fpm::SingleTargetMatch::dMatchScore);
+        .def_readonly("dMatchScore", &fpm::SingleTargetMatch::dMatchScore)
+        .def_readonly("dScale", &fpm::SingleTargetMatch::dScale);
     py::class_<fpm::TemplateMatcher>(m, "TemplateMatcher")
         .def(py::init<int, int>(), py::arg("device") = 0, py::arg("result_capacity") = 4096)
         .def("setMaxPositions", &fpm::TemplateMatcher::setMaxPositions)
@@ -30,6 +31,8 @@ PYBIND11_MODULE(fpm_b200_pybind, m)
         .def("setMinReduceArea", &fpm::TemplateMatcher::setMinReduceArea)
         .def("setUseSIMD", &fpm::TemplateMatcher::setUseSIMD)
         .def("setSubPixelEstimation", &fpm::TemplateMatcher::setSubPixelEstimation)
+        .def("setScaleRange", &fpm::TemplateMatcher::setScaleRange)
+        .def("getScaleRange", &fpm::TemplateMatcher::getScaleRange)
         .def("getMaxPositions", &fpm::TemplateMatcher::getMaxPositions)
         .def("getMaxOverlap", &fpm::TemplateMatcher::getMaxOverlap)
         .def("getScore", &fpm::TemplateMatcher::getScore)

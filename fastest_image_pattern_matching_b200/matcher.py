@@ -8,6 +8,7 @@ is learned / the source is empty / the template does not fit / nothing is found.
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass
 from typing import List, Optional, Sequence, Tuple
 
@@ -30,6 +31,7 @@ class SingleTargetMatch:
     ptCenter: Tuple[float, float]
     dMatchedAngle: float
     dMatchScore: float
+    dScale: float = 1.0             # match scale (setScaleRange): the instance is dScale times the template's size
 
 
 def _as_u8_2d(img) -> np.ndarray:
@@ -41,12 +43,12 @@ def _as_u8_2d(img) -> np.ndarray:
     return a
 
 
-def _convert(res, n) -> List[SingleTargetMatch]:
+def _convert(res, n, scales=None) -> List[SingleTargetMatch]:
     out = []
     for i in range(n):
         r = res[i]
         out.append(SingleTargetMatch((r.ltx, r.lty), (r.rtx, r.rty), (r.rbx, r.rby), (r.lbx, r.lby),
-                                     (r.cx, r.cy), r.angle, r.score))
+                                     (r.cx, r.cy), r.angle, r.score, 1.0 if scales is None else scales[i]))
     return out
 
 
@@ -108,6 +110,19 @@ class TemplateMatcher:
         for p, v in zip((L.PARAM_TOLERANCE1, L.PARAM_TOLERANCE2, L.PARAM_TOLERANCE3, L.PARAM_TOLERANCE4), rng):
             self._set(p, v)
         self._set(L.PARAM_TOLERANCE_RANGE, 1)
+
+    def setScaleRange(self, lo: float, hi: float):
+        """Match instances lo..hi times the template's size (FPM_PARAM_SCALE_MIN / MAX, each in [0.5, 2]; default 1, 1; a
+        match refuses lo > hi).  Result rectangles have the scaled size and dScale reports each one's scale.  Both values are
+        checked before either is set, so a refused call leaves the range as it was."""
+        for name, v in (("FPM_PARAM_SCALE_MIN", lo), ("FPM_PARAM_SCALE_MAX", hi)):
+            if not (math.isfinite(float(v)) and 0.5 <= float(v) <= 2.0):
+                raise FpmError("%s must lie in [0.5, 2], got %r" % (name, v))
+        self._set(L.PARAM_SCALE_MIN, lo)
+        self._set(L.PARAM_SCALE_MAX, hi)
+
+    def getScaleRange(self) -> Tuple[float, float]:
+        return self._get(L.PARAM_SCALE_MIN), self._get(L.PARAM_SCALE_MAX)
 
     def getLastExecutionTime(self) -> float:
         """seconds, like the reference (include/TemplateMatcher.h:40)"""
@@ -271,9 +286,11 @@ class TemplateMatcher:
         s = _as_u8_2d(sourceImage)
         cap = self.result_capacity
         res = (L.fpm_result * cap)()
-        n = C.c_int(0)
-        self._check(self._lib.fpm_match(self._h, s.ctypes.data, s.shape[1], s.shape[0], s.strides[0], res, cap, C.byref(n)))
-        return _convert(res, min(n.value, cap))
+        sc = (C.c_double * cap)()
+        n = (C.c_int * 1)()
+        self._check(self._lib.fpm_match_scaled(self._h, s.ctypes.data, 0, 1, s.shape[1], s.shape[0], s.strides[0],
+                                               s.strides[0] * s.shape[0], res, sc, cap, n))
+        return _convert(res, min(n[0], cap), sc)
 
     # ---- image ingest (SURVEY 8f rank 4): decode on the device, match without a pixel copy ----
     def ingestBmp(self, file_bytes) -> tuple:
@@ -314,8 +331,12 @@ class TemplateMatcher:
         cap = self.result_capacity
         res = (L.fpm_result * cap)()
         n = C.c_int(0)
-        self._check(self._lib.fpm_match_ingested(self._h, res, cap, C.byref(n)))
-        return _convert(res, min(n.value, cap))
+        if self.ingestedCount() != 1:                     # fpm_match_ingested's refusal and message
+            self._check(self._lib.fpm_match_ingested(self._h, res, cap, C.byref(n)))
+        sc = (C.c_double * cap)()
+        cnt = (C.c_int * 1)()
+        self._check(self._lib.fpm_match_ingested_scaled(self._h, res, sc, cap, cnt))
+        return _convert(res, min(cnt[0], cap), sc)
 
     def learnIngested(self) -> bool:
         self._check(self._lib.fpm_learn_ingested(self._h))
@@ -361,8 +382,9 @@ class TemplateMatcher:
         cap = self.result_capacity
         res = (L.fpm_result * (cap * max(B, 1)))()
         n = (C.c_int * max(B, 1))()
-        self._check(self._lib.fpm_match_ingested_batch(self._h, res, cap, n))
-        return [_convert(res[b * cap:(b + 1) * cap], min(n[b], cap)) for b in range(B)]
+        sc = (C.c_double * (cap * max(B, 1)))()
+        self._check(self._lib.fpm_match_ingested_scaled(self._h, res, sc, cap, n))
+        return [_convert(res[b * cap:(b + 1) * cap], min(n[b], cap), sc[b * cap:(b + 1) * cap]) for b in range(B)]
 
     def matchBatch(self, frames: np.ndarray) -> List[List[SingleTargetMatch]]:
         """frames: [B, H, W] uint8 in host memory (pinned for full PCIe speed)."""
@@ -372,9 +394,10 @@ class TemplateMatcher:
         B, H, W = f.shape
         cap = self.result_capacity
         res = (L.fpm_result * (cap * B))()
+        sc = (C.c_double * (cap * B))()
         n = (C.c_int * B)()
-        self._check(self._lib.fpm_match_batch(self._h, f.ctypes.data, B, W, H, f.strides[1], f.strides[0], res, cap, n))
-        return [_convert(res[b * cap:(b + 1) * cap], min(n[b], cap)) for b in range(B)]
+        self._check(self._lib.fpm_match_scaled(self._h, f.ctypes.data, 0, B, W, H, f.strides[1], f.strides[0], res, sc, cap, n))
+        return [_convert(res[b * cap:(b + 1) * cap], min(n[b], cap), sc[b * cap:(b + 1) * cap]) for b in range(B)]
 
     def matchBatchRaw(self, ptr: int, B: int, W: int, H: int, stride: int, frame_stride: int, on_device: bool,
                       res=None, counts=None):

@@ -70,6 +70,20 @@ enum fpm_param {
                                            only H2D traffic), 0 = on the host (sequential; its coefficients are uploaded) */
     FPM_PARAM_JPEG_PASSES = 24,    /* read-only: synchronisation passes of the last JPEG ingest (0 = decoded on the host); a batch iterates
                                       as one, so this is the count of its slowest file */
+    FPM_PARAM_SCALE_MIN = 25,
+    FPM_PARAM_SCALE_MAX = 26,      /* match scale range [SCALE_MIN, SCALE_MAX], default [1, 1]: an instance s times the template's size is
+                                      found by resampling the source by 1/s around each level's centre (getRotationMatrix2D(c, angle, 1/s))
+                                      with the same template pyramid.  Values outside [0.5, 2] or not finite are refused (FPM_ERR_INVALID);
+                                      min > max is refused at match time (the setters run in either order).
+                                      Schedule: ds = 2 / max(w, h) of the top template level; {min} when min == max (a fixed
+                                      magnification), else n = ceil(log(max/min) / log1p(ds)) + 1 scales min * exp(k log(max/min) / (n-1)),
+                                      the last exactly max.  Top-layer pose slot k * n_angles + a (scale-major).  Descent: scales
+                                      s / (1 + ds_L), s, s * (1 + ds_L) (range) or s (fixed) x the usual angles, best = first strict
+                                      maximum; sub-pixel uses the three angle evals of the best scale.  Results are the rectangles of the
+                                      scaled size (w * s, h * s) in every result convention; [1, 1] is the unscaled matcher bit for bit.
+                                      fpm_match_scaled reports each record's scale.  Template sets of more than one template,
+                                      fpm_match_sharded*, fpm_match_set_sharded* and fpm_stage_* refuse any range other than [1, 1].
+                                      FPM_PARAM_TENSOR_CORES = 6 takes the mode-1 route at any range other than [1, 1]. */
     FPM_PARAM_COUNT_
 };
 
@@ -215,6 +229,14 @@ int fpm_ingest_jpeg_batch(fpm_handle* h, const uint8_t* data, const size_t* offs
 int fpm_ingested_count(const fpm_handle* h);
 int fpm_ingested_frame_pixels(fpm_handle* h, int index, uint8_t* out);
 int fpm_match_ingested_batch(fpm_handle* h, fpm_result* out, int cap, int* counts);
+
+/* Scale-tolerant matching (FPM_PARAM_SCALE_MIN / MAX): the records of fpm_match_batch (src_on_device = 0) /
+ * fpm_match_batch_device (1) / fpm_match_ingested_batch, plus the scale of each record in scales[] at the same index as in out
+ * (frame b's record i at b * cap + i): the exact schedule / descent value, 1.0 at the range [1, 1].  scales may be NULL.
+ * Refused like the single-template entry points on a set of more than one template. */
+int fpm_match_scaled(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                     size_t frame_stride, fpm_result* out, double* scales, int cap, int* counts);
+int fpm_match_ingested_scaled(fpm_handle* h, fpm_result* out, double* scales, int cap, int* counts);
 
 /* getLastExecutionTime (include/TemplateMatcher.h:40), milliseconds of the last match call. */
 double fpm_last_time_ms(const fpm_handle* h);

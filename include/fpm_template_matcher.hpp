@@ -10,6 +10,7 @@
 
 #include <stdexcept>
 #include <string>
+#include <utility>
 #include <vector>
 
 #ifdef FPM_WITH_OPENCV
@@ -29,6 +30,7 @@ struct SingleTargetMatch {
 #endif
     double dMatchedAngle;
     double dMatchScore;
+    double dScale = 1.0;     // match scale (setScaleRange): the instance is dScale times the template's size
 };
 
 class TemplateMatcher {
@@ -50,6 +52,18 @@ public:
     void setMinReduceArea(int v) { fpm_set_param(h_, FPM_PARAM_MIN_REDUCE_AREA, v); }
     void setUseSIMD(bool v) { fpm_set_param(h_, FPM_PARAM_USE_SIMD, v ? 1 : 0); }
     void setSubPixelEstimation(bool v) { fpm_set_param(h_, FPM_PARAM_SUBPIXEL, v ? 1 : 0); }
+    // match instances lo..hi times the template's size (each in [0.5, 2]); false when refused, and then the range is unchanged
+    bool setScaleRange(double lo, double hi)
+    {
+        const double old = fpm_get_param(h_, FPM_PARAM_SCALE_MIN);
+        if (fpm_set_param(h_, FPM_PARAM_SCALE_MIN, lo) != 0) return false;
+        if (fpm_set_param(h_, FPM_PARAM_SCALE_MAX, hi) != 0) { fpm_set_param(h_, FPM_PARAM_SCALE_MIN, old); return false; }
+        return true;
+    }
+    std::pair<double, double> getScaleRange() const
+    {
+        return {fpm_get_param(h_, FPM_PARAM_SCALE_MIN), fpm_get_param(h_, FPM_PARAM_SCALE_MAX)};
+    }
     int getMaxPositions() const { return (int)fpm_get_param(h_, FPM_PARAM_MAX_POSITIONS); }
     double getMaxOverlap() const { return fpm_get_param(h_, FPM_PARAM_MAX_OVERLAP); }
     double getScore() const { return fpm_get_param(h_, FPM_PARAM_SCORE); }
@@ -78,15 +92,17 @@ public:
         std::vector<SingleTargetMatch> out;
         if (!src || w <= 0 || h <= 0) return out;
         std::vector<fpm_result> r((size_t)cap_);
+        std::vector<double> sc((size_t)cap_);
         int n = 0;
-        if (fpm_match(h_, src, w, h, stride, r.data(), cap_, &n) != FPM_OK) throw std::runtime_error(fpm_last_error(h_));
+        if (fpm_match_scaled(h_, src, 0, 1, w, h, stride, (size_t)stride * h, r.data(), sc.data(), cap_, &n) != FPM_OK)
+            throw std::runtime_error(fpm_last_error(h_));
         if (n > cap_) n = cap_;
         out.resize((size_t)n);
         for (int i = 0; i < n; i++) {
             out[i].ptLT = {r[i].ltx, r[i].lty}; out[i].ptRT = {r[i].rtx, r[i].rty};
             out[i].ptRB = {r[i].rbx, r[i].rby}; out[i].ptLB = {r[i].lbx, r[i].lby};
             out[i].ptCenter = {r[i].cx, r[i].cy};
-            out[i].dMatchedAngle = r[i].angle; out[i].dMatchScore = r[i].score;
+            out[i].dMatchedAngle = r[i].angle; out[i].dMatchScore = r[i].score; out[i].dScale = sc[i];
         }
         return out;
     }
