@@ -43,6 +43,10 @@ SIGNATURES = {
     "fpm_match_ingested_set_batch": (_i, [_vp, _vp, _i, _vp]),
     "fpm_match_set_batch_merged": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _d, _vp, _vp, _i, _vp, _vp]),
     "fpm_match_ingested_set_batch_merged": (_i, [_vp, _d, _vp, _vp, _i, _vp, _vp]),
+    "fpm_match_set_scaled": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _vp, _vp, _i, _vp]),
+    "fpm_match_ingested_set_scaled": (_i, [_vp, _vp, _vp, _i, _vp]),
+    "fpm_match_set_scaled_merged": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _sz, _d, _vp, _vp, _vp, _i, _vp, _vp]),
+    "fpm_match_ingested_set_scaled_merged": (_i, [_vp, _d, _vp, _vp, _vp, _i, _vp, _vp]),
     "fpm_is_learned": (_i, [_vp]),
     "fpm_clear": (None, [_vp]),
     "fpm_match": (_i, [_vp, _vp, _i, _i, _i, _vp, _i, _pi]),
@@ -98,6 +102,10 @@ SIGNATURES = {
     "fpm_match_set_sharded_merged": (_i, [_vp, _vp, _i, _i, _i, _i, _d, _vp, _vp, _i, _vp, _vp]),
     "fpm_match_set_sharded_virtual": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _i, _vp]),
     "fpm_match_set_sharded_merged_virtual": (_i, [_vp, _i, _vp, _i, _i, _i, _d, _vp, _vp, _i, _vp, _vp]),
+    "fpm_match_set_sharded_scaled": (_i, [_vp, _vp, _i, _i, _i, _i, _vp, _vp, _i, _vp]),
+    "fpm_match_set_sharded_scaled_merged": (_i, [_vp, _vp, _i, _i, _i, _i, _d, _vp, _vp, _vp, _i, _vp, _vp]),
+    "fpm_match_set_sharded_scaled_virtual": (_i, [_vp, _i, _vp, _i, _i, _i, _vp, _vp, _i, _vp]),
+    "fpm_match_set_sharded_scaled_merged_virtual": (_i, [_vp, _i, _vp, _i, _i, _i, _d, _vp, _vp, _vp, _i, _vp, _vp]),
     "fpm_shard_angle_range": (_i, [_i, _i, _i, _pi, _pi]),
     "fpm_collective_count": (C.c_longlong, [_vp]),
     "fpm_dbg_pyrdown": (_i, [_vp, _vp, _i, _i, _i, _vp]),

@@ -19,6 +19,7 @@
 #include <cstring>
 #include <dlfcn.h>
 #include <map>
+#include <memory>
 #include <mutex>
 #include <new>
 #include <string>
@@ -161,15 +162,16 @@ struct TopPlan {                  // cached per (source size, parameters); alway
 // Templates of a set with the same level-0 size, border colour and masked-ness: they share the top layer, the angle schedule, the
 // canvases, the ROI sizes and the NMS rectangle, and run through the pipeline together as virtual images
 // v = frame * n + member.  The group being matched lives in the handle's fields (tpl, border, tpl0_w/h, members, plan,
-// d_jobs_top, d_angles, d_ftx, d_fty); group 0 is there at rest, the others are swapped in for their pass.
+// d_jobs_top, d_angles, d_ftx, d_fty, d_scales); group 0 is there at rest, the others are swapped in for their pass.  Groups of
+// different top-level sizes have different scale schedules, so the slot scales belong to the group like its plan.
 struct TplGroup {
     std::vector<int> members;      // set indices, ascending
     std::vector<TplLevelHost> tpl; // levels (statistics and pixels of members[0])
     int border = 0, w0 = 0, h0 = 0;
     bool masked = false;           // its members carry masks (a group is all masked or all unmasked)
     TopPlan plan;
-    DevBuf d_jobs_top, d_angles, d_ftx, d_fty;
-    void release() { d_jobs_top.release(); d_angles.release(); d_ftx.release(); d_fty.release(); }
+    DevBuf d_jobs_top, d_angles, d_ftx, d_fty, d_scales;
+    void release() { d_jobs_top.release(); d_angles.release(); d_ftx.release(); d_fty.release(); d_scales.release(); }
 };
 
 struct SetTpl { std::vector<uint8_t> px, mask; int w = 0, h = 0; };   // mask: 0/1 bytes (w*h), empty = unmasked
@@ -239,10 +241,12 @@ struct fpm_handle {
     int shard_upload = 1;          // FPM_PARAM_SHARD_UPLOAD: host frame uploaded as 1/N row slices + NVLink allgather
     DevBuf d_gpicks, d_grefined;   // allgather buffers: one fixed-size block per rank, consumed in place by the kernels
     FpmRefined* ref_out = nullptr; // where run_refine appends (null: d_refined / counters[CNT_REFINED])
-    // fpm_match_scaled: run_final writes the scale of the record written at out_base[i] to scales_out[i] (out_base: the caller's
-    // whole output array, so chunks, split halves and their twin handle all index it the same way)
+    // fpm_match_scaled and the scaled set calls: run_final / run_set_merge write the scale of the record written at out_base[i]
+    // to scales_out[i] (out_base: the caller's whole output array, so chunks, split halves, their twin handle and the ranks of
+    // the virtual angle-sharded calls all index it the same way)
     double* scales_out = nullptr;
     const fpm_result* scales_base = nullptr;
+    const char* scaled_fn = nullptr;   // the call in flight returns scales: a set matches at any range, refusals name this call
     int* ref_cnt = nullptr;
     // one call's layout of the rank blocks, the same on every rank: block = picks of every group that runs
     // [group][template][chunk angle][MaxPos+5], then their counts [group][template][chunk angle]; refined block = one
@@ -895,7 +899,7 @@ struct GroupScope {
         std::swap(h->tpl, G.tpl); std::swap(h->members, G.members); std::swap(h->border, G.border);
         std::swap(h->tpl0_w, G.w0); std::swap(h->tpl0_h, G.h0); std::swap(h->plan, G.plan);
         std::swap(h->d_jobs_top, G.d_jobs_top); std::swap(h->d_angles, G.d_angles);
-        std::swap(h->d_ftx, G.d_ftx); std::swap(h->d_fty, G.d_fty);
+        std::swap(h->d_ftx, G.d_ftx); std::swap(h->d_fty, G.d_fty); std::swap(h->d_scales, G.d_scales);
     }
     GroupScope(fpm_handle* hh, size_t gg) : h(hh), g(gg) { if (g) swap(h, h->groups[g]); }
     ~GroupScope() { if (g) swap(h, h->groups[g]); }
@@ -1546,6 +1550,7 @@ int run_set_merge(fpm_handle* h, int batch, int n_set, int n_groups, const Merge
         for (int i = 0; i < m; i++) {
             const FpmResultDev& r = h_rec[(size_t)b * ocap + i];
             fpm_result& o = out[(size_t)b * cap + i];
+            if (h->scales_out) h->scales_out[&o - h->scales_base] = r.scale;
             o.score = r.score; o.angle = r.angle; o.cx = r.cx; o.cy = r.cy;
             o.ltx = r.ltx; o.lty = r.lty; o.rtx = r.rtx; o.rty = r.rty;
             o.rbx = r.rbx; o.rby = r.rby; o.lbx = r.lbx; o.lby = r.lby;
@@ -1574,7 +1579,8 @@ int runnable_groups(const fpm_handle* h, int w, int hgt, std::vector<char>& run)
 // device lists of the merge for the groups that run (run[g]) over `batch` frames, header zeroed on the stream
 int merge_setup(fpm_handle* h, int batch, int cap, int n_set, const std::vector<char>& run, MergeDev* md)
 {
-    // list capacity: a group's list of a frame never exceeds its candidate list, n_angles * (MaxPos + 5) entries
+    // list capacity: a group's list of a frame never exceeds its candidate list, (MaxPos + 5) entries per pose slot (angle x
+    // scale of the schedule)
     const size_t n_groups = h->groups.size();
     int longest = 0;
     for (size_t g = 0; g < n_groups; g++) {
@@ -1584,7 +1590,10 @@ int merge_setup(fpm_handle* h, int batch, int cap, int n_set, const std::vector<
         longest = std::max(longest, h->plan.n_ang * (h->max_pos + FPM_MATCH_CANDIDATE_NUM));
     }
     md->lcap = std::min(cap, longest);
-    if ((long long)n_set * md->lcap >= (1ll << 30)) { h->err = "merged set results: n_set * list capacity too large"; return FPM_ERR_LIMIT; }
+    if ((long long)n_set * md->lcap >= (1ll << 30)) {
+        h->err = "merged set results: n_set * list capacity (min(cap, pose slots x (MaxPos + 5))) too large";
+        return FPM_ERR_LIMIT;
+    }
     md->ocap = std::min(cap, n_set * md->lcap);
     const MergedLayout lay(batch, n_set, md->ocap, (int)n_groups);
     CK(h->d_mlists.ensure((size_t)batch * n_set * std::max(md->lcap, 1) * sizeof(FpmResultDev)));
@@ -1597,8 +1606,10 @@ int merge_setup(fpm_handle* h, int batch, int cap, int n_set, const std::vector<
 }
 
 // The match scale range (FPM_PARAM_SCALE_MIN / MAX), checked at match time because the two setters may run in either order:
-// min <= max, and [1, 1] on the calls that do not carry a scale (scaled_ok = false: template sets of more than one template, the
-// angle-sharded calls, fpm_stage_*).
+// min <= max, and [1, 1] on the calls that do not carry a scale (scaled_ok = false: fpm_match_set_batch* and
+// fpm_match_ingested_set_batch* on sets of more than one template, fpm_match_sharded*, fpm_match_set_sharded* without _scaled,
+// fpm_stage_*).  The calls that return each record's scale accept any range: fpm_match_scaled, fpm_match_ingested_scaled,
+// fpm_match_set_scaled*, fpm_match_ingested_set_scaled* and fpm_match_set_sharded_scaled*.
 int refuse_scale(const fpm_handle* h, const char* fn, bool scaled_ok)
 {
     if (h->scale_min == 1.0 && h->scale_max == 1.0) return FPM_OK;
@@ -1624,7 +1635,7 @@ int match_device(fpm_handle* h, const uint8_t* d_src, int batch, int w, int hgt,
     if (mg && mg->set_counts) std::fill(mg->set_counts, mg->set_counts + (size_t)batch * n_set, 0);
     if (!h->learned) return FPM_OK;                          // :99-101 -> empty
     const bool is_set = fpm_set_size(h) > 1;
-    int rc = refuse_scale(h, is_set ? "fpm_match_set_batch" : "fpm_match", !is_set);
+    int rc = refuse_scale(h, h->scaled_fn ? h->scaled_fn : is_set ? "fpm_match_set_batch" : "fpm_match", !is_set || h->scaled_fn);
     if (rc) return rc;
     rc = ensure_learned_for_mra(h);
     if (rc) return rc;
@@ -2016,7 +2027,7 @@ void fpm_destroy(fpm_handle* h)
     cudaStreamSynchronize(h->copy_stream);
     cudaStreamSynchronize(h->aux_stream);
     DevBuf* bufs[] = {&h->d_gpicks, &h->d_grefined, &h->d_tpl, &h->d_tsh, &h->d_raw, &h->d_inv, &h->d_numer, &h->d_totS, &h->d_totQ, &h->d_ingest_raw, &h->d_ingest, &h->d_src, &h->d_pyr, &h->d_rot, &h->d_score, &h->d_blkv, &h->d_blkl, &h->d_picks, &h->d_pickcnt,
-                      &h->d_jobs_top, &h->d_angles, &h->d_ftx, &h->d_fty, &h->d_off, &h->d_keys, &h->d_cand[0], &h->d_cand[1],
+                      &h->d_jobs_top, &h->d_angles, &h->d_ftx, &h->d_fty, &h->d_scales, &h->d_off, &h->d_keys, &h->d_cand[0], &h->d_cand[1],
                       &h->d_candcnt, &h->d_toppt, &h->d_counters, &h->d_jobs_ref, &h->d_roi, &h->d_rowsum, &h->d_rowS, &h->d_rowQ,
                       &h->d_pairs, &h->d_refined, &h->d_rects, &h->d_del, &h->d_idmap, &h->d_results, &h->d_rescnt, &h->d_trace, &h->d_trace_sc,
                       &h->d_dbg[0], &h->d_dbg[1], &h->d_dbg[2], &h->d_dbg[3], &h->d_members, &h->d_mlists, &h->d_merged};
@@ -2277,7 +2288,7 @@ int match_batch_device(fpm_handle* h, const uint8_t* d_src, int batch, int width
         // the other half's kernels fill the device.
         rc = ensure_twin(h);
         if (rc) return rc;
-        h->twin->scales_out = h->scales_out; h->twin->scales_base = h->scales_base;
+        h->twin->scales_out = h->scales_out; h->twin->scales_base = h->scales_base; h->twin->scaled_fn = h->scaled_fn;
         const int b0 = batch / 2;
         int rc2 = FPM_OK;
         const SetMerge mg2 = mg ? mg->shifted(b0, cap, n_set) : SetMerge{};
@@ -2391,13 +2402,36 @@ int fpm_match_batch(fpm_handle* h, const uint8_t* src, int batch, int width, int
     return match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, n);
 }
 
+namespace {
+int check_merge_args(fpm_handle* h, const char* fn, double max_overlap, int cap, const int* labels)
+{
+    if (!std::isfinite(max_overlap)) { h->err = std::string(fn) + ": max_overlap must be finite"; return FPM_ERR_INVALID; }
+    if (cap > 0 && !labels) { h->err = std::string(fn) + ": labels is NULL while cap > 0"; return FPM_ERR_INVALID; }
+    return FPM_OK;
+}
+
+// fpm_match_set_batch / fpm_match_set_batch_merged (mg) and their scaled twins; fn names the call in the refusals
+int match_set(fpm_handle* h, const char* fn, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+              size_t frame_stride, fpm_result* out, int cap, int* counts, const SetMerge* mg)
+{
+    if (h->trace && fpm_set_size(h) > 1) {
+        h->err = std::string(fn) + ": FPM_PARAM_TRACE is not supported for a set of more than one template";
+        return FPM_ERR_INVALID;
+    }
+    if (mg) {
+        if (int rc = check_merge_args(h, fn, mg->max_overlap, cap, mg->labels)) return rc;
+        if (mg->set_counts && batch > 0) std::fill(mg->set_counts, mg->set_counts + (size_t)batch * std::max(fpm_set_size(h), 1), 0);
+    }
+    return src_on_device ? match_batch_device(h, src, batch, width, height, stride, frame_stride, out, cap, counts, mg)
+                         : match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, counts, mg);
+}
+}  // namespace
+
 int fpm_match_set_batch(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
                         size_t frame_stride, fpm_result* out, int cap, int* counts)
 {
     if (!h) return FPM_ERR_INVALID;
-    if (h->trace && fpm_set_size(h) > 1) { h->err = "fpm_match_set_batch: FPM_PARAM_TRACE is not supported for a set of more than one template"; return FPM_ERR_INVALID; }
-    return src_on_device ? match_batch_device(h, src, batch, width, height, stride, frame_stride, out, cap, counts)
-                         : match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, counts);
+    return match_set(h, "fpm_match_set_batch", src, src_on_device, batch, width, height, stride, frame_stride, out, cap, counts, nullptr);
 }
 
 int fpm_match_set_batch_merged(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
@@ -2405,13 +2439,9 @@ int fpm_match_set_batch_merged(fpm_handle* h, const uint8_t* src, int src_on_dev
                                int* set_counts)
 {
     if (!h) return FPM_ERR_INVALID;
-    if (h->trace && fpm_set_size(h) > 1) { h->err = "fpm_match_set_batch_merged: FPM_PARAM_TRACE is not supported for a set of more than one template"; return FPM_ERR_INVALID; }
-    if (!std::isfinite(max_overlap)) { h->err = "fpm_match_set_batch_merged: max_overlap must be finite"; return FPM_ERR_INVALID; }
-    if (cap > 0 && !labels) { h->err = "fpm_match_set_batch_merged: labels is NULL while cap > 0"; return FPM_ERR_INVALID; }
-    if (set_counts && batch > 0) std::fill(set_counts, set_counts + (size_t)batch * std::max(fpm_set_size(h), 1), 0);
     const SetMerge mg{max_overlap, labels, set_counts};
-    return src_on_device ? match_batch_device(h, src, batch, width, height, stride, frame_stride, out, cap, counts, &mg)
-                         : match_batch_host(h, src, batch, width, height, stride, frame_stride, out, cap, counts, &mg);
+    return match_set(h, "fpm_match_set_batch_merged", src, src_on_device, batch, width, height, stride, frame_stride, out, cap,
+                     counts, &mg);
 }
 
 int fpm_match(fpm_handle* h, const uint8_t* src, int width, int height, int stride, fpm_result* out, int cap, int* n)
@@ -3246,16 +3276,28 @@ int fpm_ingested_pixels(fpm_handle* h, uint8_t* out)
 }
 
 namespace {
-// fpm_match_scaled / fpm_match_ingested_scaled: the scale of every record written during the call goes to scales
+// the calls that return scales: the scale of every record written during the call goes to scales; fn (the scaled set calls)
+// lets a set of more than one template match at any range
 struct ScalesOut {
     fpm_handle* h;
-    ScalesOut(fpm_handle* hh, fpm_result* out, double* scales) : h(hh) { h->scales_out = scales; h->scales_base = out; }
+    ScalesOut(fpm_handle* hh, fpm_result* out, double* scales, const char* fn = nullptr) : h(hh)
+    {
+        h->scales_out = scales; h->scales_base = out; h->scaled_fn = fn;
+    }
     ~ScalesOut()
     {
-        h->scales_out = nullptr; h->scales_base = nullptr;
-        if (h->twin) { h->twin->scales_out = nullptr; h->twin->scales_base = nullptr; }
+        h->scales_out = nullptr; h->scales_base = nullptr; h->scaled_fn = nullptr;
+        if (h->twin) { h->twin->scales_out = nullptr; h->twin->scales_base = nullptr; h->twin->scaled_fn = nullptr; }
     }
 };
+
+// the frames of the last ingest x the set, through match_set
+int match_ingested_set(fpm_handle* h, const char* fn, fpm_result* out, int cap, int* counts, const SetMerge* mg)
+{
+    if (h->ingest_count <= 0) { h->err = "no ingested frame"; return FPM_ERR_INVALID; }
+    return match_set(h, fn, h->d_ingest.as<uint8_t>(), 1, h->ingest_count, h->ingest_w, h->ingest_h, h->ingest_pitch,
+                     (size_t)h->ingest_pitch * h->ingest_h, out, cap, counts, mg);
+}
 }  // namespace
 
 int fpm_match_scaled(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
@@ -3274,6 +3316,44 @@ int fpm_match_ingested_scaled(fpm_handle* h, fpm_result* out, double* scales, in
     if (int rc = refuse_set(h, "fpm_match_ingested_scaled")) return rc;
     ScalesOut so(h, out, scales);
     return fpm_match_ingested_set_batch(h, out, cap, counts);
+}
+
+int fpm_match_set_scaled(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                         size_t frame_stride, fpm_result* out, double* scales, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    const char* fn = "fpm_match_set_scaled";
+    ScalesOut so(h, out, scales, fn);
+    return match_set(h, fn, src, src_on_device, batch, width, height, stride, frame_stride, out, cap, counts, nullptr);
+}
+
+int fpm_match_ingested_set_scaled(fpm_handle* h, fpm_result* out, double* scales, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    const char* fn = "fpm_match_ingested_set_scaled";
+    ScalesOut so(h, out, scales, fn);
+    return match_ingested_set(h, fn, out, cap, counts, nullptr);
+}
+
+int fpm_match_set_scaled_merged(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                                size_t frame_stride, double max_overlap, fpm_result* out, double* scales, int* labels, int cap,
+                                int* counts, int* set_counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    const char* fn = "fpm_match_set_scaled_merged";
+    const SetMerge mg{max_overlap, labels, set_counts};
+    ScalesOut so(h, out, scales, fn);
+    return match_set(h, fn, src, src_on_device, batch, width, height, stride, frame_stride, out, cap, counts, &mg);
+}
+
+int fpm_match_ingested_set_scaled_merged(fpm_handle* h, double max_overlap, fpm_result* out, double* scales, int* labels, int cap,
+                                         int* counts, int* set_counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    const char* fn = "fpm_match_ingested_set_scaled_merged";
+    const SetMerge mg{max_overlap, labels, set_counts};
+    ScalesOut so(h, out, scales, fn);
+    return match_ingested_set(h, fn, out, cap, counts, &mg);
 }
 
 int fpm_match_ingested(fpm_handle* h, fpm_result* out, int cap, int* n)
@@ -3631,10 +3711,11 @@ int fpm_shard_angle_range(int n_angles, int nranks, int rank, int* a0, int* a1)
 long long fpm_collective_count(const fpm_handle* h) { return h ? h->collectives : 0; }
 
 namespace {
-// refusals shared by the whole-set sharded calls (fpm_match_set_batch's, plus a missing communicator)
-int check_set_sharded(fpm_handle* h, const char* fn, int cap, const void* out, const int* n)
+// refusals shared by the whole-set sharded calls (fpm_match_set_batch's, plus a missing communicator); scaled: the _scaled
+// calls, which accept any scale range
+int check_set_sharded(fpm_handle* h, const char* fn, int cap, const void* out, const int* n, bool scaled = false)
 {
-    if (int rc = refuse_scale(h, fn, false)) return rc;
+    if (int rc = refuse_scale(h, fn, scaled)) return rc;
     if (h->trace && fpm_set_size(h) > 1) {
         h->err = std::string(fn) + ": FPM_PARAM_TRACE is not supported for a set of more than one template";
         return FPM_ERR_INVALID;
@@ -3647,15 +3728,8 @@ int check_set_sharded(fpm_handle* h, const char* fn, int cap, const void* out, c
     return FPM_OK;
 }
 
-int check_merge_args(fpm_handle* h, const char* fn, double max_overlap, int cap, const int* labels)
-{
-    if (!std::isfinite(max_overlap)) { h->err = std::string(fn) + ": max_overlap must be finite"; return FPM_ERR_INVALID; }
-    if (cap > 0 && !labels) { h->err = std::string(fn) + ": labels is NULL while cap > 0"; return FPM_ERR_INVALID; }
-    return FPM_OK;
-}
-
 // refusals of the virtual-rank drivers: every handle present, none with a communicator, one set size on all of them
-int check_virtual(fpm_handle* const* hs, int nranks, const char* fn, bool whole_set)
+int check_virtual(fpm_handle* const* hs, int nranks, const char* fn, bool whole_set, bool scaled = false)
 {
     if (!hs || nranks < 1) return FPM_ERR_INVALID;
     for (int r = 0; r < nranks; r++)
@@ -3665,7 +3739,7 @@ int check_virtual(fpm_handle* const* hs, int nranks, const char* fn, bool whole_
         return FPM_ERR_INVALID;
     };
     for (int r = 0; r < nranks; r++)
-        if (int rc = refuse_scale(hs[r], fn, false)) return rc;
+        if (int rc = refuse_scale(hs[r], fn, scaled)) return rc;
     for (int r = 0; r < nranks; r++) {
         if (hs[r]->nccl_comm) return whole_set ? refuse("the handle of rank " + std::to_string(r) + " has a communicator") : FPM_ERR_INVALID;
         if (!whole_set) {
@@ -3700,54 +3774,105 @@ int fpm_match_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* 
     return match_set_sharded_virtual(hs, nranks, src, width, height, stride, out, cap, n, 1, nullptr, false);
 }
 
+namespace {
+// fpm_match_set_sharded* (mg: merged; scaled: the _scaled calls, which accept any range and write each record's scale)
+int set_sharded(fpm_handle* h, const char* fn, bool scaled, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                fpm_result* out, double* scales, int cap, int* counts, const SetMerge* mg)
+{
+    if (int rc = check_set_sharded(h, fn, cap, out, counts, scaled)) return rc;
+    if (mg) if (int rc = check_merge_args(h, fn, mg->max_overlap, cap, mg->labels)) return rc;
+    const int n_set = std::max(fpm_set_size(h), 1);
+    std::fill(counts, counts + (mg ? 1 : n_set), 0);
+    if (mg && mg->set_counts) std::fill(mg->set_counts, mg->set_counts + n_set, 0);
+    ScalesOut so(h, out, scales, scaled ? fn : nullptr);
+    return match_set_sharded(h, src, width, height, stride, src_on_device, out, cap, counts, mg);
+}
+
+// fpm_match_set_sharded*_virtual: mg holds the caller's whole labels / set_counts arrays, split here into the ranks' merges
+int set_sharded_virtual(fpm_handle* const* hs, int nranks, const char* fn, bool scaled, const uint8_t* src, int width, int height,
+                        int stride, fpm_result* out, double* scales, int cap, int* counts, const SetMerge* mg)
+{
+    if (int rc = check_virtual(hs, nranks, fn, true, scaled)) return rc;
+    for (int r = 0; r < nranks; r++) {
+        if (int rc = check_set_sharded(hs[r], fn, cap, out, counts, scaled)) return rc;
+        if (mg) if (int rc = check_merge_args(hs[r], fn, mg->max_overlap, cap, mg->labels)) return rc;
+    }
+    const int n_set = std::max(fpm_set_size(hs[0]), 1), n_rows = mg ? 1 : n_set;
+    std::fill(counts, counts + (size_t)nranks * n_rows, 0);
+    if (mg && mg->set_counts) std::fill(mg->set_counts, mg->set_counts + (size_t)nranks * n_set, 0);
+    std::vector<SetMerge> mgs;
+    for (int r = 0; mg && r < nranks; r++)
+        mgs.push_back(SetMerge{mg->max_overlap, mg->labels ? mg->labels + (size_t)r * cap : nullptr,
+                               mg->set_counts ? mg->set_counts + (size_t)r * n_set : nullptr});
+    std::vector<std::unique_ptr<ScalesOut>> so;            // every rank indexes the whole out / scales arrays
+    for (int r = 0; r < nranks; r++) so.emplace_back(new ScalesOut(hs[r], out, scales, scaled ? fn : nullptr));
+    return match_set_sharded_virtual(hs, nranks, src, width, height, stride, out, cap, counts, n_rows, mg ? mgs.data() : nullptr, true);
+}
+}  // namespace
+
 int fpm_match_set_sharded(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
                           fpm_result* out, int cap, int* counts)
 {
     if (!h) return FPM_ERR_INVALID;
-    if (int rc = check_set_sharded(h, "fpm_match_set_sharded", cap, out, counts)) return rc;
-    std::fill(counts, counts + std::max(fpm_set_size(h), 1), 0);
-    return match_set_sharded(h, src, width, height, stride, src_on_device, out, cap, counts, nullptr);
+    return set_sharded(h, "fpm_match_set_sharded", false, src, width, height, stride, src_on_device, out, nullptr, cap, counts, nullptr);
 }
 
 int fpm_match_set_sharded_merged(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
                                  double max_overlap, fpm_result* out, int* labels, int cap, int* count, int* set_counts)
 {
     if (!h) return FPM_ERR_INVALID;
-    if (int rc = check_set_sharded(h, "fpm_match_set_sharded_merged", cap, out, count)) return rc;
-    if (int rc = check_merge_args(h, "fpm_match_set_sharded_merged", max_overlap, cap, labels)) return rc;
-    *count = 0;
-    if (set_counts) std::fill(set_counts, set_counts + std::max(fpm_set_size(h), 1), 0);
     const SetMerge mg{max_overlap, labels, set_counts};
-    return match_set_sharded(h, src, width, height, stride, src_on_device, out, cap, count, &mg);
+    return set_sharded(h, "fpm_match_set_sharded_merged", false, src, width, height, stride, src_on_device, out, nullptr, cap, count, &mg);
 }
 
 int fpm_match_set_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
                                   fpm_result* out, int cap, int* counts)
 {
-    if (int rc = check_virtual(hs, nranks, "fpm_match_set_sharded_virtual", true)) return rc;
-    for (int r = 0; r < nranks; r++)
-        if (int rc = check_set_sharded(hs[r], "fpm_match_set_sharded_virtual", cap, out, counts)) return rc;
-    const int n_set = std::max(fpm_set_size(hs[0]), 1);
-    std::fill(counts, counts + (size_t)nranks * n_set, 0);
-    return match_set_sharded_virtual(hs, nranks, src, width, height, stride, out, cap, counts, n_set, nullptr, true);
+    return set_sharded_virtual(hs, nranks, "fpm_match_set_sharded_virtual", false, src, width, height, stride, out, nullptr, cap,
+                               counts, nullptr);
 }
 
 int fpm_match_set_sharded_merged_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height,
                                          int stride, double max_overlap, fpm_result* out, int* labels, int cap, int* count,
                                          int* set_counts)
 {
-    if (int rc = check_virtual(hs, nranks, "fpm_match_set_sharded_merged_virtual", true)) return rc;
-    for (int r = 0; r < nranks; r++) {
-        if (int rc = check_set_sharded(hs[r], "fpm_match_set_sharded_merged_virtual", cap, out, count)) return rc;
-        if (int rc = check_merge_args(hs[r], "fpm_match_set_sharded_merged_virtual", max_overlap, cap, labels)) return rc;
-    }
-    const int n_set = std::max(fpm_set_size(hs[0]), 1);
-    std::fill(count, count + nranks, 0);
-    if (set_counts) std::fill(set_counts, set_counts + (size_t)nranks * n_set, 0);
-    std::vector<SetMerge> mg(nranks);
-    for (int r = 0; r < nranks; r++)
-        mg[r] = SetMerge{max_overlap, labels ? labels + (size_t)r * cap : nullptr, set_counts ? set_counts + (size_t)r * n_set : nullptr};
-    return match_set_sharded_virtual(hs, nranks, src, width, height, stride, out, cap, count, 1, mg.data(), true);
+    const SetMerge mg{max_overlap, labels, set_counts};
+    return set_sharded_virtual(hs, nranks, "fpm_match_set_sharded_merged_virtual", false, src, width, height, stride, out, nullptr,
+                               cap, count, &mg);
+}
+
+int fpm_match_set_sharded_scaled(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                                 fpm_result* out, double* scales, int cap, int* counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    return set_sharded(h, "fpm_match_set_sharded_scaled", true, src, width, height, stride, src_on_device, out, scales, cap, counts,
+                       nullptr);
+}
+
+int fpm_match_set_sharded_scaled_merged(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                                        double max_overlap, fpm_result* out, double* scales, int* labels, int cap, int* count,
+                                        int* set_counts)
+{
+    if (!h) return FPM_ERR_INVALID;
+    const SetMerge mg{max_overlap, labels, set_counts};
+    return set_sharded(h, "fpm_match_set_sharded_scaled_merged", true, src, width, height, stride, src_on_device, out, scales, cap,
+                       count, &mg);
+}
+
+int fpm_match_set_sharded_scaled_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
+                                         fpm_result* out, double* scales, int cap, int* counts)
+{
+    return set_sharded_virtual(hs, nranks, "fpm_match_set_sharded_scaled_virtual", true, src, width, height, stride, out, scales,
+                               cap, counts, nullptr);
+}
+
+int fpm_match_set_sharded_scaled_merged_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height,
+                                                int stride, double max_overlap, fpm_result* out, double* scales, int* labels, int cap,
+                                                int* count, int* set_counts)
+{
+    const SetMerge mg{max_overlap, labels, set_counts};
+    return set_sharded_virtual(hs, nranks, "fpm_match_set_sharded_scaled_merged_virtual", true, src, width, height, stride, out,
+                               scales, cap, count, &mg);
 }
 
 // ---- stage kernels for parity tests ----------------------------------------------------

@@ -191,58 +191,76 @@ class TemplateMatcher:
 
     def patternSetSize(self) -> int: return int(self._lib.fpm_set_size(self._h))
 
-    def _set_results(self, res, counts, B, T):
+    # scaled=True on the set methods: the scaled set calls (fpm_match_set_scaled*, fpm_match_ingested_set_scaled*,
+    # fpm_match_set_sharded_scaled*), which match at the handle's scale range (setScaleRange) and fill dScale; the default
+    # calls match at [1, 1] only and refuse any other range
+    def _set_results(self, res, counts, B, T, scales=None):
         cap = self.result_capacity
-        return [[_convert(res[(b * T + t) * cap:(b * T + t + 1) * cap], min(counts[b * T + t], cap)) for t in range(T)]
+        return [[_convert(res[(b * T + t) * cap:(b * T + t + 1) * cap], min(counts[b * T + t], cap),
+                          None if scales is None else scales[(b * T + t) * cap:(b * T + t + 1) * cap]) for t in range(T)]
                 for b in range(B)]
 
     def matchSetBatchRaw(self, ptr: int, B: int, W: int, H: int, stride: int, frame_stride: int, on_device: bool,
-                         res=None, counts=None):
-        """Pointer-level set match: returns (results ctypes array [B][T][cap], counts [B][T])."""
+                         res=None, counts=None, scaled: bool = False, scales=None):
+        """Pointer-level set match: returns (results ctypes array [B][T][cap], counts [B][T]), and with scaled=True
+        (fpm_match_set_scaled) also the scales [B][T][cap] at the indices of the results."""
         cap, T = self.result_capacity, max(self.patternSetSize(), 1)
         if res is None:
             res = (L.fpm_result * (cap * B * T))()
         if counts is None:
             counts = (C.c_int * (B * T))()
-        self._check(self._lib.fpm_match_set_batch(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride, res, cap,
-                                                  counts))
-        return res, counts
+        if not scaled:
+            self._check(self._lib.fpm_match_set_batch(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride, res, cap,
+                                                      counts))
+            return res, counts
+        if scales is None:
+            scales = (C.c_double * (cap * B * T))()
+        self._check(self._lib.fpm_match_set_scaled(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride, res, scales,
+                                                   cap, counts))
+        return res, counts, scales
 
-    def matchSetBatch(self, frames: np.ndarray) -> List[List[List[SingleTargetMatch]]]:
+    def matchSetBatch(self, frames: np.ndarray, scaled: bool = False) -> List[List[List[SingleTargetMatch]]]:
         """frames: [B, H, W] uint8 in host memory -> [frame][template][results]."""
         f = np.asarray(frames)
         if f.ndim != 3 or f.dtype != np.uint8 or f.strides[2] != 1:
             raise FpmError("frames must be a [B,H,W] uint8 array with unit pixel stride")
         B, H, W = f.shape
         T = max(self.patternSetSize(), 1)
-        res, counts = self.matchSetBatchRaw(f.ctypes.data, B, W, H, f.strides[1], f.strides[0], False)
-        return self._set_results(res, counts, B, T)
+        out = self.matchSetBatchRaw(f.ctypes.data, B, W, H, f.strides[1], f.strides[0], False, scaled=scaled)
+        return self._set_results(out[0], out[1], B, T, out[2] if scaled else None)
 
-    def matchSet(self, sourceImage) -> List[List[SingleTargetMatch]]:
+    def matchSet(self, sourceImage, scaled: bool = False) -> List[List[SingleTargetMatch]]:
         """one host image -> [template][results]"""
-        return self.matchSetBatch(_as_u8_2d(sourceImage)[None])[0]
+        return self.matchSetBatch(_as_u8_2d(sourceImage)[None], scaled=scaled)[0]
 
-    def matchIngestedSetBatch(self) -> List[List[List[SingleTargetMatch]]]:
+    def matchIngestedSetBatch(self, scaled: bool = False) -> List[List[List[SingleTargetMatch]]]:
         """the frames of the last ingest x the set: [frame][template][results]"""
         B, T, cap = self.ingestedCount(), max(self.patternSetSize(), 1), self.result_capacity
         res = (L.fpm_result * (cap * max(B, 1) * T))()
         counts = (C.c_int * (max(B, 1) * T))()
-        self._check(self._lib.fpm_match_ingested_set_batch(self._h, res, cap, counts))
-        return self._set_results(res, counts, B, T)
+        if not scaled:
+            self._check(self._lib.fpm_match_ingested_set_batch(self._h, res, cap, counts))
+            return self._set_results(res, counts, B, T)
+        sc = (C.c_double * (cap * max(B, 1) * T))()
+        self._check(self._lib.fpm_match_ingested_set_scaled(self._h, res, sc, cap, counts))
+        return self._set_results(res, counts, B, T, sc)
 
     # ---- merged set results: one labelled list per frame, rotated-rectangle NMS across templates ----
-    def _merged_results(self, res, labels, counts, B):
+    def _merged_results(self, res, labels, counts, B, scales=None):
         cap = self.result_capacity
         out = []
         for b in range(B):
             m = min(counts[b], cap)
-            out.append(list(zip(labels[b * cap:b * cap + m], _convert(res[b * cap:(b + 1) * cap], m))))
+            out.append(list(zip(labels[b * cap:b * cap + m],
+                                _convert(res[b * cap:(b + 1) * cap], m, None if scales is None else scales[b * cap:(b + 1) * cap]))))
         return out
 
     def matchSetBatchMergedRaw(self, ptr: int, B: int, W: int, H: int, stride: int, frame_stride: int, on_device: bool,
-                               max_overlap: float, res=None, labels=None, counts=None, set_counts=None):
+                               max_overlap: float, res=None, labels=None, counts=None, set_counts=None, scaled: bool = False,
+                               scales=None):
         """Pointer-level merged set match (fpm_match_set_batch_merged): returns (results ctypes array [B][cap], labels [B][cap],
-        counts [B], set_counts [B][T]: the per-template totals)."""
+        counts [B], set_counts [B][T]: the per-template totals), and with scaled=True (fpm_match_set_scaled_merged) also the
+        scales [B][cap]."""
         cap, T = self.result_capacity, max(self.patternSetSize(), 1)
         if res is None:
             res = (L.fpm_result * (cap * B))()
@@ -252,32 +270,43 @@ class TemplateMatcher:
             counts = (C.c_int * B)()
         if set_counts is None:
             set_counts = (C.c_int * (B * T))()
-        self._check(self._lib.fpm_match_set_batch_merged(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride,
-                                                         float(max_overlap), res, labels, cap, counts, set_counts))
-        return res, labels, counts, set_counts
+        if not scaled:
+            self._check(self._lib.fpm_match_set_batch_merged(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride,
+                                                             float(max_overlap), res, labels, cap, counts, set_counts))
+            return res, labels, counts, set_counts
+        if scales is None:
+            scales = (C.c_double * (cap * B))()
+        self._check(self._lib.fpm_match_set_scaled_merged(self._h, ptr, 1 if on_device else 0, B, W, H, stride, frame_stride,
+                                                          float(max_overlap), res, scales, labels, cap, counts, set_counts))
+        return res, labels, counts, set_counts, scales
 
-    def matchSetBatchMerged(self, frames: np.ndarray, max_overlap: float) -> List[List[Tuple[int, SingleTargetMatch]]]:
+    def matchSetBatchMerged(self, frames: np.ndarray, max_overlap: float,
+                            scaled: bool = False) -> List[List[Tuple[int, SingleTargetMatch]]]:
         """frames: [B, H, W] uint8 in host memory -> per frame one list of (set index, result), score descending, after NMS
         across templates with the overlap threshold max_overlap (the per-template lists keep MaxOverlap)."""
         f = np.asarray(frames)
         if f.ndim != 3 or f.dtype != np.uint8 or f.strides[2] != 1:
             raise FpmError("frames must be a [B,H,W] uint8 array with unit pixel stride")
         B, H, W = f.shape
-        res, labels, counts, _ = self.matchSetBatchMergedRaw(f.ctypes.data, B, W, H, f.strides[1], f.strides[0], False, max_overlap)
-        return self._merged_results(res, labels, counts, B)
+        out = self.matchSetBatchMergedRaw(f.ctypes.data, B, W, H, f.strides[1], f.strides[0], False, max_overlap, scaled=scaled)
+        return self._merged_results(out[0], out[1], out[2], B, out[4] if scaled else None)
 
-    def matchSetMerged(self, sourceImage, max_overlap: float) -> List[Tuple[int, SingleTargetMatch]]:
+    def matchSetMerged(self, sourceImage, max_overlap: float, scaled: bool = False) -> List[Tuple[int, SingleTargetMatch]]:
         """one host image -> [(set index, result)]"""
-        return self.matchSetBatchMerged(_as_u8_2d(sourceImage)[None], max_overlap)[0]
+        return self.matchSetBatchMerged(_as_u8_2d(sourceImage)[None], max_overlap, scaled=scaled)[0]
 
-    def matchIngestedSetBatchMerged(self, max_overlap: float) -> List[List[Tuple[int, SingleTargetMatch]]]:
+    def matchIngestedSetBatchMerged(self, max_overlap: float, scaled: bool = False) -> List[List[Tuple[int, SingleTargetMatch]]]:
         """the frames of the last ingest x the set, merged: [frame][(set index, result)]"""
         B, T, cap = self.ingestedCount(), max(self.patternSetSize(), 1), self.result_capacity
         res = (L.fpm_result * (cap * max(B, 1)))()
         labels = (C.c_int * (cap * max(B, 1)))()
         counts = (C.c_int * max(B, 1))()
-        self._check(self._lib.fpm_match_ingested_set_batch_merged(self._h, float(max_overlap), res, labels, cap, counts, None))
-        return self._merged_results(res, labels, counts, B)
+        if not scaled:
+            self._check(self._lib.fpm_match_ingested_set_batch_merged(self._h, float(max_overlap), res, labels, cap, counts, None))
+            return self._merged_results(res, labels, counts, B)
+        sc = (C.c_double * (cap * max(B, 1)))()
+        self._check(self._lib.fpm_match_ingested_set_scaled_merged(self._h, float(max_overlap), res, sc, labels, cap, counts, None))
+        return self._merged_results(res, labels, counts, B, sc)
 
     # ---- match (src/TemplateMatcher.cpp:97-437) ----
     def match(self, sourceImage) -> List[SingleTargetMatch]:
@@ -608,20 +637,28 @@ class TemplateMatcher:
         self._check(self._lib.fpm_match_sharded(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0, res, cap, C.byref(n)))
         return _convert(res, min(n.value, cap))
 
-    def matchSetSharded(self, sourceImage=None, ptr=None, shape=None, stride=None, on_device=False) -> List[List[SingleTargetMatch]]:
-        """collective, the whole template set against one frame (fpm_match_set_sharded): every rank passes the SAME frame and
-        receives the same [template][results] lists, equal to matchSet on one GPU"""
+    def matchSetSharded(self, sourceImage=None, ptr=None, shape=None, stride=None, on_device=False,
+                        scaled: bool = False) -> List[List[SingleTargetMatch]]:
+        """collective, the whole template set against one frame (fpm_match_set_sharded, scaled: fpm_match_set_sharded_scaled):
+        every rank passes the SAME frame and receives the same [template][results] lists, equal to matchSet on one GPU"""
         cap, T = self.result_capacity, max(self.patternSetSize(), 1)
         res, counts = (L.fpm_result * (cap * T))(), (C.c_int * T)()
         if ptr is None:
             s = _as_u8_2d(sourceImage)
             ptr, shape, stride = s.ctypes.data, s.shape, s.strides[0]
-        self._check(self._lib.fpm_match_set_sharded(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0, res, cap, counts))
-        return self._set_results(res, counts, 1, T)[0]
+        if not scaled:
+            self._check(self._lib.fpm_match_set_sharded(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0, res, cap,
+                                                        counts))
+            return self._set_results(res, counts, 1, T)[0]
+        sc = (C.c_double * (cap * T))()
+        self._check(self._lib.fpm_match_set_sharded_scaled(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0, res, sc,
+                                                           cap, counts))
+        return self._set_results(res, counts, 1, T, sc)[0]
 
     def matchSetShardedMerged(self, sourceImage=None, max_overlap: Optional[float] = None, ptr=None, shape=None, stride=None,
-                              on_device=False) -> List[Tuple[int, SingleTargetMatch]]:
-        """collective, merged as matchSetMerged (fpm_match_set_sharded_merged): [(set index, result)] on every rank"""
+                              on_device=False, scaled: bool = False) -> List[Tuple[int, SingleTargetMatch]]:
+        """collective, merged as matchSetMerged (fpm_match_set_sharded_merged, scaled: fpm_match_set_sharded_scaled_merged):
+        [(set index, result)] on every rank"""
         if max_overlap is None:
             raise FpmError("matchSetShardedMerged needs max_overlap")
         cap, T = self.result_capacity, max(self.patternSetSize(), 1)
@@ -629,9 +666,14 @@ class TemplateMatcher:
         if ptr is None:
             s = _as_u8_2d(sourceImage)
             ptr, shape, stride = s.ctypes.data, s.shape, s.strides[0]
-        self._check(self._lib.fpm_match_set_sharded_merged(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0,
-                                                           float(max_overlap), res, labels, cap, count, set_counts))
-        return self._merged_results(res, labels, count, 1)[0]
+        if not scaled:
+            self._check(self._lib.fpm_match_set_sharded_merged(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0,
+                                                               float(max_overlap), res, labels, cap, count, set_counts))
+            return self._merged_results(res, labels, count, 1)[0]
+        sc = (C.c_double * cap)()
+        self._check(self._lib.fpm_match_set_sharded_scaled_merged(self._h, ptr, shape[1], shape[0], stride, 1 if on_device else 0,
+                                                                  float(max_overlap), res, sc, labels, cap, count, set_counts))
+        return self._merged_results(res, labels, count, 1, sc)[0]
 
     # ---- angle-sharded stage API ----
     def stageNumAngles(self, W, H) -> int: return self._lib.fpm_stage_num_angles(self._h, W, H)
@@ -727,32 +769,44 @@ def match_sharded_virtual(matchers, sourceImage):
     return [_convert(res[i * cap:(i + 1) * cap], min(counts[i], cap)) for i in range(n)]
 
 
-def match_set_sharded_virtual(matchers, sourceImage, max_overlap=None):
+def match_set_sharded_virtual(matchers, sourceImage, max_overlap=None, scaled=False):
     """fpm_match_set_sharded_virtual: the whole template set against one frame, angle-sharded over the given handles of ONE
     device as the ranks.  Returns one result per rank (they must all be equal): [template][results], or with max_overlap
-    the merged [(set index, result)] list (fpm_match_set_sharded_merged_virtual)."""
+    the merged [(set index, result)] list (fpm_match_set_sharded_merged_virtual).  scaled=True: the _scaled calls, which match
+    at the handles' scale range and fill dScale."""
     s = _as_u8_2d(sourceImage)
     lib = matchers[0]._lib
     n = len(matchers)
     cap = min(m.result_capacity for m in matchers)
     T = max(matchers[0].patternSetSize(), 1)
     hs = (C.c_void_p * n)(*[m._h for m in matchers])
+    args = (hs, n, s.ctypes.data, s.shape[1], s.shape[0], s.strides[0])
+    sc = None
+    name = "fpm_match_set_sharded%s%s_virtual" % ("_scaled" if scaled else "", "" if max_overlap is None else "_merged")
+    fn = getattr(lib, name)
     if max_overlap is None:
         res, counts = (L.fpm_result * (cap * n * T))(), (C.c_int * (n * T))()
-        rc = lib.fpm_match_set_sharded_virtual(hs, n, s.ctypes.data, s.shape[1], s.shape[0], s.strides[0], res, cap, counts)
+        if scaled:
+            sc = (C.c_double * (cap * n * T))()
+            rc = fn(*args, res, sc, cap, counts)
+        else:
+            rc = fn(*args, res, cap, counts)
     else:
         res, labels, counts, set_counts = (L.fpm_result * (cap * n))(), (C.c_int * (cap * n))(), (C.c_int * n)(), (C.c_int * (n * T))()
-        rc = lib.fpm_match_set_sharded_merged_virtual(hs, n, s.ctypes.data, s.shape[1], s.shape[0], s.strides[0], float(max_overlap),
-                                                      res, labels, cap, counts, set_counts)
+        if scaled:
+            sc = (C.c_double * (cap * n))()
+            rc = fn(*args, float(max_overlap), res, sc, labels, cap, counts, set_counts)
+        else:
+            rc = fn(*args, float(max_overlap), res, labels, cap, counts, set_counts)
     if rc != 0:
         errs = [lib.fpm_last_error(m._h).decode() for m in matchers]
-        raise FpmError("fpm_match_set_sharded%s_virtual error %d: %s" % ("" if max_overlap is None else "_merged", rc,
-                                                                         "; ".join(e for e in errs if e)))
+        raise FpmError("%s error %d: %s" % (name, rc, "; ".join(e for e in errs if e)))
+
+    def conv(i, m):
+        return _convert(res[i * cap:(i + 1) * cap], m, None if sc is None else sc[i * cap:(i + 1) * cap])
     if max_overlap is None:
-        return [[_convert(res[(r * T + t) * cap:(r * T + t + 1) * cap], min(counts[r * T + t], cap)) for t in range(T)]
-                for r in range(n)]
-    return [list(zip(labels[r * cap:r * cap + min(counts[r], cap)], _convert(res[r * cap:(r + 1) * cap], min(counts[r], cap))))
-            for r in range(n)]
+        return [[conv(r * T + t, min(counts[r * T + t], cap)) for t in range(T)] for r in range(n)]
+    return [list(zip(labels[r * cap:r * cap + min(counts[r], cap)], conv(r, min(counts[r], cap)))) for r in range(n)]
 
 
 # ---- multi-template matching ("NCC-based OCR", MatchTool/MatchToolDlg.cpp:718-770) --------------------------
@@ -798,7 +852,8 @@ class GlyphReader:
     """One learned TemplateMatcher per glyph; read(image) = the upstream OCR loop: match every glyph, collect the
     centres with their letter, assemble lines.  readBatch(frames) reads many frames with one handle holding all glyphs as
     a template set (created on first use).  masks (optional): {letter: mask} for glyphs matched under a don't-care mask,
-    e.g. their strokes; glyphs without an entry are unmasked."""
+    e.g. their strokes; glyphs without an entry are unmasked.  scale_range=(lo, hi) among the params reads text printed lo..hi
+    times the glyphs' size (setScaleRange on every handle; readBatch then uses the scaled set calls)."""
 
     def __init__(self, templates: dict, masks: Optional[dict] = None, device: int = 0, result_capacity: int = 256, **params):
         self.letters = [ch for ch in OCR_LETTERS if ch in templates] + sorted(k for k in templates if k not in OCR_LETTERS)
@@ -820,9 +875,11 @@ class GlyphReader:
     def _new_matcher(self):
         m = TemplateMatcher(self._device, result_capacity=self._capacity)
         for k, v in self._params.items():
+            if k == "scale_range" and v is None:             # no range: the unscaled matcher
+                continue
             {"max_pos": m.setMaxPositions, "max_overlap": m.setMaxOverlap, "score": m.setScore,
              "tolerance_angle": m.setToleranceAngle, "min_reduce_area": m.setMinReduceArea, "use_simd": m.setUseSIMD,
-             "sub_pixel": m.setSubPixelEstimation}[k](v)
+             "sub_pixel": m.setSubPixelEstimation, "scale_range": lambda r: m.setScaleRange(*r)}[k](v)
         return m
 
     def _assemble(self, per, line_tol):
@@ -842,10 +899,11 @@ class GlyphReader:
             self._set_matcher = self._new_matcher()
             self._set_matcher.learnPatternSet(self._templates, self._masks if any(m is not None for m in self._masks) else None)
         f = np.ascontiguousarray(np.stack([_as_u8_2d(x) for x in frames]) if isinstance(frames, (list, tuple)) else frames, np.uint8)
+        scaled = self._params.get("scale_range") is not None
         if merge_overlap is None:
-            return [self._assemble(per, line_tol) for per in self._set_matcher.matchSetBatch(f)]
+            return [self._assemble(per, line_tol) for per in self._set_matcher.matchSetBatch(f, scaled=scaled)]
         out = []
-        for merged in self._set_matcher.matchSetBatchMerged(f, merge_overlap):
+        for merged in self._set_matcher.matchSetBatchMerged(f, merge_overlap, scaled=scaled):
             per = [[] for _ in self.letters]
             for t, r in merged:
                 per[t].append(r)

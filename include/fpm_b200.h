@@ -81,8 +81,10 @@ enum fpm_param {
                                       s / (1 + ds_L), s, s * (1 + ds_L) (range) or s (fixed) x the usual angles, best = first strict
                                       maximum; sub-pixel uses the three angle evals of the best scale.  Results are the rectangles of the
                                       scaled size (w * s, h * s) in every result convention; [1, 1] is the unscaled matcher bit for bit.
-                                      fpm_match_scaled reports each record's scale.  Template sets of more than one template,
-                                      fpm_match_sharded*, fpm_match_set_sharded* and fpm_stage_* refuse any range other than [1, 1].
+                                      fpm_match_scaled reports each record's scale; for template sets fpm_match_set_scaled*,
+                                      fpm_match_ingested_set_scaled* and fpm_match_set_sharded_scaled* do.  fpm_match_set_batch*
+                                      and fpm_match_ingested_set_batch* on sets of more than one template, fpm_match_sharded*, the
+                                      fpm_match_set_sharded* calls without _scaled and fpm_stage_* refuse any range other than [1, 1].
                                       FPM_PARAM_TENSOR_CORES = 6 takes the mode-1 route at any range other than [1, 1]. */
     FPM_PARAM_COUNT_
 };
@@ -116,7 +118,9 @@ int fpm_learn(fpm_handle* h, const uint8_t* tpl, int width, int height, int stri
  * There is no NMS across templates.
  * A handle holding more than one template refuses every single-template entry point with FPM_ERR_INVALID and a message:
  * fpm_match*, fpm_match_ingested*, fpm_learn_ingested, fpm_match_multi, fpm_match_sharded*, fpm_stage_*, fpm_tpl_* (and
- * fpm_match_set_batch with FPM_PARAM_TRACE on).  fpm_match_set_sharded* run a set in the angle-sharded mode.  FPM_PARAM_MIN_REDUCE_AREA changed after learning re-learns the whole set. */
+ * fpm_match_set_batch with FPM_PARAM_TRACE on).  fpm_match_set_sharded* run a set in the angle-sharded mode.  FPM_PARAM_MIN_REDUCE_AREA changed after learning re-learns the whole set.
+ * A scale range other than [1, 1] (FPM_PARAM_SCALE_MIN / MAX) is matched on a set by the calls that return each record's scale:
+ * fpm_match_set_scaled, fpm_match_ingested_set_scaled, their _merged twins and fpm_match_set_sharded_scaled*. */
 int fpm_learn_set(fpm_handle* h, int n, const uint8_t* const* tpls, const int* widths, const int* heights, const int* strides);
 /* fpm_learn_set with a don't-care mask per template: masks[i] (u8, template i's size, mask_strides[i] bytes per row,
  * nonzero = kept) or NULL for an unmasked member; masks == NULL is fpm_learn_set.  Each masked member is learned exactly as
@@ -162,6 +166,20 @@ int fpm_match_set_batch_merged(fpm_handle* h, const uint8_t* src, int src_on_dev
 /* the frames left by the last ingest x the set, merged as in fpm_match_set_batch_merged */
 int fpm_match_ingested_set_batch_merged(fpm_handle* h, double max_overlap, fpm_result* out, int* labels, int cap, int* counts,
                                         int* set_counts);
+/* Scale-tolerant template sets: each call is its twin above (fpm_match_set_batch, fpm_match_ingested_set_batch and the two
+ * _merged calls) at any scale range (FPM_PARAM_SCALE_MIN / MAX, [1, 1] included), plus the scale of each record in scales[] at
+ * the same index as in out (scales may be NULL).  For every (b, t) the records and scales are bit for bit those a handle
+ * holding only template t returns through fpm_match_scaled with the same parameters and range; the merged calls merge those
+ * lists as fpm_match_set_batch_merged does, so the NMS across templates compares the scaled rectangles.  Each group of the set
+ * runs its own scale schedule (ds = 2 / max of its top level).  Refusals as the twin's, and min > max. */
+int fpm_match_set_scaled(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                         size_t frame_stride, fpm_result* out, double* scales, int cap, int* counts);
+int fpm_match_ingested_set_scaled(fpm_handle* h, fpm_result* out, double* scales, int cap, int* counts);
+int fpm_match_set_scaled_merged(fpm_handle* h, const uint8_t* src, int src_on_device, int batch, int width, int height, int stride,
+                                size_t frame_stride, double max_overlap, fpm_result* out, double* scales, int* labels, int cap,
+                                int* counts, int* set_counts);
+int fpm_match_ingested_set_scaled_merged(fpm_handle* h, double max_overlap, fpm_result* out, double* scales, int* labels, int cap,
+                                         int* counts, int* set_counts);
 
 /* isPatternLearned / clearPattern (include/TemplateMatcher.h:43-46). */
 int fpm_is_learned(const fpm_handle* h);
@@ -330,6 +348,21 @@ int fpm_match_set_sharded_virtual(fpm_handle* const* hs, int nranks, const uint8
 int fpm_match_set_sharded_merged_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height,
                                          int stride, double max_overlap, fpm_result* out, int* labels, int cap, int* count,
                                          int* set_counts);
+/* The _scaled twins of the four calls above: any scale range, and each record's scale in scales[] at the same index as in out
+ * (NULL: not written).  On every rank the lists and scales are bit-identical to what fpm_match_set_scaled (_merged) returns for
+ * the frame on one GPU.  The ranks shard the pose slots (angle x scale, scale-major) of every group's schedule; the collectives
+ * are those of the unscaled call.  Refusals as the twin's, and min > max.  On a set of one, fpm_match_set_sharded_scaled is the
+ * angle-sharded single-template scaled match (fpm_match_sharded itself keeps refusing ranges). */
+int fpm_match_set_sharded_scaled(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                                 fpm_result* out, double* scales, int cap, int* counts);
+int fpm_match_set_sharded_scaled_merged(fpm_handle* h, const uint8_t* src, int width, int height, int stride, int src_on_device,
+                                        double max_overlap, fpm_result* out, double* scales, int* labels, int cap, int* count,
+                                        int* set_counts);
+int fpm_match_set_sharded_scaled_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height, int stride,
+                                         fpm_result* out, double* scales, int cap, int* counts);
+int fpm_match_set_sharded_scaled_merged_virtual(fpm_handle* const* hs, int nranks, const uint8_t* src, int width, int height,
+                                                int stride, double max_overlap, fpm_result* out, double* scales, int* labels, int cap,
+                                                int* count, int* set_counts);
 /* contiguous chunk [a0, a1) of an n_angles schedule swept by `rank` (host arithmetic, no device needed) */
 int fpm_shard_angle_range(int n_angles, int nranks, int rank, int* a0, int* a1);
 /* number of NCCL collectives issued by this handle since creation */
